@@ -19,12 +19,17 @@ torch.distributed only launches, hands out the library's NCCL id, and reduces th
   cpu_baseline  the f64 CPU oracle (a port: the Rust reference cannot be built here) on a bounded sample
   --impl reference  times that same CPU restatement, all host threads, as the reference arm (loads nothing of the product)
   --inproc  one process, N GPUs: rtiow_ctx_create(N) + rtiow_render
+  --dump-outputs DIR  after the timed steps, the frame of the last one as DIR/frame.npy (float32, see dump_frame)
+
+bench.py writes nothing into the repository: the tree may be read-only.
 """
 from __future__ import annotations
 
 import argparse
+import ctypes
 import json
 import os
+import signal
 import subprocess
 import sys
 import threading
@@ -35,6 +40,7 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True                                # no __pycache__ next to the modules imported from the tree
 os.environ.setdefault("NCCL_DEBUG_FILE", "/dev/stderr")      # NCCL's version banner must not land on stdout: ONE JSON line there
 
 WORKLOAD = dict(name="RTIOW Part 1 final scene (seeded random_scene), 1200x675, 500 spp, depth 50", width=1200, height=675, spp=500,
@@ -77,7 +83,11 @@ def parse():
                          "pixels into rank 0's frame over NVLink (CUDA IPC mapping) + a 1-int NCCL all-reduce as barrier; 'auto' = fused when the mapping works")
     ap.add_argument("--scan", default="auto", choices=["auto", "fp32", "tensor"], help="sphere filter backend (rtiow_ctx_set_scan_backend)")
     ap.add_argument("--inproc", action="store_true", help="one process driving --gpus N devices through rtiow_ctx_create(N) + rtiow_render (no torchrun)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frame the timed path returned in its last step to DIR/frame.npy (float32; a seeded pixel sample above 64 MB)")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     name, w, h, spp, grid, mode = CONFIGS[a.config]
     a.workload = name if (a.width, a.height, a.spp) == (None, None, None) else f"{name} [overridden size]"
     a.width, a.height, a.spp = a.width or w, a.height or h, a.spp or spp
@@ -94,10 +104,14 @@ class ClockSampler:
     def __init__(self, gpu_index: int):
         self.idx, self.proc, self.lines = gpu_index, None, []
 
+    @staticmethod
+    def _die_with_parent():
+        ctypes.CDLL(None).prctl(1, signal.SIGTERM)              # PR_SET_PDEATHSIG: the sampler never outlives bench.py, even when it fails
+
     def start(self):
         try:
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "200", "-i", str(self.idx)],
-                                         stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+                                         stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True, preexec_fn=self._die_with_parent)
             self.t = threading.Thread(target=lambda: self.lines.extend(self.proc.stdout), daemon=True)
             self.t.start()
         except OSError:
@@ -108,6 +122,7 @@ class ClockSampler:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
         time.sleep(0.25)
         self.proc.terminate()
+        self.proc.wait(timeout=10)
         self.t.join(timeout=2)
         sm, mx, reasons, power = [], [], set(), []
         for ln in self.lines:
@@ -134,6 +149,26 @@ def make_config(args, n_spheres):
             "cache": "GPU arm: L2 flushed (160 MiB device fill) between timed steps"}
 
 
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_frame(out_dir, frame):
+    """--dump-outputs: the RGBA8 frame (top-down, [H, W, 4]) a caller of the timed path receives, as out_dir/frame.npy in float32,
+    so that two builds can be compared output for output (the inputs are fixed by the seeds of WORKLOAD).  A frame whose float32
+    copy exceeds DUMP_LIMIT_BYTES (cfg5) is written as a fixed, seeded sample of its pixels: frame.npy [k, 4] and, in
+    frame_pixels.npy (float64), the linear index y * W + x of each sampled pixel."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    H, W, C = frame.shape
+    if frame.size * 4 <= DUMP_LIMIT_BYTES:
+        np.save(out / "frame.npy", frame.astype(np.float32))
+        return
+    k = (DUMP_LIMIT_BYTES - 4096) // (C * 4 + 8)                          # 4 KiB: the two .npy headers
+    idx = np.sort(np.random.default_rng(0).choice(H * W, size=k, replace=False))
+    np.save(out / "frame.npy", frame.reshape(H * W, C)[idx].astype(np.float32))
+    np.save(out / "frame_pixels.npy", idx.astype(np.float64))
+
+
 # ----------------------------------------------------------------------------------------------- CPU arms
 def oracle_module(native=True):
     """the checker / CPU baseline: bench.py is one of the places allowed to load oracle/.  For the TIMED legs the oracle is
@@ -147,9 +182,9 @@ def time_oracle(o, sc, W, H, spp, seed):
     cam = o.camera_new((13, 2, 3), (0, 0, 0), (0, 1, 0), 20.0, W / H, 0.1, 10.0)
     t0 = time.perf_counter()
     # n_threads explicit: torchrun exports OMP_NUM_THREADS=1, the reference arm must use every host core
-    _, _, cnt = o.render(sc, cam, W, H, spp, seed=seed, sampler=o.SAMPLER_REJECTION, n_threads=o.host_threads())
+    img, _, cnt = o.render(sc, cam, W, H, spp, seed=seed, sampler=o.SAMPLER_REJECTION, n_threads=o.host_threads())
     dt = time.perf_counter() - t0
-    return W * H * spp / dt / 1e6, dt, cnt
+    return W * H * spp / dt / 1e6, dt, cnt, img
 
 
 def run_reference(args, rank):
@@ -167,8 +202,10 @@ def run_reference(args, rank):
         time_oracle(o, sc, W, H, 1, 1)
     t0 = time.perf_counter()
     for k in range(args.steps):
-        time_oracle(o, sc, W, H, spp, 1 + k)
+        img = time_oracle(o, sc, W, H, spp, 1 + k)[3]
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_frame(args.dump_outputs, img)
     v = W * H * spp * args.steps / dt / 1e6
     sample = (f"each step renders {W}x{H} @ {spp} spp ({W * H * spp / 1e6:.2f} M paths) of the {args.spp} spp workload; Mpaths/s does not depend on spp; "
               f"f64 C restatement (gcc -O2 -march={march}, OpenMP rows), NOT `cargo run --release`: no rustc in this image")
@@ -301,11 +338,8 @@ def run_ours(args, rank, local_rank, world):
 
     for _ in range(args.warmup):
         flush.fill_(1)
-        st = step_device()
+        step_device()
     barrier()
-    gather_note = ctx.gather_info()
-    per_step_launches = st["kernel_launches"]                                       # render + finalize (+ de-interleave): OUR kernels, not NCCL's
-    backend_tensor = st["scan_backend"] == capi.SCAN_TENSOR
     clocks = ClockSampler(local_rank)
     if rank == 0:
         clocks.start()
@@ -318,14 +352,20 @@ def run_ours(args, rank, local_rank, world):
     # the library times every frame's kernel with its own event pair and rtiow_ctx_synchronize returns the mean
     for k in range(args.steps):
         flush.fill_(1)                                                             # evict L2 between timed iterations
-        ctx.render_rank_enqueue(cam, prm)
+        frame_ptr = ctx.render_rank_enqueue(cam, prm)
         if (k + 1) % 512 == 0 and k + 1 < args.steps:                              # the library keeps one event pair per enqueued frame (<= 1024)
             st = ctx.synchronize()
             kernel_ms += [st["kernel_ms"]] * 512; rays.append(st["rays_traced"])
     e1.record(stream)
     st = ctx.synchronize()
-    kernel_ms += [st["kernel_ms"]] * (args.steps % 512 or min(args.steps, 512)); rays.append(st["rays_traced"])
+    tail = args.steps % 512 or min(args.steps, 512)                                # frames since the last synchronize
+    kernel_ms += [st["kernel_ms"]] * tail; rays.append(st["rays_traced"])
     barrier()
+    per_step_launches = st["kernel_launches"] // tail                              # render + finalize (+ de-interleave): OUR kernels, not NCCL's
+    backend_tensor = st["scan_backend"] == capi.SCAN_TENSOR
+    gather_note = ctx.gather_info()
+    # the last timed frame, as the caller of rtiow_render_rank_enqueue has it: rank 0 holds the whole frame in HBM
+    frame = capi.device_to_host(frame_ptr, W * H * 4).reshape(H, W, 4) if args.dump_outputs and rank == 0 else None
     total_ms = maxr(e0.elapsed_time(e1))
     clk = clocks.stop() if rank == 0 else None
     ms_per_step = total_ms / args.steps
@@ -351,7 +391,7 @@ def run_ours(args, rank, local_rank, world):
         sc = o.Scene(**scene)
         cores = o.host_threads()
         s_spp = args.cpu_sample_spp or max(1, min(spp, int(2 * cores * (1200 * 675) / (W * H) * 530 / n_spheres)))   # ~10-30 s of CPU work
-        v, dt, _ = time_oracle(o, sc, W, H, s_spp, 1)
+        v, dt, _, _ = time_oracle(o, sc, W, H, s_spp, 1)
         cpu = {"value": v, "unit": "Mpaths/s", "cores": cores, "kind": "port",
                "sample": f"{W}x{H} @ {s_spp} spp ({W * H * s_spp / 1e6:.1f} M paths, {dt:.1f} s) of the {spp} spp workload; f64 C restatement (gcc -O2 -march={march}), OpenMP rows"}
 
@@ -380,6 +420,8 @@ def run_ours(args, rank, local_rank, world):
         }
         if cpu:
             out["cpu_baseline"] = cpu
+        if frame is not None:
+            dump_frame(args.dump_outputs, frame)
         emit_json(out)
     if world > 1:
         dist.destroy_process_group()
@@ -410,6 +452,8 @@ def run_inproc(args):
         kms.append(st["kernel_ms"])
     dt = (time.perf_counter() - t0) / args.steps
     clk = clocks.stop()
+    if args.dump_outputs:
+        dump_frame(args.dump_outputs, out)
     paths = W * H * spp
     emit_json({"impl": "ours-inproc", "metric": "Mpaths/s", "value": paths / dt / 1e6, "unit": "Mpaths/s", "n_gpus": n, "steps": args.steps, "warmup": args.warmup,
                "ms_per_step": dt * 1e3, "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic",

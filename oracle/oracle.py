@@ -8,6 +8,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import subprocess
+import tempfile
 from pathlib import Path
 
 import numpy as np
@@ -20,7 +21,6 @@ SAMPLER_REJECTION, SAMPLER_DIRECT = 0, 1
 
 
 _SCENE_SO = _HERE / "build" / "librtiow_scene.so"
-_NATIVE_SO = _HERE / "build" / "native" / "librtiow_oracle.so"
 
 
 def build(force: bool = False) -> Path:
@@ -35,13 +35,16 @@ def build(force: bool = False) -> Path:
 
 def use_native_build() -> bool:
     """bench.py's timed CPU legs: rebuild the oracle with -march=native ON THE BOX THAT RUNS IT (the committed recipe builds for
-    baseline x86-64 because the .so travels) and switch lib() to it.  Returns False (and keeps the baseline build) if gcc fails."""
+    baseline x86-64 because the .so travels) and switch lib() to it.  The build goes to a temporary directory, removed once the
+    library is loaded: bench.py writes nothing into the tree.  Returns False (and keeps the baseline build) if gcc fails."""
     global _lib
-    try:
-        subprocess.run(["make", "-C", str(_HERE), "-B", "MARCH=native", "BUILD=build/native", "build/native/librtiow_oracle.so"], check=True, capture_output=True)
-    except (subprocess.CalledProcessError, OSError):
-        return False
-    _lib = C.CDLL(str(_NATIVE_SO))
+    with tempfile.TemporaryDirectory(prefix="rtiow_oracle_") as td:
+        so = Path(td) / "librtiow_oracle.so"
+        try:
+            subprocess.run(["make", "-C", str(_HERE), "-B", "MARCH=native", f"BUILD={td}", str(so)], check=True, capture_output=True)
+        except (subprocess.CalledProcessError, OSError):
+            return False
+        _lib = C.CDLL(str(so))
     _declare(_lib)
     return True
 

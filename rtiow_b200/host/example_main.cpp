@@ -7,6 +7,7 @@
 #include <chrono>
 #include <cstdlib>
 #include <cstring>
+#include <filesystem>
 #include <iostream>
 
 #include "rtiow.hpp"
@@ -66,14 +67,18 @@ static int selftest()
       expect(c == a && seen == std::vector<uint32_t>({ 2, 4, 6, 8 }) && first == render(cam, random_scene(1), q), "render_progressive: passes, preview and final frame");
       try { render_progressive(cam, random_scene(1), p, 4, [](uint32_t, uint32_t, uint32_t, const std::vector<uint8_t>&) { return true; }); expect(false, "cancel must throw"); }
       catch (const RenderError& e) { expect(e.kind == RenderError::Cancelled, "callback returning true -> RenderError::Cancelled"); } }
+    // the files below go to a private directory: a fixed name in the shared temporary directory may belong to another user
+    std::string dir = (std::filesystem::temp_directory_path() / "rtiow_selftest_XXXXXX").string();
+    if (!mkdtemp(dir.data())) { std::cerr << "FAIL: cannot create a temporary directory\nselftest FAILED\n"; return 1; }
     // scene files: the world survives a round trip bit for bit, and both filter backends render it
-    { save_scene(random_scene(1), "/tmp/rtiow_selftest_scene.txt");
-      expect(render(cam, load_scene("/tmp/rtiow_selftest_scene.txt"), p) == a, "scene file round trip renders the same frame");
+    { save_scene(random_scene(1), dir + "/scene.txt");
+      expect(render(cam, load_scene(dir + "/scene.txt"), p) == a, "scene file round trip renders the same frame");
       RenderParams q = p; q.scan = RTIOW_SCAN_FP32; rtiow_stats sq{};
       std::vector<uint8_t> f = render(cam, random_scene(1), q, &sq); size_t diff = 0;
       for (size_t i = 0; i < f.size(); ++i) diff += f[i] != a[i];
       expect(sq.scan_backend == RTIOW_SCAN_FP32 && diff <= f.size() / 1000, "FP32 filter backend renders the same frame (up to last-bit path differences)"); }
-    expect(write_png("/tmp/rtiow_selftest.png", 160, 90, a) && write_ppm("/tmp/rtiow_selftest.ppm", 160, 90, a), "PNG/PPM written");
+    expect(write_png(dir + "/selftest.png", 160, 90, a) && write_ppm(dir + "/selftest.ppm", 160, 90, a), "PNG/PPM written");
+    std::error_code ec; std::filesystem::remove_all(dir, ec);
     std::cout << (bad ? "selftest FAILED\n" : "selftest ok\n");
     return bad ? 1 : 0;
 }

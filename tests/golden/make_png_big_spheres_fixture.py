@@ -1,7 +1,7 @@
 """Generates tests/golden/png_big_spheres.json from the reference's only result-bearing artefact,
-/root/reference/rtiow_part1_final.png (1200x800 RGBA8).
+rtiow_part1_final.png of Druthyn/rtiow (1200x800 RGBA8):
 
-Run in the build container (the GPU box has no /root/reference):  python tests/golden/make_png_big_spheres_fixture.py
+    python tests/golden/make_png_big_spheres_fixture.py path/to/rtiow_part1_final.png
 
 random_scene (main.rs:59-102) is random in its small spheres only: the ground (main.rs:62-64) and the three unit spheres —
 glass at (0,1,0), Lambertian (0.4,0.2,0.1) at (-4,1,0), Metal (0.7,0.6,0.5) fuzz 0 at (4,1,0) (main.rs:93-99) — are fixed, and so
@@ -21,12 +21,13 @@ We keep 9x9-pixel block means (the render is converged: block std <= ~1 LSB) on 
 and smoothness in the PNG itself.
 """
 import json
+import sys
 from pathlib import Path
 
 import numpy as np
 from PIL import Image
 
-SRC = Path("/root/reference/rtiow_part1_final.png")
+SRC = Path(sys.argv[1])
 OUT = Path(__file__).with_name("png_big_spheres.json")
 
 im = np.array(Image.open(SRC)).astype(float)

@@ -1,7 +1,7 @@
 """Generates tests/golden/png_sky_rows.json from the reference's only result-bearing artefact,
-/root/reference/rtiow_part1_final.png (1200x800 RGBA8).
+rtiow_part1_final.png of Druthyn/rtiow (1200x800 RGBA8):
 
-Run in the build container (the GPU box has no /root/reference):  python tests/golden/make_png_sky_fixture.py
+    python tests/golden/make_png_sky_fixture.py path/to/rtiow_part1_final.png
 
 The scene in that render is random (main.rs:60), but pixels that only see sky are a deterministic function of
 Camera::new (camera.rs:17-45) + the miss branch of ray_color (main.rs:54-56) + Color::to_rgba (vec3.rs:404-420) +
@@ -9,12 +9,13 @@ the row flip (main.rs:141-145), up to +-1 LSB of Monte-Carlo jitter inside the p
 from the top rows, which are row-uniform (no geometry reaches them).
 """
 import json
+import sys
 from pathlib import Path
 
 import numpy as np
 from PIL import Image
 
-SRC = Path("/root/reference/rtiow_part1_final.png")
+SRC = Path(sys.argv[1])
 OUT = Path(__file__).with_name("png_sky_rows.json")
 
 im = np.array(Image.open(SRC))

@@ -13,8 +13,8 @@ ROOT = Path(__file__).resolve().parent.parent
 
 
 @pytest.mark.parametrize("path", sorted(str(p.relative_to(ROOT)) for p in list((ROOT / "tools").glob("*.py")) + [ROOT / "bench.py", ROOT / "__graft_entry__.py"]))
-def test_scripts_compile(path):
-    py_compile.compile(str(ROOT / path), doraise=True)
+def test_scripts_compile(path, tmp_path):
+    py_compile.compile(str(ROOT / path), cfile=str(tmp_path / "compiled.pyc"), doraise=True)      # the byte code goes to tmp_path, not into the tree
 
 
 def _bench():
