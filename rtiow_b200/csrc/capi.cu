@@ -57,21 +57,22 @@ extern "C" int rtiow_device_count(int* out)
 // ------------------------------------------------------------------------------------------------
 // context
 // ------------------------------------------------------------------------------------------------
-template <typename U> struct DevBuf {
+// a buffer that only grows: device memory, or page-locked host memory (the staging buffers of the H2D / D2H copies)
+template <typename U, bool kHost> struct Buf {
     U* p = nullptr; size_t n = 0;
     cudaError_t resize(size_t count)
     {
         if (count <= n && p) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr; n = 0;
-        cudaError_t e = cudaMalloc(&p, std::max<size_t>(count, 1) * sizeof(U));
+        release();
+        const size_t bytes = std::max<size_t>(count, 1) * sizeof(U);
+        cudaError_t e = kHost ? cudaMallocHost((void**)&p, bytes) : cudaMalloc((void**)&p, bytes);
         if (e == cudaSuccess) n = count;
         return e;
     }
-    void release() { if (p) cudaFree(p); p = nullptr; n = 0; }
+    void release() { if (p) { if (kHost) cudaFreeHost(p); else cudaFree(p); } p = nullptr; n = 0; }
 };
-
-template <typename U> struct DevPtr { unsigned char* raw; U* p() const { return reinterpret_cast<U*>(raw); } };   // a typed view into the scene blob
+template <typename U> using DevBuf = Buf<U, false>;
+template <typename U> using HostBuf = Buf<U, true>;
 
 struct DeviceState {
     int device = 0;
@@ -90,8 +91,8 @@ struct DeviceState {
     // frame
     DevBuf<unsigned long long> accum; DevBuf<unsigned long long> counters;   // [0]=work [1]=rays
     DevBuf<uint32_t> tiles; DevBuf<uint32_t> gathered; DevBuf<uint32_t> frame;
-    uint8_t* pinned = nullptr; size_t pinned_bytes = 0;
-    unsigned long long* pinned_cnt = nullptr;
+    HostBuf<uint8_t> pinned;                           // staging of the frame's D2H copy when the caller's buffer is pageable
+    HostBuf<unsigned long long> pinned_cnt;            // the counters after the frame
     // measurement
     DevBuf<uint4> flush; DevBuf<float> probe;
     int last_backend = RTIOW_SCAN_FP32;                // which filter the last render launch used (rtiow_stats.scan_backend)
@@ -100,8 +101,7 @@ struct DeviceState {
 struct rtiow_ctx {
     std::vector<DeviceState> dev;
     int scan_backend = RTIOW_SCAN_AUTO;  // rtiow_ctx_set_scan_backend
-    size_t scene_bytes = 0;
-    unsigned char* scene_stage = nullptr; size_t scene_stage_bytes = 0;   // page-locked staging blob of rtiow_scene_upload
+    HostBuf<unsigned char> scene_stage;  // page-locked staging blob of rtiow_scene_upload
     bool peer_ok = true;                 // every device can store into device 0's memory (NVLink P2P): fused epilogue + gather
     // the gather of the row tiles (rtiow_ctx_set_gather)
     int gather = RTIOW_GATHER_AUTO;
@@ -139,7 +139,7 @@ static int init_device(DeviceState& d, int device)
     CU(cudaStreamCreateWithFlags(&d.stream, cudaStreamNonBlocking));
     CU(cudaEventCreate(&d.ev0)); CU(cudaEventCreate(&d.ev1)); CU(cudaEventCreateWithFlags(&d.ev_done, cudaEventDisableTiming));
     CU(d.counters.resize(2));
-    CU(cudaMallocHost(&d.pinned_cnt, 2 * sizeof(unsigned long long)));
+    CU(d.pinned_cnt.resize(2));
     return RTIOW_OK;
 }
 
@@ -334,15 +334,14 @@ extern "C" void rtiow_ctx_destroy(rtiow_ctx* c)
         d.scene_blob.release();
         d.accum.release(); d.counters.release(); d.tiles.release(); d.gathered.release(); d.frame.release();
         d.flush.release(); d.probe.release();
-        if (d.pinned) cudaFreeHost(d.pinned);
-        if (d.pinned_cnt) cudaFreeHost(d.pinned_cnt);
+        d.pinned.release(); d.pinned_cnt.release();
         if (d.ev0) cudaEventDestroy(d.ev0);
         if (d.ev1) cudaEventDestroy(d.ev1);
         if (d.ev_done) cudaEventDestroy(d.ev_done);
         for (auto& ev : d.ring) { cudaEventDestroy(ev.first); cudaEventDestroy(ev.second); }
         if (d.stream && d.owns_stream) cudaStreamDestroy(d.stream);
     }
-    if (c->scene_stage) cudaFreeHost(c->scene_stage);
+    c->scene_stage.release();
     delete c;
 }
 
@@ -353,51 +352,30 @@ extern "C" void rtiow_ctx_destroy(rtiow_ctx* c)
 // root of rays leaving the surface lose more than t_min = 1e-4 (main.rs:44) in f32.
 static const double kBigRadius = 8.0;
 
-extern "C" int rtiow_scene_upload(rtiow_ctx* c, const rtiow_spheres* s, const rtiow_materials* m)
+static int check_scene(const rtiow_spheres* s, const rtiow_materials* m)
 {
-    if (!c || !s || !m) return fail(RTIOW_ERR_INVALID_ARG, "NULL argument");
     if (s->n > 0 && (!s->cx || !s->cy || !s->cz || !s->radius || !s->mat_index)) return fail(RTIOW_ERR_INVALID_ARG, "NULL sphere array");
     if (m->n > 0 && (!m->kind || !m->albedo_r || !m->albedo_g || !m->albedo_b || !m->param)) return fail(RTIOW_ERR_INVALID_ARG, "NULL material array");
     if (s->n > (1u << 30)) return fail(RTIOW_ERR_INVALID_ARG, "too many spheres");
-    const int n = (int)s->n;
-    for (int i = 0; i < n; ++i) {
+    for (int i = 0; i < (int)s->n; ++i) {
         if (s->mat_index[i] >= m->n) return fail(RTIOW_ERR_INVALID_ARG, "sphere %d: material index %u out of range (%u)", i, s->mat_index[i], m->n);
         if (m->kind[s->mat_index[i]] > RTIOW_MAT_DIELECTRIC) return fail(RTIOW_ERR_UNSUPPORTED, "sphere %d: material kind %u has no GPU implementation", i, m->kind[s->mat_index[i]]);
         if (!(std::isfinite(s->cx[i]) && std::isfinite(s->cy[i]) && std::isfinite(s->cz[i]) && std::isfinite(s->radius[i])))
             return fail(RTIOW_ERR_INVALID_ARG, "sphere %d: non-finite centre or radius", i);
     }
-    std::vector<float4> sph(n), mat(n); std::vector<double4> sphd(n), matd(n); std::vector<uint8_t> kind(n);
-    std::vector<int> small_ids, big_ids;
-    for (int i = 0; i < n; ++i) {
-        const uint32_t mi = s->mat_index[i];
-        sphd[i] = make_double4(s->cx[i], s->cy[i], s->cz[i], s->radius[i]);
-        sph[i] = make_float4((float)s->cx[i], (float)s->cy[i], (float)s->cz[i], (float)s->radius[i]);
-        matd[i] = make_double4(m->albedo_r[mi], m->albedo_g[mi], m->albedo_b[mi], m->param[mi]);
-        mat[i] = make_float4((float)m->albedo_r[mi], (float)m->albedo_g[mi], (float)m->albedo_b[mi], (float)m->param[mi]);
-        kind[i] = (uint8_t)m->kind[mi];
-        const double reach = std::sqrt(s->cx[i] * s->cx[i] + s->cy[i] * s->cy[i] + s->cz[i] * s->cz[i]) + std::fabs(s->radius[i]);
-        if (std::fabs(s->radius[i]) > kBigRadius || reach > 4096.0) big_ids.push_back(i); else small_ids.push_back(i);
-    }
-    const int ns = (int)small_ids.size(), nb = (int)big_ids.size();
-    std::vector<int> order(small_ids);
-    while (order.size() % 32) order.push_back(-1);
-    const int np = (int)order.size();
-    if (np > 65535 * 32) return fail(RTIOW_ERR_UNSUPPORTED, "scene too large");
-    // R: radius of the sphere around the coordinate origin on which the filter places its line point (rt_scene.cuh);
-    // it bounds every small sphere, so a line that misses it can hit none of them
-    double R = 1.0, rmax = 0.0;
-    for (int id : small_ids) {
-        const float4 v = sph[id];
-        R = std::max(R, std::sqrt((double)v.x * v.x + (double)v.y * v.y + (double)v.z * v.z) + std::fabs((double)v.w));
-        rmax = std::max(rmax, std::fabs((double)v.w));
-    }
-    const float R2f = (float)(R * R * (1.0 + 1e-6));
-    const double R2 = (double)R2f;
-    std::vector<float> table(RT_TABLE_FLOATS(np), 0.0f); std::vector<float4> small(np); std::vector<int> small_idx(np);
+    return RTIOW_OK;
+}
+
+// The FP32 filter's table of the small spheres (rt_scene.cuh): records of 4 spheres [cx0..3][cy0..3][cz0..3][K0..3], then the
+// look-ahead record.  small = the first ns entries are spheres, the rest padding; R2 = the squared bounding radius of the filter.
+static std::vector<float> filter_table(const std::vector<float4>& small, int ns, double R2)
+{
+    const int np = (int)small.size();
+    std::vector<float> table(RT_TABLE_FLOATS(np), 0.0f);
     for (int p = 0; p < np; ++p) {
-        float* rec = table.data() + (size_t)(p >> 2) * 16 + (p & 3);          // record of 4 spheres: [cx0..3][cy0..3][cz0..3][K0..3]
-        if (order[p] >= 0) {
-            const float4 v = sph[order[p]];
+        float* rec = table.data() + (size_t)(p >> 2) * 16 + (p & 3);
+        if (p < ns) {
+            const float4 v = small[p];
             rec[0] = v.x; rec[4] = v.y; rec[8] = v.z;
             // K = |c|^2 - r^2 + R^2 of the f32 sphere, in f64, lowered by the filter slack (RT_FILTER_SLACK, rt_scene.cuh)
             // and rounded toward -inf: the filter may only err towards keeping a sphere
@@ -405,16 +383,19 @@ extern "C" int rtiow_scene_upload(rtiow_ctx* c, const rtiow_spheres* s, const rt
             const double K = c2 - r2 + R2 - (double)RT_FILTER_SLACK * (c2 + r2 + R2) - 1e-30;
             float Kf = (float)K; if ((double)Kf > K) Kf = std::nextafterf(Kf, -INFINITY);
             rec[12] = Kf;
-            small[p] = v; small_idx[p] = order[p];
         } else {       // padding: C = 1e30 can never be reached by hb^2
             rec[0] = 0; rec[4] = 0; rec[8] = 0; rec[12] = 1e30f;
-            small[p] = make_float4(0, 0, 0, 0); small_idx[p] = -1;
         }
     }
     for (int k = 0; k < 4; ++k) table[(size_t)np * 4 + 12 + k] = 1e30f;        // the look-ahead record: never hit, never used
-    std::vector<double4> big(nb); for (int b = 0; b < nb; ++b) big[b] = sphd[big_ids[b]];
-    // f32 fast path of the large spheres: centre as hi + lo floats, K = |c|^2 - r^2 (from f64) as hi + lo; only offered when the
-    // radius is a float and the centre's lo part is one too (anything else keeps the f64 routine for every ray)
+    return table;
+}
+
+// f32 fast path of the large spheres: centre as hi + lo floats, K = |c|^2 - r^2 (from f64) as hi + lo; only offered (*ok) when the
+// radius is a float and the centre's lo part is one too (anything else keeps the f64 routine for every ray)
+static std::vector<float4> big_sphere_records(const std::vector<double4>& big, bool* ok)
+{
+    const int nb = (int)big.size();
     std::vector<float4> bigf(3 * (size_t)nb); bool bigf_ok = nb > 0;
     for (int b = 0; b < nb; ++b) {
         const double4 v = big[b];
@@ -425,91 +406,138 @@ extern "C" int rtiow_scene_upload(rtiow_ctx* c, const rtiow_spheres* s, const rt
         bigf_ok = bigf_ok && (double)r == v.w && (double)hx + (double)lx == v.x && (double)hy + (double)ly == v.y && (double)hz + (double)lz == v.z && std::isfinite(Kh);
         bigf[3 * b] = make_float4(hx, hy, hz, r); bigf[3 * b + 1] = make_float4(lx, ly, lz, Kh); bigf[3 * b + 2] = make_float4(Kl, 0.f, 0.f, 0.f);
     }
-    // Tensor-core filter (rt_umma.cuh): per small sphere the 11 features of the bilinear discriminant, scaled by powers of
-    // two chosen from the bounding radius, split hi/lo in fp16, in the canonical K-major layout.  S_0 carries the slack that
-    // bounds the 3-product split and the fp32 accumulation (tools/probe_umma_filter.cu measures 1.15e-6 R^2; 1.5625e-5 R^2 here).
-    // Enabled when the image fits beside the candidate lists in one CTA's shared memory and the slack stays below the
-    // mean r^2 (a scene spread over a huge radius would pass every sphere near the line; the FP32 filter handles those).
-    std::vector<unsigned char> ubimg; int u_npad = 0; umma::FeatScale u_sc{ 1.0f, 1.0f, 1.0f, 1.0f };
-    {
-        using Shape = UmmaShape<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
-        const int npad = (ns + RT_UMMA_CHUNK - 1) / RT_UMMA_CHUNK * RT_UMMA_CHUNK;
-        const double Rp = std::exp2(std::ceil(std::log2(R)));
-        const double slack = 1.5625e-5 * R * R;
-        double mean_r2 = 0; for (int id : small_ids) mean_r2 += (double)sph[id].w * sph[id].w;
-        mean_r2 = ns ? mean_r2 / ns : 0.0;
-        // fp16 accumulator (RT_UMMA_D16): |D| <= 4 R^2 for a line that meets the bounding sphere; it must stay finite in fp16
-        const bool d_fits = !RT_UMMA_D16 || 4.0 * R * R < 60000.0;
-        if (ns > 0 && npad < 65536 && Shape::smem_bytes(npad) <= 227 * 1024 && Rp <= 8192.0 && slack <= mean_r2 && d_fits) {
-            u_npad = npad;
-            u_sc = umma::FeatScale{ (float)Rp, 1.0f, (float)(Rp * 0.5), (float)(1.0 / Rp) };
-            const size_t blk = RT_UMMA_B_BLOCK_BYTES(npad);
-            ubimg.assign(2 * blk, 0);
-            // sphere j of `small` sits in column col(j) of the image: with the fp16 accumulator the columns of a 32-sphere word are
-            // permuted so that the packed sign collection (umma::sign_word16) returns bit 31 - k for sphere k, as the funnel shifts do
-            // K slots of the two blocks: umma::b2_feature (block 0 = B1: every hi feature + the hi parts that meet the ray's lo
-            // parts of features 10 and 0..3; block 1 = B2: the lo parts of features 0..9 + the hi parts that meet lo_4..lo_9)
-            auto put_all = [&](int j, const double (&S)[11]) {
-                const uint32_t col = RT_UMMA_D16 ? (((uint32_t)j & ~31u) | umma::d16_column((uint32_t)j & 31u)) : (uint32_t)j;
-                for (int b = 0; b < 2; ++b)
-                    for (int s = 0; s < 16; ++s) {
-                        int feat; bool is_lo; umma::b2_feature(b, s, &feat, &is_lo);
-                        const float x = (float)S[feat]; const __half h = __float2half_rn(x); const __half l = __float2half_rn(x - __half2float(h));
-                        memcpy(&ubimg[b * blk + umma::b_offset(col, s)], is_lo ? &l : &h, 2);
-                    }
-            };
-            for (int j = 0; j < npad; ++j) {
-                double S[11] = { 0 };
-                if (j < ns) {                     // position j of `small` (list order); the f32 sphere the precise test sees
-                    const float4 v = sph[order[j]];
-                    const double x = v.x, y = v.y, z = v.z, r = v.w;
-                    S[0] = (r * r - (x * x + y * y + z * z) + slack) / u_sc.s0;
-                    S[1] = x / u_sc.s1; S[2] = y / u_sc.s1; S[3] = z / u_sc.s1;
-                    S[4] = x * x / u_sc.s4; S[5] = y * y / u_sc.s4; S[6] = z * z / u_sc.s4;
-                    S[7] = x * y / u_sc.s4; S[8] = x * z / u_sc.s4; S[9] = y * z / u_sc.s4;
-                } else {
-                    S[0] = -4.0 * Rp * Rp / u_sc.s0;                  // padding: never passes, whatever the ray
-                }
-                S[10] = 1.0 / u_sc.s10;                               // a power of two: no lo part (the two-product form relies on it)
-                put_all(j, S);
+    *ok = bigf_ok;
+    return bigf;
+}
+
+// Tensor-core filter (rt_umma.cuh): per small sphere the 11 features of the bilinear discriminant, scaled by powers of
+// two chosen from the bounding radius, split hi/lo in fp16, in the canonical K-major layout.  S_0 carries the slack that
+// bounds the 3-product split and the fp32 accumulation (tools/probe_umma_filter.cu measures 1.15e-6 R^2; 1.5625e-5 R^2 here).
+// Enabled when the image fits beside the candidate lists in one CTA's shared memory and the slack stays below the
+// mean r^2 (a scene spread over a huge radius would pass every sphere near the line; the FP32 filter handles those).
+// Returns the padded sphere count u_npad, or 0 (and no image) when the scene does not qualify.
+static int tensor_image(const std::vector<float4>& small, int ns, double R, std::vector<unsigned char>* img, umma::FeatScale* u_sc)
+{
+    using Shape = UmmaShape<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
+    const int npad = (ns + RT_UMMA_CHUNK - 1) / RT_UMMA_CHUNK * RT_UMMA_CHUNK;
+    const double Rp = std::exp2(std::ceil(std::log2(R)));
+    const double slack = 1.5625e-5 * R * R;
+    double mean_r2 = 0; for (int j = 0; j < ns; ++j) mean_r2 += (double)small[j].w * small[j].w;
+    mean_r2 = ns ? mean_r2 / ns : 0.0;
+    // fp16 accumulator (RT_UMMA_D16): |D| <= 4 R^2 for a line that meets the bounding sphere; it must stay finite in fp16
+    const bool d_fits = !RT_UMMA_D16 || 4.0 * R * R < 60000.0;
+    if (!(ns > 0 && npad < 65536 && Shape::smem_bytes(npad) <= 227 * 1024 && Rp <= 8192.0 && slack <= mean_r2 && d_fits)) return 0;
+    *u_sc = umma::FeatScale{ (float)Rp, 1.0f, (float)(Rp * 0.5), (float)(1.0 / Rp) };
+    const size_t blk = RT_UMMA_B_BLOCK_BYTES(npad);
+    img->assign(2 * blk, 0);
+    // sphere j of `small` sits in column col(j) of the image: with the fp16 accumulator the columns of a 32-sphere word are
+    // permuted so that the packed sign collection (umma::sign_word16) returns bit 31 - k for sphere k, as the funnel shifts do
+    // K slots of the two blocks: umma::b2_feature (block 0 = B1: every hi feature + the hi parts that meet the ray's lo
+    // parts of features 10 and 0..3; block 1 = B2: the lo parts of features 0..9 + the hi parts that meet lo_4..lo_9)
+    auto put_all = [&](int j, const double (&S)[11]) {
+        const uint32_t col = RT_UMMA_D16 ? (((uint32_t)j & ~31u) | umma::d16_column((uint32_t)j & 31u)) : (uint32_t)j;
+        for (int b = 0; b < 2; ++b)
+            for (int s = 0; s < 16; ++s) {
+                int feat; bool is_lo; umma::b2_feature(b, s, &feat, &is_lo);
+                const float x = (float)S[feat]; const __half h = __float2half_rn(x); const __half l = __float2half_rn(x - __half2float(h));
+                memcpy(&(*img)[b * blk + umma::b_offset(col, s)], is_lo ? &l : &h, 2);
             }
+    };
+    for (int j = 0; j < npad; ++j) {
+        double S[11] = { 0 };
+        if (j < ns) {                     // position j of `small` (list order); the f32 sphere the precise test sees
+            const float4 v = small[j];
+            const double x = v.x, y = v.y, z = v.z, r = v.w;
+            S[0] = (r * r - (x * x + y * y + z * z) + slack) / u_sc->s0;
+            S[1] = x / u_sc->s1; S[2] = y / u_sc->s1; S[3] = z / u_sc->s1;
+            S[4] = x * x / u_sc->s4; S[5] = y * y / u_sc->s4; S[6] = z * z / u_sc->s4;
+            S[7] = x * y / u_sc->s4; S[8] = x * z / u_sc->s4; S[9] = y * z / u_sc->s4;
+        } else {
+            S[0] = -4.0 * Rp * Rp / u_sc->s0;                 // padding: never passes, whatever the ray
         }
+        S[10] = 1.0 / u_sc->s10;                              // a power of two: no lo part (the two-product form relies on it)
+        put_all(j, S);
     }
-    // layout of the blob: every array at a 256-byte boundary
+    return npad;
+}
+
+// The scene's arrays in one allocation, each at a 256-byte boundary.  put() appends an array and returns its offset in the
+// guise of a pointer; rebase() turns such offsets into addresses in a device's copy of the blob.
+struct SceneBlob {
     struct Part { const void* src; size_t bytes, off; };
-    Part parts[12] = {
-        { table.data(), table.size() * sizeof(float), 0 }, { small.data(), (size_t)np * sizeof(float4), 0 }, { small_idx.data(), (size_t)np * sizeof(int), 0 },
-        { big.data(), (size_t)nb * sizeof(double4), 0 }, { big_ids.data(), (size_t)nb * sizeof(int), 0 },
-        { sph.data(), (size_t)n * sizeof(float4), 0 }, { sphd.data(), (size_t)n * sizeof(double4), 0 }, { mat.data(), (size_t)n * sizeof(float4), 0 },
-        { matd.data(), (size_t)n * sizeof(double4), 0 }, { kind.data(), (size_t)n * sizeof(uint8_t), 0 },
-        { ubimg.data(), ubimg.size(), 0 }, { bigf.data(), bigf.size() * sizeof(float4), 0 } };
-    size_t blob_bytes = 0, payload = 0;
-    for (auto& pt : parts) { pt.off = blob_bytes; blob_bytes += (pt.bytes + 255) & ~(size_t)255; payload += pt.bytes; }
-    if (c->scene_stage_bytes < blob_bytes) {
-        if (c->scene_stage) cudaFreeHost(c->scene_stage);
-        c->scene_stage = nullptr; c->scene_stage_bytes = 0;
-        CU(cudaMallocHost(&c->scene_stage, blob_bytes)); c->scene_stage_bytes = blob_bytes;
+    std::vector<Part> parts; size_t bytes = 0;
+    template <typename U> const U* put(const std::vector<U>& v)
+    {
+        const Part pt{ v.data(), v.size() * sizeof(U), bytes };
+        parts.push_back(pt);
+        bytes += (pt.bytes + 255) & ~(size_t)255;
+        return reinterpret_cast<const U*>(pt.off);
     }
-    for (auto& pt : parts) if (pt.bytes) memcpy(c->scene_stage + pt.off, pt.src, pt.bytes);
-    c->scene_bytes = 0;
+    void write(unsigned char* dst) const { for (const Part& pt : parts) if (pt.bytes) memcpy(dst + pt.off, pt.src, pt.bytes); }
+};
+static SceneDev rebase(SceneDev s, const unsigned char* blob)
+{
+    auto at = [blob](auto& p) { p = reinterpret_cast<std::remove_reference_t<decltype(p)>>(blob + reinterpret_cast<uintptr_t>(p)); };
+    at(s.table); at(s.small); at(s.small_idx); at(s.big); at(s.big_idx); at(s.sph); at(s.sphd); at(s.mat); at(s.matd); at(s.kind); at(s.u_bimg); at(s.bigf);
+    return s;
+}
+
+extern "C" int rtiow_scene_upload(rtiow_ctx* c, const rtiow_spheres* s, const rtiow_materials* m)
+{
+    if (!c || !s || !m) return fail(RTIOW_ERR_INVALID_ARG, "NULL argument");
+    int rc = check_scene(s, m); if (rc) return rc;
+    const int n = (int)s->n;
+    std::vector<float4> sph(n), mat(n); std::vector<double4> sphd(n), matd(n); std::vector<uint8_t> kind(n);
+    std::vector<int> small_idx, big_idx;
+    for (int i = 0; i < n; ++i) {
+        const uint32_t mi = s->mat_index[i];
+        sphd[i] = make_double4(s->cx[i], s->cy[i], s->cz[i], s->radius[i]);
+        sph[i] = make_float4((float)s->cx[i], (float)s->cy[i], (float)s->cz[i], (float)s->radius[i]);
+        matd[i] = make_double4(m->albedo_r[mi], m->albedo_g[mi], m->albedo_b[mi], m->param[mi]);
+        mat[i] = make_float4((float)m->albedo_r[mi], (float)m->albedo_g[mi], (float)m->albedo_b[mi], (float)m->param[mi]);
+        kind[i] = (uint8_t)m->kind[mi];
+        const double reach = std::sqrt(s->cx[i] * s->cx[i] + s->cy[i] * s->cy[i] + s->cz[i] * s->cz[i]) + std::fabs(s->radius[i]);
+        if (std::fabs(s->radius[i]) > kBigRadius || reach > 4096.0) big_idx.push_back(i); else small_idx.push_back(i);
+    }
+    const int ns = (int)small_idx.size(), nb = (int)big_idx.size();
+    while (small_idx.size() % 32) small_idx.push_back(-1);                  // whole 32-sphere words; padding never hits
+    const int np = (int)small_idx.size();
+    if (np > 65535 * 32) return fail(RTIOW_ERR_UNSUPPORTED, "scene too large");
+    std::vector<float4> small(np);
+    for (int p = 0; p < ns; ++p) small[p] = sph[small_idx[p]];
+    // R: radius of the sphere around the coordinate origin on which the filter places its line point (rt_scene.cuh);
+    // it bounds every small sphere, so a line that misses it can hit none of them
+    double R = 1.0, rmax = 0.0;
+    for (int p = 0; p < ns; ++p) {
+        const float4 v = small[p];
+        R = std::max(R, std::sqrt((double)v.x * v.x + (double)v.y * v.y + (double)v.z * v.z) + std::fabs((double)v.w));
+        rmax = std::max(rmax, std::fabs((double)v.w));
+    }
+    const float R2f = (float)(R * R * (1.0 + 1e-6));
+    const std::vector<float> table = filter_table(small, ns, (double)R2f);
+    std::vector<double4> big(nb); for (int b = 0; b < nb; ++b) big[b] = sphd[big_idx[b]];
+    bool bigf_ok = false;
+    const std::vector<float4> bigf = big_sphere_records(big, &bigf_ok);
+    SceneDev sc{};
+    std::vector<unsigned char> ubimg;
+    sc.u_sc = umma::FeatScale{ 1.0f, 1.0f, 1.0f, 1.0f };
+    sc.u_npad = tensor_image(small, ns, R, &ubimg, &sc.u_sc);
+    SceneBlob blob;                      // the pointers of `sc` hold offsets into the blob until rebase()
+    sc.table = blob.put(table); sc.small = blob.put(small); sc.small_idx = blob.put(small_idx); sc.big = blob.put(big); sc.big_idx = blob.put(big_idx);
+    sc.sph = blob.put(sph); sc.sphd = blob.put(sphd); sc.mat = blob.put(mat); sc.matd = blob.put(matd); sc.kind = blob.put(kind);
+    sc.u_bimg = blob.put(ubimg); sc.bigf = blob.put(bigf);
+    sc.np = np; sc.n_rec = (ns + 3) / 4; sc.nb = nb; sc.n = n;
+    sc.filter_R2 = R2f; sc.filter_sigma = (float)(16.0 * 5.9604644775390625e-08 * std::max(rmax, 1e-3));
+    CU(c->scene_stage.resize(blob.bytes));
+    blob.write(c->scene_stage.p);
     for (auto& d : c->dev) {
         CU(cudaSetDevice(d.device));
-        CU(d.scene_blob.resize(blob_bytes));
-        CU(cudaMemcpyAsync(d.scene_blob.p, c->scene_stage, blob_bytes, cudaMemcpyHostToDevice, d.stream));
+        CU(d.scene_blob.resize(blob.bytes));
+        CU(cudaMemcpyAsync(d.scene_blob.p, c->scene_stage.p, blob.bytes, cudaMemcpyHostToDevice, d.stream));
         CU(cudaStreamSynchronize(d.stream));
-        const size_t bytes = payload;
-        unsigned char* B = d.scene_blob.p;
-        struct { DevPtr<float> table; DevPtr<float4> small; DevPtr<int> small_idx; DevPtr<double4> big; DevPtr<int> big_idx; DevPtr<float4> sph; DevPtr<double4> sphd;
-                 DevPtr<float4> mat; DevPtr<double4> matd; DevPtr<uint8_t> kind; DevPtr<unsigned char> ubimg; DevPtr<float4> bigf; } dd = {
-            { B + parts[0].off }, { B + parts[1].off }, { B + parts[2].off }, { B + parts[3].off }, { B + parts[4].off }, { B + parts[5].off }, { B + parts[6].off },
-            { B + parts[7].off }, { B + parts[8].off }, { B + parts[9].off }, { B + parts[10].off }, { B + parts[11].off } };
-        d.scene.table = dd.table.p(); d.scene.small = dd.small.p(); d.scene.small_idx = dd.small_idx.p(); d.scene.np = np; d.scene.n_rec = (ns + 3) / 4;
-        d.scene.filter_R2 = R2f; d.scene.filter_sigma = (float)(16.0 * 5.9604644775390625e-08 * std::max(rmax, 1e-3));
-        d.scene.big = dd.big.p(); d.scene.big_idx = dd.big_idx.p(); d.scene.nb = nb;
-        d.scene.sph = dd.sph.p(); d.scene.sphd = dd.sphd.p(); d.scene.mat = dd.mat.p(); d.scene.matd = dd.matd.p(); d.scene.kind = dd.kind.p(); d.scene.n = n;
-        d.scene.u_bimg = dd.ubimg.p(); d.scene.u_npad = u_npad; d.scene.u_sc = u_sc; d.scene.bigf = bigf_ok ? dd.bigf.p() : nullptr;
+        d.scene = rebase(sc, d.scene_blob.p);
+        if (!bigf_ok) d.scene.bigf = nullptr;          // the records stay in the blob; the f64 routine handles every large sphere
         d.has_scene = true;
-        c->scene_bytes = bytes;
     }
     return RTIOW_OK;
 }
@@ -609,23 +637,35 @@ extern "C" int rtiow_tile_buffer_bytes(const rtiow_params* p, int world, size_t*
 // ------------------------------------------------------------------------------------------------
 // launch configuration
 // ------------------------------------------------------------------------------------------------
-struct ScanCfg { int variant; size_t smem; };   // 0: smem 256x4, 1: smem 512x1 (large scenes), 2: global-memory scene
+// Which filter a scan runs.  F32: the tensor-core one when the scene qualifies (rtiow_scene_upload) and the caller did not ask
+// otherwise, else the FP32 one with its table in shared memory (Smem; Wide: a table too large for 256-thread CTAs, beside the
+// candidate lists of one wide CTA per SM) or read from global memory.  F64 tests every sphere.
+enum class Scan { F64, Tensor, Smem, Wide, Global };
+using UShape = UmmaShape<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
 static size_t cand_bytes(int threads) { return (size_t)threads * RT_CAND_CAP * sizeof(uint16_t); }
-static ScanCfg pick_cfg(int np)
+struct ScanPlan {
+    Scan scan;
+    size_t scene_smem;      // shared memory of the scene: the FP32 table (Smem, Wide), the tensor kernels' whole layout (Tensor), else 0
+    // dynamic shared memory of a CTA of `threads` threads: the FP32 filters add a candidate list per thread
+    size_t smem(int threads) const { return scan == Scan::F64 || scan == Scan::Tensor ? scene_smem : scene_smem + cand_bytes(threads); }
+};
+static int plan_scan(const rtiow_ctx* c, const DeviceState& d, int precision, ScanPlan* plan)
 {
-    const size_t table = RT_TABLE_FLOATS(np) * sizeof(float);
-    if (table + cand_bytes(256) <= 56 * 1024) return { 0, table + cand_bytes(256) };
-    if (table + cand_bytes(512) <= 227 * 1024) return { 1, table + cand_bytes(512) };
-    return { 2, cand_bytes(256) };
+    if (precision == RTIOW_PRECISION_F64) { *plan = { Scan::F64, 0 }; return RTIOW_OK; }
+    if (d.scene.u_npad > 0 && c->scan_backend != RTIOW_SCAN_FP32) { *plan = { Scan::Tensor, UShape::smem_bytes(d.scene.u_npad) }; return RTIOW_OK; }
+    if (c->scan_backend == RTIOW_SCAN_TENSOR)
+        return fail(RTIOW_ERR_UNSUPPORTED, "RTIOW_SCAN_TENSOR requested but the scene does not qualify for the tensor-core filter (too many / too widely spread small spheres)");
+    const size_t table = RT_TABLE_FLOATS(d.scene.np) * sizeof(float);
+    if (table + cand_bytes(256) <= 56 * 1024) *plan = { Scan::Smem, table };
+    else if (table + cand_bytes(512) <= 227 * 1024) *plan = { Scan::Wide, table };
+    else *plan = { Scan::Global, 0 };
+    return RTIOW_OK;
 }
 
-template <typename K> static int prep_kernel(K kernel, size_t smem, int threads, int sms, int* grid)
+// more dynamic shared memory than the default 48 KB has to be allowed per kernel
+template <typename K> static int allow_smem(K kernel, size_t smem)
 {
     if (smem > 48 * 1024) CU(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int per_sm = 0;
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem));
-    if (per_sm < 1) return fail(RTIOW_ERR_CUDA, "kernel does not fit on an SM (smem %zu)", smem);
-    *grid = per_sm * sms;
     return RTIOW_OK;
 }
 
@@ -643,34 +683,63 @@ template <typename T> static void size_fetch(RenderArgs<T>& a, int grid, int thr
     const uint64_t cap = std::max<uint32_t>(1u, 256u / a.chunk_samples);
     a.chunks_per_fetch = (uint32_t)std::min<uint64_t>(cap, std::max<uint64_t>(1, want));
     a.guided_div = (uint32_t)std::max<uint64_t>(1, 2 * n_warps);
-#ifdef RTIOW_TUNING                      // experiment builds only (tools/ab.sh): the product library reads no environment
-    if (const char* t = getenv("RTIOW_TUNE_GUIDED")) a.guided_div = (uint32_t)std::max(1, atoi(t));
-#endif
 }
 
-// which filter runs: the tensor-core one when the scene qualifies (rtiow_scene_upload) and the caller did not ask otherwise
-static bool use_tensor_scan(const rtiow_ctx* c, const DeviceState& d) { return d.scene.u_npad > 0 && c->scan_backend != RTIOW_SCAN_FP32; }
-static int check_scan_backend(const rtiow_ctx* c, const DeviceState& d)
+// a persistent render kernel: as many CTAs as fit on the SMs at once
+template <typename T, typename K> static int launch_persistent(K kernel, RenderArgs<T>& a, int threads, size_t smem, int sms, cudaStream_t st)
 {
-    if (c->scan_backend == RTIOW_SCAN_TENSOR && d.scene.u_npad == 0)
-        return fail(RTIOW_ERR_UNSUPPORTED, "RTIOW_SCAN_TENSOR requested but the scene does not qualify for the tensor-core filter (too many / too widely spread small spheres)");
+    int rc = allow_smem(kernel, smem); if (rc) return rc;
+    int per_sm = 0;
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem));
+    if (per_sm < 1) return fail(RTIOW_ERR_CUDA, "kernel does not fit on an SM (smem %zu)", smem);
+    const int grid = per_sm * sms;
+    size_fetch(a, grid, threads);
+    kernel<<<grid, threads, smem, st>>>(a);
     return RTIOW_OK;
 }
 
+template <typename T> static int launch_render_kernel(const ScanPlan& plan, const DeviceState& d, RenderArgs<T>& a, cudaStream_t st)
+{
+    if constexpr (std::is_same<T, double>::value) {
+        return launch_persistent(render_kernel<double, false, 256, 2>, a, 256, plan.smem(256), d.sms, st);
+    } else {
+        switch (plan.scan) {
+        case Scan::Tensor: {     // one CTA per SM (it owns all of TMEM), G groups of 128 rays + G issuer warps
+            auto k = render_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
+            const size_t smem = plan.smem(UShape::kRenderThreads);
+            int rc = allow_smem(k, smem); if (rc) return rc;
+            size_fetch(a, d.sms, UShape::kRayThreads);          // the work is shared among the ray threads, not the whole block
+            k<<<d.sms, UShape::kRenderThreads, smem, st>>>(a);
+            return RTIOW_OK;
+        }
+        case Scan::Smem:         // 3 CTAs x 256 threads x 80 registers fills the 64K-register file
+            return launch_persistent(render_kernel<float, true, 256, 3>, a, 256, plan.smem(256), d.sms, st);
+        case Scan::Wide:         // one CTA per SM, 24 warps at 80 registers (+2.5 % over 512 threads at 104) when their lists fit
+            if (plan.smem(768) <= 227 * 1024) return launch_persistent(render_kernel<float, true, 768, 1>, a, 768, plan.smem(768), d.sms, st);
+            return launch_persistent(render_kernel<float, true, 512, 1>, a, 512, plan.smem(512), d.sms, st);
+        case Scan::Global:
+            return launch_persistent(render_kernel<float, false, 256, 4>, a, 256, plan.smem(256), d.sms, st);
+        case Scan::F64:
+            break;
+        }
+        return fail(RTIOW_ERR_INVALID_ARG, "an F64 scan plan for an F32 render");
+    }
+}
+
+// where a device's epilogue stores its pixels: its rows in rank-local order into a tile buffer, or into their top-down places in
+// a whole frame that may live on another GPU (fused quantise + gather: finalize_to_frame_kernel)
+struct Dest { uint32_t* p; bool whole_frame; };
+
 template <typename T>
-static int launch_render(const rtiow_ctx* c, DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, uint32_t rank, uint32_t world, uint32_t* d_tiles,
-                         cudaStream_t st, uint32_t* launches, uint32_t* peer_frame, SampleRange sr)
+static int launch_render(const ScanPlan& plan, DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, uint32_t rank, uint32_t world, SampleRange sr,
+                         Dest dst, cudaStream_t st, uint32_t* launches)
 {
     RenderArgs<T> a;
     a.scene = d.scene; a.cam = to_dev_camera<T>(*cam);
     a.width = p->width; a.height = p->height; a.spp = sr.count; a.smp_begin = sr.begin; a.max_depth = p->max_depth; a.t_min = (T)p->t_min; a.key = philox_key(p->seed);
     a.inv_wm1 = (T)(1.0 / (double)(p->width - 1)); a.inv_hm1 = (T)(1.0 / (double)(p->height - 1));
     a.rank = rank; a.world = world; a.tile_rows = tile_rows_of(p); a.local_rows = rows_of_rank(p->height, tile_rows_of(p), world, rank);
-    uint32_t chunk = 64u;
-#ifdef RTIOW_TUNING
-    if (const char* t = getenv("RTIOW_TUNE_CHUNK")) chunk = (uint32_t)std::max(1, atoi(t));
-#endif
-    a.chunk_samples = std::min<uint32_t>(sr.count, chunk);
+    a.chunk_samples = std::min<uint32_t>(sr.count, 64u);
     a.chunks_per_pixel = (sr.count + a.chunk_samples - 1) / a.chunk_samples;
     a.chunks_per_fetch = std::max<uint32_t>(1u, 256u / a.chunk_samples);
     const uint64_t n_lp = (uint64_t)a.local_rows * p->width;
@@ -680,85 +749,70 @@ static int launch_render(const rtiow_ctx* c, DeviceState& d, const rtiow_camera*
     if (sr.begin == 0) CU(cudaMemsetAsync(d.accum.p, 0, 3 * n_lp * sizeof(unsigned long long), st));     // later passes add to the same sums
     CU(cudaMemsetAsync(d.counters.p, 0, 2 * sizeof(unsigned long long), st));
     if (n_lp == 0) return RTIOW_OK;
-    int grid = 0;
-    if (sizeof(T) == 8) {
-        d.last_backend = RTIOW_SCAN_FP32;
-        auto k = render_kernel<T, false, 256, 2>;
-        int rc = prep_kernel(k, 0, 256, d.sms, &grid); if (rc) return rc;
-        size_fetch(a, grid, 256);
-        k<<<grid, 256, 0, st>>>(a);
-    } else if (use_tensor_scan(c, d)) {
-        // sphere filter on the tensor cores: one CTA per SM (it owns all of TMEM), G groups of 128 rays + G issuer warps
-        if constexpr (std::is_same<T, float>::value) {
-            using Shape = UmmaShape<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
-            auto k = render_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
-            const size_t sm = Shape::smem_bytes(d.scene.u_npad);
-            CU(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-            grid = d.sms;
-            size_fetch(a, grid, Shape::kRayThreads);
-            k<<<grid, Shape::kRenderThreads, sm, st>>>(a);
-            d.last_backend = RTIOW_SCAN_TENSOR;
-        }
-    } else {
-        const ScanCfg cfg = pick_cfg(d.scene.np);
-        int min_ctas = 3;                                       // 3 CTAs x 256 threads x 80 registers fills the 64K-register file
-#ifdef RTIOW_TUNING
-        if (const char* t = getenv("RTIOW_TUNE_MIN_CTAS")) min_ctas = atoi(t);
-#endif
-        d.last_backend = RTIOW_SCAN_FP32;
-        if (cfg.variant == 0 && min_ctas == 3) {
-            auto k = render_kernel<T, true, 256, 3>;
-            int rc = prep_kernel(k, cfg.smem, 256, d.sms, &grid); if (rc) return rc;
-            size_fetch(a, grid, 256);
-            k<<<grid, 256, cfg.smem, st>>>(a);
-        } else if (cfg.variant == 0 && min_ctas == 2) {
-            auto k = render_kernel<T, true, 256, 2>;
-            int rc = prep_kernel(k, cfg.smem, 256, d.sms, &grid); if (rc) return rc;
-            size_fetch(a, grid, 256);
-            k<<<grid, 256, cfg.smem, st>>>(a);
-        } else if (cfg.variant == 0) {
-            auto k = render_kernel<T, true, 256, 4>;
-            int rc = prep_kernel(k, cfg.smem, 256, d.sms, &grid); if (rc) return rc;
-            size_fetch(a, grid, 256);
-            k<<<grid, 256, cfg.smem, st>>>(a);
-        } else if (cfg.variant == 1 && cfg.smem - cand_bytes(512) + cand_bytes(768) <= 227 * 1024) {
-            auto k = render_kernel<T, true, 768, 1>;              // one CTA per SM, 24 warps at 80 registers (+2.5 % over 512 threads at 104)
-            const size_t sm = cfg.smem - cand_bytes(512) + cand_bytes(768);
-            int rc = prep_kernel(k, sm, 768, d.sms, &grid); if (rc) return rc;
-            size_fetch(a, grid, 768);
-            k<<<grid, 768, sm, st>>>(a);
-        } else if (cfg.variant == 1) {
-            auto k = render_kernel<T, true, 512, 1>;
-            int rc = prep_kernel(k, cfg.smem, 512, d.sms, &grid); if (rc) return rc;
-            size_fetch(a, grid, 512);
-            k<<<grid, 512, cfg.smem, st>>>(a);
-        } else {
-            auto k = render_kernel<T, false, 256, 4>;
-            int rc = prep_kernel(k, cfg.smem, 256, d.sms, &grid); if (rc) return rc;
-            size_fetch(a, grid, 256);
-            k<<<grid, 256, cfg.smem, st>>>(a);
-        }
-    }
+    d.last_backend = plan.scan == Scan::Tensor ? RTIOW_SCAN_TENSOR : RTIOW_SCAN_FP32;
+    int rc = launch_render_kernel(plan, d, a, st); if (rc) return rc;
     CU(cudaGetLastError());
-    if (peer_frame)      // fused quantise + gather: stores go to rank 0's frame through peer memory
-        finalize_to_frame_kernel<<<(unsigned)((n_lp + 255) / 256), 256, 0, st>>>(d.accum.p, (uint32_t)n_lp, sr.begin + sr.count, p->alpha, p->width, tile_rows_of(p), world, rank, peer_frame);
+    if (dst.whole_frame)
+        finalize_to_frame_kernel<<<(unsigned)((n_lp + 255) / 256), 256, 0, st>>>(d.accum.p, (uint32_t)n_lp, sr.begin + sr.count, p->alpha, p->width, tile_rows_of(p), world, rank, dst.p);
     else
-        finalize_kernel<<<(unsigned)((n_lp + 255) / 256), 256, 0, st>>>(d.accum.p, (uint32_t)n_lp, sr.begin + sr.count, p->alpha, d_tiles);
+        finalize_kernel<<<(unsigned)((n_lp + 255) / 256), 256, 0, st>>>(d.accum.p, (uint32_t)n_lp, sr.begin + sr.count, p->alpha, dst.p);
     CU(cudaGetLastError());
     *launches += 2;
     return RTIOW_OK;
 }
 
-static int render_tiles(const rtiow_ctx* c, DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, uint32_t rank, uint32_t world, uint32_t* d_tiles,
-                        cudaStream_t st, uint32_t* launches, uint32_t* peer_frame = nullptr, const SampleRange* range = nullptr)
+// One device's part of a frame: samples `sr` of the rows {y : (y / tile_rows) % world == rank}, quantised into `dst`, with the
+// events e0 / e1 around the work and its kernel launches added to *launches
+static int render_step(const rtiow_ctx* c, DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, uint32_t rank, uint32_t world, SampleRange sr,
+                       Dest dst, cudaStream_t st, cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches)
 {
     if (!d.has_scene) return fail(RTIOW_ERR_INVALID_ARG, "no scene uploaded (call rtiow_scene_upload first)");
     CU(cudaSetDevice(d.device));
-    const SampleRange sr = range ? *range : SampleRange{ 0u, p->spp };
-    if (p->precision != RTIOW_PRECISION_F64) { int rc = check_scan_backend(c, d); if (rc) return rc; }
-    return p->precision == RTIOW_PRECISION_F64 ? launch_render<double>(c, d, cam, p, rank, world, d_tiles, st, launches, peer_frame, sr)
-                                               : launch_render<float>(c, d, cam, p, rank, world, d_tiles, st, launches, peer_frame, sr);
+    ScanPlan plan;
+    int rc = plan_scan(c, d, p->precision, &plan); if (rc) return rc;
+    CU(cudaEventRecord(e0, st));
+    rc = plan.scan == Scan::F64 ? launch_render<double>(plan, d, cam, p, rank, world, sr, dst, st, launches)
+                                : launch_render<float>(plan, d, cam, p, rank, world, sr, dst, st, launches);
+    if (rc) return rc;
+    CU(cudaEventRecord(e1, st));
+    return RTIOW_OK;
 }
+
+// a frame on one device: its rank-local order IS top-down
+static int render_single(const rtiow_ctx* c, DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, SampleRange sr, cudaStream_t st,
+                         cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches, const uint32_t** d_frame)
+{
+    CU(d.tiles.resize((size_t)p->width * p->height));
+    int rc = render_step(c, d, cam, p, 0, 1, sr, Dest{ d.tiles.p, false }, st, e0, e1, launches); if (rc) return rc;
+    *d_frame = d.tiles.p;
+    return RTIOW_OK;
+}
+
+// The frame's D2H copy.  A caller's buffer that is page-locked itself (cudaHostAlloc / cudaHostRegister, torch pin_memory) takes
+// the DMA directly; pageable memory goes through the device's staging buffer, and finish() copies it over after the stream
+// synchronisation (0.3 ms for the 3.2 MB headline frame).
+struct FrameCopy {
+    uint8_t* out = nullptr; const uint8_t* staged = nullptr; size_t bytes = 0;
+    int start(DeviceState& d, uint8_t* dst, const uint32_t* d_frame, size_t n, cudaStream_t st)
+    {
+        out = dst; bytes = n;
+        if (!host_is_pinned(dst)) { CU(d.pinned.resize(n)); staged = d.pinned.p; }
+        CU(cudaMemcpyAsync(staged ? d.pinned.p : dst, d_frame, n, cudaMemcpyDeviceToHost, st));
+        return RTIOW_OK;
+    }
+    void finish() const { if (staged) memcpy(out, staged, bytes); }
+};
+
+// what a render call reports; the scene's sphere count and the filter used come from device d
+static rtiow_stats make_stats(const DeviceState& d, double kernel_ms, double total_ms, uint64_t paths, uint64_t rays, uint32_t launches, uint32_t n_gpus,
+                              uint64_t h2d_bytes, uint64_t d2h_bytes)
+{
+    rtiow_stats s; memset(&s, 0, sizeof s);
+    s.kernel_ms = kernel_ms; s.total_ms = total_ms; s.paths = paths; s.rays_traced = rays; s.sphere_tests = rays * (uint64_t)d.scene.n;
+    s.h2d_bytes = h2d_bytes; s.d2h_bytes = d2h_bytes; s.kernel_launches = launches; s.n_gpus = n_gpus; s.scan_backend = (uint32_t)d.last_backend;
+    return s;
+}
+static const uint64_t kCallH2D = sizeof(rtiow_camera) + sizeof(rtiow_params);     // a frame's only input: the camera and the params
 
 static double now_ms()
 {
@@ -778,19 +832,14 @@ static int render_rank(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_params
     cudaStream_t st = stream ? (cudaStream_t)stream : d.stream;
     const double t0 = now_ms();
     uint32_t launches = 0;
-    if (stats) CU(cudaEventRecord(d.ev0, st));
-    rc = render_tiles(c, d, cam, p, (uint32_t)rank, (uint32_t)world, to_frame ? nullptr : (uint32_t*)dst, st, &launches, to_frame ? (uint32_t*)dst : nullptr);
+    rc = render_step(c, d, cam, p, (uint32_t)rank, (uint32_t)world, SampleRange{ 0u, p->spp }, Dest{ (uint32_t*)dst, to_frame }, st, d.ev0, d.ev1, &launches);
     if (rc) return rc;
     if (stats) {
-        CU(cudaEventRecord(d.ev1, st));
-        CU(cudaMemcpyAsync(d.pinned_cnt, d.counters.p, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(d.pinned_cnt.p, d.counters.p, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
         CU(cudaStreamSynchronize(st));
         float ms = 0; CU(cudaEventElapsedTime(&ms, d.ev0, d.ev1));
-        memset(stats, 0, sizeof *stats);
-        stats->kernel_ms = ms; stats->total_ms = now_ms() - t0;
-        stats->paths = (uint64_t)rows_of_rank(p->height, tile_rows_of(p), world, rank) * p->width * p->spp;
-        stats->rays_traced = d.pinned_cnt[1]; stats->sphere_tests = stats->rays_traced * (uint64_t)d.scene.n;
-        stats->kernel_launches = launches; stats->n_gpus = 1; stats->scan_backend = (uint32_t)d.last_backend;
+        *stats = make_stats(d, ms, now_ms() - t0, (uint64_t)rows_of_rank(p->height, tile_rows_of(p), world, rank) * p->width * p->spp, d.pinned_cnt.p[1],
+                            launches, 1, 0, 0);
     }
     return RTIOW_OK;
 }
@@ -838,19 +887,9 @@ static int render_frame(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_param
     DeviceState& d0 = c->dev[0];
     uint32_t launches = 0;
     CU(cudaSetDevice(d0.device));
-    const bool direct = host_is_pinned(out_rgba);           // a page-locked caller buffer takes the DMA directly (no staging copy)
-    if (!direct && d0.pinned_bytes < frame_bytes) {
-        if (d0.pinned) cudaFreeHost(d0.pinned);
-        d0.pinned = nullptr; d0.pinned_bytes = 0;
-        CU(cudaMallocHost(&d0.pinned, frame_bytes)); d0.pinned_bytes = frame_bytes;
-    }
     const uint32_t* d_final = nullptr;
     if (world == 1) {
-        CU(d0.tiles.resize(tile_px));
-        CU(cudaEventRecord(d0.ev0, d0.stream));
-        rc = render_tiles(c, d0, cam, p, 0, 1, d0.tiles.p, d0.stream, &launches, nullptr, &sr); if (rc) return rc;
-        CU(cudaEventRecord(d0.ev1, d0.stream));
-        d_final = d0.tiles.p;                                  // world == 1: rank-local order IS top-down
+        rc = render_single(c, d0, cam, p, sr, d0.stream, d0.ev0, d0.ev1, &launches, &d_final); if (rc) return rc;
     } else {
         // interleaved row tiles on every GPU.  Three gathers:
         //   fused (default with NVLink peer access, every B200 box): each rank's epilogue stores its pixels straight into device
@@ -873,12 +912,10 @@ static int render_frame(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_param
         for (uint32_t r = 0; r < world; ++r) {
             DeviceState& d = c->dev[r];
             CU(cudaSetDevice(d.device));
-            uint32_t* dst = nullptr;
-            if (use_nccl) { CU(d.tiles.resize(tile_px)); CU(d.gathered.resize(tile_px * world)); dst = d.tiles.p; }
-            else if (!fused) { if (r == 0) dst = d0.gathered.p; else { CU(d.tiles.resize(tile_px)); dst = d.tiles.p; } }
-            CU(cudaEventRecord(d.ev0, d.stream));
-            rc = render_tiles(c, d, cam, p, r, world, dst, d.stream, &launches, fused ? d0.frame.p : nullptr, &sr); if (rc) return rc;
-            CU(cudaEventRecord(d.ev1, d.stream));
+            Dest dst{ d0.frame.p, true };
+            if (use_nccl) { CU(d.tiles.resize(tile_px)); CU(d.gathered.resize(tile_px * world)); dst = Dest{ d.tiles.p, false }; }
+            else if (!fused) { if (r == 0) dst = Dest{ d0.gathered.p, false }; else { CU(d.tiles.resize(tile_px)); dst = Dest{ d.tiles.p, false }; } }
+            rc = render_step(c, d, cam, p, r, world, sr, dst, d.stream, d.ev0, d.ev1, &launches); if (rc) return rc;
             if (r != 0 && !use_nccl) {
                 if (!fused) {
                     const size_t bytes = (size_t)rows_of_rank(p->height, tile_rows_of(p), world, r) * p->width * 4;
@@ -910,27 +947,23 @@ static int render_frame(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_param
         c->gather_note = note;
         d_final = d0.frame.p;
     }
-    CU(cudaMemcpyAsync(direct ? out_rgba : d0.pinned, d_final, frame_bytes, cudaMemcpyDeviceToHost, d0.stream));
-    CU(cudaMemcpyAsync(d0.pinned_cnt, d0.counters.p, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, d0.stream));
+    FrameCopy copy;
+    rc = copy.start(d0, out_rgba, d_final, frame_bytes, d0.stream); if (rc) return rc;
+    CU(cudaMemcpyAsync(d0.pinned_cnt.p, d0.counters.p, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, d0.stream));
     CU(cudaStreamSynchronize(d0.stream));
-    if (!direct) memcpy(out_rgba, d0.pinned, frame_bytes);
+    copy.finish();
     if (stats) {
-        memset(stats, 0, sizeof *stats);
         float ms = 0; CU(cudaEventElapsedTime(&ms, d0.ev0, d0.ev1));
-        uint64_t rays = d0.pinned_cnt[1];
+        uint64_t rays = d0.pinned_cnt.p[1];
         for (uint32_t r = 1; r < world; ++r) {
             DeviceState& d = c->dev[r];
             CU(cudaSetDevice(d.device));
-            CU(cudaMemcpyAsync(d.pinned_cnt, d.counters.p, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, d.stream));
+            CU(cudaMemcpyAsync(d.pinned_cnt.p, d.counters.p, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, d.stream));
             CU(cudaStreamSynchronize(d.stream));
-            rays += d.pinned_cnt[1];
+            rays += d.pinned_cnt.p[1];
             float mr = 0; CU(cudaEventElapsedTime(&mr, d.ev0, d.ev1)); ms = std::max(ms, mr);          // the slowest device's kernels
         }
-        stats->kernel_ms = ms; stats->total_ms = now_ms() - t0;
-        stats->paths = (uint64_t)p->width * p->height * sr.count;
-        stats->rays_traced = rays; stats->sphere_tests = rays * (uint64_t)d0.scene.n;
-        stats->h2d_bytes = sizeof(rtiow_camera) + sizeof(rtiow_params); stats->d2h_bytes = frame_bytes + 16;
-        stats->kernel_launches = launches; stats->n_gpus = world; stats->scan_backend = (uint32_t)d0.last_backend;
+        *stats = make_stats(d0, ms, now_ms() - t0, (uint64_t)p->width * p->height * sr.count, rays, launches, world, kCallH2D, frame_bytes + 16);
     }
     return RTIOW_OK;
 }
@@ -1069,7 +1102,7 @@ static int ensure_nccl_buffers(rtiow_ctx* c, size_t tile_px, cudaStream_t st)
 }
 
 static int render_rank_impl(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_params* p, uint8_t* out_rgba, const void** d_frame_out, rtiow_stats* stats,
-                            bool enqueue_only = false)
+                            bool enqueue_only)
 {
     if (!c || !cam) return fail(RTIOW_ERR_INVALID_ARG, "NULL argument");
     int rc = check_params(p); if (rc) return rc;
@@ -1097,11 +1130,7 @@ static int render_rank_impl(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_p
     }
     bool frame_here = true;                                 // d_final holds the whole frame on THIS rank
     if (world == 1) {
-        CU(d.tiles.resize(tile_px));
-        CU(cudaEventRecord(e0, st));
-        rc = render_tiles(c, d, cam, p, 0, 1, d.tiles.p, st, &launches); if (rc) return rc;
-        CU(cudaEventRecord(e1, st));
-        d_final = d.tiles.p;
+        rc = render_single(c, d, cam, p, SampleRange{ 0u, p->spp }, st, e0, e1, &launches, &d_final); if (rc) return rc;
         c->gather_note = "single GPU: no gather";
     } else {
         bool fused = false;
@@ -1117,9 +1146,7 @@ static int render_rank_impl(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_p
             // it is the frame-complete barrier.  Two frames alternate, so rank 0's copy-out of frame k is ordered (by its stream
             // and the barrier of frame k+1) before anybody writes that buffer again in frame k+2.
             uint32_t* fr = c->ipc_frame + (size_t)(c->ipc_parity & 1u) * npx; c->ipc_parity ^= 1u;
-            CU(cudaEventRecord(e0, st));
-            rc = render_tiles(c, d, cam, p, rank, world, nullptr, st, &launches, fr); if (rc) return rc;
-            CU(cudaEventRecord(e1, st));
+            rc = render_step(c, d, cam, p, rank, world, SampleRange{ 0u, p->spp }, Dest{ fr, true }, st, e0, e1, &launches); if (rc) return rc;
             rc = nccl_barrier(c, st); if (rc) return rc;
             d_final = fr; frame_here = rank == 0;
             snprintf(note, sizeof note, "one process per GPU x%u: epilogue stores into rank 0's frame over NVLink (CUDA IPC mapping made inside librtiow_cuda.so) + "
@@ -1129,9 +1156,7 @@ static int render_rank_impl(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_p
             uint32_t* tiles = c->nccl_tiles ? c->nccl_tiles : d.tiles.p;
             uint32_t* gathered = c->nccl_gathered ? c->nccl_gathered : d.gathered.p;
             CU(d.frame.resize(npx));
-            CU(cudaEventRecord(e0, st));
-            rc = render_tiles(c, d, cam, p, rank, world, tiles, st, &launches); if (rc) return rc;
-            CU(cudaEventRecord(e1, st));
+            rc = render_step(c, d, cam, p, rank, world, SampleRange{ 0u, p->spp }, Dest{ tiles, false }, st, e0, e1, &launches); if (rc) return rc;
             NC(g_nccl.AllGather(tiles, gathered, tile_px * 4, ncclUint8, c->comm, st));      // one per frame, equal (padded) counts: SURVEY §8(e)
             deinterleave_kernel<<<(unsigned)((npx + 255) / 256), 256, 0, st>>>(gathered, p->width, p->height, tile_rows_of(p), world, tile_px, d.frame.p);
             CU(cudaGetLastError());
@@ -1143,19 +1168,9 @@ static int render_rank_impl(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_p
         }
         c->gather_note = note;
     }
-    // a caller's frame buffer that is page-locked itself (cudaHostAlloc / cudaHostRegister, torch pin_memory) takes the DMA directly;
-    // pageable memory goes through the ctx's pinned staging buffer and one host memcpy (0.3 ms for the 3.2 MB headline frame)
-    bool direct = false;
-    if (out_rgba && frame_here) {
-        direct = host_is_pinned(out_rgba);
-        if (!direct && d.pinned_bytes < frame_bytes) {
-            if (d.pinned) cudaFreeHost(d.pinned);
-            d.pinned = nullptr; d.pinned_bytes = 0;
-            CU(cudaMallocHost(&d.pinned, frame_bytes)); d.pinned_bytes = frame_bytes;
-        }
-        CU(cudaMemcpyAsync(direct ? out_rgba : d.pinned, d_final, frame_bytes, cudaMemcpyDeviceToHost, st));
-    }
-    CU(cudaMemcpyAsync(d.pinned_cnt, d.counters.p, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    FrameCopy copy;
+    if (out_rgba && frame_here) { rc = copy.start(d, out_rgba, d_final, frame_bytes, st); if (rc) return rc; }
+    CU(cudaMemcpyAsync(d.pinned_cnt.p, d.counters.p, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
     if (enqueue_only) {                                     // no host synchronisation: rtiow_ctx_synchronize collects the stats
         ++d.ring_used;
         d.enq_paths = (uint64_t)rows_of_rank(p->height, tile_rows_of(p), world, rank) * p->width * p->spp;
@@ -1164,28 +1179,24 @@ static int render_rank_impl(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_p
         return RTIOW_OK;
     }
     CU(cudaStreamSynchronize(st));
-    if (out_rgba && frame_here && !direct) memcpy(out_rgba, d.pinned, frame_bytes);
+    copy.finish();
     if (d_frame_out) *d_frame_out = frame_here ? d_final : nullptr;
     if (stats) {
-        memset(stats, 0, sizeof *stats);
         float ms = 0; CU(cudaEventElapsedTime(&ms, d.ev0, d.ev1));
-        stats->kernel_ms = ms; stats->total_ms = now_ms() - t0;
-        stats->paths = (uint64_t)rows_of_rank(p->height, tile_rows_of(p), world, rank) * p->width * p->spp;
-        stats->rays_traced = d.pinned_cnt[1]; stats->sphere_tests = stats->rays_traced * (uint64_t)d.scene.n;
-        stats->h2d_bytes = sizeof(rtiow_camera) + sizeof(rtiow_params); stats->d2h_bytes = (out_rgba && frame_here ? frame_bytes : 0) + 16;
-        stats->kernel_launches = launches; stats->n_gpus = world; stats->scan_backend = (uint32_t)d.last_backend;
+        *stats = make_stats(d, ms, now_ms() - t0, (uint64_t)rows_of_rank(p->height, tile_rows_of(p), world, rank) * p->width * p->spp, d.pinned_cnt.p[1],
+                            launches, world, kCallH2D, copy.bytes + 16);
     }
     return RTIOW_OK;
 }
 
 extern "C" int rtiow_render_rank(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_params* p, uint8_t* out_rgba, rtiow_stats* stats)
 {
-    return render_rank_impl(c, cam, p, out_rgba, nullptr, stats);
+    return render_rank_impl(c, cam, p, out_rgba, nullptr, stats, false);
 }
 extern "C" int rtiow_render_rank_device(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_params* p, const void** d_frame, rtiow_stats* stats)
 {
     if (!d_frame) return fail(RTIOW_ERR_INVALID_ARG, "d_frame is NULL");
-    return render_rank_impl(c, cam, p, nullptr, d_frame, stats);
+    return render_rank_impl(c, cam, p, nullptr, d_frame, stats, false);
 }
 
 // Frames back to back without a host round trip per frame (an animation, a bench's timed loop): the render kernel, the epilogue /
@@ -1206,13 +1217,9 @@ extern "C" int rtiow_ctx_synchronize(rtiow_ctx* c, rtiow_stats* stats)
         memset(stats, 0, sizeof *stats);
         double sum = 0;
         for (size_t i = 0; i < d.ring_used; ++i) { float ms = 0; CU(cudaEventElapsedTime(&ms, d.ring[i].first, d.ring[i].second)); sum += ms; }
-        if (d.ring_used) {
-            stats->kernel_ms = sum / (double)d.ring_used;            // mean over the frames enqueued since the last synchronize
-            stats->paths = d.enq_paths;                              // of the last frame, like rays_traced
-            stats->rays_traced = d.pinned_cnt[1]; stats->sphere_tests = stats->rays_traced * (uint64_t)d.scene.n;
-            stats->kernel_launches = d.enq_launches; stats->n_gpus = d.enq_world; stats->scan_backend = (uint32_t)d.last_backend;
-            stats->h2d_bytes = (sizeof(rtiow_camera) + sizeof(rtiow_params)) * d.ring_used; stats->d2h_bytes = 16 * d.ring_used;
-        }
+        // the mean kernel time of the frames enqueued since the last synchronize; paths and rays of the last one
+        if (d.ring_used)
+            *stats = make_stats(d, sum / (double)d.ring_used, 0.0, d.enq_paths, d.pinned_cnt.p[1], d.enq_launches, d.enq_world, kCallH2D * d.ring_used, 16 * d.ring_used);
     }
     d.ring_used = 0; d.enq_launches = 0;
     return RTIOW_OK;
@@ -1277,34 +1284,27 @@ extern "C" int rtiow_hitlist_batch(rtiow_ctx* c, int precision, int64_t n, const
     BATCH_PROLOGUE();
     if (!d.has_scene) return fail(RTIOW_ERR_INVALID_ARG, "no scene uploaded");
     if (!orig || !dir || !hit || !index || !t || !p || !normal || !front_face) return fail(RTIOW_ERR_INVALID_ARG, "NULL array");
-    if (precision == RTIOW_PRECISION_F32) { int rc = check_scan_backend(c, d); if (rc) return rc; }
+    ScanPlan plan;
+    int rc = plan_scan(c, d, precision, &plan); if (rc) return rc;
     if (n == 0) return RTIOW_OK;
-    SceneDev scene = d.scene;
     double *dor, *dd, *dt, *dp, *dn; int32_t *dh, *di, *dff;
     CU(S.in(orig, N3, &dor)); CU(S.in(dir, N3, &dd));
     CU(S.out(n, &dh)); CU(S.out(n, &di)); CU(S.out(n, &dt)); CU(S.out(N3, &dp)); CU(S.out(N3, &dn)); CU(S.out(n, &dff));
-    if (precision == RTIOW_PRECISION_F64) {
-        hitlist_kernel<double, false, 256><<<grid, 256, 0, d.stream>>>(scene, n, dor, dd, t_min, dh, di, dt, dp, dn, dff);
-    } else if (use_tensor_scan(c, d)) {
-        using Shape = UmmaShape<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
-        auto k = hitlist_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
-        const size_t sm = Shape::smem_bytes(d.scene.u_npad);
-        CU(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-        k<<<(unsigned)((n + Shape::kRayThreads - 1) / Shape::kRayThreads), Shape::kThreads, sm, d.stream>>>(scene, n, dor, dd, t_min, dh, di, dt, dp, dn, dff);
-    } else {
-        const ScanCfg cfg = pick_cfg(d.scene.np);
-        if (cfg.variant == 0) {
-            auto k = hitlist_kernel<float, true, 256>;
-            if (cfg.smem > 48 * 1024) CU(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cfg.smem));
-            k<<<grid, 256, cfg.smem, d.stream>>>(scene, n, dor, dd, t_min, dh, di, dt, dp, dn, dff);
-        } else if (cfg.variant == 1) {
-            auto k = hitlist_kernel<float, true, 512>;
-            CU(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cfg.smem));
-            k<<<(unsigned)((n + 511) / 512), 512, cfg.smem, d.stream>>>(scene, n, dor, dd, t_min, dh, di, dt, dp, dn, dff);
-        } else {
-            hitlist_kernel<float, false, 256><<<grid, 256, cfg.smem, d.stream>>>(scene, n, dor, dd, t_min, dh, di, dt, dp, dn, dff);
-        }
+    // one ray per thread, `rays` of them in a CTA of `threads`
+    auto launch = [&](auto k, int rays, int threads) -> int {
+        const size_t smem = plan.smem(threads);
+        int rc = allow_smem(k, smem); if (rc) return rc;
+        k<<<(unsigned)((n + rays - 1) / rays), threads, smem, d.stream>>>(d.scene, n, dor, dd, t_min, dh, di, dt, dp, dn, dff);
+        return RTIOW_OK;
+    };
+    switch (plan.scan) {
+    case Scan::F64: rc = launch(hitlist_kernel<double, false, 256>, 256, 256); break;
+    case Scan::Tensor: rc = launch(hitlist_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK>, UShape::kRayThreads, UShape::kThreads); break;
+    case Scan::Smem: rc = launch(hitlist_kernel<float, true, 256>, 256, 256); break;
+    case Scan::Wide: rc = launch(hitlist_kernel<float, true, 512>, 512, 512); break;
+    case Scan::Global: rc = launch(hitlist_kernel<float, false, 256>, 256, 256); break;
     }
+    if (rc) return rc;
     CU(cudaGetLastError());
     CU(S.back(hit, dh, n)); CU(S.back(index, di, n)); CU(S.back(t, dt, n)); CU(S.back(p, dp, N3)); CU(S.back(normal, dn, N3)); CU(S.back(front_face, dff, n));
     CU(cudaStreamSynchronize(d.stream));
@@ -1407,9 +1407,9 @@ extern "C" int rtiow_ray_color_trace_batch(rtiow_ctx* c, int precision, int64_t 
     BATCH_PROLOGUE();
     if (!d.has_scene) return fail(RTIOW_ERR_INVALID_ARG, "no scene uploaded");
     if (!orig || !dir || !pixel || !sample || !color) return fail(RTIOW_ERR_INVALID_ARG, "NULL array");
-    if (precision == RTIOW_PRECISION_F32) { int rc = check_scan_backend(c, d); if (rc) return rc; }
+    ScanPlan plan;
+    int rc = plan_scan(c, d, precision, &plan); if (rc) return rc;
     if (n == 0) return RTIOW_OK;
-    SceneDev scene = d.scene;
     double *dor, *dd, *dcol; uint32_t *dpx, *dsm; unsigned long long* dr;
     CU(S.in(orig, N3, &dor)); CU(S.in(dir, N3, &dd)); CU(S.in(pixel, n, &dpx)); CU(S.in(sample, n, &dsm));
     CU(S.out(N3, &dcol)); CU(S.out(n, &dr));
@@ -1417,28 +1417,21 @@ extern "C" int rtiow_ray_color_trace_batch(rtiow_ctx* c, int precision, int64_t 
     int32_t* dti = nullptr; double* dtr = nullptr;
     if (trace_index && n_tr) { CU(S.out(n_tr, &dti)); CU(cudaMemsetAsync(dti, 0xff, n_tr * sizeof(int32_t), d.stream)); }   // -1: no ray at this depth
     if (trace_ray && n_tr) CU(S.out(n_tr * 6, &dtr));
-    if (precision == RTIOW_PRECISION_F64) {
-        ray_color_kernel<double, false, 256><<<grid, 256, 0, d.stream>>>(scene, n, dor, dd, dpx, dsm, seed, max_depth, t_min, dcol, dr, dti, dtr);
-    } else if (use_tensor_scan(c, d)) {
-        using Shape = UmmaShape<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
-        auto k = ray_color_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
-        const size_t sm = Shape::smem_bytes(d.scene.u_npad);
-        CU(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-        k<<<(unsigned)((n + Shape::kRayThreads - 1) / Shape::kRayThreads), Shape::kThreads, sm, d.stream>>>(scene, n, dor, dd, dpx, dsm, seed, max_depth, t_min, dcol, dr, dti, dtr);
-    } else {
-        const ScanCfg cfg = pick_cfg(d.scene.np);
-        if (cfg.variant == 0) {
-            auto k = ray_color_kernel<float, true, 256>;
-            if (cfg.smem > 48 * 1024) CU(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cfg.smem));
-            k<<<grid, 256, cfg.smem, d.stream>>>(scene, n, dor, dd, dpx, dsm, seed, max_depth, t_min, dcol, dr, dti, dtr);
-        } else if (cfg.variant == 1) {
-            auto k = ray_color_kernel<float, true, 512>;
-            CU(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cfg.smem));
-            k<<<(unsigned)((n + 511) / 512), 512, cfg.smem, d.stream>>>(scene, n, dor, dd, dpx, dsm, seed, max_depth, t_min, dcol, dr, dti, dtr);
-        } else {
-            ray_color_kernel<float, false, 256><<<grid, 256, cfg.smem, d.stream>>>(scene, n, dor, dd, dpx, dsm, seed, max_depth, t_min, dcol, dr, dti, dtr);
-        }
+    // one path per thread, `rays` of them in a CTA of `threads`
+    auto launch = [&](auto k, int rays, int threads) -> int {
+        const size_t smem = plan.smem(threads);
+        int rc = allow_smem(k, smem); if (rc) return rc;
+        k<<<(unsigned)((n + rays - 1) / rays), threads, smem, d.stream>>>(d.scene, n, dor, dd, dpx, dsm, seed, max_depth, t_min, dcol, dr, dti, dtr);
+        return RTIOW_OK;
+    };
+    switch (plan.scan) {
+    case Scan::F64: rc = launch(ray_color_kernel<double, false, 256>, 256, 256); break;
+    case Scan::Tensor: rc = launch(ray_color_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK>, UShape::kRayThreads, UShape::kThreads); break;
+    case Scan::Smem: rc = launch(ray_color_kernel<float, true, 256>, 256, 256); break;
+    case Scan::Wide: rc = launch(ray_color_kernel<float, true, 512>, 512, 512); break;
+    case Scan::Global: rc = launch(ray_color_kernel<float, false, 256>, 256, 256); break;
     }
+    if (rc) return rc;
     CU(cudaGetLastError());
     CU(S.back(color, dcol, N3));
     if (rays) CU(S.back((unsigned long long*)rays, dr, n));
