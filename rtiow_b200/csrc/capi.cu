@@ -453,7 +453,9 @@ static int tensor_image(const std::vector<float4>& small, int ns, double R, std:
             S[4] = x * x / u_sc->s4; S[5] = y * y / u_sc->s4; S[6] = z * z / u_sc->s4;
             S[7] = x * y / u_sc->s4; S[8] = x * z / u_sc->s4; S[9] = y * z / u_sc->s4;
         } else {
-            S[0] = -4.0 * Rp * Rp / u_sc->s0;                 // padding: never passes, whatever the ray
+            // padding: never passes, whatever the ray.  Its D = -2 Rp^2 - |f_perp|^2 (+ sigma) stays within
+            // |D| <= 2 Rp^2 + R^2 < 65504, finite in fp16 up to the largest R that d_fits admits (Rp = 128)
+            S[0] = -2.0 * Rp * Rp / u_sc->s0;
         }
         S[10] = 1.0 / u_sc->s10;                              // a power of two: no lo part (the two-product form relies on it)
         put_all(j, S);

@@ -149,16 +149,27 @@ def test_hitlist_ties_and_order(ctx, oracle):
         assert rel_err(got["t"], ref["t"]).max() < TOL[prec]
 
 
+@pytest.mark.parametrize("backend", ["fp32", "tensor"])
 @pytest.mark.parametrize("n_spheres", [0, 1, 31, 32, 33, 1024 + 7])
-def test_hitlist_ragged_scene_sizes(ctx, oracle, n_spheres):
-    """empty world, sizes straddling the 32-sphere word and the 1024-sphere segment"""
+def test_hitlist_ragged_scene_sizes(ctx, capi, oracle, n_spheres, backend):
+    """empty world, sizes straddling the 32-sphere word and the 1024-sphere segment, on each filter (SCAN_AUTO would pick the
+    tensor filter for all of them)"""
     rng = np.random.default_rng(n_spheres)
     c = f32(rng.uniform(-6, 6, (n_spheres, 3))); r = f32(rng.uniform(0.05, 0.6, n_spheres))
     sc = oracle.Scene(c, r, np.zeros(n_spheres, np.uint32), [0], [[1, 1, 1]], [0])
     ctx.upload_scene(c, r, np.zeros(n_spheres, np.uint32), [0], [[1, 1, 1]], [0])
     o = f32(rng.uniform(-9, 9, (5000, 3))); d = f32(rng.normal(size=(5000, 3)))
     ref = oracle.world_hit_batch(sc, o, d)
-    got = ctx.hitlist_batch(o, d, 1e-4)
+    ctx.set_scan_backend(capi.SCAN_TENSOR if backend == "tensor" else capi.SCAN_FP32)
+    try:
+        if backend == "tensor" and n_spheres == 0:          # an empty world does not qualify for the tensor filter
+            with pytest.raises(capi.RtiowError) as e:
+                ctx.hitlist_batch(o, d, 1e-4)
+            assert e.value.code == capi.ERR_UNSUPPORTED
+            return
+        got = ctx.hitlist_batch(o, d, 1e-4)
+    finally:
+        ctx.set_scan_backend(capi.SCAN_AUTO)
     want = np.where(ref["hit"] == 1, ref["index"], -1)
     assert (got["index"] == want).mean() > 0.999
     m = (got["index"] == want) & (want >= 0)

@@ -13,6 +13,9 @@ No GPU and no library call besides the seeded scene generator: the GPU counterpa
 (bit-identical hits from the FP32 and the tensor filter) and tools/probe_umma_filter.cu (the same error measured on the B200).
 """
 import numpy as np
+import pytest
+
+import scan_scenes
 
 f16, f32 = np.float16, np.float32
 
@@ -64,7 +67,7 @@ def sphere_image(center, radius, npad, R_scene, sc):
     S[:n, 1:4] = c / s1
     S[:n, 4:7] = c * c / s4
     S[:n, 7] = c[:, 0] * c[:, 1] / s4; S[:n, 8] = c[:, 0] * c[:, 2] / s4; S[:n, 9] = c[:, 1] * c[:, 2] / s4
-    S[n:, 0] = -4.0 * Rp * Rp / s0
+    S[n:, 0] = -2.0 * Rp * Rp / s0      # padding: D = -2 Rp^2 - |f|^2 (+ sigma), |D| <= 2 Rp^2 + R^2 < 65504 wherever d_fits holds
     S[:, 10] = 1.0 / s10
     hi, lo = split(S.astype(f32))
     assert not lo[:, 10].any(), "S_10 is a power of two: the two-product form relies on its lo part being zero"
@@ -107,15 +110,31 @@ def test_d16_column_inverts_the_packed_sign_order():
         assert 8 * b + j == 31 - k
 
 
-def test_contraction_reproduces_the_discriminant_and_never_drops_a_hit(capi):
-    scene = capi.random_scene(1)
-    small = np.abs(scene["radius"]) <= 8.0                                     # the r = 1000 ground goes to the large-sphere test
-    c, r = scene["center"][small], scene["radius"][small]
+def restate(c, r, o, d):
+    """the filter of closest_hit_umma on the small spheres (c, r) and unit rays (o, d), all f32 values:
+    -> D [rays, npad] (the contraction, f64 copy), the f64 discriminant [rays, ns], live rows, slack, R"""
     R_scene = float((np.linalg.norm(c, axis=1) + np.abs(r)).max())
     Rp = 2.0 ** np.ceil(np.log2(R_scene))
     sc = (Rp, 1.0, Rp * 0.5, 1.0 / Rp)                                        # umma::FeatScale {s0, s1, s4, s10}
     npad = -(-len(c) // 64) * 64
     B, slack = sphere_image(c, r, npad, R_scene, sc)
+    # closest_hit_umma: foot point of the coordinate origin (orthogonalised twice), liveness against the bounding sphere
+    a = (d * d).sum(1)
+    f = o - d * ((o * d).sum(1) / a)[:, None]
+    f = f - d * ((f * d).sum(1) / a)[:, None]
+    live = (f * f).sum(1) < R_scene * R_scene * (1 + 1e-6)
+    row1, row2 = ray_rows(f, d, live, 0.0, sc)
+    D = contraction(row1, row2, B).astype(np.float64)
+    oc = c[None, :, :].astype(f32).astype(np.float64) - o[:, None, :]
+    hb = (oc * d[:, None, :]).sum(2)
+    disc = hb * hb - a[:, None] * ((oc * oc).sum(2) - (r.astype(f32).astype(np.float64) ** 2)[None, :])        # sphere.rs:24 (quarter form)
+    return D, disc, live, slack, R_scene
+
+
+def test_contraction_reproduces_the_discriminant_and_never_drops_a_hit(capi):
+    scene = capi.random_scene(1)
+    small = np.abs(scene["radius"]) <= 8.0                                     # the r = 1000 ground goes to the large-sphere test
+    c, r = scene["center"][small], scene["radius"][small]
 
     rng = np.random.default_rng(7)
     n = 4096
@@ -127,20 +146,10 @@ def test_contraction_reproduces_the_discriminant_and_never_drops_a_hit(capi):
     d[-256:] = np.array([0.0, 1.0, 0.0]) + 0.01 * rng.standard_normal((256, 3)); o[-256:, 0] += 60.0       # far outside, heading up
     o = o.astype(f32).astype(np.float64)
     d = (d / np.linalg.norm(d, axis=1, keepdims=True)).astype(f32).astype(np.float64)
-
-    # closest_hit_umma: foot point of the coordinate origin (orthogonalised twice), liveness against the bounding sphere
     a = (d * d).sum(1)
-    f = o - d * ((o * d).sum(1) / a)[:, None]
-    f = f - d * ((f * d).sum(1) / a)[:, None]
-    R2 = R_scene * R_scene * (1 + 1e-6)
-    live = (f * f).sum(1) < R2
-    assert live[:-256].mean() > 0.9 and not live[-256:].any()
-    row1, row2 = ray_rows(f, d, live, 0.0, sc)
-    D = contraction(row1, row2, B).astype(np.float64)
 
-    oc = c[None, :, :].astype(f32).astype(np.float64) - o[:, None, :]
-    hb = (oc * d[:, None, :]).sum(2)
-    disc = hb * hb - a[:, None] * ((oc * oc).sum(2) - (r.astype(f32).astype(np.float64) ** 2)[None, :])        # sphere.rs:24 (quarter form)
+    D, disc, live, slack, R_scene = restate(c, r, o, d)
+    assert live[:-256].mean() > 0.9 and not live[-256:].any()
     nreal = len(c)
     # 1. padding and dead rows never pass
     assert (D[:, nreal:] < 0).all()
@@ -157,3 +166,27 @@ def test_contraction_reproduces_the_discriminant_and_never_drops_a_hit(capi):
     assert passed.sum() <= 1.25 * hit.sum()
     # 4. a ray that hits nothing far away still cannot overflow the fp16 result: |D| <= 4 R^2 << 65504
     assert np.isfinite(D).all() and 4 * R_scene * R_scene < 60000
+
+
+@pytest.mark.parametrize("name", ["ball-R122.4", "compact-3137", "row-r0.4"])
+def test_contraction_at_the_selection_boundaries(capi, name):
+    """the scenes at the edges of the tensor filter's rules (tests/scan_scenes.py): R just under 122.47 (Rp = 128, 4 R^2 just
+    under 60000, padding columns past the last word of small spheres), the largest image (npad 3200, 63 padding columns), and
+    the slack just below the mean r^2.  No sphere with discriminant >= 0 is dropped, every column of every ray stays finite
+    in fp16, and the padding columns stay negative."""
+    arrays = scan_scenes.sparse_ball(122.4) if name == "ball-R122.4" else scan_scenes.build(name, capi)
+    info = scan_scenes.scene_info(arrays)
+    assert info["failing"] == [], info["failing"]
+    k = info["small"]
+    c, r = arrays["center"][k], arrays["radius"][k]
+    o, d = scan_scenes.rays(name, arrays)
+    d = (d / np.linalg.norm(d, axis=1, keepdims=True)).astype(f32).astype(np.float64)
+    D, disc, live, _, _ = restate(c, r, o, d)
+    ns = len(c)
+    assert live.mean() > 0.5
+    assert not ((disc >= 0) & live[:, None] & (D[:, :ns] < 0)).any(), "the filter dropped a sphere whose discriminant is >= 0"
+    assert np.isfinite(D[:, :ns]).all()
+    pad = D[:, ns:]
+    assert pad.shape[1] == info["npad"] - ns > 0
+    assert np.isfinite(pad).all(), f"{(~np.isfinite(pad)).sum()} padding entries overflow fp16"
+    assert (pad < 0).all()
