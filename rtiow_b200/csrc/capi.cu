@@ -424,8 +424,8 @@ static int tensor_image(const std::vector<float4>& small, int ns, double R, std:
     const double slack = 1.5625e-5 * R * R;
     double mean_r2 = 0; for (int j = 0; j < ns; ++j) mean_r2 += (double)small[j].w * small[j].w;
     mean_r2 = ns ? mean_r2 / ns : 0.0;
-    // fp16 accumulator (RT_UMMA_D16): |D| <= 4 R^2 for a line that meets the bounding sphere; it must stay finite in fp16
-    const bool d_fits = !RT_UMMA_D16 || 4.0 * R * R < 60000.0;
+    // fp16 accumulator: |D| <= 4 R^2 for a line that meets the bounding sphere; it must stay finite in fp16
+    const bool d_fits = 4.0 * R * R < 60000.0;
     if (!(ns > 0 && npad < 65536 && Shape::smem_bytes(npad) <= 227 * 1024 && Rp <= 8192.0 && slack <= mean_r2 && d_fits)) return 0;
     *u_sc = umma::FeatScale{ (float)Rp, 1.0f, (float)(Rp * 0.5), (float)(1.0 / Rp) };
     const size_t blk = RT_UMMA_B_BLOCK_BYTES(npad);
@@ -435,7 +435,7 @@ static int tensor_image(const std::vector<float4>& small, int ns, double R, std:
     // K slots of the two blocks: umma::b2_feature (block 0 = B1: every hi feature + the hi parts that meet the ray's lo
     // parts of features 10 and 0..3; block 1 = B2: the lo parts of features 0..9 + the hi parts that meet lo_4..lo_9)
     auto put_all = [&](int j, const double (&S)[11]) {
-        const uint32_t col = RT_UMMA_D16 ? (((uint32_t)j & ~31u) | umma::d16_column((uint32_t)j & 31u)) : (uint32_t)j;
+        const uint32_t col = ((uint32_t)j & ~31u) | umma::d16_column((uint32_t)j & 31u);
         for (int b = 0; b < 2; ++b)
             for (int s = 0; s < 16; ++s) {
                 int feat; bool is_lo; umma::b2_feature(b, s, &feat, &is_lo);

@@ -120,34 +120,64 @@ __device__ __forceinline__ void candidate_self(V3<T> dhat, T inv_a, T t_min, V3<
 // A word is 512 contiguous bytes: every LDS.128 of the unrolled word is [base + immediate].
 #define RT_TABLE_FLOATS(np) (4 * (size_t)(np) + 16)
 
+// The line gate of both filters (this one and the tensor-core filter of rt_umma_scan.cuh): f, the foot point of the
+// coordinate origin on the line, orthogonalised twice (the second pass removes the O(u |o|) component along dhat that the
+// first leaves when the origin is far away); sigma = 16 u r_max |o|_1, as the foot point of a far origin is only known to
+// ~4 u |o|; live: the line enters the R-sphere widened by sigma.  A line that misses it can hit no small sphere.
+struct LineGate {
+    V3<float> f;
+    float sigma;
+    bool live;
+};
+__device__ __forceinline__ LineGate line_gate(V3<float> o, V3<float> dhat, float inv_a, float R2, float sigma_per_len)
+{
+    LineGate g;
+    g.f = o - dhat * (dot(o, dhat) * inv_a);
+    g.f = g.f - dhat * (dot(g.f, dhat) * inv_a);
+    g.sigma = sigma_per_len * (fabsf(o.x) + fabsf(o.y) + fabsf(o.z));
+    g.live = length_squared(g.f) < R2 + g.sigma;
+    return g;
+}
+
 struct FilterRay {
     float M2PX, M2PY, M2PZ, DX, DY, DZ, NPD;
 };
 __device__ __forceinline__ FilterRay make_filter_ray(V3<float> o, V3<float> dhat, float inv_a, float R2, float sigma_per_len)
 {
-    // foot point of the coordinate origin on the line, orthogonalised twice: the second pass removes the O(u |o|)
-    // component along dhat that the first leaves when the origin is far away
-    V3<float> f = o - dhat * (dot(o, dhat) * inv_a);
-    f = f - dhat * (dot(f, dhat) * inv_a);
-    const float ff = length_squared(f);
-    // |p|^2 = R^2 + sigma, sigma = 16 u r_max |o|_1: the foot point of a far origin is only known to ~4 u |o|
-    const float sigma = sigma_per_len * (fabsf(o.x) + fabsf(o.y) + fabsf(o.z));
-    const float h2 = (R2 + sigma) - ff;
-    const bool inside = h2 > 0.0f;                          // the line enters the R-sphere
-    const float s = inside ? sqrtf(h2 * inv_a) : 0.0f;
-    const V3<float> p = f - dhat * s;                       // where the line enters the R-sphere
+    const LineGate g = line_gate(o, dhat, inv_a, R2, sigma_per_len);
+    // |p|^2 = R^2 + sigma
+    const float s = g.live ? sqrtf(((R2 + g.sigma) - length_squared(g.f)) * inv_a) : 0.0f;
+    const V3<float> p = g.f - dhat * s;                     // where the line enters the R-sphere
     FilterRay r;
     // A line that misses the R-sphere (an origin far out on the ground, heading for the sky) can hit no small sphere:
     // with p = 0 the filter computes (c.d)^2 - K <= |c|^2 - (|c|^2 - r^2 + R^2) < 0 for every sphere, as R >= |c| + |r|.
     // (Keeping the foot point instead would stay conservative, but |p|^2 - R^2 would act as slack and let through every
     // sphere within that distance of the line — hundreds of false candidates per such ray.)
-    const float live = inside ? 1.0f : 0.0f;
+    const float live = g.live ? 1.0f : 0.0f;
     r.M2PX = -2.0f * live * p.x; r.M2PY = -2.0f * live * p.y; r.M2PZ = -2.0f * live * p.z;
     // opaque to the compiler: otherwise it keeps p and re-multiplies by -2 in every 32-sphere word (3 FMUL per word)
     asm volatile("" : "+f"(r.M2PX), "+f"(r.M2PY), "+f"(r.M2PZ));
     r.DX = dhat.x; r.DY = dhat.y; r.DZ = dhat.z;
     r.NPD = -live * dot(p, dhat);
     return r;
+}
+
+// One 4-sphere record of the filter: the sign bits of the 4 disc' shifted into m, the record's last sphere in bit 0.
+__device__ __forceinline__ unsigned filter_record(unsigned m, float4 cx, float4 cy, float4 cz, float4 kk, const FilterRay& f)
+{
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+        const float2 X = h ? make_float2(cx.z, cx.w) : make_float2(cx.x, cx.y);
+        const float2 Y = h ? make_float2(cy.z, cy.w) : make_float2(cy.x, cy.y);
+        const float2 Z = h ? make_float2(cz.z, cz.w) : make_float2(cz.x, cz.y);
+        const float2 K = h ? make_float2(kk.z, kk.w) : make_float2(kk.x, kk.y);
+        const float2 hb = ffma2(X, bc2(f.DX), ffma2(Y, bc2(f.DY), ffma2(Z, bc2(f.DZ), bc2(f.NPD))));
+        const float2 C = ffma2(X, bc2(f.M2PX), ffma2(Y, bc2(f.M2PY), ffma2(Z, bc2(f.M2PZ), K)));
+        const float2 disc = ffma2(hb, hb, neg2(C));
+        m = __funnelshift_l(__float_as_uint(disc.x), m, 1);
+        m = __funnelshift_l(__float_as_uint(disc.y), m, 1);
+    }
+    return m;
 }
 
 // One 32-sphere word of the filter: 8 records, software-pipelined one record ahead (the ~30-cycle shared-memory latency
@@ -159,18 +189,7 @@ __device__ __forceinline__ unsigned filter_word(const float4* __restrict__ rec, 
     for (int q = 0; q < 8; ++q) {
         const float4 cx = ncx, cy = ncy, cz = ncz, kk = nkk;
         ncx = rec[4 * q + 4]; ncy = rec[4 * q + 5]; ncz = rec[4 * q + 6]; nkk = rec[4 * q + 7];
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-            const float2 X = h ? make_float2(cx.z, cx.w) : make_float2(cx.x, cx.y);
-            const float2 Y = h ? make_float2(cy.z, cy.w) : make_float2(cy.x, cy.y);
-            const float2 Z = h ? make_float2(cz.z, cz.w) : make_float2(cz.x, cz.y);
-            const float2 K = h ? make_float2(kk.z, kk.w) : make_float2(kk.x, kk.y);
-            const float2 hb = ffma2(X, bc2(f.DX), ffma2(Y, bc2(f.DY), ffma2(Z, bc2(f.DZ), bc2(f.NPD))));
-            const float2 C = ffma2(X, bc2(f.M2PX), ffma2(Y, bc2(f.M2PY), ffma2(Z, bc2(f.M2PZ), K)));
-            const float2 disc = ffma2(hb, hb, neg2(C));
-            m = __funnelshift_l(__float_as_uint(disc.x), m, 1);
-            m = __funnelshift_l(__float_as_uint(disc.y), m, 1);
-        }
+        m = filter_record(m, cx, cy, cz, kk, f);
     }
     return m;
 }
@@ -194,21 +213,32 @@ __device__ __noinline__ unsigned filter_tail(const float4* __restrict__ rec, int
     for (int q = 0; q < n_rec; ++q, rec += 4, sa += 64u) {
         const float4 cx = ncx, cy = ncy, cz = ncz, kk = nkk;
         ncx = ld_rec(rec, sa, 4, kSmem); ncy = ld_rec(rec, sa, 5, kSmem); ncz = ld_rec(rec, sa, 6, kSmem); nkk = ld_rec(rec, sa, 7, kSmem);
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-            const float2 X = h ? make_float2(cx.z, cx.w) : make_float2(cx.x, cx.y);
-            const float2 Y = h ? make_float2(cy.z, cy.w) : make_float2(cy.x, cy.y);
-            const float2 Z = h ? make_float2(cz.z, cz.w) : make_float2(cz.x, cz.y);
-            const float2 K = h ? make_float2(kk.z, kk.w) : make_float2(kk.x, kk.y);
-            const float2 hb = ffma2(X, bc2(f.DX), ffma2(Y, bc2(f.DY), ffma2(Z, bc2(f.DZ), bc2(f.NPD))));
-            const float2 C = ffma2(X, bc2(f.M2PX), ffma2(Y, bc2(f.M2PY), ffma2(Z, bc2(f.M2PZ), K)));
-            const float2 disc = ffma2(hb, hb, neg2(C));
-            m = __funnelshift_l(__float_as_uint(disc.x), m, 1);
-            m = __funnelshift_l(__float_as_uint(disc.y), m, 1);
-        }
+        m = filter_record(m, cx, cy, cz, kk, f);
     }
     const int absent = 32 - 4 * n_rec;                       // spheres of the word that were not filtered: marked "not passed"
     return (m << absent) | ((1u << absent) - 1u);
+}
+
+// The precise test of small sphere p, unless it is the one the ray starts on (candidate_self tests that one).
+__device__ __forceinline__ void candidate_small(const float4* __restrict__ small, int p, V3<float> o, V3<float> dhat, float inv_a, float t_min,
+                                                int self_pos, float* t_best, int* p_best)
+{
+    if (p != self_pos) { const float4 s = small[p]; candidate<float, true>(o, dhat, inv_a, t_min, mk(s.x, s.y, s.z), s.w, p, t_best, p_best); }
+}
+
+// Candidate collection of both filters: the survivors of one pass word (bit (31-k) set: sphere p0 + k passed) go onto the lane's
+// list (slot k at cand[k * stride]) as positions relative to `base`, and once the list holds RT_CAND_CAP, straight to the precise
+// test.  uint16 slots: the FP32 table can hold more than 65 535 spheres, so that scan lists positions relative to its segment.
+__device__ __forceinline__ void collect(unsigned pass, int p0, int base, uint16_t* cand, int stride, int* nc, const float4* __restrict__ small,
+                                        V3<float> o, V3<float> dhat, float inv_a, float t_min, int self_pos, float* t_best, int* p_best)
+{
+    while (pass) {
+        const int k = __clz(pass);
+        pass &= ~(0x80000000u >> k);
+        const int p = p0 + k;
+        if (*nc < RT_CAND_CAP) { cand[*nc * stride] = (uint16_t)(p - base); ++*nc; }
+        else candidate_small(small, p, o, dhat, inv_a, t_min, self_pos, t_best, p_best);
+    }
 }
 
 template <bool kSmem>
@@ -229,70 +259,37 @@ __device__ __forceinline__ void scan_small(const float* __restrict__ table, int 
     do {
         const int w1 = min(w0 + RT_SEG_WORDS, n_words);
         int nc = 0;
-        for (int w = w0; w < w1; ++w, rec += 32) {
-            unsigned c = ~filter_word(rec, f, ncx, ncy, ncz, nkk);      // bit (31-k) set: sphere 32w+k passed the filter
-            while (c) {
-                const int k = __clz(c);
-                c &= ~(0x80000000u >> k);
-                const int p = (w << 5) + k;
-                if (nc < RT_CAND_CAP) { cand[nc * cand_stride] = (uint16_t)(p - (w0 << 5)); ++nc; }
-                else if (p != self_pos) { const float4 s = small[p]; candidate<float, true>(o, dhat, inv_a, t_min, mk(s.x, s.y, s.z), s.w, p, &tb, &pb); }
-            }
-        }
+        for (int w = w0; w < w1; ++w, rec += 32)
+            collect(~filter_word(rec, f, ncx, ncy, ncz, nkk), w << 5, w0 << 5, cand, cand_stride, &nc, small, o, dhat, inv_a, t_min, self_pos, &tb, &pb);
         if (w1 == n_words && n_tail) {                                   // the partial word: survivors go straight to the precise test
             unsigned c = ~filter_tail<kSmem>(reinterpret_cast<const float4*>(table) + (size_t)n_words * 32, n_tail, f);
             while (c) {
                 const int k = __clz(c);
                 c &= ~(0x80000000u >> k);
-                const int p = (n_words << 5) + k;
-                if (p != self_pos) { const float4 s = small[p]; candidate<float, true>(o, dhat, inv_a, t_min, mk(s.x, s.y, s.z), s.w, p, &tb, &pb); }
+                candidate_small(small, (n_words << 5) + k, o, dhat, inv_a, t_min, self_pos, &tb, &pb);
             }
         }
         const int nmax = __reduce_max_sync(RT_FULL, nc);
-        for (int k = 0; k < nmax; ++k) {
-            if (k < nc) {
-                const int p = (w0 << 5) + cand[k * cand_stride];
-                if (p != self_pos) { const float4 s = small[p]; candidate<float, true>(o, dhat, inv_a, t_min, mk(s.x, s.y, s.z), s.w, p, &tb, &pb); }
-            }
-        }
+        for (int k = 0; k < nmax; ++k)
+            if (k < nc) candidate_small(small, (w0 << 5) + cand[k * cand_stride], o, dhat, inv_a, t_min, self_pos, &tb, &pb);
         w0 = w1;
     } while (w0 < n_words);
     *p_best = pb; *t_best = tb;
 }
 
-// The spheres too large for f32 (|oc|^2 - r^2 of sphere.rs:22 cancels: the r = 1000 ground, main.rs:64), tested in f64 against
-// the closest hit so far.  Not inlined: once per ray, and kept out of the scan's register allocation.
-__device__ __noinline__ HitF big_spheres_hit(const double4* __restrict__ big, const int* __restrict__ big_idx, int nb, V3<float> o, V3<float> dhat,
-                                             float t_min, int self_code, V3<float> self_n, HitF h)
+struct HitD {            // the large spheres' closest hit, t kept in f64 for the merge
+    double t;
+    int idx;
+    int code;
+};
+
+// The spheres too large for f32 (|oc|^2 - r^2 of sphere.rs:22 cancels: the r = 1000 ground, main.rs:64), tested in f64.
+// Not inlined: rare (a lane the f32 form does not cover), and kept out of the scan's register allocation.
+__device__ __noinline__ HitD big_spheres_best(const double4* __restrict__ big, const int* __restrict__ big_idx, int nb, V3<float> o, V3<float> dhat,
+                                              float t_min, int self_code, V3<float> self_n)
 {
     const V3<double> od = mk<double>(o.x, o.y, o.z), dd = mk<double>(dhat.x, dhat.y, dhat.z);
     const double inv_ad = 2.0 - length_squared(dd);          // 1/a for a = 1 + e, |e| < 1e-6: exact to e^2
-    double tbd = (double)h.t; int ib = h.idx;
-    for (int b = 0; b < nb; ++b) {
-        const double4 s = big[b];
-        const int before = ib; const double tbefore = tbd;
-        if (self_code == -2 - b) {
-            // self_n is unit to f32 rounding (|sn|^2 = 1 + e, |e| < 1e-6): one Newton step of 1/sqrt from the seed 1 is exact to
-            // e^2 — no f64 sqrt and division (~60 instructions on a pipe that runs at 1/32 of the FP32 rate)
-            V3<double> sn = mk<double>(self_n.x, self_n.y, self_n.z);
-            sn = sn * (1.5 - 0.5 * length_squared(sn));
-            candidate_self<double>(dd, inv_ad, (double)t_min, sn, s.w, big_idx[b], &tbd, &ib);
-        } else {
-            candidate<double, true>(od, dd, inv_ad, (double)t_min, mk(s.x, s.y, s.z), s.w, big_idx[b], &tbd, &ib);
-        }
-        if (ib != before || tbd != tbefore) { h.idx = ib; h.t = (float)tbd; h.code = -2 - b; }
-    }
-    return h;
-}
-
-// The same test with the result kept in f64 and no earlier hit to compare with: the tensor-core scan (rt_umma_scan.cuh) runs
-// it while the first MMA chunk is in flight and merges afterwards — (t ascending, list index descending) is a total order, so
-// the closest hit does not depend on the order in which candidates are offered.
-__device__ __noinline__ void big_spheres_best(const double4* __restrict__ big, const int* __restrict__ big_idx, int nb, V3<float> o, V3<float> dhat,
-                                              float t_min, int self_code, V3<float> self_n, double* t_out, int* idx_out, int* code_out)
-{
-    const V3<double> od = mk<double>(o.x, o.y, o.z), dd = mk<double>(dhat.x, dhat.y, dhat.z);
-    const double inv_ad = 2.0 - length_squared(dd);
     double tbd = __longlong_as_double(0x7ff0000000000000LL); int ib = -1, code = RT_SELF_NONE;
     for (int b = 0; b < nb; ++b) {
         const double4 s = big[b];
@@ -308,10 +305,11 @@ __device__ __noinline__ void big_spheres_best(const double4* __restrict__ big, c
         }
         if (ib != before || tbd != tbefore) code = -2 - b;
     }
-    *t_out = tbd; *idx_out = ib; *code_out = code;
+    HitD h; h.t = tbd; h.idx = ib; h.code = code;
+    return h;
 }
 
-// The large spheres in f32, for the tensor-core scan.  `half_b^2 - a c` (sphere.rs:24) cancels in f32 for a sphere of radius 1000
+// The large spheres in f32.  `half_b^2 - a c` (sphere.rs:24) cancels in f32 for a sphere of radius 1000
 // because c = |o - c|^2 - r^2 is formed from two numbers of size 10^6.  Expanded around the COORDINATE origin instead,
 //     C = |o|^2 - 2 o.c + K ,   K = |c|^2 - r^2  (per sphere, from f64, carried as hi + lo)
 // has terms of the size of the result whenever the origin is near the scene and outside the sphere (the ground: K = 0,
@@ -354,18 +352,31 @@ __device__ __forceinline__ void big_spheres_f32(const float4* __restrict__ bigf,
     *t_out = tb; *idx_out = ib; *code_out = code; *need64 = bad;
 }
 
-// The FP32 scan's call: the f32 form, or f64 for the lanes / scenes it does not cover, merged into the closest small-sphere hit
-// by (t ascending, list index descending) — sphere.rs:29,31 + mod.rs:61-66.  Not inlined: once per ray, and kept out of the
-// scan's register allocation (as big_spheres_hit was).
+// The large spheres' own closest hit: the f32 form, or f64 for the lanes / scenes it does not cover.
+__device__ __forceinline__ HitD big_spheres(const float4* __restrict__ bigf, const double4* __restrict__ big, const int* __restrict__ big_idx, int nb,
+                                            V3<float> o, V3<float> dhat, float t_min, int self_code, V3<float> self_n)
+{
+    bool need64 = bigf == nullptr;
+    HitD h; float tf = __int_as_float(0x7f800000); h.idx = -1; h.code = RT_SELF_NONE;
+    if (!need64) big_spheres_f32(bigf, big_idx, nb, o, dhat, t_min, self_code, self_n, &tf, &h.idx, &h.code, &need64);
+    h.t = (double)tf;
+    if (need64) h = big_spheres_best(big, big_idx, nb, o, dhat, t_min, self_code, self_n);
+    return h;
+}
+
+// The large spheres' hit merged into the small spheres' one by (t ascending, list index descending), sphere.rs:29,31 +
+// mod.rs:61-66, compared in f64.  A total order: the winner is the one a test of the large spheres seeded with h would give.
+__device__ __forceinline__ HitF merge_big(HitF h, HitD b)
+{
+    if (b.idx >= 0 && (b.t < (double)h.t || (b.t == (double)h.t && b.idx > h.idx))) { h.t = (float)b.t; h.idx = b.idx; h.code = b.code; }
+    return h;
+}
+
+// The FP32 scan's call.  Not inlined: once per ray, and kept out of the filter loop's register allocation.
 __device__ __noinline__ HitF big_spheres_merge(const float4* __restrict__ bigf, const double4* __restrict__ big, const int* __restrict__ big_idx, int nb,
                                                V3<float> o, V3<float> dhat, float t_min, int self_code, V3<float> self_n, HitF h)
 {
-    bool need64 = bigf == nullptr;
-    float tf = __int_as_float(0x7f800000); int ib = -1, cb = RT_SELF_NONE;
-    if (!need64) big_spheres_f32(bigf, big_idx, nb, o, dhat, t_min, self_code, self_n, &tf, &ib, &cb, &need64);
-    if (need64) return big_spheres_hit(big, big_idx, nb, o, dhat, t_min, self_code, self_n, h);
-    if (ib >= 0 && (tf < h.t || (tf == h.t && ib > h.idx))) { h.t = tf; h.idx = ib; h.code = cb; }
-    return h;
+    return merge_big(h, big_spheres(bigf, big, big_idx, nb, o, dhat, t_min, self_code, self_n));
 }
 
 // Closest hit of one ray against the whole scene: HittableList::hit (mod.rs:56-69).

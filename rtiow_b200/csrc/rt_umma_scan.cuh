@@ -7,8 +7,8 @@
 //                   the group's D columns (fp16 accumulator) ; tcgen05.commit -> full (mbarrier)
 //   ray threads   : wait(full) ; tcgen05.ld.pack::16b their own lane: NC discriminants of THEIR ray, two per register ;
 //                   bar.arrive(hand-back) ; sign bits -> 32-sphere words, four per instruction (sign_word16) ; survivors ->
-//                   per-lane candidate list -> precise test (sphere_roots, rt_device.cuh), exactly as the FP32 scan of
-//                   rt_scene.cuh does.
+//                   per-lane candidate list (collect, shared with the FP32 scan of rt_scene.cuh) -> precise test
+//                   (sphere_roots, rt_device.cuh).
 // The issuer is a warp of its own because tcgen05.mma issue stalls the issuing thread while the tensor pipe is busy
 // (tools/probe_umma_filter.cu: an issuer that shares a warp with an epilogue halves the throughput), and every group has
 // its own: one thread polling all groups' barriers (mbarrier.test_wait) measured 40 % slower in situ.  D is single-buffered
@@ -32,9 +32,6 @@ namespace rt {
 #endif
 #ifndef RT_UMMA_AFULL_BACKOFF_NS
 #define RT_UMMA_AFULL_BACKOFF_NS 0            // the issuer's sleep between polls while its group is in the per-ray phase (0, 100, 400 ns measured the same)
-#endif
-#ifndef RT_UMMA_D16
-#define RT_UMMA_D16 1                         // fp16 accumulator + packed sign collection (rt_umma.cuh, sign_word16); the only form left
 #endif
 #ifndef RT_UMMA_RAY_REGS
 #define RT_UMMA_RAY_REGS 72                   // setmaxnreg of the render kernel's ray warpgroups ...
@@ -234,14 +231,10 @@ __device__ __forceinline__ HitF closest_hit_umma(UmmaCtx& ux, const SceneDev& sc
     // the sphere the ray starts on is tested on its own, independently of the filter (rt_scene.cuh, candidate_self)
     if (self_code >= 0) candidate_self<float>(dhat, inv_a, t_min, self_n, sc.small[self_code].w, self_code, &tb, &pb);
 
-    // the line's foot point of the coordinate origin, orthogonalised twice (a far origin leaves O(u |o|) along dhat after one pass)
-    V3<float> f = o - dhat * (dot(o, dhat) * inv_a);
-    f = f - dhat * (dot(f, dhat) * inv_a);
-    const float sigma = sc.filter_sigma * (fabsf(o.x) + fabsf(o.y) + fabsf(o.z));     // covers the f32 error of a far origin's foot point
-    const bool live = length_squared(f) < sc.filter_R2 + sigma;                        // a line that misses the bounding sphere hits nothing
     {
+        const LineGate g = line_gate(o, dhat, inv_a, sc.filter_R2, sc.filter_sigma);
         uint32_t row1[8], row2[8];
-        ray_rows(f.x, f.y, f.z, dhat.x, dhat.y, dhat.z, live, sigma, sc.u_sc, row1, row2);
+        ray_rows(g.f.x, g.f.y, g.f.z, dhat.x, dhat.y, dhat.z, g.live, g.sigma, sc.u_sc, row1, row2);
         tmem_st8(ux.t_a + ux.lane_base, row1);
         tmem_st8(ux.t_a + 8u + ux.lane_base, row2);
     }
@@ -251,14 +244,9 @@ __device__ __forceinline__ HitF closest_hit_umma(UmmaCtx& ux, const SceneDev& sc
     RT_STAMP(5);
 
     // the large spheres while the first chunk's MMAs are in flight (later, inside the chunk loop, they delay the warp's hand-backs:
-    // DESIGN.md §7.1): f32 through the cancellation-free form (big_spheres_f32); lanes whose origin defeats it, and scenes whose
-    // large spheres are not f32-representable, take the f64 routine
-    double t_big = __longlong_as_double(0x7ff0000000000000LL); int i_big = -1, c_big = RT_SELF_NONE;
-    if (sc.nb > 0) {
-        bool need64 = sc.bigf == nullptr;
-        if (!need64) { float tf; big_spheres_f32(sc.bigf, sc.big_idx, sc.nb, o, dhat, t_min, self_code, self_n, &tf, &i_big, &c_big, &need64); t_big = (double)tf; }
-        if (need64) big_spheres_best(sc.big, sc.big_idx, sc.nb, o, dhat, t_min, self_code, self_n, &t_big, &i_big, &c_big);
-    }
+    // DESIGN.md §7.1)
+    HitD big{__longlong_as_double(0x7ff0000000000000LL), -1, RT_SELF_NONE};
+    if (sc.nb > 0) big = big_spheres(sc.bigf, sc.big, sc.big_idx, sc.nb, o, dhat, t_min, self_code, self_n);
 
     RT_STAMP(6);
     int nc = 0;
@@ -266,9 +254,6 @@ __device__ __forceinline__ HitF closest_hit_umma(UmmaCtx& ux, const SceneDev& sc
         mbar_wait_spin(ux.bar_full, ux.full_phase); ux.full_phase ^= 1u;
         RT_STAMP(10 + c);
         tc_fence_after();
-#if !RT_UMMA_D16
-#error "the fp32-accumulator scan (one SHF per sphere) was removed; see git history before the fp16-D commit"
-#endif
         uint32_t v[NC / 32][16];
 #pragma unroll
         for (int w = 0; w < NC / 32; ++w) tmem_ld16p(ux.t_d + ux.lane_base + 32u * w, v[w]);
@@ -277,22 +262,15 @@ __device__ __forceinline__ HitF closest_hit_umma(UmmaCtx& ux, const SceneDev& sc
         tc_fence_before();                                                     // hand D back to the issuer, whose next MMAs then
         umma_hand_back(ux);                                                    // overlap the sign collection
 #pragma unroll
-        for (int w = 0; w < NC / 32; ++w) {
-            unsigned pass = ~sign_word16(v[w]);                                // bit (31-k) set: sphere k of the word passed the filter
-            while (pass) {
-                const int k = __clz(pass);
-                pass &= ~(0x80000000u >> k);
-                const int p = c * NC + w * 32 + k;
-                if (nc < RT_CAND_CAP) { ux.cand[nc * kStride] = (uint16_t)p; ++nc; }
-                else if (p != self_code) { const float4 s = sc.small[p]; candidate<float, true>(o, dhat, inv_a, t_min, mk(s.x, s.y, s.z), s.w, p, &tb, &pb); }
-            }
-        }
+        for (int w = 0; w < NC / 32; ++w)                                      // ~sign_word16: bit (31-k) set when sphere k passed
+            collect(~sign_word16(v[w]), c * NC + w * 32, 0, ux.cand, kStride, &nc, sc.small, o, dhat, inv_a, t_min, self_code, &tb, &pb);
         RT_STAMP(70 + c);
     }
     RT_STAMP(7);
     // survivors through the precise test, the warp in lock step, RT_UMMA_DRAIN_ILP per round: the test is one dependent chain (load,
     // ~25 FP operations, a MUFU), so independent ones per lane divide the rounds' latency (the drain is 11 % of an iteration); all of
-    // a round's list reads and sphere loads are issued before its first test (that alone was worth 2 %)
+    // a round's list reads and sphere loads are issued before its first test (that alone was worth 2 %).  The FP32 scan's drain
+    // (scan_small) is kept apart: this form, at one survivor per round, compiles to longer code there.
     const int nmax = __reduce_max_sync(RT_FULL, nc);
     for (int k = 0; k < nmax; k += RT_UMMA_DRAIN_ILP) {
         int pp[RT_UMMA_DRAIN_ILP]; bool gg[RT_UMMA_DRAIN_ILP]; float4 ss[RT_UMMA_DRAIN_ILP];
@@ -310,10 +288,7 @@ __device__ __forceinline__ HitF closest_hit_umma(UmmaCtx& ux, const SceneDev& sc
     }
     RT_STAMP(8);
     HitF h; h.t = tb; h.idx = pb >= 0 ? sc.small_idx[pb] : -1; h.code = pb;
-    // merge with the large spheres: t ascending, then list index descending (sphere.rs:29,31 + mod.rs:61-66), compared in f64 as
-    // big_spheres_hit does
-    if (i_big >= 0 && (t_big < (double)h.t || (t_big == (double)h.t && i_big > h.idx))) { h.t = (float)t_big; h.idx = i_big; h.code = c_big; }
-    return h;
+    return merge_big(h, big);
 }
 
 }  // namespace rt

@@ -118,7 +118,7 @@ def restate(c, r, o, d):
     sc = (Rp, 1.0, Rp * 0.5, 1.0 / Rp)                                        # umma::FeatScale {s0, s1, s4, s10}
     npad = -(-len(c) // 64) * 64
     B, slack = sphere_image(c, r, npad, R_scene, sc)
-    # closest_hit_umma: foot point of the coordinate origin (orthogonalised twice), liveness against the bounding sphere
+    # line_gate (rt_scene.cuh): foot point of the coordinate origin (orthogonalised twice), liveness against the bounding sphere
     a = (d * d).sum(1)
     f = o - d * ((o * d).sum(1) / a)[:, None]
     f = f - d * ((f * d).sum(1) / a)[:, None]

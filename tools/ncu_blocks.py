@@ -28,7 +28,7 @@ src = subprocess.run(["ncu", "-i", rep, "--page", "source", "--csv", "--print-so
 rows = list(csv.reader(io.StringIO(src)))
 hdr = rows[1]; data = [r for r in rows[2:] if len(r) == len(hdr)]
 iex, ismp, iav = hdr.index("Instructions Executed"), hdr.index("# Samples"), hdr.index("Thread Instructions Executed")
-# non-inlined callees (big_spheres_hit, filter_tail) follow the kernel in ncu's listing: keep them, without line info
+# non-inlined callees (big_spheres_merge, big_spheres_best, filter_tail) follow the kernel in ncu's listing: keep them, without line info
 lines += [(0, ("callee", 0), r[1].strip()) for r in data[len(lines):]]
 assert len(data) == len(lines), (len(data), len(lines))
 def cost(op): return 2 if op.split()[-1 if op.startswith("@") else 0].startswith(("FFMA2", "FADD2", "FMUL2")) or " FFMA2" in op[:14] else 1
