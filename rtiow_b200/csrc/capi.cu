@@ -747,7 +747,7 @@ static int launch_render(const ScanPlan& plan, DeviceState& d, const rtiow_camer
     const uint64_t n_lp = (uint64_t)a.local_rows * p->width;
     a.n_chunks = n_lp * a.chunks_per_pixel;
     CU(d.accum.resize(3 * n_lp));
-    a.accum = d.accum.p; a.work_counter = d.counters.p; a.ray_counter = d.counters.p + 1; a.np_smem = 1;
+    a.accum = d.accum.p; a.work_counter = d.counters.p; a.ray_counter = d.counters.p + 1;
     if (sr.begin == 0) CU(cudaMemsetAsync(d.accum.p, 0, 3 * n_lp * sizeof(unsigned long long), st));     // later passes add to the same sums
     CU(cudaMemsetAsync(d.counters.p, 0, 2 * sizeof(unsigned long long), st));
     if (n_lp == 0) return RTIOW_OK;

@@ -32,7 +32,6 @@ template <typename T> struct RenderArgs {
     unsigned long long* accum;     // [3][local_rows*width] 32.32 fixed-point radiance sums
     unsigned long long* work_counter;
     unsigned long long* ray_counter;
-    int np_smem;                   // 1: filter SoA staged in shared memory
 };
 
 #define RT_FIX_SCALE 4294967296.0f   // 2^32
@@ -148,18 +147,14 @@ __device__ __forceinline__ void event_sample(bool camera, const Uniform4<T>& u, 
     *sa = rr * cs; *sb = rr * sn;
 }
 
-// One iteration of ray_color (main.rs:38-57) for every lane of the warp, on explicit rays (the unit-level entry point
-// rtiow_ray_color_batch): world.hit, then miss -> sky / hit -> scatter.  Returns the lane's new `active`; when the path
-// ends, *radiance receives its value (throughput x sky, or black).  The render kernel below runs the same pieces in a
-// different order (scatter of the previous hit and camera rays share one Philox block + sampler per iteration).
-template <typename T, bool kSmem>
-__device__ __forceinline__ bool bounce_step(const SceneDev& sc, const float* table, uint16_t* cand, int cand_stride, const PhiloxKey& key, int max_depth,
-                                            T t_min, bool active, PathState<T>& ps, V3<T>* radiance, int* hit_index = nullptr)
+// One iteration of ray_color (main.rs:38-57) for a lane on an explicit ray (rtiow_ray_color_batch), after the scan found
+// (t_hit, idx, code): miss -> sky / hit -> scatter.  Returns the lane's new `active`; when the path ends, *radiance receives
+// its value (throughput x sky, or black).  The render kernel below runs the same pieces in a different order (scatter of
+// the previous hit and camera rays share one Philox block + sampler per iteration).
+template <typename T>
+__device__ __forceinline__ bool bounce_step(const SceneDev& sc, const PhiloxKey& key, int max_depth, T t_min, PathState<T>& ps, T t_hit, int idx, int code,
+                                            V3<T>* radiance)
 {
-    T t_hit; int idx, code;
-    world_hit<T, kSmem>(sc, table, cand, cand_stride, ps, &t_hit, &idx, &code);
-    if (hit_index) *hit_index = idx;
-    if (!active) return false;
     if (idx < 0) {                                                            // miss: sky (main.rs:54-56)
         *radiance = ps.thr * sky<T, sizeof(T) == 4>(ps.dhat);
         return false;
@@ -243,6 +238,40 @@ __device__ __forceinline__ void accumulate(const RenderArgs<T>& a, uint32_t acc_
     }
 }
 
+// Step 2 of the render iteration (below) for one lane: the camera ray of a fresh sample, or the scatter at the pending hit
+// on sphere hit_idx at ps.o.  Returns whether the lane has a ray for this iteration's scan.
+template <typename T>
+__device__ __forceinline__ bool next_ray(const RenderArgs<T>& a, PathState<T>& ps, bool fresh, bool pending, int hit_idx, int hit_code, uint32_t px, uint32_t pj)
+{
+    const Uniform4<T> u = event_uniforms<T>(a.key, ps.pix_key, ps.smp, fresh ? 0u : (uint32_t)(a.max_depth - ps.depth) + 1u);
+    T sa, sb, z; event_sample(fresh, u, &sa, &sb, &z);
+    bool active = false;
+    if (fresh) {
+        const T su = (T(px) + u.u0) * a.inv_wm1;                 // main.rs:131
+        const T sv = (T(pj) + u.u1) * a.inv_hm1;                 // main.rs:132
+        V3<T> ro, rd; get_ray(a.cam, su, sv, sa, sb, &ro, &rd);  // main.rs:134
+        start_ray(ps, ro, rd, a.t_min);
+        ps.thr = mk<T>(1, 1, 1); ps.self_code = RT_SELF_NONE;
+        ps.depth = a.max_depth;
+        active = ps.depth > 0;                                   // main.rs:40-42
+    } else if (pending) {
+        active = scatter_at_hit(a.scene, a.t_min, ps, ps.o, hit_idx, hit_code, sa, sb, z, u.u0, u.u2);
+    }
+    return active;
+}
+
+// Step 4 for one lane after the scan found (t_hit, idx, code); on a hit the lane moves to the hit point and keeps the
+// sphere in *hit_idx, *hit_code.  Returns whether a scatter is now pending.
+template <typename T>
+__device__ __forceinline__ bool take_hit(const RenderArgs<T>& a, PathState<T>& ps, bool active, uint32_t acc_lp, T t_hit, int idx, int code,
+                                         int* hit_idx, int* hit_code)
+{
+    if (!active) return false;
+    if (idx < 0) { accumulate(a, acc_lp, ps.thr * sky<T, sizeof(T) == 4>(ps.dhat)); return false; }     // miss: sky (main.rs:54-56)
+    ps.o = ps.o + ps.dhat * t_hit; *hit_idx = idx; *hit_code = code;                                    // ray.rs:15-17
+    return true;
+}
+
 // The render kernel.  Per iteration of a warp:
 //   1. lanes without a path take the next (pixel, sample);
 //   2. ONE Philox block + ONE sincospi/sqrt per lane serve whatever event the lane is at — the camera ray of a fresh
@@ -250,6 +279,7 @@ __device__ __forceinline__ void accumulate(const RenderArgs<T>& a, uint32_t acc_
 //      common part runs once, converged, instead of once per divergent branch;
 //   3. the scan (world.hit) for all 32 lanes;
 //   4. miss -> throughput x sky is added to the pixel and the lane is free again; hit -> the lane keeps the hit for step 2.
+// Steps 2 and 4 are next_ray and take_hit, which the tensor-core kernel below calls too.
 template <typename T, bool kSmem, int kThreads, int kMinCtas>
 __global__ void __launch_bounds__(kThreads, kMinCtas) render_kernel(const RenderArgs<T> a)
 {
@@ -271,38 +301,21 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) render_kernel(const Render
         const bool fresh = assign_work(a, wc, lt_mask, pending, ps, acc_lp, &px, &pj);
         if (!__any_sync(RT_FULL, fresh || pending)) break;
 
-        const Uniform4<T> u = event_uniforms<T>(a.key, ps.pix_key, ps.smp, fresh ? 0u : (uint32_t)(a.max_depth - ps.depth) + 1u);
-        T sa, sb, z; event_sample(fresh, u, &sa, &sb, &z);
-        bool active = false;                            // the lane has a ray for this iteration's scan
-        if (fresh) {
-            const T su = (T(px) + u.u0) * a.inv_wm1;                 // main.rs:131
-            const T sv = (T(pj) + u.u1) * a.inv_hm1;                 // main.rs:132
-            V3<T> ro, rd; get_ray(a.cam, su, sv, sa, sb, &ro, &rd);  // main.rs:134
-            start_ray(ps, ro, rd, a.t_min);
-            ps.thr = mk<T>(1, 1, 1); ps.self_code = RT_SELF_NONE;
-            ps.depth = a.max_depth;
-            active = ps.depth > 0;                                   // main.rs:40-42
-        } else if (pending) {
-            active = scatter_at_hit(a.scene, a.t_min, ps, ps.o, hit_idx, hit_code, sa, sb, z, u.u0, u.u2);
-        }
-        pending = false;
-
+        const bool active = next_ray(a, ps, fresh, pending, hit_idx, hit_code, px, pj);
         n_rays_w += __popc(__ballot_sync(RT_FULL, active));          // world.hit call count (main.rs:44)
         T t_hit; int idx, code;
         world_hit<T, kSmem>(a.scene, table, cand, kThreads, ps, &t_hit, &idx, &code);
-        if (active) {
-            if (idx < 0) accumulate(a, acc_lp, ps.thr * sky<T, sizeof(T) == 4>(ps.dhat));     // miss: sky (main.rs:54-56)
-            else { ps.o = ps.o + ps.dhat * t_hit; hit_idx = idx; hit_code = code; pending = true; }   // ray.rs:15-17
-        }
+        pending = take_hit(a, ps, active, acc_lp, t_hit, idx, code, &hit_idx, &hit_code);
     }
     if (lane == 0) atomicAdd(a.ray_counter, (unsigned long long)n_rays_w);
 }
 
 // The same render loop with the sphere filter on the tensor cores (rt_umma_scan.cuh): G groups of 128 ray threads + G
-// MMA-issuer warps per CTA, one CTA per SM.  Everything per ray — work distribution, the Philox event, camera / scatter,
-// the precise test of the filter's survivors, the f64 large-sphere test, accumulation — is the code above; only the
-// filter moves from 7 FFMA2 per sphere pair to three tcgen05.mma per 128 rays x NC spheres, and the warp-level "any lane
-// alive" vote becomes a 128-thread one, because a group's 128 rays form one MMA.
+// MMA-issuer warps per CTA, one CTA per SM.  Everything per ray is the code above — work distribution (assign_work), the
+// Philox event and camera / scatter (next_ray), sky and accumulation (take_hit), and in the scan the precise test of the
+// filter's survivors and the f64 large-sphere test; only the filter moves from 7 FFMA2 per sphere pair to three
+// tcgen05.mma per 128 rays x NC spheres, and the warp-level "any lane alive" vote becomes a 128-thread one, because a
+// group's 128 rays form one MMA.
 template <int G, int NC>
 __global__ void __launch_bounds__(UmmaShape<G, NC>::kRenderThreads, 1) render_kernel_umma(const RenderArgs<float> a)
 {
@@ -332,30 +345,12 @@ __global__ void __launch_bounds__(UmmaShape<G, NC>::kRenderThreads, 1) render_ke
             if (!umma_group_any(ux, fresh || pending)) { umma_group_quit(ux); break; }
             RT_STAMP(3);
 
-            const Uniform4<float> u = event_uniforms<float>(a.key, ps.pix_key, ps.smp, fresh ? 0u : (uint32_t)(a.max_depth - ps.depth) + 1u);
-            float sa, sb, z; event_sample(fresh, u, &sa, &sb, &z);
-            bool active = false;
-            if (fresh) {
-                const float su = (float(px) + u.u0) * a.inv_wm1;             // main.rs:131
-                const float sv = (float(pj) + u.u1) * a.inv_hm1;             // main.rs:132
-                V3<float> ro, rd; get_ray(a.cam, su, sv, sa, sb, &ro, &rd);  // main.rs:134
-                start_ray(ps, ro, rd, a.t_min);
-                ps.thr = mk<float>(1, 1, 1); ps.self_code = RT_SELF_NONE;
-                ps.depth = a.max_depth;
-                active = ps.depth > 0;                                       // main.rs:40-42
-            } else if (pending) {
-                active = scatter_at_hit(a.scene, a.t_min, ps, ps.o, hit_idx, hit_code, sa, sb, z, u.u0, u.u2);
-            }
-            pending = false;
-
+            const bool active = next_ray(a, ps, fresh, pending, hit_idx, hit_code, px, pj);
             n_rays_w += __popc(__ballot_sync(RT_FULL, active));              // world.hit call count (main.rs:44)
             RT_STAMP(4);
             const HitF h = closest_hit_umma<G, NC>(ux, a.scene, ps.o, ps.dhat, ps.tmin_n, ps.self_code, ps.self_n, active);
             RT_STAMP(9);
-            if (active) {
-                if (h.idx < 0) accumulate(a, acc_lp, ps.thr * sky<float, true>(ps.dhat));                    // miss: sky (main.rs:54-56)
-                else { ps.o = ps.o + ps.dhat * h.t; hit_idx = h.idx; hit_code = h.code; pending = true; }    // ray.rs:15-17
-            }
+            pending = take_hit(a, ps, active, acc_lp, h.t, h.idx, h.code, &hit_idx, &hit_code);
         }
         if (lane == 0) atomicAdd(a.ray_counter, (unsigned long long)n_rays_w);
     }

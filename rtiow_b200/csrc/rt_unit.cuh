@@ -31,6 +31,36 @@ __global__ void sphere_hit_kernel(int64_t n, const double* center, const double*
     st3(p, i, pp); st3(normal, i, nn); front_face[i] = ff ? 1 : 0;
 }
 
+// Ray i of a hitlist batch as the scan takes it (a lane past n gets a dummy ray): ps.o, ps.dhat, ps.tmin_n, no self sphere.
+// Returns 1/|dir|, which takes t back to |dir| units; it is a division, not start_ray's rsqrtf.
+template <typename T>
+__device__ __forceinline__ T hitlist_ray(PathState<T>& ps, int64_t i, int64_t n, const double* orig, const double* dir, double t_min)
+{
+    V3<T> o = mk<T>(0, 0, 0), d = mk<T>(0, 1, 0);
+    if (i < n) { o = ld3<T>(orig, i); d = ld3<T>(dir, i); }
+    const T len = length(d), inv_len = T(1) / len;
+    ps.o = o; ps.dhat = d * inv_len; ps.tmin_n = (T)t_min * len;
+    ps.self_code = RT_SELF_NONE; ps.self_n = mk<T>(0, 1, 0);
+    return inv_len;
+}
+
+// HittableList::hit's result for ray i: the closest hit (t_hit, idx) found by the scan, with its HitRecord (mod.rs:20-30).
+// ps is taken by value: by reference, nvcc contracts hitlist_ray's |dir|^2 in another order, which moves the last bits of t.
+template <typename T>
+__device__ __forceinline__ void store_hit(const SceneDev& sc, int64_t i, const PathState<T> ps, T inv_len, T t_hit, int idx,
+                                          int32_t* hit, int32_t* index, double* t, double* p, double* normal, int32_t* front_face)
+{
+    V3<T> pp = mk<T>(0, 0, 0), nn = mk<T>(0, 0, 0); bool ff = false;
+    if (idx >= 0) {
+        V3<T> cen; T rad;
+        if (sizeof(T) == 4) { const float4 s = sc.sph[idx]; cen = mk<T>(s.x, s.y, s.z); rad = s.w; }
+        else { const double4 s = sc.sphd[idx]; cen = mk<T>(s.x, s.y, s.z); rad = s.w; }
+        pp = ps.o + ps.dhat * t_hit; hit_record(pp, cen, rad, ps.dhat, &nn, &ff);
+    }
+    hit[i] = idx >= 0; index[i] = idx; t[i] = idx >= 0 ? (double)(t_hit * inv_len) : 0.0;
+    st3(p, i, pp); st3(normal, i, nn); front_face[i] = ff ? 1 : 0;
+}
+
 // HittableList::hit (mod.rs:56-69) through the renderer's scan
 template <typename T, bool kSmem, int kThreads>
 __global__ void __launch_bounds__(kThreads) hitlist_kernel(SceneDev sc, int64_t n, const double* orig, const double* dir, double t_min,
@@ -40,31 +70,11 @@ __global__ void __launch_bounds__(kThreads) hitlist_kernel(SceneDev sc, int64_t 
     uint16_t* cand;
     const float* table = setup_scan_smem<kSmem>(smem_raw, sc, kThreads, &cand);
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const bool live = i < n;
-    V3<T> o = mk<T>(0, 0, 0), d = mk<T>(0, 1, 0);
-    if (live) { o = ld3<T>(orig, i); d = ld3<T>(dir, i); }
-    const T len = length(d), inv_len = T(1) / len;
-    const V3<T> dhat = d * inv_len;
-    const T tmin_n = (T)t_min * len;
-    T th; int idx;
-    if (sizeof(T) == 4) {
-        HitF h = closest_hit<kSmem>(sc, table, mk<float>((float)o.x, (float)o.y, (float)o.z), mk<float>((float)dhat.x, (float)dhat.y, (float)dhat.z),
-                                    (float)tmin_n, RT_SELF_NONE, mk<float>(0, 1, 0), cand, kThreads);
-        th = (T)h.t; idx = h.idx;
-    } else {
-        double td; closest_hit_f64(sc, mk<double>(o.x, o.y, o.z), mk<double>(dhat.x, dhat.y, dhat.z), (double)tmin_n, RT_SELF_NONE, mk<double>(0, 1, 0), &td, &idx);
-        th = (T)td;
-    }
-    if (!live) return;
-    V3<T> pp = mk<T>(0, 0, 0), nn = mk<T>(0, 0, 0); bool ff = false;
-    if (idx >= 0) {
-        V3<T> cen; T rad;
-        if (sizeof(T) == 4) { const float4 s = sc.sph[idx]; cen = mk<T>(s.x, s.y, s.z); rad = s.w; }
-        else { const double4 s = sc.sphd[idx]; cen = mk<T>(s.x, s.y, s.z); rad = s.w; }
-        pp = o + dhat * th; hit_record(pp, cen, rad, dhat, &nn, &ff);
-    }
-    hit[i] = idx >= 0; index[i] = idx; t[i] = idx >= 0 ? (double)(th * inv_len) : 0.0;
-    st3(p, i, pp); st3(normal, i, nn); front_face[i] = ff ? 1 : 0;
+    PathState<T> ps;
+    const T inv_len = hitlist_ray(ps, i, n, orig, dir, t_min);
+    T th; int idx, code;
+    world_hit<T, kSmem>(sc, table, cand, kThreads, ps, &th, &idx, &code);
+    if (i < n) store_hit(sc, i, ps, inv_len, th, idx, hit, index, t, p, normal, front_face);
 }
 
 // the same through the tensor-core scan (rt_umma_scan.cuh): 128 rays per group, G groups + G issuer warps per CTA
@@ -79,19 +89,11 @@ __global__ void __launch_bounds__(G * 160, 1) hitlist_kernel_umma(SceneDev sc, i
         umma_issuer<G, NC>(ux);
     } else {
         const int64_t i = (int64_t)blockIdx.x * (G * 128) + threadIdx.x;
-        const bool live = i < n;
-        V3<float> o = mk<float>(0, 0, 0), d = mk<float>(0, 1, 0);
-        if (live) { o = ld3<float>(orig, i); d = ld3<float>(dir, i); }
-        const float len = length(d), inv_len = 1.0f / len;
-        const V3<float> dhat = d * inv_len;
-        const HitF h = closest_hit_umma<G, NC>(ux, sc, o, dhat, (float)t_min * len, RT_SELF_NONE, mk<float>(0, 1, 0));
+        PathState<float> ps;
+        const float inv_len = hitlist_ray(ps, i, n, orig, dir, t_min);
+        const HitF h = closest_hit_umma<G, NC>(ux, sc, ps.o, ps.dhat, ps.tmin_n, ps.self_code, ps.self_n);
         umma_group_quit(ux);
-        if (live) {
-            V3<float> pp = mk<float>(0, 0, 0), nn = mk<float>(0, 0, 0); bool ff = false;
-            if (h.idx >= 0) { const float4 s = sc.sph[h.idx]; pp = o + dhat * h.t; hit_record(pp, mk<float>(s.x, s.y, s.z), s.w, dhat, &nn, &ff); }
-            hit[i] = h.idx >= 0; index[i] = h.idx; t[i] = h.idx >= 0 ? (double)(h.t * inv_len) : 0.0;
-            st3(p, i, pp); st3(normal, i, nn); front_face[i] = ff ? 1 : 0;
-        }
+        if (i < n) store_hit(sc, i, ps, inv_len, h.t, h.idx, hit, index, t, p, normal, front_face);
     }
     umma_teardown(tmem_base);
 }
@@ -159,6 +161,30 @@ __global__ void sampler_kernel(int64_t n, const uint32_t* pixel, const uint32_t*
     o[6] = uv.x; o[7] = uv.y; o[8] = uv.z; o[9] = bv.x; o[10] = bv.y; o[11] = bv.z;
 }
 
+// The path of ray i of a ray_color batch: throughput 1, depth max_depth, keyed (pixel[i], sample[i]).  Returns whether the
+// lane has a ray (a lane past n gets a dummy path).
+template <typename T>
+__device__ __forceinline__ bool ray_color_start(PathState<T>& ps, int64_t i, int64_t n, const double* orig, const double* dir, const uint32_t* pixel,
+                                                const uint32_t* sample, int32_t max_depth, double t_min)
+{
+    init_path(ps);
+    ps.thr = mk<T>(1, 1, 1); ps.depth = max_depth;
+    if (i < n) { start_ray(ps, ld3<T>(orig, i), ld3<T>(dir, i), (T)t_min); ps.pix_key = pixel[i]; ps.smp = sample[i]; }
+    return i < n && max_depth > 0;
+}
+
+// bounce_step for a lane whose scan found (t_hit, idx, code) for its ray nr, which goes to trace_ray / trace_idx when they
+// are given.  Returns the lane's new `active`; when the path ends, *result receives its radiance.
+template <typename T>
+__device__ __forceinline__ bool ray_color_bounce(const SceneDev& sc, const PhiloxKey& key, int32_t max_depth, double t_min, int64_t i, uint32_t& nr,
+                                                 int32_t* trace_idx, double* trace_ray, PathState<T>& ps, T t_hit, int idx, int code, V3<T>* result)
+{
+    const size_t k = (size_t)i * max_depth + nr++;                            // world.hit call count (main.rs:44)
+    if (trace_ray) { double* tr = trace_ray + k * 6; tr[0] = ps.o.x; tr[1] = ps.o.y; tr[2] = ps.o.z; tr[3] = ps.dhat.x; tr[4] = ps.dhat.y; tr[5] = ps.dhat.z; }
+    if (trace_idx) trace_idx[k] = idx;
+    return bounce_step(sc, key, max_depth, (T)t_min, ps, t_hit, idx, code, result);
+}
+
 // ray_color (main.rs:38-57): the renderer's bounce loop on explicit rays
 template <typename T, bool kSmem, int kThreads>
 __global__ void __launch_bounds__(kThreads) ray_color_kernel(SceneDev sc, int64_t n, const double* orig, const double* dir, const uint32_t* pixel,
@@ -169,29 +195,20 @@ __global__ void __launch_bounds__(kThreads) ray_color_kernel(SceneDev sc, int64_
     uint16_t* cand;
     const float* table = setup_scan_smem<kSmem>(smem_raw, sc, kThreads, &cand);
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    bool active = i < n && max_depth > 0;
-    PathState<T> ps; init_path(ps);
-    ps.thr = mk<T>(1, 1, 1); ps.depth = max_depth;
+    PathState<T> ps;
+    bool active = ray_color_start(ps, i, n, orig, dir, pixel, sample, max_depth, t_min);
     const PhiloxKey key = philox_key(seed);
     V3<T> result = mk<T>(0, 0, 0);
     uint32_t nr = 0;
-    if (i < n) { start_ray(ps, ld3<T>(orig, i), ld3<T>(dir, i), (T)t_min); ps.pix_key = pixel[i]; ps.smp = sample[i]; }
     while (__any_sync(RT_FULL, active)) {
-        V3<T> rad = mk<T>(0, 0, 0);
-        const bool was = active;
-        if (active) {
-            if (trace_ray) { double* tr = trace_ray + ((size_t)i * max_depth + nr) * 6; tr[0] = ps.o.x; tr[1] = ps.o.y; tr[2] = ps.o.z; tr[3] = ps.dhat.x; tr[4] = ps.dhat.y; tr[5] = ps.dhat.z; }
-            ++nr;                                                             // world.hit call count (main.rs:44)
-        }
-        int hit_index = -1;
-        active = bounce_step<T, kSmem>(sc, table, cand, kThreads, key, max_depth, (T)t_min, active, ps, &rad, &hit_index);
-        if (was && trace_idx) trace_idx[(size_t)i * max_depth + nr - 1] = hit_index;
-        if (was && !active) result = rad;
+        T t_hit; int idx, code;
+        world_hit<T, kSmem>(sc, table, cand, kThreads, ps, &t_hit, &idx, &code);
+        if (active) active = ray_color_bounce(sc, key, max_depth, t_min, i, nr, trace_idx, trace_ray, ps, t_hit, idx, code, &result);
     }
     if (i < n) { st3(color, i, result); if (rays) rays[i] = nr; }
 }
 
-// ray_color through the tensor-core scan: the bounce loop of bounce_step, 128 rays per group in lock step
+// ray_color through the tensor-core scan: the same bounce loop, 128 rays per group in lock step
 template <int G, int NC>
 __global__ void __launch_bounds__(G * 160, 1) ray_color_kernel_umma(SceneDev sc, int64_t n, const double* orig, const double* dir, const uint32_t* pixel,
                                                                     const uint32_t* sample, uint64_t seed, int32_t max_depth, double t_min,
@@ -204,26 +221,14 @@ __global__ void __launch_bounds__(G * 160, 1) ray_color_kernel_umma(SceneDev sc,
         umma_issuer<G, NC>(ux);
     } else {
         const int64_t i = (int64_t)blockIdx.x * (G * 128) + threadIdx.x;
-        bool active = i < n && max_depth > 0;
-        PathState<float> ps; init_path(ps);
-        ps.thr = mk<float>(1, 1, 1); ps.depth = max_depth;
+        PathState<float> ps;
+        bool active = ray_color_start(ps, i, n, orig, dir, pixel, sample, max_depth, t_min);
         const PhiloxKey key = philox_key(seed);
         V3<float> result = mk<float>(0, 0, 0);
         uint32_t nr = 0;
-        if (i < n) { start_ray(ps, ld3<float>(orig, i), ld3<float>(dir, i), (float)t_min); ps.pix_key = pixel[i]; ps.smp = sample[i]; }
         while (umma_group_any(ux, active)) {
-            if (active) {
-                if (trace_ray) { double* tr = trace_ray + ((size_t)i * max_depth + nr) * 6; tr[0] = ps.o.x; tr[1] = ps.o.y; tr[2] = ps.o.z; tr[3] = ps.dhat.x; tr[4] = ps.dhat.y; tr[5] = ps.dhat.z; }
-                ++nr;                                                             // world.hit call count (main.rs:44)
-            }
             const HitF h = closest_hit_umma<G, NC>(ux, sc, ps.o, ps.dhat, ps.tmin_n, ps.self_code, ps.self_n, active);
-            if (!active) continue;
-            if (trace_idx) trace_idx[(size_t)i * max_depth + nr - 1] = h.idx;
-            if (h.idx < 0) { result = ps.thr * sky<float, true>(ps.dhat); active = false; continue; }         // main.rs:54-56
-            const V3<float> p = ps.o + ps.dhat * h.t;                             // ray.rs:15-17
-            const Uniform4<float> u = event_uniforms<float>(key, ps.pix_key, ps.smp, (uint32_t)(max_depth - ps.depth) + 1u);
-            float sa, sb, z; event_sample(false, u, &sa, &sb, &z);
-            if (!scatter_at_hit(sc, (float)t_min, ps, p, h.idx, h.code, sa, sb, z, u.u0, u.u2)) { result = mk<float>(0, 0, 0); active = false; }
+            if (active) active = ray_color_bounce(sc, key, max_depth, t_min, i, nr, trace_idx, trace_ray, ps, h.t, h.idx, h.code, &result);
         }
         umma_group_quit(ux);
         if (i < n) { st3(color, i, result); if (rays) rays[i] = nr; }

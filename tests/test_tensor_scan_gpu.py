@@ -92,6 +92,37 @@ def test_backends_agree_on_ray_color(ctx_final, capi, restore_backend):
     assert a["rays"].max() > 5
 
 
+@pytest.mark.parametrize("backend", ["SCAN_FP32", "SCAN_TENSOR"])
+def test_ray_color_trace_records_every_ray(ctx_final, capi, final_scene, restore_backend, backend):
+    """rtiow_ray_color_trace_batch follows ray_color_batch's paths and records each ray and the sphere it hit"""
+    rng = np.random.default_rng(10)
+    n, depth = 3000, 50
+    o = np.tile([13.0, 2.0, 3.0], (n, 1))
+    d = np.stack([rng.uniform(-11, 11, n), rng.uniform(0, 1.5, n), rng.uniform(-11, 11, n)], 1) - o
+    d = d.astype(np.float32).astype(float)
+    px = rng.integers(0, 1 << 20, n).astype(np.uint32); sm = rng.integers(0, 500, n).astype(np.uint32)
+    ctx_final.set_scan_backend(getattr(capi, backend))
+    a = ctx_final.ray_color_batch(o, d, px, sm, seed=11, max_depth=depth)
+    tr = ctx_final.ray_color_trace_batch(o, d, px, sm, seed=11, max_depth=depth)
+    assert np.array_equal(a["color"], tr["color"]) and np.array_equal(a["rays"], tr["rays"])
+    rays = tr["rays"].astype(np.int64)[:, None]
+    k = np.arange(depth)[None, :]
+    assert rays.max() > 5 and (rays >= 1).all()
+    assert (tr["index"][k < rays - 1] >= 0).all()                    # every ray but a path's last one hit a sphere
+    assert (tr["index"][k >= rays] == -1).all() and (tr["ray"][k >= rays] == 0).all()
+    assert np.abs(tr["ray"][:, 0, :3] - o).max() == 0.0
+    assert np.abs(tr["ray"][:, 0, 3:] - d / np.linalg.norm(d, axis=1, keepdims=True)).max() < 1e-6
+    # ray k + 1 starts on sphere index[k].  The hit point is o + dhat t in f32: both filters put it within 4e-6 of the sphere
+    # (hit points up to 53 from the origin, where an f32 ulp is 4e-6).  The bar of 1e-4 allows 25 times that and is still
+    # far below 0.2, the smallest radius, so a ray recorded against the wrong sphere or depth fails it.
+    cen, rad = np.asarray(final_scene[0]["center"], float), np.abs(np.asarray(final_scene[0]["radius"], float))
+    bounce = k[:, :-1] < rays - 1
+    i, j = np.nonzero(bounce)
+    s = tr["index"][i, j]
+    res = np.abs(np.linalg.norm(tr["ray"][i, j + 1, :3] - cen[s], axis=1) - rad[s])
+    assert len(res) > n and res.max() < 1e-4, f"max |dist - r| {res.max():.3g}"
+
+
 def test_selection_rules(ctx, capi, scene_factory, restore_backend):
     """a scene whose sphere table does not fit one CTA's shared memory stays on the FP32 filter; forcing TENSOR is an error, not a fallback"""
     arrays, _ = scene_factory(1, 50, 0)                 # ~10.2 k spheres (BASELINE configs[3])
