@@ -156,6 +156,16 @@ void rtiow_params_default(rtiow_params* p);
  * buffer handed to ImageBuffer::from_vec at main.rs:147 — into caller-owned HOST memory. */
 int rtiow_render(rtiow_ctx* ctx, const rtiow_camera* cam, const rtiow_params* p, uint8_t* out_rgba, rtiow_stats* stats);
 
+/* Many views of one scene (turntables, animations, stereo pairs, camera sweeps) in one call: out_rgba receives n_views top-down
+ * RGBA8 frames of 4*width*height bytes each, in view order, in caller-owned HOST memory.  Frame v equals
+ * rtiow_render(ctx, &cams[v], p, ...) byte for byte, so the views share their sample streams (same seed, same pixel keys);
+ * decorrelated views are separate calls with other seeds.  One render launch per device pays the fixed per-launch cost once
+ * per batch.  An n-GPU ctx renders a contiguous block of whole views on each device.  n_views * width * height must be
+ * <= 0xfffffff0.  A rank ctx with world > 1 returns RTIOW_ERR_UNSUPPORTED.  Stats cover the whole batch (kernel_ms: the
+ * slowest device's). */
+int rtiow_render_views(rtiow_ctx* ctx, const rtiow_camera* cams, uint32_t n_views, const rtiow_params* p, uint8_t* out_rgba,
+                       rtiow_stats* stats);
+
 /* The reference shows progress per row (indicatif bar, main.rs:120,124) and the finished frame in a piston window
  * (main.rs:151-171).  The GPU equivalent: the spp samples are rendered in n_passes slices (clamped to spp); after each slice
  * on_pass(user, pass [1-based], n_passes, spp_done, rgba) receives the frame so far — out_rgba, top-down RGBA8, quantised

@@ -108,6 +108,14 @@ def render(cam: capi.Camera, world: HittableList, params: capi.Params, n_gpus: i
     return img
 
 
+def render_views(cams, world: HittableList, params: capi.Params, n_gpus: int = 1):
+    """Many cameras of one world in one call: [K,H,W,4] top-down RGBA8, frame v byte-identical to render(cams[v], ...)."""
+    with capi.Context(n_gpus) as ctx:
+        ctx.upload_scene(**world.to_arrays())
+        imgs, _ = ctx.render_views(cams, params)
+    return imgs
+
+
 def render_progressive(cam: capi.Camera, world: HittableList, params: capi.Params, n_passes: int, on_pass=None, n_gpus: int = 1):
     """render() in n_passes slices of the samples; on_pass(pass_1based, n_passes, spp_done, rgba[H,W,4]) after each — the role of
     the reference's progress bar and preview window (main.rs:120-124,151-171).  Final frame bit-identical to render()'s."""

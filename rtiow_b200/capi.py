@@ -30,7 +30,7 @@ PROGRESS_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint3
 SYMBOLS = [
     "rtiow_abi_version", "rtiow_last_error", "rtiow_device_count", "rtiow_ctx_create", "rtiow_ctx_create_on_device",
     "rtiow_ctx_destroy", "rtiow_ctx_set_scan_backend", "rtiow_nccl_unique_id", "rtiow_ctx_create_rank", "rtiow_ctx_set_gather", "rtiow_ctx_set_stream",
-    "rtiow_ctx_gather_info", "rtiow_render_rank", "rtiow_render_rank_device", "rtiow_render_rank_enqueue", "rtiow_ctx_synchronize", "rtiow_scene_upload", "rtiow_camera_new", "rtiow_params_default", "rtiow_render", "rtiow_render_progressive",
+    "rtiow_ctx_gather_info", "rtiow_render_rank", "rtiow_render_rank_device", "rtiow_render_rank_enqueue", "rtiow_ctx_synchronize", "rtiow_scene_upload", "rtiow_camera_new", "rtiow_params_default", "rtiow_render", "rtiow_render_views", "rtiow_render_progressive",
     "rtiow_tile_buffer_bytes", "rtiow_render_tiles_device", "rtiow_render_to_frame_device", "rtiow_deinterleave_device", "rtiow_sphere_hit_batch",
     "rtiow_hitlist_batch", "rtiow_scatter_batch", "rtiow_get_ray_batch", "rtiow_to_rgba_batch", "rtiow_reflect_batch",
     "rtiow_refract_batch", "rtiow_ray_color_batch", "rtiow_ray_color_trace_batch", "rtiow_sampler_batch", "rtiow_fp32_peak_probe", "rtiow_flush_l2",
@@ -119,6 +119,7 @@ def _declare(L):
         "rtiow_camera_new": (C.c_int, [P, P, P, d, d, d, d, C.POINTER(Camera)]),
         "rtiow_params_default": (None, [C.POINTER(Params)]),
         "rtiow_render": (C.c_int, [P, C.POINTER(Camera), C.POINTER(Params), P, C.POINTER(Stats)]),
+        "rtiow_render_views": (C.c_int, [P, C.POINTER(Camera), C.c_uint32, C.POINTER(Params), P, C.POINTER(Stats)]),
         "rtiow_render_progressive": (C.c_int, [P, C.POINTER(Camera), C.POINTER(Params), C.c_uint32, PROGRESS_FN, P, P, C.POINTER(Stats)]),
         "rtiow_render_rank_enqueue": (C.c_int, [P, C.POINTER(Camera), C.POINTER(Params), C.POINTER(C.c_void_p)]),
         "rtiow_ctx_synchronize": (C.c_int, [P, C.POINTER(Stats)]),
@@ -353,6 +354,28 @@ class Context:
         st = Stats()
         _check(lib().rtiow_render(self._h, C.byref(cam), C.byref(params), _p(out), C.byref(st)))
         return out, st.as_dict()
+
+    def render_views(self, cams, params: Params, out=None):
+        """rtiow_render_views: many cameras of the uploaded scene in one call -> (rgba[K,H,W,4] uint8, stats of the batch).
+        View v is byte-identical to render(cams[v], params).  `out` (K*H*W*4 contiguous uint8: a numpy array, or a CPU torch
+        tensor such as a pin_memory() one) receives the frames."""
+        cams = list(cams)
+        k = len(cams)
+        arr = (Camera * max(k, 1))(*cams)
+        shape = (k, params.height, params.width, 4)
+        if out is None:
+            out = np.empty(shape, np.uint8)
+        if isinstance(out, np.ndarray):
+            if out.dtype != np.uint8 or out.size != int(np.prod(shape)) or not out.flags.c_contiguous:
+                raise ValueError(f"out must be a C-contiguous uint8 array with {int(np.prod(shape))} elements")
+            ptr = _p(out)
+        else:                                 # a torch tensor (e.g. pinned host memory)
+            if str(out.dtype) != "torch.uint8" or out.numel() != int(np.prod(shape)) or not out.is_contiguous() or out.device.type != "cpu":
+                raise ValueError(f"out must be a contiguous CPU uint8 tensor with {int(np.prod(shape))} elements")
+            ptr = C.c_void_p(out.data_ptr())
+        st = Stats()
+        _check(lib().rtiow_render_views(self._h, arr, k, C.byref(params), ptr, C.byref(st)))
+        return out.reshape(shape), st.as_dict()
 
     def render_progressive(self, cam: Camera, params: Params, n_passes: int, on_pass=None, out: np.ndarray | None = None):
         """rtiow_render_progressive: the spp samples in n_passes slices; on_pass(pass_1based, n_passes, spp_done, rgba[H,W,4] view)

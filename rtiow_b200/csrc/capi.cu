@@ -93,6 +93,7 @@ struct DeviceState {
     DevBuf<uint32_t> tiles; DevBuf<uint32_t> gathered; DevBuf<uint32_t> frame;
     HostBuf<uint8_t> pinned;                           // staging of the frame's D2H copy when the caller's buffer is pageable
     HostBuf<unsigned long long> pinned_cnt;            // the counters after the frame
+    DevBuf<unsigned char> cams; HostBuf<unsigned char> cams_stage;   // the cameras of a batch of views (rtiow_render_views) and their staging
     // measurement
     DevBuf<uint4> flush; DevBuf<float> probe;
     int last_backend = RTIOW_SCAN_FP32;                // which filter the last render launch used (rtiow_stats.scan_backend)
@@ -334,7 +335,7 @@ extern "C" void rtiow_ctx_destroy(rtiow_ctx* c)
         d.scene_blob.release();
         d.accum.release(); d.counters.release(); d.tiles.release(); d.gathered.release(); d.frame.release();
         d.flush.release(); d.probe.release();
-        d.pinned.release(); d.pinned_cnt.release();
+        d.pinned.release(); d.pinned_cnt.release(); d.cams.release(); d.cams_stage.release();
         if (d.ev0) cudaEventDestroy(d.ev0);
         if (d.ev1) cudaEventDestroy(d.ev1);
         if (d.ev_done) cudaEventDestroy(d.ev_done);
@@ -687,8 +688,9 @@ template <typename T> static void size_fetch(RenderArgs<T>& a, int grid, int thr
     a.guided_div = (uint32_t)std::max<uint64_t>(1, 2 * n_warps);
 }
 
-// a persistent render kernel: as many CTAs as fit on the SMs at once
-template <typename T, typename K> static int launch_persistent(K kernel, RenderArgs<T>& a, int threads, size_t smem, int sms, cudaStream_t st)
+// a persistent render kernel: as many CTAs as fit on the SMs at once.  `views` is empty for a frame and the device array of the
+// cameras for a batch of views (render_views_kernel)
+template <typename T, typename K, typename... V> static int launch_persistent(K kernel, RenderArgs<T>& a, int threads, size_t smem, int sms, cudaStream_t st, V... views)
 {
     int rc = allow_smem(kernel, smem); if (rc) return rc;
     int per_sm = 0;
@@ -696,31 +698,44 @@ template <typename T, typename K> static int launch_persistent(K kernel, RenderA
     if (per_sm < 1) return fail(RTIOW_ERR_CUDA, "kernel does not fit on an SM (smem %zu)", smem);
     const int grid = per_sm * sms;
     size_fetch(a, grid, threads);
-    kernel<<<grid, threads, smem, st>>>(a);
+    kernel<<<grid, threads, smem, st>>>(a, views...);
     return RTIOW_OK;
 }
 
-template <typename T> static int launch_render_kernel(const ScanPlan& plan, const DeviceState& d, RenderArgs<T>& a, cudaStream_t st)
+// the render kernel of one scan arm: a frame's, or with kViews a batch of views' (the same loop, rt_render.cuh)
+template <bool kViews, typename T, bool kSmem, int kThreads, int kMinCtas> static auto render_entry()
+{
+    if constexpr (kViews) return render_views_kernel<T, kSmem, kThreads, kMinCtas>;
+    else return render_kernel<T, kSmem, kThreads, kMinCtas>;
+}
+template <bool kViews> static auto render_entry_umma()
+{
+    if constexpr (kViews) return render_views_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
+    else return render_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
+}
+
+template <bool kViews, typename T, typename... V>
+static int launch_render_kernel(const ScanPlan& plan, const DeviceState& d, RenderArgs<T>& a, cudaStream_t st, V... views)
 {
     if constexpr (std::is_same<T, double>::value) {
-        return launch_persistent(render_kernel<double, false, 256, 2>, a, 256, plan.smem(256), d.sms, st);
+        return launch_persistent(render_entry<kViews, double, false, 256, 2>(), a, 256, plan.smem(256), d.sms, st, views...);
     } else {
         switch (plan.scan) {
         case Scan::Tensor: {     // one CTA per SM (it owns all of TMEM), G groups of 128 rays + G issuer warps
-            auto k = render_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
+            auto k = render_entry_umma<kViews>();
             const size_t smem = plan.smem(UShape::kRenderThreads);
             int rc = allow_smem(k, smem); if (rc) return rc;
             size_fetch(a, d.sms, UShape::kRayThreads);          // the work is shared among the ray threads, not the whole block
-            k<<<d.sms, UShape::kRenderThreads, smem, st>>>(a);
+            k<<<d.sms, UShape::kRenderThreads, smem, st>>>(a, views...);
             return RTIOW_OK;
         }
         case Scan::Smem:         // 3 CTAs x 256 threads x 80 registers fills the 64K-register file
-            return launch_persistent(render_kernel<float, true, 256, 3>, a, 256, plan.smem(256), d.sms, st);
+            return launch_persistent(render_entry<kViews, float, true, 256, 3>(), a, 256, plan.smem(256), d.sms, st, views...);
         case Scan::Wide:         // one CTA per SM, 24 warps at 80 registers (+2.5 % over 512 threads at 104) when their lists fit
-            if (plan.smem(768) <= 227 * 1024) return launch_persistent(render_kernel<float, true, 768, 1>, a, 768, plan.smem(768), d.sms, st);
-            return launch_persistent(render_kernel<float, true, 512, 1>, a, 512, plan.smem(512), d.sms, st);
+            if (plan.smem(768) <= 227 * 1024) return launch_persistent(render_entry<kViews, float, true, 768, 1>(), a, 768, plan.smem(768), d.sms, st, views...);
+            return launch_persistent(render_entry<kViews, float, true, 512, 1>(), a, 512, plan.smem(512), d.sms, st, views...);
         case Scan::Global:
-            return launch_persistent(render_kernel<float, false, 256, 4>, a, 256, plan.smem(256), d.sms, st);
+            return launch_persistent(render_entry<kViews, float, false, 256, 4>(), a, 256, plan.smem(256), d.sms, st, views...);
         case Scan::F64:
             break;
         }
@@ -732,15 +747,18 @@ template <typename T> static int launch_render_kernel(const ScanPlan& plan, cons
 // a whole frame that may live on another GPU (fused quantise + gather: finalize_to_frame_kernel)
 struct Dest { uint32_t* p; bool whole_frame; };
 
+// n_views = 0: a frame (or a rank's rows of one) of camera *cam.  n_views > 0 (world 1): a batch of views, the cameras
+// cam[0 .. n_views), rendered as one frame n_views * height rows tall whose epilogue writes the views' frames one after the other.
 template <typename T>
 static int launch_render(const ScanPlan& plan, DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, uint32_t rank, uint32_t world, SampleRange sr,
-                         Dest dst, cudaStream_t st, uint32_t* launches)
+                         Dest dst, cudaStream_t st, uint32_t* launches, uint32_t n_views)
 {
     RenderArgs<T> a;
     a.scene = d.scene; a.cam = to_dev_camera<T>(*cam);
     a.width = p->width; a.height = p->height; a.spp = sr.count; a.smp_begin = sr.begin; a.max_depth = p->max_depth; a.t_min = (T)p->t_min; a.key = philox_key(p->seed);
     a.inv_wm1 = (T)(1.0 / (double)(p->width - 1)); a.inv_hm1 = (T)(1.0 / (double)(p->height - 1));
-    a.rank = rank; a.world = world; a.tile_rows = tile_rows_of(p); a.local_rows = rows_of_rank(p->height, tile_rows_of(p), world, rank);
+    a.rank = rank; a.world = world; a.tile_rows = tile_rows_of(p);
+    a.local_rows = n_views ? n_views * p->height : rows_of_rank(p->height, tile_rows_of(p), world, rank);
     a.chunk_samples = std::min<uint32_t>(sr.count, 64u);
     a.chunks_per_pixel = (sr.count + a.chunk_samples - 1) / a.chunk_samples;
     a.chunks_per_fetch = std::max<uint32_t>(1u, 256u / a.chunk_samples);
@@ -752,7 +770,18 @@ static int launch_render(const ScanPlan& plan, DeviceState& d, const rtiow_camer
     CU(cudaMemsetAsync(d.counters.p, 0, 2 * sizeof(unsigned long long), st));
     if (n_lp == 0) return RTIOW_OK;
     d.last_backend = plan.scan == Scan::Tensor ? RTIOW_SCAN_TENSOR : RTIOW_SCAN_FP32;
-    int rc = launch_render_kernel(plan, d, a, st); if (rc) return rc;
+    int rc;
+    if (n_views) {              // the cameras go up in one copy; only a path's first ray reads its view's camera
+        const size_t bytes = (size_t)n_views * sizeof(CameraT<T>);
+        CU(d.cams_stage.resize(bytes)); CU(d.cams.resize(bytes));
+        CameraT<T>* staged = reinterpret_cast<CameraT<T>*>(d.cams_stage.p);
+        for (uint32_t v = 0; v < n_views; ++v) staged[v] = to_dev_camera<T>(cam[v]);
+        CU(cudaMemcpyAsync(d.cams.p, staged, bytes, cudaMemcpyHostToDevice, st));
+        rc = launch_render_kernel<true>(plan, d, a, st, reinterpret_cast<const CameraT<T>*>(d.cams.p));
+    } else {
+        rc = launch_render_kernel<false>(plan, d, a, st);
+    }
+    if (rc) return rc;
     CU(cudaGetLastError());
     if (dst.whole_frame)
         finalize_to_frame_kernel<<<(unsigned)((n_lp + 255) / 256), 256, 0, st>>>(d.accum.p, (uint32_t)n_lp, sr.begin + sr.count, p->alpha, p->width, tile_rows_of(p), world, rank, dst.p);
@@ -764,28 +793,29 @@ static int launch_render(const ScanPlan& plan, DeviceState& d, const rtiow_camer
 }
 
 // One device's part of a frame: samples `sr` of the rows {y : (y / tile_rows) % world == rank}, quantised into `dst`, with the
-// events e0 / e1 around the work and its kernel launches added to *launches
+// events e0 / e1 around the work and its kernel launches added to *launches.  n_views > 0: the batch of views cam[0 .. n_views)
+// (launch_render).
 static int render_step(const rtiow_ctx* c, DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, uint32_t rank, uint32_t world, SampleRange sr,
-                       Dest dst, cudaStream_t st, cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches)
+                       Dest dst, cudaStream_t st, cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches, uint32_t n_views = 0)
 {
     if (!d.has_scene) return fail(RTIOW_ERR_INVALID_ARG, "no scene uploaded (call rtiow_scene_upload first)");
     CU(cudaSetDevice(d.device));
     ScanPlan plan;
     int rc = plan_scan(c, d, p->precision, &plan); if (rc) return rc;
     CU(cudaEventRecord(e0, st));
-    rc = plan.scan == Scan::F64 ? launch_render<double>(plan, d, cam, p, rank, world, sr, dst, st, launches)
-                                : launch_render<float>(plan, d, cam, p, rank, world, sr, dst, st, launches);
+    rc = plan.scan == Scan::F64 ? launch_render<double>(plan, d, cam, p, rank, world, sr, dst, st, launches, n_views)
+                                : launch_render<float>(plan, d, cam, p, rank, world, sr, dst, st, launches, n_views);
     if (rc) return rc;
     CU(cudaEventRecord(e1, st));
     return RTIOW_OK;
 }
 
-// a frame on one device: its rank-local order IS top-down
+// a frame on one device: its rank-local order IS top-down (and a batch of n_views views is their frames one after the other)
 static int render_single(const rtiow_ctx* c, DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, SampleRange sr, cudaStream_t st,
-                         cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches, const uint32_t** d_frame)
+                         cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches, const uint32_t** d_frame, uint32_t n_views = 0)
 {
-    CU(d.tiles.resize((size_t)p->width * p->height));
-    int rc = render_step(c, d, cam, p, 0, 1, sr, Dest{ d.tiles.p, false }, st, e0, e1, launches); if (rc) return rc;
+    CU(d.tiles.resize((size_t)p->width * p->height * std::max<uint32_t>(n_views, 1)));
+    int rc = render_step(c, d, cam, p, 0, 1, sr, Dest{ d.tiles.p, false }, st, e0, e1, launches, n_views); if (rc) return rc;
     *d_frame = d.tiles.p;
     return RTIOW_OK;
 }
@@ -975,6 +1005,52 @@ extern "C" int rtiow_render(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_p
     if (!c || !cam || !out_rgba) return fail(RTIOW_ERR_INVALID_ARG, "NULL argument");
     int rc = check_params(p); if (rc) return rc;
     return render_frame(c, cam, p, SampleRange{ 0u, p->spp }, out_rgba, stats);
+}
+
+// Many cameras of one scene (turntables, stereo pairs, camera sweeps) in one render launch per device: CTA start-up, the
+// end-of-frame tail, the memsets, the epilogue, the copy and the synchronisation are paid once per batch instead of once per
+// view.  A device renders its views as one frame n_views * height rows tall in which every row keeps its own view's pixel keys
+// (rt_render.cuh, assign_work), so frame v is byte-identical to rtiow_render(cams[v]).  An n-GPU ctx gives device r the whole
+// views [r K / n, (r + 1) K / n), copied straight into their place in out_rgba: no gather.
+extern "C" int rtiow_render_views(rtiow_ctx* c, const rtiow_camera* cams, uint32_t n_views, const rtiow_params* p, uint8_t* out_rgba, rtiow_stats* stats)
+{
+    if (!c || !cams || !out_rgba) return fail(RTIOW_ERR_INVALID_ARG, "NULL argument");
+    int rc = check_params(p); if (rc) return rc;
+    if (n_views == 0) return fail(RTIOW_ERR_INVALID_ARG, "n_views must be >= 1");
+    if ((uint64_t)n_views * p->width * p->height > 0xfffffff0ull) return fail(RTIOW_ERR_INVALID_ARG, "batch too large: n_views * width * height must be <= 0xfffffff0");
+    if (c->world > 1) return fail(RTIOW_ERR_UNSUPPORTED, "rtiow_render_views: a rank ctx with world > 1 renders collective frames (rtiow_render_rank), not batches of views");
+    const double t0 = now_ms();
+    const uint32_t n_dev = (uint32_t)c->dev.size();
+    const size_t frame_bytes = (size_t)p->width * p->height * 4;
+    std::vector<FrameCopy> copies(n_dev);
+    uint32_t launches = 0;
+    int first = -1;                                         // the first device that renders: its scene and scan backend go into the stats
+    for (uint32_t r = 0; r < n_dev; ++r) {
+        const uint32_t v0 = (uint32_t)((uint64_t)r * n_views / n_dev), v1 = (uint32_t)((uint64_t)(r + 1) * n_views / n_dev);
+        if (v0 == v1) continue;                             // more devices than views
+        DeviceState& d = c->dev[r];
+        CU(cudaSetDevice(d.device));
+        const uint32_t* d_frames = nullptr;
+        rc = render_single(c, d, cams + v0, p, SampleRange{ 0u, p->spp }, d.stream, d.ev0, d.ev1, &launches, &d_frames, v1 - v0); if (rc) return rc;
+        rc = copies[r].start(d, out_rgba + v0 * frame_bytes, d_frames, (v1 - v0) * frame_bytes, d.stream); if (rc) return rc;
+        CU(cudaMemcpyAsync(d.pinned_cnt.p, d.counters.p, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, d.stream));
+        if (first < 0) first = (int)r;
+    }
+    float ms = 0; uint64_t rays = 0; uint32_t used = 0;
+    for (uint32_t r = 0; r < n_dev; ++r) {
+        if (!copies[r].out) continue;
+        DeviceState& d = c->dev[r];
+        CU(cudaSetDevice(d.device));
+        CU(cudaStreamSynchronize(d.stream));
+        copies[r].finish();
+        float mr = 0; CU(cudaEventElapsedTime(&mr, d.ev0, d.ev1)); ms = std::max(ms, mr);          // the slowest device's kernels
+        rays += d.pinned_cnt.p[1]; ++used;
+    }
+    CU(cudaSetDevice(c->dev[0].device));
+    if (stats)
+        *stats = make_stats(c->dev[first], ms, now_ms() - t0, (uint64_t)n_views * p->width * p->height * p->spp, rays, launches, n_dev,
+                            (uint64_t)n_views * sizeof(rtiow_camera) + sizeof(rtiow_params), (uint64_t)n_views * frame_bytes + 16 * used);
+    return RTIOW_OK;
 }
 
 // The per-pass preview the reference gets from its progress bar and piston window (main.rs:120-124,151-171): the spp samples

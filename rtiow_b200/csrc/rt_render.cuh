@@ -169,16 +169,19 @@ __device__ __forceinline__ bool bounce_step(const SceneDev& sc, const PhiloxKey&
 // ---- the pixel/sample loop's bookkeeping (main.rs:122-135) ---------------------------------------------------------
 // warp-uniform cursor over the work: chunks (<= 256 samples of ONE pixel) fetched from a global atomic counter
 struct WorkCursor {
-    uint32_t cs = 0, ce = 0, c_lp = 0, c_x = 0, c_y = 0;
+    uint32_t cs = 0, ce = 0, c_lp = 0, c_x = 0, c_y = 0, c_v = 0;
     unsigned long long cc = 0, cce = 0;
     bool exhausted = false;
 };
 
 // Every lane whose slot is free (`busy` false) takes the next (pixel, sample) of the warp's chunk (main.rs:130).  Returns
 // true for the lanes that received one; their pixel column / bottom-up row come back in *px, *pj.
-template <typename T>
+// kViews: the launch renders a batch of views (rtiow_render_views) on one device as ONE frame n_views * height rows tall, so
+// local row lr is row lr % height of view lr / height.  *pv receives the view; pj and the Philox pixel key are those of the
+// row within the view, exactly as the view's own frame computes them, which makes every view byte-identical to it.
+template <bool kViews, typename T>
 __device__ __forceinline__ bool assign_work(const RenderArgs<T>& a, WorkCursor& wc, unsigned lt_mask, bool busy, PathState<T>& ps, uint32_t& acc_lp,
-                                            uint32_t* px, uint32_t* pj)
+                                            uint32_t* px, uint32_t* pj, uint32_t* pv)
 {
     bool fresh = false;
     unsigned need = __ballot_sync(RT_FULL, !busy);
@@ -208,6 +211,7 @@ __device__ __forceinline__ bool assign_work(const RenderArgs<T>& a, WorkCursor& 
             const uint32_t lr = wc.c_lp / a.width;
             wc.c_x = wc.c_lp - lr * a.width;
             wc.c_y = local_to_global_row(lr, a.tile_rows, a.world, a.rank);
+            if (kViews) { wc.c_v = lr / a.height; wc.c_y = lr - wc.c_v * a.height; }
         }
         const uint32_t avail = wc.ce - wc.cs;
         const uint32_t r = __popc(need & lt_mask);
@@ -216,6 +220,7 @@ __device__ __forceinline__ bool assign_work(const RenderArgs<T>& a, WorkCursor& 
             acc_lp = wc.c_lp;
             ps.smp = a.smp_begin + wc.cs + r;
             *px = wc.c_x;
+            *pv = wc.c_v;
             *pj = a.height - 1u - wc.c_y;                            // j = 0 is the bottom row (main.rs:132,141-145)
             ps.pix_key = *pj * a.width + wc.c_x;
         }
@@ -239,9 +244,11 @@ __device__ __forceinline__ void accumulate(const RenderArgs<T>& a, uint32_t acc_
 }
 
 // Step 2 of the render iteration (below) for one lane: the camera ray of a fresh sample, or the scatter at the pending hit
-// on sphere hit_idx at ps.o.  Returns whether the lane has a ray for this iteration's scan.
-template <typename T>
-__device__ __forceinline__ bool next_ray(const RenderArgs<T>& a, PathState<T>& ps, bool fresh, bool pending, int hit_idx, int hit_code, uint32_t px, uint32_t pj)
+// on sphere hit_idx at ps.o.  Returns whether the lane has a ray for this iteration's scan.  The camera is a.cam, or with
+// kViews the camera of the sample's view pv.
+template <bool kViews, typename T>
+__device__ __forceinline__ bool next_ray(const RenderArgs<T>& a, const CameraT<T>* cams, PathState<T>& ps, bool fresh, bool pending, int hit_idx, int hit_code,
+                                         uint32_t px, uint32_t pj, uint32_t pv)
 {
     const Uniform4<T> u = event_uniforms<T>(a.key, ps.pix_key, ps.smp, fresh ? 0u : (uint32_t)(a.max_depth - ps.depth) + 1u);
     T sa, sb, z; event_sample(fresh, u, &sa, &sb, &z);
@@ -249,7 +256,8 @@ __device__ __forceinline__ bool next_ray(const RenderArgs<T>& a, PathState<T>& p
     if (fresh) {
         const T su = (T(px) + u.u0) * a.inv_wm1;                 // main.rs:131
         const T sv = (T(pj) + u.u1) * a.inv_hm1;                 // main.rs:132
-        V3<T> ro, rd; get_ray(a.cam, su, sv, sa, sb, &ro, &rd);  // main.rs:134
+        const CameraT<T>& cam = kViews ? cams[pv] : a.cam;
+        V3<T> ro, rd; get_ray(cam, su, sv, sa, sb, &ro, &rd);    // main.rs:134
         start_ray(ps, ro, rd, a.t_min);
         ps.thr = mk<T>(1, 1, 1); ps.self_code = RT_SELF_NONE;
         ps.depth = a.max_depth;
@@ -279,9 +287,10 @@ __device__ __forceinline__ bool take_hit(const RenderArgs<T>& a, PathState<T>& p
 //      common part runs once, converged, instead of once per divergent branch;
 //   3. the scan (world.hit) for all 32 lanes;
 //   4. miss -> throughput x sky is added to the pixel and the lane is free again; hit -> the lane keeps the hit for step 2.
-// Steps 2 and 4 are next_ray and take_hit, which the tensor-core kernel below calls too.
-template <typename T, bool kSmem, int kThreads, int kMinCtas>
-__global__ void __launch_bounds__(kThreads, kMinCtas) render_kernel(const RenderArgs<T> a)
+// Steps 2 and 4 are next_ray and take_hit, which the tensor-core kernel below calls too.  render_kernel renders a frame
+// (or a rank's rows of one); render_views_kernel runs the same loop over a batch of views, one camera per view in `cams`.
+template <typename T, bool kSmem, int kThreads, bool kViews>
+__device__ __forceinline__ void render_loop(const RenderArgs<T>& a, const CameraT<T>* cams)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     uint16_t* cand;
@@ -297,11 +306,11 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) render_kernel(const Render
     WorkCursor wc;
 
     for (;;) {
-        uint32_t px = 0, pj = 0;
-        const bool fresh = assign_work(a, wc, lt_mask, pending, ps, acc_lp, &px, &pj);
+        uint32_t px = 0, pj = 0, pv = 0;
+        const bool fresh = assign_work<kViews>(a, wc, lt_mask, pending, ps, acc_lp, &px, &pj, &pv);
         if (!__any_sync(RT_FULL, fresh || pending)) break;
 
-        const bool active = next_ray(a, ps, fresh, pending, hit_idx, hit_code, px, pj);
+        const bool active = next_ray<kViews>(a, cams, ps, fresh, pending, hit_idx, hit_code, px, pj, pv);
         n_rays_w += __popc(__ballot_sync(RT_FULL, active));          // world.hit call count (main.rs:44)
         T t_hit; int idx, code;
         world_hit<T, kSmem>(a.scene, table, cand, kThreads, ps, &t_hit, &idx, &code);
@@ -310,14 +319,25 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) render_kernel(const Render
     if (lane == 0) atomicAdd(a.ray_counter, (unsigned long long)n_rays_w);
 }
 
+template <typename T, bool kSmem, int kThreads, int kMinCtas>
+__global__ void __launch_bounds__(kThreads, kMinCtas) render_kernel(const RenderArgs<T> a)
+{
+    render_loop<T, kSmem, kThreads, false>(a, nullptr);
+}
+template <typename T, bool kSmem, int kThreads, int kMinCtas>
+__global__ void __launch_bounds__(kThreads, kMinCtas) render_views_kernel(const RenderArgs<T> a, const CameraT<T>* __restrict__ cams)
+{
+    render_loop<T, kSmem, kThreads, true>(a, cams);
+}
+
 // The same render loop with the sphere filter on the tensor cores (rt_umma_scan.cuh): G groups of 128 ray threads + G
 // MMA-issuer warps per CTA, one CTA per SM.  Everything per ray is the code above — work distribution (assign_work), the
 // Philox event and camera / scatter (next_ray), sky and accumulation (take_hit), and in the scan the precise test of the
 // filter's survivors and the f64 large-sphere test; only the filter moves from 7 FFMA2 per sphere pair to three
 // tcgen05.mma per 128 rays x NC spheres, and the warp-level "any lane alive" vote becomes a 128-thread one, because a
 // group's 128 rays form one MMA.
-template <int G, int NC>
-__global__ void __launch_bounds__(UmmaShape<G, NC>::kRenderThreads, 1) render_kernel_umma(const RenderArgs<float> a)
+template <int G, int NC, bool kViews>
+__device__ __forceinline__ void render_loop_umma(const RenderArgs<float>& a, const CameraT<float>* cams)
 {
     extern __shared__ __align__(1024) unsigned char smem_umma[];
     uint32_t tmem_base;
@@ -338,14 +358,14 @@ __global__ void __launch_bounds__(UmmaShape<G, NC>::kRenderThreads, 1) render_ke
         uint32_t n_rays_w = 0;
         WorkCursor wc;
         for (;;) {
-            uint32_t px = 0, pj = 0;
+            uint32_t px = 0, pj = 0, pv = 0;
             RT_STAMP(1);
-            const bool fresh = assign_work(a, wc, lt_mask, pending, ps, acc_lp, &px, &pj);
+            const bool fresh = assign_work<kViews>(a, wc, lt_mask, pending, ps, acc_lp, &px, &pj, &pv);
             RT_STAMP(2);
             if (!umma_group_any(ux, fresh || pending)) { umma_group_quit(ux); break; }
             RT_STAMP(3);
 
-            const bool active = next_ray(a, ps, fresh, pending, hit_idx, hit_code, px, pj);
+            const bool active = next_ray<kViews>(a, cams, ps, fresh, pending, hit_idx, hit_code, px, pj, pv);
             n_rays_w += __popc(__ballot_sync(RT_FULL, active));              // world.hit call count (main.rs:44)
             RT_STAMP(4);
             const HitF h = closest_hit_umma<G, NC>(ux, a.scene, ps.o, ps.dhat, ps.tmin_n, ps.self_code, ps.self_n, active);
@@ -355,6 +375,17 @@ __global__ void __launch_bounds__(UmmaShape<G, NC>::kRenderThreads, 1) render_ke
         if (lane == 0) atomicAdd(a.ray_counter, (unsigned long long)n_rays_w);
     }
     umma_teardown(tmem_base);
+}
+
+template <int G, int NC>
+__global__ void __launch_bounds__(UmmaShape<G, NC>::kRenderThreads, 1) render_kernel_umma(const RenderArgs<float> a)
+{
+    render_loop_umma<G, NC, false>(a, nullptr);
+}
+template <int G, int NC>
+__global__ void __launch_bounds__(UmmaShape<G, NC>::kRenderThreads, 1) render_views_kernel_umma(const RenderArgs<float> a, const CameraT<float>* __restrict__ cams)
+{
+    render_loop_umma<G, NC, true>(a, cams);
 }
 
 // Color::to_rgba (vec3.rs:404-420) + the row flip (main.rs:141-145): fixed-point sums -> top-down

@@ -3,7 +3,10 @@
 // into flags (SURVEY §8f #3).  No preview window (main.rs:151-171 cannot run headless).
 //
 //   rtiow_host_example [--width W] [--height H] [--spp N] [--depth D] [--seed S] [--scene-seed S] [--gpus G]
-//                      [--grid HALF_EXTENT] [--materials 0..3] [--f64] [--passes N] [--out image.png|image.ppm] [--selftest]
+//                      [--grid HALF_EXTENT] [--materials 0..3] [--f64] [--passes N] [--views N] [--out image.png|image.ppm] [--selftest]
+// --views N renders N cameras orbiting the look-at point about the vertical axis in one call and writes out_000.png ...
+// (with --out, the frames are named after its stem: --out orbit.ppm writes orbit_000.ppm ...).
+#include <algorithm>
 #include <chrono>
 #include <cstdlib>
 #include <cstring>
@@ -30,6 +33,13 @@ static Color ray_color(const Ray& r, const HittableList& world, int depth)
 struct Unknown : Hit {   // a shape the GPU path does not know
     std::optional<HitRecord> hit(const Ray&, double, double) const override { return std::nullopt; }
 };
+
+// the reference camera (main.rs:108-118) turned by `angle` radians about the vertical axis through the look-at point
+static Camera orbit_camera(double angle, double aspect)
+{
+    const double c = std::cos(angle), s = std::sin(angle);
+    return Camera(Point3(13 * c + 3 * s, 2, 3 * c - 13 * s), Point3(0, 0, 0), Vec3(0, 1, 0), 20.0, aspect, 0.1, 10.0);
+}
 
 static int selftest()
 {
@@ -67,6 +77,20 @@ static int selftest()
       expect(c == a && seen == std::vector<uint32_t>({ 2, 4, 6, 8 }) && first == render(cam, random_scene(1), q), "render_progressive: passes, preview and final frame");
       try { render_progressive(cam, random_scene(1), p, 4, [](uint32_t, uint32_t, uint32_t, const std::vector<uint8_t>&) { return true; }); expect(false, "cancel must throw"); }
       catch (const RenderError& e) { expect(e.kind == RenderError::Cancelled, "callback returning true -> RenderError::Cancelled"); } }
+    // a batch of views: three orbit cameras in one call, each frame byte-identical to its own render()
+    { std::vector<Camera> cams = { orbit_camera(0.0, 16.0 / 9.0), orbit_camera(2.0, 16.0 / 9.0), orbit_camera(4.0, 16.0 / 9.0) };
+      rtiow_stats sv{};
+      std::vector<uint8_t> v = render_views(cams, random_scene(1), p, &sv);
+      const size_t fb = size_t(4) * p.width * p.height;
+      bool same = v.size() == 3 * fb;
+      uint64_t rays = 0;
+      for (size_t k = 0; k < cams.size() && same; ++k) {
+          rtiow_stats sk{};
+          same = std::equal(v.begin() + k * fb, v.begin() + (k + 1) * fb, render(cams[k], random_scene(1), p, &sk).begin());
+          rays += sk.rays_traced;
+      }
+      expect(same && std::equal(v.begin(), v.begin() + fb, a.begin()), "render_views: every view equals its own render() byte for byte");
+      expect(sv.paths == 3ull * p.width * p.height * p.spp && sv.rays_traced == rays, "render_views stats: paths and rays of the batch"); }
     // the files below go to a private directory: a fixed name in the shared temporary directory may belong to another user
     std::string dir = (std::filesystem::temp_directory_path() / "rtiow_selftest_XXXXXX").string();
     if (!mkdtemp(dir.data())) { std::cerr << "FAIL: cannot create a temporary directory\nselftest FAILED\n"; return 1; }
@@ -87,7 +111,7 @@ int main(int argc, char** argv)
 {
     RenderParams p; p.width = 200; p.height = 133;                       // main.rs:24-28
     uint64_t scene_seed = 1; int grid = 11, materials = 0; std::string out = "image.png";     // main.rs:177
-    bool explicit_h = false; uint32_t passes = 0; std::string scene_file, dump_scene;
+    bool explicit_h = false, explicit_out = false; uint32_t passes = 0, views = 0; std::string scene_file, dump_scene;
     for (int i = 1; i < argc; ++i) {
         auto next = [&]() -> const char* { if (i + 1 >= argc) { std::cerr << "missing value for " << argv[i] << "\n"; std::exit(2); } return argv[++i]; };
         if (!std::strcmp(argv[i], "--width")) p.width = std::atoi(next());
@@ -101,7 +125,8 @@ int main(int argc, char** argv)
         else if (!std::strcmp(argv[i], "--materials")) materials = std::atoi(next());
         else if (!std::strcmp(argv[i], "--f64")) p.f64 = true;
         else if (!std::strcmp(argv[i], "--passes")) passes = uint32_t(std::atoi(next()));
-        else if (!std::strcmp(argv[i], "--out")) out = next();
+        else if (!std::strcmp(argv[i], "--views")) views = uint32_t(std::atoi(next()));
+        else if (!std::strcmp(argv[i], "--out")) { out = next(); explicit_out = true; }
         else if (!std::strcmp(argv[i], "--scene")) scene_file = next();               // render the world of a scene file instead of random_scene
         else if (!std::strcmp(argv[i], "--dump-scene")) dump_scene = next();          // write the world to a scene file (for the oracle / a cargo build)
         else if (!std::strcmp(argv[i], "--scan")) { const char* v = next(); p.scan = !std::strcmp(v, "fp32") ? RTIOW_SCAN_FP32 : !std::strcmp(v, "tensor") ? RTIOW_SCAN_TENSOR : RTIOW_SCAN_AUTO; }
@@ -115,6 +140,24 @@ int main(int argc, char** argv)
         if (!dump_scene.empty()) { save_scene(world, dump_scene); std::cout << dump_scene << " written (" << world.iter().size() << " spheres)\n"; }
         Camera cam(Point3(13, 2, 3), Point3(0, 0, 0), Vec3(0, 1, 0), 20.0, double(p.width) / double(p.height), 0.1, 10.0);   // main.rs:108-118
         rtiow_stats st{};
+        const bool ppm = out.size() > 4 && out.substr(out.size() - 4) == ".ppm";
+        if (views > 0) {                                                  // an orbit of `views` cameras in one call
+            std::vector<Camera> cams;
+            for (uint32_t k = 0; k < views; ++k) cams.push_back(orbit_camera(2.0 * 3.14159265358979323846 * k / views, double(p.width) / double(p.height)));
+            std::vector<uint8_t> frames = render_views(cams, world, p, &st);
+            std::cout << views << " views of " << p.width << "x" << p.height << " @ " << p.spp << " spp on " << st.n_gpus << " GPU(s): kernel " << st.kernel_ms
+                      << " ms, " << double(st.paths) / st.kernel_ms / 1e3 << " Mpaths/s\n";
+            const std::string stem = explicit_out ? out.substr(0, out.rfind('.') == std::string::npos ? out.size() : out.rfind('.')) : "out";
+            const size_t fb = size_t(4) * p.width * p.height;
+            for (uint32_t k = 0; k < views; ++k) {
+                char name[32]; std::snprintf(name, sizeof name, "_%03u", k);
+                const std::string path = stem + name + (ppm ? ".ppm" : ".png");
+                std::vector<uint8_t> f(frames.begin() + k * fb, frames.begin() + (k + 1) * fb);
+                if (!(ppm ? write_ppm(path, p.width, p.height, f) : write_png(path, p.width, p.height, f))) { std::cerr << "could not write " << path << "\n"; return 1; }
+                std::cout << path << " saved\n";
+            }
+            return 0;
+        }
         auto t0 = std::chrono::steady_clock::now();
         // main.rs:122-145; with --passes N the progress the reference shows as a bar (main.rs:120,124) is printed per pass
         std::vector<uint8_t> pixels = passes == 0 ? render(cam, world, p, &st)
@@ -124,7 +167,7 @@ int main(int argc, char** argv)
         std::cout << "\nDone.\n";                                        // main.rs:149
         std::cout << p.width << "x" << p.height << " @ " << p.spp << " spp on " << st.n_gpus << " GPU(s): kernel " << st.kernel_ms << " ms, call " << ms
                   << " ms (incl. ctx + upload), " << double(st.paths) / st.kernel_ms / 1e3 << " Mpaths/s, " << double(st.rays_traced) / double(st.paths) << " rays/path\n";
-        bool ok = out.size() > 4 && out.substr(out.size() - 4) == ".ppm" ? write_ppm(out, p.width, p.height, pixels) : write_png(out, p.width, p.height, pixels);
+        bool ok = ppm ? write_ppm(out, p.width, p.height, pixels) : write_png(out, p.width, p.height, pixels);
         if (!ok) { std::cerr << "could not write " << out << "\n"; return 1; }
         std::cout << out << " saved to working directory\n";             // main.rs:196
     } catch (const RenderError& e) {

@@ -287,9 +287,10 @@ inline int progress_trampoline(void* user, uint32_t pass, uint32_t n_passes, uin
 }
 }  // namespace detail
 
-// The world as the GPU sees it + one render call; n_passes == 0: rtiow_render, else rtiow_render_progressive.
+// The world as the GPU sees it + one render call; n_passes == 0: rtiow_render, else rtiow_render_progressive; with `views`:
+// rtiow_render_views of those cameras (cam is not used).
 inline std::vector<uint8_t> render_impl(const Camera& cam, const HittableList& world, const RenderParams& p, rtiow_stats* stats, uint32_t n_passes,
-                                        const ProgressFn* on_pass)
+                                        const ProgressFn* on_pass, const std::vector<Camera>* views = nullptr)
 {
     std::vector<double> cx, cy, cz, rad, ar, ag, ab, prm; std::vector<uint32_t> mi, kind;
     std::vector<const Scatter*> seen;
@@ -317,8 +318,11 @@ inline std::vector<uint8_t> render_impl(const Camera& cam, const HittableList& w
     rtiow_params rp; rtiow_params_default(&rp);
     rp.width = p.width; rp.height = p.height; rp.spp = p.spp; rp.max_depth = p.max_depth; rp.t_min = p.t_min; rp.seed = p.seed; rp.alpha = p.alpha;
     rp.precision = p.f64 ? RTIOW_PRECISION_F64 : RTIOW_PRECISION_F32; rp.tile_rows = p.tile_rows;
-    std::vector<uint8_t> out(size_t(4) * p.width * p.height);
-    if (n_passes == 0) check(rtiow_render(ctx, &cam.raw(), &rp, out.data(), stats));
+    std::vector<uint8_t> out(size_t(4) * p.width * p.height * (views ? views->size() : 1));
+    if (views) {
+        std::vector<rtiow_camera> raw; for (const Camera& v : *views) raw.push_back(v.raw());
+        check(rtiow_render_views(ctx, raw.data(), uint32_t(raw.size()), &rp, out.data(), stats));
+    } else if (n_passes == 0) check(rtiow_render(ctx, &cam.raw(), &rp, out.data(), stats));
     else {
         detail::ProgressCtx pc{ on_pass, &out };
         check(rtiow_render_progressive(ctx, &cam.raw(), &rp, n_passes, on_pass && *on_pass ? detail::progress_trampoline : nullptr, &pc, out.data(), stats));
@@ -332,6 +336,14 @@ inline std::vector<uint8_t> render_impl(const Camera& cam, const HittableList& w
 inline std::vector<uint8_t> render(const Camera& cam, const HittableList& world, const RenderParams& p, rtiow_stats* stats = nullptr)
 {
     return render_impl(cam, world, p, stats, 0, nullptr);
+}
+
+// render_views(): many cameras of one world in one call (a turntable, a stereo pair, a camera sweep).  Returns the views'
+// top-down RGBA8 frames one after the other, 4*W*H bytes each; frame v is byte-identical to render(cams[v], world, p).
+inline std::vector<uint8_t> render_views(const std::vector<Camera>& cams, const HittableList& world, const RenderParams& p, rtiow_stats* stats = nullptr)
+{
+    if (cams.empty()) throw RenderError(RTIOW_ERR_INVALID_ARG, "render_views needs at least one camera");
+    return render_impl(cams.front(), world, p, stats, 0, nullptr, &cams);
 }
 
 // render_progressive(): the same frame in n_passes slices of the samples, with a preview after each — what the reference's

@@ -58,6 +58,24 @@ pub fn render(cam: &Camera, world: &HittableList, p: &RenderParams) -> Result<Ve
     render_impl(cam, world, p, 0, None)
 }
 
+/// Many cameras of one world in one call (a turntable, a stereo pair, a camera sweep): the views' top-down RGBA8 frames one
+/// after the other, `4*width*height` bytes each.  Frame `v` is byte-identical to `render(&cams[v], world, p)`.
+pub fn render_views(cams: &[Camera], world: &HittableList, p: &RenderParams) -> Result<Vec<u8>, RenderError> {
+    unsafe {
+        let mut raw: *mut sys::rtiow_ctx = ptr::null_mut();
+        let rc = sys::rtiow_ctx_create(p.n_gpus, &mut raw);
+        if rc != sys::RTIOW_OK { return Err(err(rc)); }
+        let ctx = Ctx(raw);
+        upload(&ctx, world)?;
+        let prm = raw_params(p);
+        let raw_cams: Vec<sys::rtiow_camera> = cams.iter().map(|c| c.raw()).collect();
+        let mut pixels = vec![0u8; 4 * p.width as usize * p.height as usize * cams.len()];
+        let rc = sys::rtiow_render_views(ctx.0, raw_cams.as_ptr(), cams.len() as u32, &prm, pixels.as_mut_ptr(), ptr::null_mut());
+        if rc != sys::RTIOW_OK { return Err(err(rc)); }
+        Ok(pixels)
+    }
+}
+
 /// The same frame in `n_passes` slices of the samples, with the frame so far handed to `on_pass(pass, n_passes, spp_done, rgba)`
 /// after each — the role of the indicatif bar (main.rs:120,124) and the piston preview window (main.rs:151-171).  The returned
 /// frame is bit-identical to `render`'s.  `on_pass` returning `true` stops the render: `Err(RenderError::Cancelled)`.
