@@ -197,7 +197,7 @@ extern "C" void rtiow_ctx_destroy(rtiow_ctx* c);
 // bench under torchrun: torch's bundled libnccl.so.2) shares it instead of mapping a second copy with the same soname.
 // ------------------------------------------------------------------------------------------------
 struct NcclApi {
-    void* h = nullptr; int version = 0;
+    void* h = nullptr; char version[16] = "";          // "2.27.3": named in the gathers' notes (rtiow_ctx_gather_info)
     ncclResult_t (*GetVersion)(int*) = nullptr;
     ncclResult_t (*GetUniqueId)(ncclUniqueId*) = nullptr;
     ncclResult_t (*CommInitRank)(ncclComm_t*, int, ncclUniqueId, int) = nullptr;
@@ -235,7 +235,8 @@ static int nccl_load()
     if (!a.GetVersion || !a.GetUniqueId || !a.CommInitRank || !a.CommInitAll || !a.CommDestroy || !a.AllGather || !a.AllReduce || !a.Broadcast ||
         !a.GroupStart || !a.GroupEnd || !a.GetErrorString)
         return fail(RTIOW_ERR_NCCL, "the NCCL library that was loaded lacks a required symbol");
-    a.GetVersion(&a.version);
+    int v = 0; a.GetVersion(&v);
+    snprintf(a.version, sizeof a.version, "%d.%d.%d", v / 10000, (v / 100) % 100, v % 100);
     g_nccl = a;
     return RTIOW_OK;
 }
@@ -307,21 +308,35 @@ extern "C" int rtiow_ctx_gather_info(rtiow_ctx* c, char* buf, size_t n)
     return RTIOW_OK;
 }
 
-static void release_gather(rtiow_ctx* c)
+// rank 0's frame of the fused gather: rank 0 frees what it allocated, the other ranks unmap it
+static void drop_ipc_frame(rtiow_ctx* c)
 {
-    if (c->dev.empty()) return;
-    cudaSetDevice(c->dev[0].device);
+    if (c->ipc_frame) { if (c->ipc_owner) cudaFree(c->ipc_frame); else cudaIpcCloseMemHandle(c->ipc_frame); }
+    c->ipc_frame = nullptr;
+}
+// the ncclMemAlloc buffers of the NCCL gather and their windows; afterwards no buffers are ready (nccl_tile_px = 0)
+static void drop_nccl_buffers(rtiow_ctx* c)
+{
     if (c->windows_registered && g_nccl.CommWindowDeregister && c->comm) {
         if (c->win_tiles) g_nccl.CommWindowDeregister(c->comm, (ncclWindow_t)c->win_tiles);
         if (c->win_gathered) g_nccl.CommWindowDeregister(c->comm, (ncclWindow_t)c->win_gathered);
     }
     if (c->nccl_tiles && g_nccl.MemFree) g_nccl.MemFree(c->nccl_tiles);
     if (c->nccl_gathered && g_nccl.MemFree) g_nccl.MemFree(c->nccl_gathered);
-    if (c->ipc_frame) { if (c->ipc_owner) cudaFree(c->ipc_frame); else cudaIpcCloseMemHandle(c->ipc_frame); }
+    c->win_tiles = c->win_gathered = nullptr; c->windows_registered = false;
+    c->nccl_tiles = c->nccl_gathered = nullptr; c->nccl_tile_px = 0;
+}
+
+static void release_gather(rtiow_ctx* c)
+{
+    if (c->dev.empty()) return;
+    cudaSetDevice(c->dev[0].device);
+    drop_nccl_buffers(c);
+    drop_ipc_frame(c);
     if (c->d_flag) cudaFree(c->d_flag);
     if (c->comm) g_nccl.CommDestroy(c->comm);
     for (size_t i = 0; i < c->comms.size(); ++i) { cudaSetDevice(c->dev[i].device); if (c->comms[i]) g_nccl.CommDestroy(c->comms[i]); }
-    c->comms.clear(); c->comm = nullptr; c->d_flag = nullptr; c->ipc_frame = nullptr; c->nccl_tiles = c->nccl_gathered = nullptr;
+    c->comms.clear(); c->comm = nullptr; c->d_flag = nullptr;
 }
 
 extern "C" void rtiow_ctx_destroy(rtiow_ctx* c)
@@ -749,9 +764,10 @@ struct Dest { uint32_t* p; bool whole_frame; };
 
 // n_views = 0: a frame (or a rank's rows of one) of camera *cam.  n_views > 0 (world 1): a batch of views, the cameras
 // cam[0 .. n_views), rendered as one frame n_views * height rows tall whose epilogue writes the views' frames one after the other.
+// *paths: the paths launched, local rows x width x samples.
 template <typename T>
 static int launch_render(const ScanPlan& plan, DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, uint32_t rank, uint32_t world, SampleRange sr,
-                         Dest dst, cudaStream_t st, uint32_t* launches, uint32_t n_views)
+                         Dest dst, cudaStream_t st, uint32_t* launches, uint64_t* paths, uint32_t n_views)
 {
     RenderArgs<T> a;
     a.scene = d.scene; a.cam = to_dev_camera<T>(*cam);
@@ -764,6 +780,7 @@ static int launch_render(const ScanPlan& plan, DeviceState& d, const rtiow_camer
     a.chunks_per_fetch = std::max<uint32_t>(1u, 256u / a.chunk_samples);
     const uint64_t n_lp = (uint64_t)a.local_rows * p->width;
     a.n_chunks = n_lp * a.chunks_per_pixel;
+    *paths = n_lp * sr.count;
     CU(d.accum.resize(3 * n_lp));
     a.accum = d.accum.p; a.work_counter = d.counters.p; a.ray_counter = d.counters.p + 1;
     if (sr.begin == 0) CU(cudaMemsetAsync(d.accum.p, 0, 3 * n_lp * sizeof(unsigned long long), st));     // later passes add to the same sums
@@ -792,19 +809,44 @@ static int launch_render(const ScanPlan& plan, DeviceState& d, const rtiow_camer
     return RTIOW_OK;
 }
 
+// What one device launched for a call (render_step): where, between which events and how many paths (0 for a rank without
+// rows), and the D2H copy of its frame when the call starts one.  A caller's buffer that is page-locked itself (cudaHostAlloc /
+// cudaHostRegister, torch pin_memory) takes the DMA directly; pageable memory goes through the device's staging buffer, and
+// finish_call copies it over after the stream synchronisation (0.3 ms for the 3.2 MB headline frame).
+struct Part {
+    DeviceState* d = nullptr; cudaStream_t st = nullptr; cudaEvent_t e0 = nullptr, e1 = nullptr;
+    uint64_t paths = 0;
+    uint8_t* out = nullptr; const uint8_t* staged = nullptr; size_t copy_bytes = 0;
+    int start_copy(uint8_t* dst, const uint32_t* d_frame, size_t n)
+    {
+        out = dst; copy_bytes = n;
+        if (!host_is_pinned(dst)) { CU(d->pinned.resize(n)); staged = d->pinned.p; }
+        CU(cudaMemcpyAsync(staged ? d->pinned.p : dst, d_frame, n, cudaMemcpyDeviceToHost, st));
+        return RTIOW_OK;
+    }
+    // the counters after the part's work into d->pinned_cnt: the last thing a call puts on the part's stream
+    int read_counters() const
+    {
+        CU(cudaSetDevice(d->device));
+        CU(cudaMemcpyAsync(d->pinned_cnt.p, d->counters.p, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+        return RTIOW_OK;
+    }
+};
+
 // One device's part of a frame: samples `sr` of the rows {y : (y / tile_rows) % world == rank}, quantised into `dst`, with the
 // events e0 / e1 around the work and its kernel launches added to *launches.  n_views > 0: the batch of views cam[0 .. n_views)
 // (launch_render).
 static int render_step(const rtiow_ctx* c, DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, uint32_t rank, uint32_t world, SampleRange sr,
-                       Dest dst, cudaStream_t st, cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches, uint32_t n_views = 0)
+                       Dest dst, cudaStream_t st, cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches, Part* part, uint32_t n_views = 0)
 {
     if (!d.has_scene) return fail(RTIOW_ERR_INVALID_ARG, "no scene uploaded (call rtiow_scene_upload first)");
     CU(cudaSetDevice(d.device));
     ScanPlan plan;
     int rc = plan_scan(c, d, p->precision, &plan); if (rc) return rc;
+    *part = Part{ &d, st, e0, e1 };
     CU(cudaEventRecord(e0, st));
-    rc = plan.scan == Scan::F64 ? launch_render<double>(plan, d, cam, p, rank, world, sr, dst, st, launches, n_views)
-                                : launch_render<float>(plan, d, cam, p, rank, world, sr, dst, st, launches, n_views);
+    rc = plan.scan == Scan::F64 ? launch_render<double>(plan, d, cam, p, rank, world, sr, dst, st, launches, &part->paths, n_views)
+                                : launch_render<float>(plan, d, cam, p, rank, world, sr, dst, st, launches, &part->paths, n_views);
     if (rc) return rc;
     CU(cudaEventRecord(e1, st));
     return RTIOW_OK;
@@ -812,28 +854,23 @@ static int render_step(const rtiow_ctx* c, DeviceState& d, const rtiow_camera* c
 
 // a frame on one device: its rank-local order IS top-down (and a batch of n_views views is their frames one after the other)
 static int render_single(const rtiow_ctx* c, DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, SampleRange sr, cudaStream_t st,
-                         cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches, const uint32_t** d_frame, uint32_t n_views = 0)
+                         cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches, Part* part, const uint32_t** d_frame, uint32_t n_views = 0)
 {
     CU(d.tiles.resize((size_t)p->width * p->height * std::max<uint32_t>(n_views, 1)));
-    int rc = render_step(c, d, cam, p, 0, 1, sr, Dest{ d.tiles.p, false }, st, e0, e1, launches, n_views); if (rc) return rc;
+    int rc = render_step(c, d, cam, p, 0, 1, sr, Dest{ d.tiles.p, false }, st, e0, e1, launches, part, n_views); if (rc) return rc;
     *d_frame = d.tiles.p;
     return RTIOW_OK;
 }
 
-// The frame's D2H copy.  A caller's buffer that is page-locked itself (cudaHostAlloc / cudaHostRegister, torch pin_memory) takes
-// the DMA directly; pageable memory goes through the device's staging buffer, and finish() copies it over after the stream
-// synchronisation (0.3 ms for the 3.2 MB headline frame).
-struct FrameCopy {
-    uint8_t* out = nullptr; const uint8_t* staged = nullptr; size_t bytes = 0;
-    int start(DeviceState& d, uint8_t* dst, const uint32_t* d_frame, size_t n, cudaStream_t st)
-    {
-        out = dst; bytes = n;
-        if (!host_is_pinned(dst)) { CU(d.pinned.resize(n)); staged = d.pinned.p; }
-        CU(cudaMemcpyAsync(staged ? d.pinned.p : dst, d_frame, n, cudaMemcpyDeviceToHost, st));
-        return RTIOW_OK;
-    }
-    void finish() const { if (staged) memcpy(out, staged, bytes); }
-};
+// the world tile buffers of a gather, one after the other in rank-local order, into the top-down frame
+static int deinterleave(const uint32_t* gathered, const rtiow_params* p, uint32_t world, uint32_t* frame, cudaStream_t st)
+{
+    const size_t npx = (size_t)p->width * p->height;
+    const size_t tile_px = (size_t)max_rows_per_rank(p->height, tile_rows_of(p), world) * p->width;
+    deinterleave_kernel<<<(unsigned)((npx + 255) / 256), 256, 0, st>>>(gathered, p->width, p->height, tile_rows_of(p), world, tile_px, frame);
+    CU(cudaGetLastError());
+    return RTIOW_OK;
+}
 
 // what a render call reports; the scene's sphere count and the filter used come from device d
 static rtiow_stats make_stats(const DeviceState& d, double kernel_ms, double total_ms, uint64_t paths, uint64_t rays, uint32_t launches, uint32_t n_gpus,
@@ -851,6 +888,26 @@ static double now_ms()
     return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count();
 }
 
+// The end of a synchronous call: every part's counters are read back, its stream synchronised and its frame copy finished.
+// *stats (when asked for) gets the slowest part's kernel time and the parts' summed paths and rays, and the scene and filter of
+// the first part's device (make_stats).
+static int finish_call(Part* parts, size_t n, double t0, uint32_t launches, uint32_t n_gpus, uint64_t h2d_bytes, uint64_t d2h_bytes, rtiow_stats* stats)
+{
+    for (size_t i = 0; i < n; ++i) { int rc = parts[i].read_counters(); if (rc) return rc; }
+    float ms = 0; uint64_t paths = 0, rays = 0;
+    for (size_t i = 0; i < n; ++i) {
+        const Part& pt = parts[i];
+        CU(cudaSetDevice(pt.d->device));
+        CU(cudaStreamSynchronize(pt.st));
+        if (pt.staged) memcpy(pt.out, pt.staged, pt.copy_bytes);
+        float mp = 0; if (stats) CU(cudaEventElapsedTime(&mp, pt.e0, pt.e1));
+        ms = std::max(ms, mp); paths += pt.paths; rays += pt.d->pinned_cnt.p[1];          // the slowest device's kernels
+    }
+    CU(cudaSetDevice(parts[0].d->device));
+    if (stats) *stats = make_stats(*parts[0].d, ms, now_ms() - t0, paths, rays, launches, n_gpus, h2d_bytes, d2h_bytes);
+    return RTIOW_OK;
+}
+
 // shared body of the two per-rank entry points: this rank's rows into a tile buffer (rank-local order), or — with `to_frame` —
 // straight into their top-down place in a whole frame that may live on another GPU (finalize_to_frame_kernel)
 static int render_rank(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_params* p, int rank, int world, void* dst, bool to_frame, void* stream,
@@ -864,16 +921,10 @@ static int render_rank(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_params
     cudaStream_t st = stream ? (cudaStream_t)stream : d.stream;
     const double t0 = now_ms();
     uint32_t launches = 0;
-    rc = render_step(c, d, cam, p, (uint32_t)rank, (uint32_t)world, SampleRange{ 0u, p->spp }, Dest{ (uint32_t*)dst, to_frame }, st, d.ev0, d.ev1, &launches);
+    Part part;
+    rc = render_step(c, d, cam, p, (uint32_t)rank, (uint32_t)world, SampleRange{ 0u, p->spp }, Dest{ (uint32_t*)dst, to_frame }, st, d.ev0, d.ev1, &launches, &part);
     if (rc) return rc;
-    if (stats) {
-        CU(cudaMemcpyAsync(d.pinned_cnt.p, d.counters.p, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        float ms = 0; CU(cudaEventElapsedTime(&ms, d.ev0, d.ev1));
-        *stats = make_stats(d, ms, now_ms() - t0, (uint64_t)rows_of_rank(p->height, tile_rows_of(p), world, rank) * p->width * p->spp, d.pinned_cnt.p[1],
-                            launches, 1, 0, 0);
-    }
-    return RTIOW_OK;
+    return stats ? finish_call(&part, 1, t0, launches, 1, 0, 0, stats) : RTIOW_OK;      // without stats the call stays asynchronous
 }
 
 extern "C" int rtiow_render_tiles_device(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_params* p, int rank, int world, void* d_tiles,
@@ -899,12 +950,7 @@ extern "C" int rtiow_deinterleave_device(rtiow_ctx* c, const void* d_gathered, c
     if (world < 1) return fail(RTIOW_ERR_INVALID_ARG, "bad world");
     DeviceState& d = c->dev[0];
     CU(cudaSetDevice(d.device));
-    cudaStream_t st = stream ? (cudaStream_t)stream : d.stream;
-    const size_t npx = (size_t)p->width * p->height;
-    const size_t tile_px = (size_t)max_rows_per_rank(p->height, tile_rows_of(p), world) * p->width;
-    deinterleave_kernel<<<(unsigned)((npx + 255) / 256), 256, 0, st>>>((const uint32_t*)d_gathered, p->width, p->height, tile_rows_of(p), (uint32_t)world, tile_px, (uint32_t*)d_frame);
-    CU(cudaGetLastError());
-    return RTIOW_OK;
+    return deinterleave((const uint32_t*)d_gathered, p, (uint32_t)world, (uint32_t*)d_frame, stream ? (cudaStream_t)stream : d.stream);
 }
 
 // THE drop-in call (main.rs:122-145)
@@ -919,9 +965,10 @@ static int render_frame(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_param
     DeviceState& d0 = c->dev[0];
     uint32_t launches = 0;
     CU(cudaSetDevice(d0.device));
+    std::vector<Part> parts(world);
     const uint32_t* d_final = nullptr;
     if (world == 1) {
-        rc = render_single(c, d0, cam, p, sr, d0.stream, d0.ev0, d0.ev1, &launches, &d_final); if (rc) return rc;
+        rc = render_single(c, d0, cam, p, sr, d0.stream, d0.ev0, d0.ev1, &launches, &parts[0], &d_final); if (rc) return rc;
     } else {
         // interleaved row tiles on every GPU.  Three gathers:
         //   fused (default with NVLink peer access, every B200 box): each rank's epilogue stores its pixels straight into device
@@ -947,7 +994,7 @@ static int render_frame(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_param
             Dest dst{ d0.frame.p, true };
             if (use_nccl) { CU(d.tiles.resize(tile_px)); CU(d.gathered.resize(tile_px * world)); dst = Dest{ d.tiles.p, false }; }
             else if (!fused) { if (r == 0) dst = Dest{ d0.gathered.p, false }; else { CU(d.tiles.resize(tile_px)); dst = Dest{ d.tiles.p, false }; } }
-            rc = render_step(c, d, cam, p, r, world, sr, dst, d.stream, d.ev0, d.ev1, &launches); if (rc) return rc;
+            rc = render_step(c, d, cam, p, r, world, sr, dst, d.stream, d.ev0, d.ev1, &launches, &parts[r]); if (rc) return rc;
             if (r != 0 && !use_nccl) {
                 if (!fused) {
                     const size_t bytes = (size_t)rows_of_rank(p->height, tile_rows_of(p), world, r) * p->width * 4;
@@ -968,9 +1015,7 @@ static int render_frame(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_param
         CU(cudaSetDevice(d0.device));
         if (!use_nccl) for (uint32_t r = 1; r < world; ++r) CU(cudaStreamWaitEvent(d0.stream, c->dev[r].ev_done, 0));
         if (!fused) {
-            const size_t npx = (size_t)p->width * p->height;
-            deinterleave_kernel<<<(unsigned)((npx + 255) / 256), 256, 0, d0.stream>>>(d0.gathered.p, p->width, p->height, tile_rows_of(p), world, tile_px, d0.frame.p);
-            CU(cudaGetLastError());
+            rc = deinterleave(d0.gathered.p, p, world, d0.frame.p, d0.stream); if (rc) return rc;
             ++launches;
         }
         char note[160];
@@ -979,25 +1024,8 @@ static int render_frame(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_param
         c->gather_note = note;
         d_final = d0.frame.p;
     }
-    FrameCopy copy;
-    rc = copy.start(d0, out_rgba, d_final, frame_bytes, d0.stream); if (rc) return rc;
-    CU(cudaMemcpyAsync(d0.pinned_cnt.p, d0.counters.p, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, d0.stream));
-    CU(cudaStreamSynchronize(d0.stream));
-    copy.finish();
-    if (stats) {
-        float ms = 0; CU(cudaEventElapsedTime(&ms, d0.ev0, d0.ev1));
-        uint64_t rays = d0.pinned_cnt.p[1];
-        for (uint32_t r = 1; r < world; ++r) {
-            DeviceState& d = c->dev[r];
-            CU(cudaSetDevice(d.device));
-            CU(cudaMemcpyAsync(d.pinned_cnt.p, d.counters.p, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, d.stream));
-            CU(cudaStreamSynchronize(d.stream));
-            rays += d.pinned_cnt.p[1];
-            float mr = 0; CU(cudaEventElapsedTime(&mr, d.ev0, d.ev1)); ms = std::max(ms, mr);          // the slowest device's kernels
-        }
-        *stats = make_stats(d0, ms, now_ms() - t0, (uint64_t)p->width * p->height * sr.count, rays, launches, world, kCallH2D, frame_bytes + 16);
-    }
-    return RTIOW_OK;
+    rc = parts[0].start_copy(out_rgba, d_final, frame_bytes); if (rc) return rc;
+    return finish_call(parts.data(), world, t0, launches, world, kCallH2D, frame_bytes + 16, stats);
 }
 
 extern "C" int rtiow_render(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_params* p, uint8_t* out_rgba, rtiow_stats* stats)
@@ -1022,35 +1050,21 @@ extern "C" int rtiow_render_views(rtiow_ctx* c, const rtiow_camera* cams, uint32
     const double t0 = now_ms();
     const uint32_t n_dev = (uint32_t)c->dev.size();
     const size_t frame_bytes = (size_t)p->width * p->height * 4;
-    std::vector<FrameCopy> copies(n_dev);
+    std::vector<Part> parts;                                // of the devices that render: the first one's scene and scan backend go into the stats
     uint32_t launches = 0;
-    int first = -1;                                         // the first device that renders: its scene and scan backend go into the stats
     for (uint32_t r = 0; r < n_dev; ++r) {
         const uint32_t v0 = (uint32_t)((uint64_t)r * n_views / n_dev), v1 = (uint32_t)((uint64_t)(r + 1) * n_views / n_dev);
         if (v0 == v1) continue;                             // more devices than views
         DeviceState& d = c->dev[r];
         CU(cudaSetDevice(d.device));
         const uint32_t* d_frames = nullptr;
-        rc = render_single(c, d, cams + v0, p, SampleRange{ 0u, p->spp }, d.stream, d.ev0, d.ev1, &launches, &d_frames, v1 - v0); if (rc) return rc;
-        rc = copies[r].start(d, out_rgba + v0 * frame_bytes, d_frames, (v1 - v0) * frame_bytes, d.stream); if (rc) return rc;
-        CU(cudaMemcpyAsync(d.pinned_cnt.p, d.counters.p, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, d.stream));
-        if (first < 0) first = (int)r;
+        Part part;
+        rc = render_single(c, d, cams + v0, p, SampleRange{ 0u, p->spp }, d.stream, d.ev0, d.ev1, &launches, &part, &d_frames, v1 - v0); if (rc) return rc;
+        rc = part.start_copy(out_rgba + v0 * frame_bytes, d_frames, (v1 - v0) * frame_bytes); if (rc) return rc;
+        parts.push_back(part);
     }
-    float ms = 0; uint64_t rays = 0; uint32_t used = 0;
-    for (uint32_t r = 0; r < n_dev; ++r) {
-        if (!copies[r].out) continue;
-        DeviceState& d = c->dev[r];
-        CU(cudaSetDevice(d.device));
-        CU(cudaStreamSynchronize(d.stream));
-        copies[r].finish();
-        float mr = 0; CU(cudaEventElapsedTime(&mr, d.ev0, d.ev1)); ms = std::max(ms, mr);          // the slowest device's kernels
-        rays += d.pinned_cnt.p[1]; ++used;
-    }
-    CU(cudaSetDevice(c->dev[0].device));
-    if (stats)
-        *stats = make_stats(c->dev[first], ms, now_ms() - t0, (uint64_t)n_views * p->width * p->height * p->spp, rays, launches, n_dev,
-                            (uint64_t)n_views * sizeof(rtiow_camera) + sizeof(rtiow_params), (uint64_t)n_views * frame_bytes + 16 * used);
-    return RTIOW_OK;
+    return finish_call(parts.data(), parts.size(), t0, launches, n_dev, (uint64_t)n_views * sizeof(rtiow_camera) + sizeof(rtiow_params),
+                       (uint64_t)n_views * frame_bytes + 16 * parts.size(), stats);
 }
 
 // The per-pass preview the reference gets from its progress bar and piston window (main.rs:120-124,151-171): the spp samples
@@ -1112,7 +1126,7 @@ static int ensure_ipc_frame(rtiow_ctx* c, size_t npx, cudaStream_t st)
 {
     if (c->ipc_state == -1 || (c->ipc_state == 1 && c->ipc_frame_px == npx)) return RTIOW_OK;
     CU(cudaStreamSynchronize(st));
-    if (c->ipc_frame) { if (c->ipc_owner) cudaFree(c->ipc_frame); else cudaIpcCloseMemHandle(c->ipc_frame); c->ipc_frame = nullptr; }
+    drop_ipc_frame(c);
     int ok = 1;
     cudaIpcMemHandle_t h; memset(&h, 0, sizeof h);
     if (c->rank == 0) {
@@ -1136,26 +1150,21 @@ static int ensure_ipc_frame(rtiow_ctx* c, size_t npx, cudaStream_t st)
     int all = 0;
     int rc = nccl_vote_min(c, ok, &all, st); if (rc) return rc;
     if (!all) {         // some rank could not map the frame (no peer access / IPC across containers): every rank falls back together
-        if (c->ipc_frame) { if (c->ipc_owner) cudaFree(c->ipc_frame); else cudaIpcCloseMemHandle(c->ipc_frame); c->ipc_frame = nullptr; }
+        drop_ipc_frame(c);
         c->ipc_state = -1;
     } else { c->ipc_state = 1; c->ipc_frame_px = npx; c->ipc_parity = 0; }
     return RTIOW_OK;
 }
 
 // tile + gathered buffers of the NCCL gather; allocated with ncclMemAlloc and registered as a symmetric window when the
-// library offers it (NCCL >= 2.27: zero-copy all-gather over NVLink), plain cudaMalloc otherwise.  Collective.
+// library offers it (NCCL >= 2.27: zero-copy all-gather over NVLink), plain cudaMalloc otherwise.  Collective; once buffers of
+// tile_px are ready, from either allocator, later frames of that size go straight on (no synchronisation, no vote).
 static int ensure_nccl_buffers(rtiow_ctx* c, size_t tile_px, cudaStream_t st)
 {
     DeviceState& d = c->dev[0];
-    if (c->nccl_tile_px == tile_px && c->nccl_tiles) return RTIOW_OK;
+    if (c->nccl_tile_px == tile_px) return RTIOW_OK;
     CU(cudaStreamSynchronize(st));
-    if (c->windows_registered && g_nccl.CommWindowDeregister) {
-        if (c->win_tiles) g_nccl.CommWindowDeregister(c->comm, (ncclWindow_t)c->win_tiles);
-        if (c->win_gathered) g_nccl.CommWindowDeregister(c->comm, (ncclWindow_t)c->win_gathered);
-    }
-    c->win_tiles = c->win_gathered = nullptr; c->windows_registered = false;
-    if (c->nccl_tiles && g_nccl.MemFree) { g_nccl.MemFree(c->nccl_tiles); g_nccl.MemFree(c->nccl_gathered); }
-    c->nccl_tiles = c->nccl_gathered = nullptr; c->nccl_tile_px = 0;
+    drop_nccl_buffers(c);
     int ok = 0;
     if (g_nccl.MemAlloc && g_nccl.MemFree && g_nccl.CommWindowRegister && g_nccl.CommWindowDeregister) {
         ok = g_nccl.MemAlloc((void**)&c->nccl_tiles, tile_px * 4) == ncclSuccess && g_nccl.MemAlloc((void**)&c->nccl_gathered, tile_px * 4 * c->world) == ncclSuccess;
@@ -1170,9 +1179,7 @@ static int ensure_nccl_buffers(rtiow_ctx* c, size_t tile_px, cudaStream_t st)
         c->win_tiles = wt; c->win_gathered = wg; c->windows_registered = reg && wt && wg;
         if (!reg) cudaGetLastError();
     } else {
-        if (c->nccl_tiles) g_nccl.MemFree(c->nccl_tiles);
-        if (c->nccl_gathered) g_nccl.MemFree(c->nccl_gathered);
-        c->nccl_tiles = c->nccl_gathered = nullptr;
+        drop_nccl_buffers(c);
         CU(d.tiles.resize(tile_px)); CU(d.gathered.resize(tile_px * c->world));
     }
     c->nccl_tile_px = tile_px;
@@ -1206,9 +1213,10 @@ static int render_rank_impl(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_p
         }
         e0 = d.ring[d.ring_used].first; e1 = d.ring[d.ring_used].second;
     }
+    Part part;
     bool frame_here = true;                                 // d_final holds the whole frame on THIS rank
     if (world == 1) {
-        rc = render_single(c, d, cam, p, SampleRange{ 0u, p->spp }, st, e0, e1, &launches, &d_final); if (rc) return rc;
+        rc = render_single(c, d, cam, p, SampleRange{ 0u, p->spp }, st, e0, e1, &launches, &part, &d_final); if (rc) return rc;
         c->gather_note = "single GPU: no gather";
     } else {
         bool fused = false;
@@ -1224,47 +1232,35 @@ static int render_rank_impl(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_p
             // it is the frame-complete barrier.  Two frames alternate, so rank 0's copy-out of frame k is ordered (by its stream
             // and the barrier of frame k+1) before anybody writes that buffer again in frame k+2.
             uint32_t* fr = c->ipc_frame + (size_t)(c->ipc_parity & 1u) * npx; c->ipc_parity ^= 1u;
-            rc = render_step(c, d, cam, p, rank, world, SampleRange{ 0u, p->spp }, Dest{ fr, true }, st, e0, e1, &launches); if (rc) return rc;
+            rc = render_step(c, d, cam, p, rank, world, SampleRange{ 0u, p->spp }, Dest{ fr, true }, st, e0, e1, &launches, &part); if (rc) return rc;
             rc = nccl_barrier(c, st); if (rc) return rc;
             d_final = fr; frame_here = rank == 0;
             snprintf(note, sizeof note, "one process per GPU x%u: epilogue stores into rank 0's frame over NVLink (CUDA IPC mapping made inside librtiow_cuda.so) + "
-                     "1-int ncclAllReduce as the frame-complete barrier (NCCL %d.%d.%d)", world, g_nccl.version / 10000, (g_nccl.version / 100) % 100, g_nccl.version % 100);
+                     "1-int ncclAllReduce as the frame-complete barrier (NCCL %s)", world, g_nccl.version);
         } else {
             rc = ensure_nccl_buffers(c, tile_px, st); if (rc) return rc;
             uint32_t* tiles = c->nccl_tiles ? c->nccl_tiles : d.tiles.p;
             uint32_t* gathered = c->nccl_gathered ? c->nccl_gathered : d.gathered.p;
             CU(d.frame.resize(npx));
-            rc = render_step(c, d, cam, p, rank, world, SampleRange{ 0u, p->spp }, Dest{ tiles, false }, st, e0, e1, &launches); if (rc) return rc;
+            rc = render_step(c, d, cam, p, rank, world, SampleRange{ 0u, p->spp }, Dest{ tiles, false }, st, e0, e1, &launches, &part); if (rc) return rc;
             NC(g_nccl.AllGather(tiles, gathered, tile_px * 4, ncclUint8, c->comm, st));      // one per frame, equal (padded) counts: SURVEY §8(e)
-            deinterleave_kernel<<<(unsigned)((npx + 255) / 256), 256, 0, st>>>(gathered, p->width, p->height, tile_rows_of(p), world, tile_px, d.frame.p);
-            CU(cudaGetLastError());
+            rc = deinterleave(gathered, p, world, d.frame.p, st); if (rc) return rc;
             ++launches;
             d_final = d.frame.p;
-            snprintf(note, sizeof note, "one process per GPU x%u: tile buffers + ncclAllGather inside librtiow_cuda.so (NCCL %d.%d.%d%s) + de-interleave", world,
-                     g_nccl.version / 10000, (g_nccl.version / 100) % 100, g_nccl.version % 100,
-                     c->windows_registered ? ", buffers from ncclMemAlloc registered as a symmetric window" : "");
+            snprintf(note, sizeof note, "one process per GPU x%u: tile buffers + ncclAllGather inside librtiow_cuda.so (NCCL %s%s) + de-interleave", world,
+                     g_nccl.version, c->windows_registered ? ", buffers from ncclMemAlloc registered as a symmetric window" : "");
         }
         c->gather_note = note;
     }
-    FrameCopy copy;
-    if (out_rgba && frame_here) { rc = copy.start(d, out_rgba, d_final, frame_bytes, st); if (rc) return rc; }
-    CU(cudaMemcpyAsync(d.pinned_cnt.p, d.counters.p, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    if (d_frame_out) *d_frame_out = frame_here ? d_final : nullptr;
+    if (out_rgba && frame_here) { rc = part.start_copy(out_rgba, d_final, frame_bytes); if (rc) return rc; }
     if (enqueue_only) {                                     // no host synchronisation: rtiow_ctx_synchronize collects the stats
+        rc = part.read_counters(); if (rc) return rc;
         ++d.ring_used;
-        d.enq_paths = (uint64_t)rows_of_rank(p->height, tile_rows_of(p), world, rank) * p->width * p->spp;
-        d.enq_launches += launches; d.enq_world = world;
-        if (d_frame_out) *d_frame_out = frame_here ? d_final : nullptr;
+        d.enq_paths = part.paths; d.enq_launches += launches; d.enq_world = world;
         return RTIOW_OK;
     }
-    CU(cudaStreamSynchronize(st));
-    copy.finish();
-    if (d_frame_out) *d_frame_out = frame_here ? d_final : nullptr;
-    if (stats) {
-        float ms = 0; CU(cudaEventElapsedTime(&ms, d.ev0, d.ev1));
-        *stats = make_stats(d, ms, now_ms() - t0, (uint64_t)rows_of_rank(p->height, tile_rows_of(p), world, rank) * p->width * p->spp, d.pinned_cnt.p[1],
-                            launches, world, kCallH2D, copy.bytes + 16);
-    }
-    return RTIOW_OK;
+    return finish_call(&part, 1, t0, launches, world, kCallH2D, part.copy_bytes + 16, stats);
 }
 
 extern "C" int rtiow_render_rank(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_params* p, uint8_t* out_rgba, rtiow_stats* stats)
