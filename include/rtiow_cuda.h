@@ -62,7 +62,9 @@ typedef struct {
 } rtiow_spheres;
 
 /* Arc<dyn Scatter> records (materials.rs).  param = fuzz (Metal, NOT clamped, materials.rs:40-45)
- * or ir (Dialectric); ignored for Lambertian.  albedo ignored for Dialectric. */
+ * or ir (Dialectric); ignored for Lambertian.  albedo ignored for Dialectric.
+ * The albedo of a Lambertian or Metal material and the param of a Metal or Dialectric one must be finite when a sphere
+ * uses the material (RTIOW_ERR_INVALID_ARG otherwise), as the sphere centres and radii must; ignored fields may be anything. */
 typedef struct {
     const uint32_t* kind;                                   /* rtiow_material_kind */
     const double* albedo_r; const double* albedo_g; const double* albedo_b;
@@ -81,7 +83,9 @@ typedef struct {
     uint32_t width, height;       /* IMAGE_WIDTH / IMAGE_HEIGHT (main.rs:25-26); both >= 2 */
     uint32_t spp;                 /* SAMPLES_PER_PIXEL (main.rs:27) */
     int32_t  max_depth;           /* MAX_DEPTH (main.rs:28): at most max_depth rays per path */
-    double   t_min;               /* 0.0001 at main.rs:44 */
+    double   t_min;               /* 0.0001 at main.rs:44; >= 0.  Below ~1e-12 (0 included) the reference's own
+                                     self-intersections depend on the last bit of its f64 rounding, and no f32 render
+                                     can be compared with it there */
     uint64_t seed;                /* Philox key; the reference's thread_rng is unseedable */
     uint8_t  alpha;               /* 255 at main.rs:137 */
     uint8_t  precision;           /* rtiow_precision */

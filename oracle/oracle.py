@@ -131,6 +131,8 @@ def _declare(L):
         ("o_direct_disk", None, [d, d, C.POINTER(d), C.POINTER(d)]),
         ("o_direct_unit_vector", Vec3, [d, d]), ("o_direct_in_unit_sphere", Vec3, [d, d, d]),
         ("o_render", C.c_int, [C.POINTER(World), C.POINTER(Camera), C.POINTER(RenderParams), P, P, C.POINTER(Counters)]),
+        ("o_render_margins", C.c_int, [C.POINTER(World), C.POINTER(Camera), C.POINTER(RenderParams), P, P, P,
+                                       C.POINTER(Counters)]),
         ("o_path_radiance", Vec3, [C.POINTER(World), C.POINTER(Camera), C.POINTER(RenderParams), u32, u32, u32,
                                    C.POINTER(Counters)]),
         ("o_sphere_hit_batch", None, [i64] + [P] * 11),
@@ -300,6 +302,40 @@ def render(scene: Scene, cam: Camera, width, height, spp, max_depth=50, t_min=1e
     if rc != 0:
         raise ValueError("o_render: invalid arguments")
     return out, acc, dict(rays=int(cnt.rays), sphere_tests=int(cnt.sphere_tests))
+
+
+def render_margins(scene: Scene, cam: Camera, width, height, spp, max_depth=50, t_min=1e-4, seed=1, alpha=255, n_threads=0,
+                   rows=None):
+    """render(..., sampler=SAMPLER_DIRECT, want_accum=True) and each pixel's knife-edge margin (o_render_margins,
+    rtiow_oracle.h).  Returns (rgba[H,W,4], accum[H,W,3], margin[H,W], counters dict)."""
+    rb, re = (0, 0) if rows is None else rows
+    prm = RenderParams(width, height, spp, max_depth, t_min, seed, alpha, SAMPLER_DIRECT, n_threads, rb, re)
+    out = np.zeros((height, width, 4), np.uint8)
+    acc = np.zeros((height, width, 3))
+    mg = np.full((height, width), np.inf)
+    cnt = Counters()
+    if lib().o_render_margins(C.byref(scene.world), C.byref(cam), C.byref(prm), _p(out), _p(acc), _p(mg), C.byref(cnt)) != 0:
+        raise ValueError("o_render_margins: invalid arguments")
+    return out, acc, mg, dict(rays=int(cnt.rays), sphere_tests=int(cnt.sphere_tests))
+
+
+# A pixel is robust -- an f32 render must give it the oracle's exact bytes -- when no ray of its paths comes within TAU of a
+# decision (margin >= TAU, o_render_margins) and its exact value 256 sqrt(clamp(sum / spp, 0, 0.999)) is more than DELTA
+# from an integer in every channel (or exactly 0: black paths add nothing on either side).
+# TAU: the margins are relative distances, and an f32 evaluation of a root, a dot product or a unit vector errs by a few
+# eps32 = 6e-8 relative to its inputs, times the growth the margin is already divided by; TAU = 2e-5 is ~300 eps32.
+# DELTA: a pixel's value in f32 carries the relative error of its path colours (~1e-6 on long chains, the sky term of a
+# unit vector); at 255 that is ~3e-4, and DELTA = 0.01 leaves a factor 30.
+MARGIN_TAU = 2e-5
+VALUE_DELTA = 0.01
+
+
+def robust_pixels(accum, margin, spp, tau=MARGIN_TAU, delta=VALUE_DELTA):
+    """bool[H, W]: the pixels whose bytes an f32 render must reproduce exactly (see MARGIN_TAU)"""
+    v = 256.0 * np.sqrt(np.clip(np.asarray(accum) / spp, 0.0, 0.999))
+    frac = np.abs(v - np.round(v))
+    exact = (frac > delta) | (np.asarray(accum) == 0.0)
+    return (np.asarray(margin) >= tau) & exact.all(axis=-1)
 
 
 # ---- worlds: the seeded scene builder and scene files, from the HOST-ONLY build of rtiow_b200/csrc/scene_gen.cpp ----------

@@ -407,6 +407,165 @@ int o_render(const o_world* w, const o_camera* cam, const o_render_params* p, ui
     return 0;
 }
 
+/* ============================== knife-edge margins ========================================= */
+/* See rtiow_oracle.h (o_render_margins) for what the margins measure and why.  Nothing below feeds back into the path: the
+ * radiance is computed by the same calls, in the same order, as o_ray_color's. */
+
+/* error growth at distance L along a ray whose origin was left by a bounce of kind k (O_MARGIN_K_*) on a sphere of radius r */
+static double o_grow(double g, double k_over_r, double L) { return g * (1.0 + k_over_r * fmax(L, 0.0)); }
+
+static int o_same_sphere(const o_sphere* a, const o_sphere* b)
+{
+    return a->center.x == b->center.x && a->center.y == b->center.y && a->center.z == b->center.z && a->radius == b->radius;
+}
+
+/* the hit scan's margin of one ray (o_world_hit with t_win the winner's root, INFINITY on a miss): grazing spheres in
+ * [t_min, t_win], roots near t_min and the gap between the two smallest accepted roots, each divided by the growth at the
+ * sphere's distance.  `self`: the sphere the ray starts on, whose near-zero root is no decision (and whose far root the
+ * renderer computes without a discriminant); a coincident twin of it has the same roots in f64. */
+static double o_hit_margin(const o_world* w, const o_ray* r, double t_min, double t_win, int32_t self, double g, double k_over_r)
+{
+    const double a = o_length_squared(r->dir), dl = sqrt(a), lo = o_length(r->orig);
+    double m = INFINITY, t1 = INFINITY, t2 = INFINITY, len1 = 0.0, len2 = 0.0;
+    int32_t i1 = -1;
+    for (int32_t i = 0; i < w->n_spheres; ++i) {
+        const o_sphere* s = &w->spheres[i];
+        const int is_self = self >= 0 && o_same_sphere(s, &w->spheres[self]);     /* the sphere, or a coincident twin */
+        const o_vec3 oc = o_sub(r->orig, s->center);
+        const double hb = o_dot(oc, r->dir), ar = fabs(s->radius);
+        const double disc = hb * hb - a * (o_length_squared(oc) - s->radius * s->radius);
+        const double len = lo + o_length(oc) + ar;              /* the lengths the sphere's roots are computed from */
+        const double tca = -hb / a;
+        if (disc < 0.0) {                                        /* a near miss in front of the winner */
+            if (!is_self && tca >= t_min && tca <= t_win)
+                m = fmin(m, (-disc / a) / (ar * len) / o_grow(g, k_over_r, tca * dl));
+            continue;
+        }
+        const double sq = sqrt(disc), t0 = (-hb - sq) / a, tf = (-hb + sq) / a;
+        const double tacc = t0 >= t_min ? t0 : tf >= t_min ? tf : tca;
+        const double gi = o_grow(g, k_over_r, tacc * dl);
+        if (!is_self && ((t0 >= t_min && t0 <= t_win) || (tf >= t_min && tf <= t_win)))
+            m = fmin(m, (disc / a) / (ar * len) / gi);           /* grazing */
+        for (int k = 0; k < 2; ++k) {                            /* roots near t_min */
+            const double t = k ? tf : t0;
+            if (is_self && fabs(t) <= fabs(k ? t0 : tf)) continue;
+            m = fmin(m, fabs(t - t_min) * dl / len / gi);
+        }
+        if (t0 >= t_min || tf >= t_min) {                        /* the two smallest accepted roots; a coincident twin ties exactly */
+            if (i1 >= 0 && o_same_sphere(s, &w->spheres[i1])) {
+                if (tacc <= t1) { t1 = tacc; i1 = i; }
+            } else if (tacc < t1) {
+                t2 = t1; len2 = len1; t1 = tacc; len1 = len; i1 = i;
+            } else if (tacc < t2) {
+                t2 = tacc; len2 = len;
+            }
+        }
+    }
+    if (isfinite(t2)) m = fmin(m, (t2 - t1) * dl / fmax(len1, len2) / o_grow(g, k_over_r, t1 * dl));
+    return m;
+}
+
+/* o_ray_color in DIRECT mode, plus the smallest margin of every ray of the path in *margin.  self: the sphere the ray
+ * starts on (-1 for a camera ray); g, k_over_r: the error growth of the ray's origin and of its direction per unit length */
+static o_vec3 o_ray_color_m(const o_ray* r, const o_world* w, int32_t depth, double t_min, o_rng* g, uint32_t bounce,
+                            o_counters* cnt, int32_t self, double gr, double k_over_r, double* margin)
+{
+    if (depth <= 0) return o_v(0, 0, 0);
+
+    o_hit_record rec;
+    int32_t idx = -1;
+    if (cnt) { cnt->rays++; cnt->sphere_tests += (uint64_t)w->n_spheres; }
+    if (o_world_hit(w, r, t_min, INFINITY, &rec, &idx)) {
+        const o_material* m = &w->materials[rec.mat];
+        const double dl = o_length(r->dir);
+        *margin = fmin(*margin, o_hit_margin(w, r, t_min, rec.t, self, gr, k_over_r));
+        const double gh = o_grow(gr, k_over_r, rec.t * dl);          /* growth at the hit point */
+        o_vec3 sample = o_v(0, 0, 0);
+        double u[4];
+        uint64_t seed = ((uint64_t)g->key[1] << 32) | g->key[0];
+        o_direct_uniforms(seed, g->pixel, g->sample, bounce + 1u, u);
+        if (m->kind == O_MAT_LAMBERTIAN) sample = o_direct_unit_vector(u[0], u[1]);
+        else if (m->kind == O_MAT_METAL) sample = o_direct_in_unit_sphere(u[0], u[1], u[2]);
+        else sample = o_v(u[0], 0, 0);
+        o_vec3 att; o_ray scat;
+        const int some = o_scatter(m, r, &rec, sample, &att, &scat);
+        /* the scatter's own decision, and the growth of the direction error it passes on */
+        const double ar = fabs(w->spheres[idx].radius);
+        double k_next = O_MARGIN_K_SPECULAR, amp = 1.0;
+        if (m->kind == O_MAT_LAMBERTIAN) {
+            *margin = fmin(*margin, o_length(o_add(rec.normal, o_unit_vector(sample))) / gh);     /* the near-zero fallback */
+            k_next = O_MARGIN_K_LAMBERTIAN;
+        } else if (m->kind == O_MAT_METAL) {
+            const double sl = o_length(scat.dir);
+            *margin = fmin(*margin, (sl > 0.0 ? fabs(o_dot(scat.dir, rec.normal)) / sl : 0.0) / gh);   /* absorption */
+        } else {
+            const double ratio = rec.front_face ? 1.0 / m->param : m->param;
+            const o_vec3 ud = o_unit_vector(r->dir);
+            const double cos_theta = fmin(1.0, -o_dot(ud, rec.normal));
+            const double sin_theta = sqrt(1.0 - cos_theta * cos_theta);
+            *margin = fmin(*margin, fabs(ratio * sin_theta - 1.0) / gh);                                    /* TIR */
+            if (ratio * sin_theta <= 1.0) {
+                *margin = fmin(*margin, fabs(o_reflectance(cos_theta, ratio) - sample.x) / gh);             /* Schlick */
+                if (o_reflectance(cos_theta, ratio) <= sample.x) {    /* refracted: Snell's law amplifies the angle's error */
+                    const double cos_out = sqrt(fmax(1.0 - ratio * ratio * sin_theta * sin_theta, 1e-300));
+                    amp = fmax(1.0, ratio * cos_theta / cos_out);
+                }
+            }
+        }
+        if (some) {
+            return o_mul_v(att, o_ray_color_m(&scat, w, depth - 1, t_min, g, bounce + 1u, cnt, idx, gh * amp,
+                                              k_next / ar, margin));
+        }
+        return o_v(0, 0, 0);
+    }
+    *margin = fmin(*margin, o_hit_margin(w, r, t_min, INFINITY, self, gr, k_over_r));
+    o_vec3 unit_direction = o_unit_vector(r->dir);
+    double t = 0.5 * (unit_direction.y + 1.0);
+    return o_add(o_mul_s(o_v(1, 1, 1), 1.0 - t), o_mul_s(o_v(0.5, 0.7, 1.0), t));
+}
+
+int o_render_margins(const o_world* w, const o_camera* cam, const o_render_params* p, uint8_t* out_rgba, double* accum,
+                     double* margin, o_counters* cnt)
+{
+    if (!w || !cam || !p || !out_rgba || !margin || p->width < 2 || p->height < 2 || p->spp == 0 || p->sampler != O_SAMPLER_DIRECT)
+        return -1;
+    uint32_t rb = p->row_begin, re = p->row_end;
+    if (rb == 0 && re == 0) re = p->height;
+    if (re > p->height || rb > re) return -1;
+    uint64_t rays = 0, tests = 0;
+#ifdef _OPENMP
+    int nt = p->n_threads > 0 ? p->n_threads : omp_get_max_threads();
+#pragma omp parallel for schedule(dynamic, 1) num_threads(nt) reduction(+ : rays, tests)
+#endif
+    for (int64_t y = (int64_t)rb; y < (int64_t)re; ++y) {
+        uint32_t j = p->height - 1u - (uint32_t)y;
+        o_counters c = { 0, 0 };
+        for (uint32_t i = 0; i < p->width; ++i) {
+            o_vec3 pixel_color = o_v(0, 0, 0);
+            double mg = INFINITY;
+            for (uint32_t s = 0; s < p->spp; ++s) {
+                /* o_path_radiance with the DIRECT sampler */
+                o_rng g;
+                o_rng_init(&g, p->seed, j * p->width + i, s, p->sampler);
+                double u4[4], dx, dy;
+                o_direct_uniforms(p->seed, g.pixel, g.sample, 0u, u4);
+                o_direct_disk(u4[2], u4[3], &dx, &dy);
+                double u = ((double)i + u4[0]) / (double)(p->width - 1);
+                double v = ((double)j + u4[1]) / (double)(p->height - 1);
+                o_ray r = o_camera_get_ray(cam, u, v, dx, dy);
+                pixel_color = o_add(pixel_color, o_ray_color_m(&r, w, p->max_depth, p->t_min, &g, 0u, &c, -1, 1.0, 0.0, &mg));
+            }
+            size_t px = (size_t)y * p->width + i;
+            o_to_rgba(pixel_color, p->alpha, p->spp, out_rgba + 4 * px);
+            if (accum) { accum[3 * px] = pixel_color.x; accum[3 * px + 1] = pixel_color.y; accum[3 * px + 2] = pixel_color.z; }
+            margin[px] = mg;
+        }
+        rays += c.rays; tests += c.sphere_tests;
+    }
+    if (cnt) { cnt->rays = rays; cnt->sphere_tests = tests; }
+    return 0;
+}
+
 /* ============================== batch helpers ============================================= */
 
 static o_vec3 ld3(const double* a, int64_t i) { return o_v(a[3 * i], a[3 * i + 1], a[3 * i + 2]); }

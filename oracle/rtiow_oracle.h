@@ -152,6 +152,30 @@ typedef struct {
 int o_render(const o_world* w, const o_camera* cam, const o_render_params* p, uint8_t* out_rgba,
              double* accum, o_counters* cnt);
 
+/* o_render with the DIRECT sampler (the same bytes, sums and counters), plus margin[H][W] (top-down): how far each pixel is
+ * from a decision an f32 render could take the other way.  It is the smallest margin over every ray of the pixel's paths;
+ * a ray's margin is the smallest of these normalised distances from a decision boundary, each divided by the ray's error
+ * growth (below):
+ *   grazing    |r^2 - dist(centre, line)^2| / (|r| L) for every sphere with a root in [t_min, t_winner], or whose line
+ *              passes outside it with tca in that range (a near miss in front of the winner);
+ *   t_min      |root - t_min| |dir| / L for every root of every sphere (not the near-zero root of the sphere the ray
+ *              starts on, which the renderer drops without computing it);
+ *   near tie   (t2 - t1) |dir| / L between the two smallest accepted roots (not between coincident spheres, which tie
+ *              exactly in f32 too);
+ *   dielectric |ratio sin(theta) - 1| and, when it can refract, |reflectance - xi|;
+ *   metal      dot(d, n) / |d| (the absorption test);
+ *   lambertian |n + unit(sample)| (the near-zero fallback).
+ * L = |o| + |o - c| + |r| is the size of the numbers the sphere's roots are computed from: f32 rounding moves a root by
+ * about eps32 L.  The growth starts at 1 on the camera ray and is multiplied at every hit by 1 + k L_next / |r| (L_next:
+ * the distance from the hit to the point of the next ray being judged; k = O_MARGIN_K_SPECULAR for a mirror or glass
+ * bounce, whose direction turns by twice the normal's error, O_MARGIN_K_LAMBERTIAN for a diffuse one, whose direction is
+ * offset by the normal's), and by Snell's amplification ratio cos(theta) / cos(theta_out) on a refraction.  Without the
+ * growth, long mirror and glass chains look robust where an f32 render leaves them. */
+#define O_MARGIN_K_SPECULAR 2.0
+#define O_MARGIN_K_LAMBERTIAN 1.0
+int o_render_margins(const o_world* w, const o_camera* cam, const o_render_params* p, uint8_t* out_rgba, double* accum,
+                     double* margin, o_counters* cnt);
+
 /* one path: pixel (i, j) with j=0 the BOTTOM row (main.rs:131-135), sample index s */
 o_vec3 o_path_radiance(const o_world* w, const o_camera* cam, const o_render_params* p,
                        uint32_t i, uint32_t j, uint32_t s, o_counters* cnt);

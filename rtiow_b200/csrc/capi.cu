@@ -16,6 +16,7 @@
 #include <cstring>
 #include <cstdlib>
 #include <string>
+#include <tuple>
 #include <type_traits>
 #include <vector>
 #include <utility>
@@ -379,6 +380,15 @@ static int check_scene(const rtiow_spheres* s, const rtiow_materials* m)
         if (!(std::isfinite(s->cx[i]) && std::isfinite(s->cy[i]) && std::isfinite(s->cz[i]) && std::isfinite(s->radius[i])))
             return fail(RTIOW_ERR_INVALID_ARG, "sphere %d: non-finite centre or radius", i);
     }
+    // a non-finite albedo or param that a sphere's material reads would turn the reference's pixel black through NaN, while the
+    // render drops the sample (to_fix); Dielectric ignores its albedo and Lambertian its param (materials.rs), so those may be anything
+    for (int i = 0; i < (int)s->n; ++i) {
+        const uint32_t k = s->mat_index[i], kind = m->kind[k];
+        if (kind != RTIOW_MAT_DIELECTRIC && !(std::isfinite(m->albedo_r[k]) && std::isfinite(m->albedo_g[k]) && std::isfinite(m->albedo_b[k])))
+            return fail(RTIOW_ERR_INVALID_ARG, "sphere %d: material %u has a non-finite albedo", i, k);
+        if (kind != RTIOW_MAT_LAMBERTIAN && !std::isfinite(m->param[k]))
+            return fail(RTIOW_ERR_INVALID_ARG, "sphere %d: material %u has a non-finite param", i, k);
+    }
     return RTIOW_OK;
 }
 
@@ -507,6 +517,15 @@ extern "C" int rtiow_scene_upload(rtiow_ctx* c, const rtiow_spheres* s, const rt
     const int n = (int)s->n;
     std::vector<float4> sph(n), mat(n); std::vector<double4> sphd(n), matd(n); std::vector<uint8_t> kind(n);
     std::vector<int> small_idx, big_idx;
+    // A sphere with a later twin (the same centre and radius) never wins: the reference computes the same root for both, and
+    // the later index takes every tie (mod.rs:61-66).  It is left out of every scan.  Kept in, it would compete with the
+    // twin a ray starts on, whose root the scan takes exactly (candidate_self) while its own carries the origin's rounding.
+    std::vector<int> order(n);
+    for (int i = 0; i < n; ++i) order[i] = i;
+    const auto key = [s](int i) { return std::make_tuple(s->cx[i], s->cy[i], s->cz[i], s->radius[i]); };
+    std::sort(order.begin(), order.end(), [&](int a, int b) { return key(a) < key(b) || (key(a) == key(b) && a < b); });
+    std::vector<uint8_t> shadowed(n, 0);
+    for (int k = 0; k + 1 < n; ++k) shadowed[order[k]] = key(order[k]) == key(order[k + 1]);
     for (int i = 0; i < n; ++i) {
         const uint32_t mi = s->mat_index[i];
         sphd[i] = make_double4(s->cx[i], s->cy[i], s->cz[i], s->radius[i]);
@@ -515,7 +534,9 @@ extern "C" int rtiow_scene_upload(rtiow_ctx* c, const rtiow_spheres* s, const rt
         mat[i] = make_float4((float)m->albedo_r[mi], (float)m->albedo_g[mi], (float)m->albedo_b[mi], (float)m->param[mi]);
         kind[i] = (uint8_t)m->kind[mi];
         const double reach = std::sqrt(s->cx[i] * s->cx[i] + s->cy[i] * s->cy[i] + s->cz[i] * s->cz[i]) + std::fabs(s->radius[i]);
-        if (std::fabs(s->radius[i]) > kBigRadius || reach > 4096.0) big_idx.push_back(i); else small_idx.push_back(i);
+        if (shadowed[i]) sphd[i].w = NAN;        // the f64 scan tests every sphere: a NaN root loses every comparison in candidate
+        else if (std::fabs(s->radius[i]) > kBigRadius || reach > 4096.0) big_idx.push_back(i);
+        else small_idx.push_back(i);
     }
     const int ns = (int)small_idx.size(), nb = (int)big_idx.size();
     while (small_idx.size() % 32) small_idx.push_back(-1);                  // whole 32-sphere words; padding never hits
@@ -780,6 +801,8 @@ static int launch_render(const ScanPlan& plan, DeviceState& d, const rtiow_camer
     a.chunks_per_fetch = std::max<uint32_t>(1u, 256u / a.chunk_samples);
     const uint64_t n_lp = (uint64_t)a.local_rows * p->width;
     a.n_chunks = n_lp * a.chunks_per_pixel;
+    a.sample_cap = (T)std::min(1e9, (double)p->spp);        // the whole frame's spp: every pass of a progressive render adds the same
+    a.saturate = p->spp > 65535u;
     *paths = n_lp * sr.count;
     CU(d.accum.resize(3 * n_lp));
     a.accum = d.accum.p; a.work_counter = d.counters.p; a.ray_counter = d.counters.p + 1;

@@ -29,6 +29,8 @@ template <typename T> struct RenderArgs {
     uint32_t chunks_per_fetch;     // chunks per fetch from the work counter while plenty are left ...
     uint32_t guided_div;           // ... and (chunks left) / guided_div towards the end (guided_div = 2 x warps of the grid)
     uint64_t n_chunks;
+    T sample_cap;                  // min(1e9, the frame's total spp): the largest value a sample adds (to_fix)
+    uint32_t saturate;             // total spp > 65535: sums could pass 2^32, accumulate with add_saturating
     unsigned long long* accum;     // [3][local_rows*width] 32.32 fixed-point radiance sums
     unsigned long long* work_counter;
     unsigned long long* ray_counter;
@@ -36,15 +38,17 @@ template <typename T> struct RenderArgs {
 
 #define RT_FIX_SCALE 4294967296.0f   // 2^32
 
-__device__ __forceinline__ unsigned long long to_fix(float c)
+// A sample's 32.32 value, clamped to [0, cap].  NaN/negative -> 0: a poisoned sample contributes nothing (the reference would
+// turn the whole pixel black through NaN -> `as u8` = 0, vec3.rs:415-417; the upload rejects non-finite materials, so only
+// an overflow to inf x 0 can make one).  cap = min(1e9, total spp) changes no byte: a sample of >= spp alone brings the
+// pixel's mean to >= 1, which quantises to 255 with or without the clamp (vec3.rs:404-420).
+__device__ __forceinline__ unsigned long long to_fix(float c, float cap)
 {
-    // NaN/negative -> 0, saturating: a poisoned sample contributes nothing (the reference would
-    // turn the whole pixel black through NaN -> `as u8` = 0, vec3.rs:415-417; measure-zero event)
-    return __float2ull_rn(fminf(fmaxf(c, 0.0f), 1.0e9f) * RT_FIX_SCALE);
+    return __float2ull_rn(fminf(fmaxf(c, 0.0f), cap) * RT_FIX_SCALE);
 }
-__device__ __forceinline__ unsigned long long to_fix(double c)
+__device__ __forceinline__ unsigned long long to_fix(double c, double cap)
 {
-    return __double2ull_rn(fmin(fmax(c, 0.0), 1.0e9) * 4294967296.0);
+    return __double2ull_rn(fmin(fmax(c, 0.0), cap) * 4294967296.0);
 }
 
 // local row -> global top-down row under the interleaved-tile partition
@@ -230,16 +234,31 @@ __device__ __forceinline__ bool assign_work(const RenderArgs<T>& a, WorkCursor& 
     return fresh;
 }
 
+// One channel's add, saturating at 2^64 - 1 (a sum of 2^32: any spp below 2^32 quantises it to 255, as the reference's
+// unbounded f64 sum would be).  An add that wraps sees old + v < old and raises the sum to the maximum; any later add wraps
+// again and does the same, so whatever the order of the adds, a channel that passed 2^32 ends at 2^64 - 1 and every other
+// one holds its exact sum.  It waits for the old value, so it is only used where a sum can pass 2^32 (RenderArgs::saturate).
+__device__ __forceinline__ void add_saturating(unsigned long long* sum, unsigned long long v)
+{
+    const unsigned long long old = atomicAdd(sum, v);
+    if (old + v < old) atomicMax(sum, ~0ull);
+}
+
 // pixel_color += ray_color (main.rs:135): 32.32 fixed-point RED.ADD.U64 straight into the frame's accumulators
-// (integer adds commute: any order, any GPU count, same bits); black paths add nothing
+// (integer adds commute: any order, any GPU count, same bits); black paths add nothing.  With every sample clamped to
+// sample_cap <= spp, a channel's sum stays below spp^2 <= 65535^2 < 2^32 and cannot wrap; larger spp saturate instead.
 template <typename T>
 __device__ __forceinline__ void accumulate(const RenderArgs<T>& a, uint32_t acc_lp, V3<T> rad)
 {
     if (rad.x != T(0) || rad.y != T(0) || rad.z != T(0)) {
         const size_t n_lp = (size_t)a.local_rows * a.width;
-        atomicAdd(a.accum + acc_lp, to_fix(rad.x));
-        atomicAdd(a.accum + n_lp + acc_lp, to_fix(rad.y));
-        atomicAdd(a.accum + 2 * n_lp + acc_lp, to_fix(rad.z));
+        unsigned long long* const sum = a.accum + acc_lp;
+        const unsigned long long vx = to_fix(rad.x, a.sample_cap), vy = to_fix(rad.y, a.sample_cap), vz = to_fix(rad.z, a.sample_cap);
+        if (a.saturate) {
+            add_saturating(sum, vx); add_saturating(sum + n_lp, vy); add_saturating(sum + 2 * n_lp, vz);
+        } else {
+            atomicAdd(sum, vx); atomicAdd(sum + n_lp, vy); atomicAdd(sum + 2 * n_lp, vz);
+        }
     }
 }
 

@@ -285,3 +285,12 @@ def test_unsupported_and_invalid_scene(ctx, capi):
     with pytest.raises(capi.RtiowError) as e:
         ctx.upload_scene([[np.nan, 0, 0]], [1.0], [0], [0], [[1, 1, 1]], [0])
     assert e.value.code == capi.ERR_INVALID_ARG
+    # a non-finite field a sphere's material reads: the reference's pixel would be black, the render's would not
+    for kind, albedo, param in ((1, [[1, np.nan, 1]], [0]), (0, [[1, 1, np.inf]], [0]), (1, [[1, 1, 1]], [np.nan]),
+                                (2, [[1, 1, 1]], [-np.inf])):
+        with pytest.raises(capi.RtiowError) as e:
+            ctx.upload_scene([[0, 0, 0]], [1.0], [0], [kind], albedo, param)
+        assert e.value.code == capi.ERR_INVALID_ARG
+    # fields the material ignores (a Dielectric's albedo, a Lambertian's param) and materials no sphere uses may be anything
+    ctx.upload_scene([[0, 0, 0], [3, 0, 0]], [1.0, 1.0], [0, 1], [2, 0, 1], [[np.nan] * 3, [1, 1, 1], [np.inf] * 3],
+                     [1.5, np.nan, np.nan])
