@@ -46,9 +46,13 @@ typedef enum { RTIOW_PRECISION_F32 = 0, RTIOW_PRECISION_F64 = 1 } rtiow_precisio
 
 /* Where the sphere FILTER of the F32 scan runs (HittableList::hit, shapes/mod.rs:56-69: every ray against every sphere).
  * FP32: 7 packed FFMA2 per sphere pair on the CUDA cores.  TENSOR: the discriminant as a [rays x 11] x [11 x spheres]
- * contraction on the tcgen05 tensor cores (fp16 hi/lo split, fp32 accumulate in TMEM).  Both are conservative filters in
- * front of the SAME precise test, so hits, images and ray counts are identical bit for bit.  AUTO = TENSOR when the scene
- * qualifies (its small spheres fit one CTA's shared memory), else FP32. */
+ * contraction on the tcgen05 tensor cores (fp16 hi/lo split, fp16 accumulate in TMEM).  Both are conservative filters in
+ * front of the SAME precise test: a filter may pass spheres the test rejects, never drop one it accepts.  So on the same ray
+ * both find the same sphere, t, p and normal bit for bit (rtiow_hitlist_batch), and each gives exactly what its own kernel
+ * gives with the filter bypassed (rtiow_ctx_set_filter_bypass).  A render runs separately compiled kernels per backend, whose
+ * hit-point and scatter code the compiler contracts into FMAs differently, so FP32 and TENSOR frames agree on all but about
+ * 1 pixel in 10^5 and ray counts to about 1e-5; each backend's frame is byte-identical to its own frame with the filter
+ * bypassed.  AUTO = TENSOR when the scene qualifies (its small spheres fit one CTA's shared memory), else FP32. */
 typedef enum { RTIOW_SCAN_AUTO = 0, RTIOW_SCAN_FP32 = 1, RTIOW_SCAN_TENSOR = 2 } rtiow_scan_backend;
 
 /* HittableList of Sphere (shapes/mod.rs:52, shapes/sphere.rs:9-13) as a structure of arrays,
@@ -130,6 +134,11 @@ void rtiow_ctx_destroy(rtiow_ctx* ctx);
 /* Select the filter backend of every later F32 call on this ctx (render and unit-level batches).  RTIOW_SCAN_TENSOR on a
  * scene that does not qualify makes those calls return RTIOW_ERR_UNSUPPORTED (never a silent fallback). */
 int  rtiow_ctx_set_scan_backend(rtiow_ctx* ctx, int backend);
+/* Testing aid, off by default.  While on, rtiow_scene_upload builds filter inputs (the FP32 table and the tensor image) that
+ * pass every sphere for every ray, so the same kernels run the precise test on every sphere: any difference from the output
+ * with the filter on is a hit the filter dropped.  The scan arm a scene lands on does not change.  Affects later uploads only;
+ * a bypassed scene is slower to render and must be uploaded again after turning it off. */
+int  rtiow_ctx_set_filter_bypass(rtiow_ctx* ctx, int on);
 
 /* One process per GPU (MPI / torchrun style) with the gather INSIDE the library.  Rank 0 calls rtiow_nccl_unique_id and hands
  * the RTIOW_NCCL_UNIQUE_ID_BYTES bytes to every rank by any means (MPI_Bcast, a file, torch.distributed); every rank then

@@ -29,7 +29,7 @@ PROGRESS_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint3
 # every symbol include/rtiow_cuda.h declares (tests check the .so exports exactly these)
 SYMBOLS = [
     "rtiow_abi_version", "rtiow_last_error", "rtiow_device_count", "rtiow_ctx_create", "rtiow_ctx_create_on_device",
-    "rtiow_ctx_destroy", "rtiow_ctx_set_scan_backend", "rtiow_nccl_unique_id", "rtiow_ctx_create_rank", "rtiow_ctx_set_gather", "rtiow_ctx_set_stream",
+    "rtiow_ctx_destroy", "rtiow_ctx_set_scan_backend", "rtiow_ctx_set_filter_bypass", "rtiow_nccl_unique_id", "rtiow_ctx_create_rank", "rtiow_ctx_set_gather", "rtiow_ctx_set_stream",
     "rtiow_ctx_gather_info", "rtiow_render_rank", "rtiow_render_rank_device", "rtiow_render_rank_enqueue", "rtiow_ctx_synchronize", "rtiow_scene_upload", "rtiow_camera_new", "rtiow_params_default", "rtiow_render", "rtiow_render_views", "rtiow_render_progressive",
     "rtiow_tile_buffer_bytes", "rtiow_render_tiles_device", "rtiow_render_to_frame_device", "rtiow_deinterleave_device", "rtiow_sphere_hit_batch",
     "rtiow_hitlist_batch", "rtiow_scatter_batch", "rtiow_get_ray_batch", "rtiow_to_rgba_batch", "rtiow_reflect_batch",
@@ -108,6 +108,7 @@ def _declare(L):
         "rtiow_ctx_create_on_device": (C.c_int, [C.c_int, C.POINTER(P)]),
         "rtiow_ctx_destroy": (None, [P]),
         "rtiow_ctx_set_scan_backend": (C.c_int, [P, C.c_int]),
+        "rtiow_ctx_set_filter_bypass": (C.c_int, [P, C.c_int]),
         "rtiow_nccl_unique_id": (C.c_int, [P]),
         "rtiow_ctx_create_rank": (C.c_int, [C.c_int, C.c_int, C.c_int, P, C.POINTER(P)]),
         "rtiow_ctx_set_gather": (C.c_int, [P, C.c_int]),
@@ -275,6 +276,10 @@ class Context:
     def set_scan_backend(self, backend: int):
         """SCAN_AUTO / SCAN_FP32 (FFMA2 filter on the CUDA cores) / SCAN_TENSOR (tcgen05 filter): same hits, same images."""
         _check(lib().rtiow_ctx_set_scan_backend(self._h, backend))
+
+    def set_filter_bypass(self, on: bool):
+        """testing aid: scenes uploaded while on get filter images that pass every sphere (the precise test sees all of them)"""
+        _check(lib().rtiow_ctx_set_filter_bypass(self._h, int(bool(on))))
 
     def set_gather(self, mode: int):
         """GATHER_AUTO / GATHER_NCCL (tile buffers + ncclAllGather + de-interleave) / GATHER_FUSED (peer stores into rank 0's frame)"""

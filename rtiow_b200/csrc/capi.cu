@@ -103,6 +103,7 @@ struct DeviceState {
 struct rtiow_ctx {
     std::vector<DeviceState> dev;
     int scan_backend = RTIOW_SCAN_AUTO;  // rtiow_ctx_set_scan_backend
+    bool filter_bypass = false;          // rtiow_ctx_set_filter_bypass: later uploads build filter images that pass every sphere
     HostBuf<unsigned char> scene_stage;  // page-locked staging blob of rtiow_scene_upload
     bool peer_ok = true;                 // every device can store into device 0's memory (NVLink P2P): fused epilogue + gather
     // the gather of the row tiles (rtiow_ctx_set_gather)
@@ -189,6 +190,13 @@ extern "C" int rtiow_ctx_set_scan_backend(rtiow_ctx* c, int backend)
     if (!c) return fail(RTIOW_ERR_INVALID_ARG, "ctx is NULL");
     if (backend != RTIOW_SCAN_AUTO && backend != RTIOW_SCAN_FP32 && backend != RTIOW_SCAN_TENSOR) return fail(RTIOW_ERR_INVALID_ARG, "unknown scan backend %d", backend);
     c->scan_backend = backend;
+    return RTIOW_OK;
+}
+
+extern "C" int rtiow_ctx_set_filter_bypass(rtiow_ctx* c, int on)
+{
+    if (!c) return fail(RTIOW_ERR_INVALID_ARG, "ctx is NULL");
+    c->filter_bypass = on != 0;
     return RTIOW_OK;
 }
 
@@ -394,13 +402,17 @@ static int check_scene(const rtiow_spheres* s, const rtiow_materials* m)
 
 // The FP32 filter's table of the small spheres (rt_scene.cuh): records of 4 spheres [cx0..3][cy0..3][cz0..3][K0..3], then the
 // look-ahead record.  small = the first ns entries are spheres, the rest padding; R2 = the squared bounding radius of the filter.
-static std::vector<float> filter_table(const std::vector<float4>& small, int ns, double R2)
+// bypass (rtiow_ctx_set_filter_bypass): every sphere gets centre 0 and K = -1e30, so C = K and disc' = hb^2 + 1e30 > 0 for every
+// ray, live or dead (a dead line has hb = 0): the precise test sees every sphere.  Padding is unchanged and still never passes.
+static std::vector<float> filter_table(const std::vector<float4>& small, int ns, double R2, bool bypass)
 {
     const int np = (int)small.size();
     std::vector<float> table(RT_TABLE_FLOATS(np), 0.0f);
     for (int p = 0; p < np; ++p) {
         float* rec = table.data() + (size_t)(p >> 2) * 16 + (p & 3);
-        if (p < ns) {
+        if (p < ns && bypass) {
+            rec[0] = 0; rec[4] = 0; rec[8] = 0; rec[12] = -1e30f;
+        } else if (p < ns) {
             const float4 v = small[p];
             rec[0] = v.x; rec[4] = v.y; rec[8] = v.z;
             // K = |c|^2 - r^2 + R^2 of the f32 sphere, in f64, lowered by the filter slack (RT_FILTER_SLACK, rt_scene.cuh)
@@ -442,7 +454,10 @@ static std::vector<float4> big_sphere_records(const std::vector<double4>& big, b
 // Enabled when the image fits beside the candidate lists in one CTA's shared memory and the slack stays below the
 // mean r^2 (a scene spread over a huge radius would pass every sphere near the line; the FP32 filter handles those).
 // Returns the padded sphere count u_npad, or 0 (and no image) when the scene does not qualify.
-static int tensor_image(const std::vector<float4>& small, int ns, double R, std::vector<unsigned char>* img, umma::FeatScale* u_sc)
+// bypass (rtiow_ctx_set_filter_bypass): every sphere column gets S_0 = Rp^2 / s0, S_10 = -1 / s10 and zeros elsewhere (powers of
+// two: no lo parts), so D = a Rp^2 + a |f_perp|^2 - (f.d)^2 - sigma > 0 on a live row and D = Rp on a dead one: every sphere passes,
+// with |D| <= Rp^2 + R^2 + sigma, finite in fp16 wherever d_fits admits the scene.  The rules, npad and padding are unchanged.
+static int tensor_image(const std::vector<float4>& small, int ns, double R, bool bypass, std::vector<unsigned char>* img, umma::FeatScale* u_sc)
 {
     using Shape = UmmaShape<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
     const int npad = (ns + RT_UMMA_CHUNK - 1) / RT_UMMA_CHUNK * RT_UMMA_CHUNK;
@@ -471,6 +486,12 @@ static int tensor_image(const std::vector<float4>& small, int ns, double R, std:
     };
     for (int j = 0; j < npad; ++j) {
         double S[11] = { 0 };
+        if (j < ns && bypass) {
+            S[0] = Rp * Rp / u_sc->s0;
+            S[10] = -1.0 / u_sc->s10;
+            put_all(j, S);
+            continue;
+        }
         if (j < ns) {                     // position j of `small` (list order); the f32 sphere the precise test sees
             const float4 v = small[j];
             const double x = v.x, y = v.y, z = v.z, r = v.w;
@@ -553,14 +574,14 @@ extern "C" int rtiow_scene_upload(rtiow_ctx* c, const rtiow_spheres* s, const rt
         rmax = std::max(rmax, std::fabs((double)v.w));
     }
     const float R2f = (float)(R * R * (1.0 + 1e-6));
-    const std::vector<float> table = filter_table(small, ns, (double)R2f);
+    const std::vector<float> table = filter_table(small, ns, (double)R2f, c->filter_bypass);
     std::vector<double4> big(nb); for (int b = 0; b < nb; ++b) big[b] = sphd[big_idx[b]];
     bool bigf_ok = false;
     const std::vector<float4> bigf = big_sphere_records(big, &bigf_ok);
     SceneDev sc{};
     std::vector<unsigned char> ubimg;
     sc.u_sc = umma::FeatScale{ 1.0f, 1.0f, 1.0f, 1.0f };
-    sc.u_npad = tensor_image(small, ns, R, &ubimg, &sc.u_sc);
+    sc.u_npad = tensor_image(small, ns, R, c->filter_bypass, &ubimg, &sc.u_sc);
     SceneBlob blob;                      // the pointers of `sc` hold offsets into the blob until rebase()
     sc.table = blob.put(table); sc.small = blob.put(small); sc.small_idx = blob.put(small_idx); sc.big = blob.put(big); sc.big_idx = blob.put(big_idx);
     sc.sph = blob.put(sph); sc.sphd = blob.put(sphd); sc.mat = blob.put(mat); sc.matd = blob.put(matd); sc.kind = blob.put(kind);

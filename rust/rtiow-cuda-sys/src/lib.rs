@@ -94,6 +94,7 @@ extern "C" {
     pub fn rtiow_ctx_create_on_device(device: c_int, out: *mut *mut rtiow_ctx) -> c_int;
     pub fn rtiow_ctx_destroy(ctx: *mut rtiow_ctx);
     pub fn rtiow_ctx_set_scan_backend(ctx: *mut rtiow_ctx, backend: c_int) -> c_int;
+    pub fn rtiow_ctx_set_filter_bypass(ctx: *mut rtiow_ctx, on: c_int) -> c_int;
     pub fn rtiow_nccl_unique_id(out_id: *mut c_void) -> c_int;
     pub fn rtiow_ctx_create_rank(device: c_int, rank: c_int, world: c_int, nccl_unique_id: *const c_void, out: *mut *mut rtiow_ctx) -> c_int;
     pub fn rtiow_ctx_set_stream(ctx: *mut rtiow_ctx, stream: *mut c_void) -> c_int;

@@ -238,18 +238,24 @@ def per_sphere_rays(arrays, seed=0):
     return np.concatenate([o_in, o_out]), np.concatenate([d_in, d_out])
 
 
+def framing(arrays):
+    """(spheres of interest, their middle, an extent around it, a camera eye that sees them): the view of mixed_rays' camera rays"""
+    info = scene_info(arrays)
+    k_all = info["small"] if info["ns"] else np.arange(len(arrays["radius"]))
+    cs, r = arrays["center"][k_all], np.abs(arrays["radius"][k_all])
+    mid = cs.mean(0)
+    ext = float(np.percentile(np.linalg.norm(cs - mid, axis=1), 90)) + r.max() + 1.0
+    return k_all, mid, ext, mid + 1.4 * ext * _unit(np.array([0.8, 0.35, 0.5]))
+
+
 def mixed_rays(arrays, n=4000, seed=0):
     """camera rays, rays leaving sphere surfaces, origins 30 .. 2000 away aimed at a sphere, short directions, and lines that
     miss the bounding sphere of the small spheres"""
     rng = np.random.default_rng(8000 + seed)
     info = scene_info(arrays)
-    k_all = info["small"] if info["ns"] else np.arange(len(arrays["radius"]))
     c, r = arrays["center"], np.abs(arrays["radius"])
-    cs = c[k_all]
-    mid = cs.mean(0)
-    ext = float(np.percentile(np.linalg.norm(cs - mid, axis=1), 90)) + r[k_all].max() + 1.0
+    k_all, mid, ext, eye = framing(arrays)
     n_cam, n_sec, n_far, n_short, n_miss = (int(n * f) for f in (0.3, 0.3, 0.2, 0.1, 0.1))
-    eye = mid + 1.4 * ext * _unit(np.array([0.8, 0.35, 0.5]))
     o_cam = eye + 0.05 * rng.normal(size=(n_cam, 3))
     d_cam = mid + ext * _unit(rng.normal(size=(n_cam, 3))) * rng.uniform(0, 1, (n_cam, 1)) ** (1 / 3) - o_cam
     k = rng.choice(k_all, n_sec + n_short)
@@ -278,6 +284,132 @@ def row_rays(x0, x1, n=1000, seed=0):
 
 def f32(a):
     return np.asarray(a, np.float32).astype(np.float64)
+
+
+# ------------------------------------------------------------------------------------------------ silhouette rays
+# The bands in which a filter can drop a hit, as designed (DESIGN.md §1.1, §1.2), in units of the discriminant of a unit
+# direction (r^2 - dist(centre, line)^2).  Stated here rather than read from the sources, so that a changed slack cannot
+# move the bands the tests demand rays in.
+FP32_SLACK = 96 * 2.0 ** -24                    # RT_FILTER_SLACK: per unit of |c|^2 + r^2 + R^2
+TENSOR_SLACK = 1.5625e-5                        # tensor_image: per unit of R^2
+SIGMA_PER_LEN = 16 * 2.0 ** -24                 # sigma = this x max |r| x |o|_1 (rtiow_scene_upload, line_gate)
+SIL_DELTA = (-3e-2, -1e-2, -3e-3, -1e-3, -3e-4, -1e-4, -3e-5, -1e-5, 0.0, 1e-5, 3e-5, 1e-4, 3e-4, 1e-3)
+SIL_BAND = (0.01, 0.1, 0.5, 0.9)                # lines whose discriminant is this fraction of each filter's band
+SIL_BACK = (0.0, 10.0, 100.0, 1000.0, 3000.0)   # origin distance behind the line's closest point (0: 3 |r|)
+SIL_DLEN = (1e-3, 1.0, 30.0)
+
+
+def _perp(u, rng):
+    """a random unit vector perpendicular to each row of u"""
+    return _unit(np.cross(u, rng.normal(size=u.shape)))
+
+
+def _band_deltas(info, c, r):
+    """per sphere, the deltas at which r^2 - (r (1 + delta))^2 is each SIL_BAND fraction of the tensor and the FP32 band"""
+    tensor = TENSOR_SLACK * info["R"] ** 2
+    fp32 = FP32_SLACK * ((c * c).sum(1) + r * r + info["R"] ** 2)
+    disc = np.concatenate([np.multiply.outer(tensor * np.ones_like(r), SIL_BAND), np.multiply.outer(fp32, SIL_BAND)], 1)
+    return np.sqrt(np.clip(1.0 - disc / (r * r)[:, None], 0.0, None)) - 1.0
+
+
+def silhouette_rays(arrays, n_spheres=40, seed=0):
+    """rays whose line passes within a hair of a small sphere's silhouette, where a filter's rounding decides:
+      * per sampled sphere, lines |r| (1 + delta) from its centre for every SIL_DELTA and for the deltas that put the
+        discriminant at SIL_BAND fractions of each filter's band, origins SIL_BACK behind the closest point, |d| in SIL_DLEN;
+      * the same at the outermost spheres, on the side where they touch the bounding R-sphere (lines that graze it: the
+        live gate and the R^2 margin);
+      * axis-aligned directions (exact zeros), origins at the coordinate origin, and origins on sphere surfaces, aimed past a
+        sphere's silhouette or in random directions.
+    -> (o, d, target): f32-rounded rays and, per ray, the list index of the sphere whose silhouette it was built on."""
+    rng = np.random.default_rng(10000 + seed)
+    info = scene_info(arrays)
+    ks = info["small"]
+    C, Rad = np.asarray(arrays["center"], float), np.abs(np.asarray(arrays["radius"], float))
+    sample = rng.choice(ks, n_spheres, replace=len(ks) < n_spheres)       # a scene of few spheres: each one several times
+    reach = np.linalg.norm(C[ks], axis=1) + Rad[ks]
+    outer = ks[np.argsort(-reach, kind="stable")[:8]]
+    os_, ds, ts = [], [], []
+
+    def add(o, d, k):
+        os_.append(o); ds.append(d); ts.append(k)
+
+    def grid(k, radial):
+        """every (delta, back, |d|) for the spheres k; radial: the closest point lies on the far side from the coordinate origin"""
+        deltas = np.concatenate([np.tile(SIL_DELTA, (len(k), 1)), _band_deltas(info, C[k], Rad[k])], 1)
+        nd = deltas.shape[1]
+        kk = np.repeat(k, nd * len(SIL_BACK) * len(SIL_DLEN))
+        delta = np.repeat(deltas.reshape(-1), len(SIL_BACK) * len(SIL_DLEN))
+        back = np.tile(np.repeat(SIL_BACK, len(SIL_DLEN)), len(k) * nd)
+        dlen = np.tile(SIL_DLEN, len(k) * nd * len(SIL_BACK))
+        c, r = C[kk], Rad[kk]
+        if radial:
+            w = np.where(np.linalg.norm(c, axis=1)[:, None] > 0, c, rng.normal(size=c.shape))
+            w = _unit(w); u = _perp(w, rng)
+        else:
+            u = _unit(rng.normal(size=c.shape)); w = _perp(u, rng)
+        back = np.where(back == 0.0, 3.0 * r, back)
+        q = c + w * (r * (1.0 + delta))[:, None]
+        add(q - u * back[:, None], u * dlen[:, None], kk)
+
+    grid(sample, False)
+    grid(outer, True)
+    # axis-aligned: direction +-e_i, the line offset from the centre along e_j
+    for i in range(3):
+        for s in (-1.0, 1.0):
+            kk = np.repeat(sample[:20], len(SIL_DELTA) * 2)
+            delta = np.tile(SIL_DELTA, len(sample[:20]) * 2)
+            back = np.tile(np.repeat([0.0, 100.0], len(SIL_DELTA)), len(sample[:20]))
+            c, r = C[kk], Rad[kk]
+            back = np.where(back == 0.0, 3.0 * r, back)
+            e_i, e_j = np.eye(3)[i], np.eye(3)[(i + 1) % 3]
+            add(c + e_j * (r * (1.0 + delta))[:, None] - s * e_i * back[:, None], np.tile(s * e_i, (len(kk), 1)), kk)
+    # origins at the coordinate origin, aimed past a silhouette, and along the axes
+    kk = np.repeat(sample, len(SIL_DELTA))
+    delta = np.tile(SIL_DELTA, len(sample))
+    c, r = C[kk], Rad[kk]
+    w = _perp(np.where(np.linalg.norm(c, axis=1)[:, None] > 0, c, rng.normal(size=c.shape)), rng)
+    add(np.zeros_like(c), c + w * (r * (1.0 + delta))[:, None], kk)
+    axes = np.concatenate([np.eye(3), -np.eye(3)])
+    add(np.zeros((12, 3)), np.concatenate([axes, 1e-3 * axes]), np.full(12, sample[0]))
+    # origins on a sphere's surface: aimed past another sphere's silhouette, and in random directions
+    k1, k2 = np.repeat(sample, len(SIL_DELTA)), rng.choice(ks, len(sample) * len(SIL_DELTA))
+    o = C[k1] + _unit(rng.normal(size=(len(k1), 3))) * Rad[k1][:, None]
+    w = _perp(C[k2] - o, rng)
+    add(o, C[k2] + w * (Rad[k2] * (1.0 + np.tile(SIL_DELTA, len(sample))))[:, None] - o, k2)
+    add(o, _unit(rng.normal(size=o.shape)) * rng.uniform(0.5, 2.0, (len(o), 1)), k1)
+    o, d, t = np.concatenate(os_), np.concatenate(ds), np.concatenate(ts)
+    keep = np.linalg.norm(d, axis=1) > 0                # (a sphere centred on the coordinate origin has no silhouette point there)
+    return f32(o[keep]), f32(d[keep]), t[keep]
+
+
+def silhouette_bands(arrays, o, d, target):
+    """per ray, the f64 discriminant of its target sphere for the f32-rounded inputs and the unit direction, r^2 - dist^2, and
+    the two bands in which a filter may err: the tensor slack, and the FP32 slack + the ray's sigma (its origin's foot point)
+    -> dict(disc, tensor, fp32)"""
+    info = scene_info(arrays)
+    c = np.asarray(arrays["center"], float)[target]; r = np.asarray(arrays["radius"], float)[target]
+    u = d / np.linalg.norm(d, axis=1, keepdims=True)
+    x = np.cross(o - c, u)                              # dist(centre, line) without the cancellation of |oc|^2 - hb^2
+    disc = r * r - (x * x).sum(1)
+    rmax = max(float(np.abs(np.asarray(arrays["radius"], float)[info["small"]]).max()), 1e-3)
+    sigma = SIGMA_PER_LEN * rmax * np.abs(o).sum(1)
+    return dict(disc=disc, tensor=np.full(len(o), TENSOR_SLACK * info["R"] ** 2),
+                fp32=FP32_SLACK * ((c * c).sum(1) + r * r + info["R"] ** 2) + sigma)
+
+
+def band_coverage(arrays, o, d, target):
+    """how many rays fall inside each band (0 < disc <= band), and inside its first 1 %"""
+    b = silhouette_bands(arrays, o, d, target)
+    pos = b["disc"] > 0
+    return {f"{k}{tag}": int((pos & (b["disc"] <= f * b[k])).sum()) for k in ("tensor", "fp32") for tag, f in (("", 1.0), ("_1%", 0.01))}
+
+
+def assert_band_coverage(arrays, o, d, target, need=300, need_edge=50):
+    """a weak ray set fails here instead of passing vacuously"""
+    cov = band_coverage(arrays, o, d, target)
+    assert cov["tensor"] >= need and cov["fp32"] >= need, cov
+    assert cov["tensor_1%"] >= need_edge and cov["fp32_1%"] >= need_edge, cov
+    return cov
 
 
 # rays along the row of spheres that overflows the candidate lists, for the scenes that have one

@@ -16,6 +16,7 @@ import numpy as np
 import pytest
 
 import scan_scenes
+from test_parity_unit_gpu import f32_scene
 
 f16, f32 = np.float16, np.float32
 
@@ -55,8 +56,9 @@ def ray_rows(f, d, live, sigma, sc):
     return row1, row2
 
 
-def sphere_image(center, radius, npad, R_scene, sc):
-    """capi.cu: the 11 sphere features (f64 -> f32 -> fp16 hi/lo) in the two K = 16 blocks, padding entries never pass"""
+def sphere_image(center, radius, npad, R_scene, sc, bypass=False):
+    """capi.cu: the 11 sphere features (f64 -> f32 -> fp16 hi/lo) in the two K = 16 blocks, padding entries never pass.
+    bypass (rtiow_ctx_set_filter_bypass): every real column is S_0 = Rp^2 / s0, S_10 = -1 / s10 and zeros, and passes every ray"""
     s0, s1, s4, s10 = sc
     Rp = 2.0 ** np.ceil(np.log2(R_scene))
     slack = 1.5625e-5 * R_scene * R_scene
@@ -69,6 +71,9 @@ def sphere_image(center, radius, npad, R_scene, sc):
     S[:n, 7] = c[:, 0] * c[:, 1] / s4; S[:n, 8] = c[:, 0] * c[:, 2] / s4; S[:n, 9] = c[:, 1] * c[:, 2] / s4
     S[n:, 0] = -2.0 * Rp * Rp / s0      # padding: D = -2 Rp^2 - |f|^2 (+ sigma), |D| <= 2 Rp^2 + R^2 < 65504 wherever d_fits holds
     S[:, 10] = 1.0 / s10
+    if bypass:
+        S[:n] = 0.0
+        S[:n, 0] = Rp * Rp / s0; S[:n, 10] = -1.0 / s10
     hi, lo = split(S.astype(f32))
     assert not lo[:, 10].any(), "S_10 is a power of two: the two-product form relies on its lo part being zero"
     B = np.zeros((2, npad, 16), f16)
@@ -110,20 +115,22 @@ def test_d16_column_inverts_the_packed_sign_order():
         assert 8 * b + j == 31 - k
 
 
-def restate(c, r, o, d):
+def restate(c, r, o, d, bypass=False):
     """the filter of closest_hit_umma on the small spheres (c, r) and unit rays (o, d), all f32 values:
-    -> D [rays, npad] (the contraction, f64 copy), the f64 discriminant [rays, ns], live rows, slack, R"""
-    R_scene = float((np.linalg.norm(c, axis=1) + np.abs(r)).max())
+    -> D [rays, npad] (the contraction, f64 copy), the f64 discriminant [rays, ns], live rows, slack, R.
+    With bypass the image is rtiow_ctx_set_filter_bypass's and the rows carry the device's per-ray sigma."""
+    R_scene = max(1.0, float((np.linalg.norm(c, axis=1) + np.abs(r)).max()))
     Rp = 2.0 ** np.ceil(np.log2(R_scene))
     sc = (Rp, 1.0, Rp * 0.5, 1.0 / Rp)                                        # umma::FeatScale {s0, s1, s4, s10}
     npad = -(-len(c) // 64) * 64
-    B, slack = sphere_image(c, r, npad, R_scene, sc)
+    B, slack = sphere_image(c, r, npad, R_scene, sc, bypass)
     # line_gate (rt_scene.cuh): foot point of the coordinate origin (orthogonalised twice), liveness against the bounding sphere
     a = (d * d).sum(1)
     f = o - d * ((o * d).sum(1) / a)[:, None]
     f = f - d * ((f * d).sum(1) / a)[:, None]
-    live = (f * f).sum(1) < R_scene * R_scene * (1 + 1e-6)
-    row1, row2 = ray_rows(f, d, live, 0.0, sc)
+    sigma = scan_scenes.SIGMA_PER_LEN * max(float(np.abs(r).max()), 1e-3) * np.abs(o).sum(1) if bypass else 0.0
+    live = (f * f).sum(1) < R_scene * R_scene * (1 + 1e-6) + sigma
+    row1, row2 = ray_rows(f, d, live, sigma, sc)
     D = contraction(row1, row2, B).astype(np.float64)
     oc = c[None, :, :].astype(f32).astype(np.float64) - o[:, None, :]
     hb = (oc * d[:, None, :]).sum(2)
@@ -168,25 +175,84 @@ def test_contraction_reproduces_the_discriminant_and_never_drops_a_hit(capi):
     assert np.isfinite(D).all() and 4 * R_scene * R_scene < 60000
 
 
+def _unit_f32(d):
+    return (d / np.linalg.norm(d, axis=1, keepdims=True)).astype(f32).astype(np.float64)
+
+
+def _chunks(o, d, n=2048):
+    for s in range(0, len(o), n):
+        yield o[s:s + n], d[s:s + n]
+
+
+def _boundary_scene(capi, name):
+    arrays = scan_scenes.sparse_ball(122.4) if name == "ball-R122.4" else scan_scenes.build(name, capi)
+    info = scan_scenes.scene_info(arrays)
+    assert info["failing"] == [], info["failing"]
+    return arrays, info
+
+
+def test_contraction_drops_no_hit_at_silhouettes(capi):
+    """the final scene's rays grazing sphere silhouettes (scan_scenes.silhouette_rays), inside the band where the split and the
+    fp16 accumulation decide: nothing with discriminant >= 0 is dropped, and the contraction tracks disc + slack there too"""
+    scene = f32_scene(capi.random_scene(1))
+    small = np.abs(scene["radius"]) <= 8.0
+    c, r = scene["center"][small], scene["radius"][small]
+    o, d, target = scan_scenes.silhouette_rays(scene)
+    scan_scenes.assert_band_coverage(scene, o, d, target)
+    d = _unit_f32(d)
+    for oo, dd in _chunks(o, d):
+        D, disc, live, slack, _ = restate(c, r, oo, dd)
+        hit = disc >= 0
+        assert not (hit & live[:, None] & (D[:, :len(c)] < 0)).any(), "the filter dropped a sphere whose discriminant is >= 0"
+        assert not (hit & ~live[:, None]).any(), "a line the gate calls dead meets a sphere"
+        want = disc[live] + slack * (dd * dd).sum(1)[live, None]
+        near = np.abs(want) < 0.05
+        assert np.abs(D[live][:, :len(c)] - want)[near].max() < 0.25 * slack
+        assert np.isfinite(D).all()
+
+
 @pytest.mark.parametrize("name", ["ball-R122.4", "compact-3137", "row-r0.4"])
 def test_contraction_at_the_selection_boundaries(capi, name):
     """the scenes at the edges of the tensor filter's rules (tests/scan_scenes.py): R just under 122.47 (Rp = 128, 4 R^2 just
     under 60000, padding columns past the last word of small spheres), the largest image (npad 3200, 63 padding columns), and
-    the slack just below the mean r^2.  No sphere with discriminant >= 0 is dropped, every column of every ray stays finite
-    in fp16, and the padding columns stay negative."""
-    arrays = scan_scenes.sparse_ball(122.4) if name == "ball-R122.4" else scan_scenes.build(name, capi)
-    info = scan_scenes.scene_info(arrays)
-    assert info["failing"] == [], info["failing"]
+    the slack just below the mean r^2, on scan_scenes.rays and the silhouette rays.  No sphere with discriminant >= 0 is
+    dropped, every column of every ray stays finite in fp16, and the padding columns stay negative."""
+    arrays, info = _boundary_scene(capi, name)
     k = info["small"]
     c, r = arrays["center"][k], arrays["radius"][k]
     o, d = scan_scenes.rays(name, arrays)
-    d = (d / np.linalg.norm(d, axis=1, keepdims=True)).astype(f32).astype(np.float64)
-    D, disc, live, _, _ = restate(c, r, o, d)
+    o2, d2, _ = scan_scenes.silhouette_rays(arrays)
+    o, d = np.concatenate([o, o2]), _unit_f32(np.concatenate([d, d2]))
     ns = len(c)
-    assert live.mean() > 0.5
-    assert not ((disc >= 0) & live[:, None] & (D[:, :ns] < 0)).any(), "the filter dropped a sphere whose discriminant is >= 0"
-    assert np.isfinite(D[:, :ns]).all()
-    pad = D[:, ns:]
-    assert pad.shape[1] == info["npad"] - ns > 0
-    assert np.isfinite(pad).all(), f"{(~np.isfinite(pad)).sum()} padding entries overflow fp16"
-    assert (pad < 0).all()
+    n_live = 0
+    for oo, dd in _chunks(o, d):
+        D, disc, live, _, _ = restate(c, r, oo, dd)
+        n_live += live.sum()
+        assert not ((disc >= 0) & live[:, None] & (D[:, :ns] < 0)).any(), "the filter dropped a sphere whose discriminant is >= 0"
+        assert np.isfinite(D[:, :ns]).all()
+        pad = D[:, ns:]
+        assert pad.shape[1] == info["npad"] - ns > 0
+        assert np.isfinite(pad).all(), f"{(~np.isfinite(pad)).sum()} padding entries overflow fp16"
+        assert (pad < 0).all()
+    assert n_live > 0.5 * len(o)
+
+
+@pytest.mark.parametrize("name", ["ball-R122.4", "compact-3137"])
+def test_bypass_image_passes_every_sphere(capi, name):
+    """rtiow_ctx_set_filter_bypass's tensor image: every real column passes (sign bit clear) on live and dead rows alike, no
+    padding column ever passes, and every entry is finite in fp16 — at Rp = 128 (the largest |D|) and with 63 padding columns"""
+    arrays, info = _boundary_scene(capi, name)
+    k = info["small"]
+    c, r = arrays["center"][k], arrays["radius"][k]
+    o, d = scan_scenes.rays(name, arrays)
+    o2, d2, _ = scan_scenes.silhouette_rays(arrays)
+    o, d = np.concatenate([o, o2]), _unit_f32(np.concatenate([d, d2]))
+    ns = len(c)
+    n_live = n_dead = 0
+    for oo, dd in _chunks(o, d):
+        D, _, live, _, _ = restate(c, r, oo, dd, bypass=True)
+        n_live += live.sum(); n_dead += (~live).sum()
+        assert np.isfinite(D).all()
+        assert not np.signbit(D[:, :ns]).any(), f"{np.signbit(D[:, :ns]).sum()} real columns do not pass"
+        assert np.signbit(D[:, ns:]).all() and info["npad"] > ns
+    assert n_live > 1000 and n_dead > 100, (n_live, n_dead)
