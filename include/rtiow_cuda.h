@@ -169,6 +169,25 @@ void rtiow_params_default(rtiow_params* p);
  * buffer handed to ImageBuffer::from_vec at main.rs:147 — into caller-owned HOST memory. */
 int rtiow_render(rtiow_ctx* ctx, const rtiow_camera* cam, const rtiow_params* p, uint8_t* out_rgba, rtiow_stats* stats);
 
+/* A frame for a denoiser: out_rgba exactly as rtiow_render writes it (byte-identical, same rays_traced), plus float
+ * "arbitrary output variables" of the same frame.  Each float buffer is top-down, caller-owned HOST memory, and may be NULL
+ * (with all four NULL the call is rtiow_render):
+ *   out_color  [H][W][3]  mean linear radiance (before gamma): the frame's own 32.32 sums / spp.  Quantised with to_rgba
+ *                         (vec3.rs:404-420) at spp it gives out_rgba, up to float rounding next to a quantisation step.  A
+ *                         channel that saturated (spp > 65535) reads 2^32 / spp.
+ *   out_albedo [H][W][3]  mean over the spp samples of the camera ray's first hit: Lambertian / Metal albedo, Dielectric
+ *                         (1,1,1), a miss the sky value of that ray (main.rs:54-56).  Each sample is clamped to [0, 1].
+ *   out_normal [H][W][3]  mean over the spp samples of the normal HitRecord::new records at the first hit ((p - c) / r turned
+ *                         against the ray, mod.rs:20-30; a negative radius turns it inwards as the reference's does); a miss
+ *                         adds 0, so a partly covered pixel has a shorter mean normal.  Not renormalised.
+ *   out_depth  [H][W]     mean distance from the camera-ray origin to the first hit over the samples that hit; +inf when
+ *                         none did.  Each sample is clamped to [0, 65536] and kept to 2^-16.
+ * With max_depth <= 0 no camera ray is traced (main.rs:40-42): colour and albedo are 0, normal 0, depth +inf.
+ * The float buffers are bit-identical for any GPU count (integer sums).  An n-GPU ctx renders its row tiles as rtiow_render
+ * does.  A rank ctx with world > 1 returns RTIOW_ERR_UNSUPPORTED. */
+int rtiow_render_aov(rtiow_ctx* ctx, const rtiow_camera* cam, const rtiow_params* p, uint8_t* out_rgba, float* out_color,
+                     float* out_albedo, float* out_normal, float* out_depth, rtiow_stats* stats);
+
 /* Many views of one scene (turntables, animations, stereo pairs, camera sweeps) in one call: out_rgba receives n_views top-down
  * RGBA8 frames of 4*width*height bytes each, in view order, in caller-owned HOST memory.  Frame v equals
  * rtiow_render(ctx, &cams[v], p, ...) byte for byte, so the views share their sample streams (same seed, same pixel keys);

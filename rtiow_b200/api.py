@@ -108,6 +108,15 @@ def render(cam: capi.Camera, world: HittableList, params: capi.Params, n_gpus: i
     return img
 
 
+def render_aov(cam: capi.Camera, world: HittableList, params: capi.Params, n_gpus: int = 1):
+    """render() plus float AOVs for a denoiser -> (rgba[H,W,4], {"color", "albedo", "normal": [H,W,3], "depth": [H,W]} float32):
+    linear colour, and the albedo, normal and distance of each camera ray's first hit (include/rtiow_cuda.h, rtiow_render_aov)."""
+    with capi.Context(n_gpus) as ctx:
+        ctx.upload_scene(**world.to_arrays())
+        img, aovs, _ = ctx.render_aov(cam, params)
+    return img, aovs
+
+
 def render_views(cams, world: HittableList, params: capi.Params, n_gpus: int = 1):
     """Many cameras of one world in one call: [K,H,W,4] top-down RGBA8, frame v byte-identical to render(cams[v], ...)."""
     with capi.Context(n_gpus) as ctx:

@@ -95,6 +95,8 @@ struct DeviceState {
     HostBuf<uint8_t> pinned;                           // staging of the frame's D2H copy when the caller's buffer is pageable
     HostBuf<unsigned long long> pinned_cnt;            // the counters after the frame
     DevBuf<unsigned char> cams; HostBuf<unsigned char> cams_stage;   // the cameras of a batch of views (rtiow_render_views) and their staging
+    // rtiow_render_aov: the first-hit accumulators (AovArgs, rt_render.cuh) and the float buffers of finalize_aov_kernel
+    DevBuf<unsigned long long> aov_sum; DevBuf<unsigned int> aov_hits; DevBuf<float> aov_out;
     // measurement
     DevBuf<uint4> flush; DevBuf<float> probe;
     int last_backend = RTIOW_SCAN_FP32;                // which filter the last render launch used (rtiow_stats.scan_backend)
@@ -360,6 +362,7 @@ extern "C" void rtiow_ctx_destroy(rtiow_ctx* c)
         d.accum.release(); d.counters.release(); d.tiles.release(); d.gathered.release(); d.frame.release();
         d.flush.release(); d.probe.release();
         d.pinned.release(); d.pinned_cnt.release(); d.cams.release(); d.cams_stage.release();
+        d.aov_sum.release(); d.aov_hits.release(); d.aov_out.release();
         if (d.ev0) cudaEventDestroy(d.ev0);
         if (d.ev1) cudaEventDestroy(d.ev1);
         if (d.ev_done) cudaEventDestroy(d.ev_done);
@@ -745,9 +748,9 @@ template <typename T> static void size_fetch(RenderArgs<T>& a, int grid, int thr
     a.guided_div = (uint32_t)std::max<uint64_t>(1, 2 * n_warps);
 }
 
-// a persistent render kernel: as many CTAs as fit on the SMs at once.  `views` is empty for a frame and the device array of the
-// cameras for a batch of views (render_views_kernel)
-template <typename T, typename K, typename... V> static int launch_persistent(K kernel, RenderArgs<T>& a, int threads, size_t smem, int sms, cudaStream_t st, V... views)
+// a persistent render kernel: as many CTAs as fit on the SMs at once.  `extra` is the kernel's argument after RenderArgs, if any:
+// the device array of the cameras for a batch of views (render_views_kernel), the AOV accumulators (render_aov_kernel)
+template <typename T, typename K, typename... V> static int launch_persistent(K kernel, RenderArgs<T>& a, int threads, size_t smem, int sms, cudaStream_t st, V... extra)
 {
     int rc = allow_smem(kernel, smem); if (rc) return rc;
     int per_sm = 0;
@@ -755,44 +758,48 @@ template <typename T, typename K, typename... V> static int launch_persistent(K 
     if (per_sm < 1) return fail(RTIOW_ERR_CUDA, "kernel does not fit on an SM (smem %zu)", smem);
     const int grid = per_sm * sms;
     size_fetch(a, grid, threads);
-    kernel<<<grid, threads, smem, st>>>(a, views...);
+    kernel<<<grid, threads, smem, st>>>(a, extra...);
     return RTIOW_OK;
 }
 
-// the render kernel of one scan arm: a frame's, or with kViews a batch of views' (the same loop, rt_render.cuh)
-template <bool kViews, typename T, bool kSmem, int kThreads, int kMinCtas> static auto render_entry()
+// What a render launch produces, which picks the kernel of a scan arm (the same loop, rt_render.cuh): a frame, a batch of views,
+// or a frame with its first-hit AOVs
+enum class Loop { Frame, Views, Aov };
+template <Loop L, typename T, bool kSmem, int kThreads, int kMinCtas> static auto render_entry()
 {
-    if constexpr (kViews) return render_views_kernel<T, kSmem, kThreads, kMinCtas>;
+    if constexpr (L == Loop::Views) return render_views_kernel<T, kSmem, kThreads, kMinCtas>;
+    else if constexpr (L == Loop::Aov) return render_aov_kernel<T, kSmem, kThreads, kMinCtas>;
     else return render_kernel<T, kSmem, kThreads, kMinCtas>;
 }
-template <bool kViews> static auto render_entry_umma()
+template <Loop L> static auto render_entry_umma()
 {
-    if constexpr (kViews) return render_views_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
+    if constexpr (L == Loop::Views) return render_views_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
+    else if constexpr (L == Loop::Aov) return render_aov_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
     else return render_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
 }
 
-template <bool kViews, typename T, typename... V>
-static int launch_render_kernel(const ScanPlan& plan, const DeviceState& d, RenderArgs<T>& a, cudaStream_t st, V... views)
+template <Loop L, typename T, typename... V>
+static int launch_render_kernel(const ScanPlan& plan, const DeviceState& d, RenderArgs<T>& a, cudaStream_t st, V... extra)
 {
     if constexpr (std::is_same<T, double>::value) {
-        return launch_persistent(render_entry<kViews, double, false, 256, 2>(), a, 256, plan.smem(256), d.sms, st, views...);
+        return launch_persistent(render_entry<L, double, false, 256, 2>(), a, 256, plan.smem(256), d.sms, st, extra...);
     } else {
         switch (plan.scan) {
         case Scan::Tensor: {     // one CTA per SM (it owns all of TMEM), G groups of 128 rays + G issuer warps
-            auto k = render_entry_umma<kViews>();
+            auto k = render_entry_umma<L>();
             const size_t smem = plan.smem(UShape::kRenderThreads);
             int rc = allow_smem(k, smem); if (rc) return rc;
             size_fetch(a, d.sms, UShape::kRayThreads);          // the work is shared among the ray threads, not the whole block
-            k<<<d.sms, UShape::kRenderThreads, smem, st>>>(a, views...);
+            k<<<d.sms, UShape::kRenderThreads, smem, st>>>(a, extra...);
             return RTIOW_OK;
         }
         case Scan::Smem:         // 3 CTAs x 256 threads x 80 registers fills the 64K-register file
-            return launch_persistent(render_entry<kViews, float, true, 256, 3>(), a, 256, plan.smem(256), d.sms, st, views...);
+            return launch_persistent(render_entry<L, float, true, 256, 3>(), a, 256, plan.smem(256), d.sms, st, extra...);
         case Scan::Wide:         // one CTA per SM, 24 warps at 80 registers (+2.5 % over 512 threads at 104) when their lists fit
-            if (plan.smem(768) <= 227 * 1024) return launch_persistent(render_entry<kViews, float, true, 768, 1>(), a, 768, plan.smem(768), d.sms, st, views...);
-            return launch_persistent(render_entry<kViews, float, true, 512, 1>(), a, 512, plan.smem(512), d.sms, st, views...);
+            if (plan.smem(768) <= 227 * 1024) return launch_persistent(render_entry<L, float, true, 768, 1>(), a, 768, plan.smem(768), d.sms, st, extra...);
+            return launch_persistent(render_entry<L, float, true, 512, 1>(), a, 512, plan.smem(512), d.sms, st, extra...);
         case Scan::Global:
-            return launch_persistent(render_entry<kViews, float, false, 256, 4>(), a, 256, plan.smem(256), d.sms, st, views...);
+            return launch_persistent(render_entry<L, float, false, 256, 4>(), a, 256, plan.smem(256), d.sms, st, extra...);
         case Scan::F64:
             break;
         }
@@ -806,10 +813,12 @@ struct Dest { uint32_t* p; bool whole_frame; };
 
 // n_views = 0: a frame (or a rank's rows of one) of camera *cam.  n_views > 0 (world 1): a batch of views, the cameras
 // cam[0 .. n_views), rendered as one frame n_views * height rows tall whose epilogue writes the views' frames one after the other.
+// aov (n_views = 0): the launch also records every camera ray's first hit (render_aov_kernel) and a second epilogue turns the sums
+// into the float buffers of d.aov_out (finalize_aov_kernel), in this device's local row order.
 // *paths: the paths launched, local rows x width x samples.
 template <typename T>
 static int launch_render(const ScanPlan& plan, DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, uint32_t rank, uint32_t world, SampleRange sr,
-                         Dest dst, cudaStream_t st, uint32_t* launches, uint64_t* paths, uint32_t n_views)
+                         Dest dst, cudaStream_t st, uint32_t* launches, uint64_t* paths, uint32_t n_views, bool aov)
 {
     RenderArgs<T> a;
     a.scene = d.scene; a.cam = to_dev_camera<T>(*cam);
@@ -838,9 +847,14 @@ static int launch_render(const ScanPlan& plan, DeviceState& d, const rtiow_camer
         CameraT<T>* staged = reinterpret_cast<CameraT<T>*>(d.cams_stage.p);
         for (uint32_t v = 0; v < n_views; ++v) staged[v] = to_dev_camera<T>(cam[v]);
         CU(cudaMemcpyAsync(d.cams.p, staged, bytes, cudaMemcpyHostToDevice, st));
-        rc = launch_render_kernel<true>(plan, d, a, st, reinterpret_cast<const CameraT<T>*>(d.cams.p));
+        rc = launch_render_kernel<Loop::Views>(plan, d, a, st, reinterpret_cast<const CameraT<T>*>(d.cams.p));
+    } else if (aov) {
+        CU(d.aov_sum.resize(7 * n_lp)); CU(d.aov_hits.resize(n_lp)); CU(d.aov_out.resize(10 * n_lp));
+        CU(cudaMemsetAsync(d.aov_sum.p, 0, 7 * n_lp * sizeof(unsigned long long), st));
+        CU(cudaMemsetAsync(d.aov_hits.p, 0, n_lp * sizeof(unsigned int), st));
+        rc = launch_render_kernel<Loop::Aov>(plan, d, a, st, AovArgs{ d.aov_sum.p, d.aov_hits.p });
     } else {
-        rc = launch_render_kernel<false>(plan, d, a, st);
+        rc = launch_render_kernel<Loop::Frame>(plan, d, a, st);
     }
     if (rc) return rc;
     CU(cudaGetLastError());
@@ -850,6 +864,11 @@ static int launch_render(const ScanPlan& plan, DeviceState& d, const rtiow_camer
         finalize_kernel<<<(unsigned)((n_lp + 255) / 256), 256, 0, st>>>(d.accum.p, (uint32_t)n_lp, sr.begin + sr.count, p->alpha, dst.p);
     CU(cudaGetLastError());
     *launches += 2;
+    if (aov) {
+        finalize_aov_kernel<<<(unsigned)((n_lp + 255) / 256), 256, 0, st>>>(d.accum.p, d.aov_sum.p, d.aov_hits.p, (uint32_t)n_lp, sr.begin + sr.count, d.aov_out.p);
+        CU(cudaGetLastError());
+        ++*launches;
+    }
     return RTIOW_OK;
 }
 
@@ -879,9 +898,9 @@ struct Part {
 
 // One device's part of a frame: samples `sr` of the rows {y : (y / tile_rows) % world == rank}, quantised into `dst`, with the
 // events e0 / e1 around the work and its kernel launches added to *launches.  n_views > 0: the batch of views cam[0 .. n_views)
-// (launch_render).
+// (launch_render).  aov: the frame's first-hit AOVs too, left in d.aov_out (launch_render).
 static int render_step(const rtiow_ctx* c, DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, uint32_t rank, uint32_t world, SampleRange sr,
-                       Dest dst, cudaStream_t st, cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches, Part* part, uint32_t n_views = 0)
+                       Dest dst, cudaStream_t st, cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches, Part* part, uint32_t n_views = 0, bool aov = false)
 {
     if (!d.has_scene) return fail(RTIOW_ERR_INVALID_ARG, "no scene uploaded (call rtiow_scene_upload first)");
     CU(cudaSetDevice(d.device));
@@ -889,8 +908,8 @@ static int render_step(const rtiow_ctx* c, DeviceState& d, const rtiow_camera* c
     int rc = plan_scan(c, d, p->precision, &plan); if (rc) return rc;
     *part = Part{ &d, st, e0, e1 };
     CU(cudaEventRecord(e0, st));
-    rc = plan.scan == Scan::F64 ? launch_render<double>(plan, d, cam, p, rank, world, sr, dst, st, launches, &part->paths, n_views)
-                                : launch_render<float>(plan, d, cam, p, rank, world, sr, dst, st, launches, &part->paths, n_views);
+    rc = plan.scan == Scan::F64 ? launch_render<double>(plan, d, cam, p, rank, world, sr, dst, st, launches, &part->paths, n_views, aov)
+                                : launch_render<float>(plan, d, cam, p, rank, world, sr, dst, st, launches, &part->paths, n_views, aov);
     if (rc) return rc;
     CU(cudaEventRecord(e1, st));
     return RTIOW_OK;
@@ -898,10 +917,10 @@ static int render_step(const rtiow_ctx* c, DeviceState& d, const rtiow_camera* c
 
 // a frame on one device: its rank-local order IS top-down (and a batch of n_views views is their frames one after the other)
 static int render_single(const rtiow_ctx* c, DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, SampleRange sr, cudaStream_t st,
-                         cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches, Part* part, const uint32_t** d_frame, uint32_t n_views = 0)
+                         cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches, Part* part, const uint32_t** d_frame, uint32_t n_views = 0, bool aov = false)
 {
     CU(d.tiles.resize((size_t)p->width * p->height * std::max<uint32_t>(n_views, 1)));
-    int rc = render_step(c, d, cam, p, 0, 1, sr, Dest{ d.tiles.p, false }, st, e0, e1, launches, part, n_views); if (rc) return rc;
+    int rc = render_step(c, d, cam, p, 0, 1, sr, Dest{ d.tiles.p, false }, st, e0, e1, launches, part, n_views, aov); if (rc) return rc;
     *d_frame = d.tiles.p;
     return RTIOW_OK;
 }
@@ -997,9 +1016,53 @@ extern "C" int rtiow_deinterleave_device(rtiow_ctx* c, const void* d_gathered, c
     return deinterleave((const uint32_t*)d_gathered, p, (uint32_t)world, (uint32_t*)d_frame, stream ? (cudaStream_t)stream : d.stream);
 }
 
+// The host buffers of rtiow_render_aov; any may be NULL
+struct AovOut { float* color; float* albedo; float* normal; float* depth; };
+
+// Device `rank`'s rows of one float buffer of d.aov_out (`elems` floats per pixel, rank-local row order) into their top-down rows
+// of the caller's host buffer.  The rank's tiles rank, rank + world, ... sit equally spaced in the frame and back to back in
+// src, so one 2D copy moves every whole tile; the frame's last tile, which may be short, goes on its own.
+static int copy_aov_rows(float* dst, const float* src, uint32_t elems, const rtiow_params* p, uint32_t world, uint32_t rank, cudaStream_t st,
+                         uint64_t* bytes)
+{
+    const uint32_t tr = tile_rows_of(p), n_tiles = (p->height + tr - 1) / tr;
+    if (rank >= n_tiles) return RTIOW_OK;
+    const size_t row = (size_t)p->width * elems * sizeof(float), tile = tr * row;
+    const uint32_t mine = (n_tiles - 1 - rank) / world + 1, last_rows = p->height - (n_tiles - 1) * tr;
+    const uint32_t whole = mine - (rank + (mine - 1) * world == n_tiles - 1 && last_rows < tr ? 1u : 0u);
+    char* const d = reinterpret_cast<char*>(dst);
+    const char* const s = reinterpret_cast<const char*>(src);
+    if (world == 1 || whole == 1) {
+        if (whole) CU(cudaMemcpyAsync(d + rank * tile, s, whole * tile, cudaMemcpyDeviceToHost, st));
+    } else if (world * tile <= (size_t)INT32_MAX) {          // the largest pitch a 2D copy takes
+        if (whole) CU(cudaMemcpy2DAsync(d + rank * tile, world * tile, s, tile, tile, whole, cudaMemcpyDeviceToHost, st));
+    } else {
+        for (uint32_t k = 0; k < whole; ++k) CU(cudaMemcpyAsync(d + ((size_t)k * world + rank) * tile, s + k * tile, tile, cudaMemcpyDeviceToHost, st));
+    }
+    if (whole < mine) CU(cudaMemcpyAsync(d + (size_t)(n_tiles - 1) * tile, s + whole * tile, last_rows * row, cudaMemcpyDeviceToHost, st));
+    *bytes += (uint64_t)rows_of_rank(p->height, tr, world, rank) * row;
+    return RTIOW_OK;
+}
+
+// every requested AOV buffer of device `rank` (d.aov_out: colour, albedo, normal, depth of its n_lp local pixels) to the host
+static int copy_aovs(const DeviceState& d, const AovOut& aov, const rtiow_params* p, uint32_t world, uint32_t rank, uint64_t* bytes)
+{
+    const size_t n_lp = (size_t)rows_of_rank(p->height, tile_rows_of(p), world, rank) * p->width;
+    float* const dst[4] = { aov.color, aov.albedo, aov.normal, aov.depth };
+    CU(cudaSetDevice(d.device));
+    for (int b = 0; b < 4; ++b) {
+        if (!dst[b]) continue;
+        int rc = copy_aov_rows(dst[b], d.aov_out.p + 3 * b * n_lp, b < 3 ? 3u : 1u, p, world, rank, d.stream, bytes); if (rc) return rc;
+    }
+    return RTIOW_OK;
+}
+
 // THE drop-in call (main.rs:122-145)
-// One launch per device over the sample range `sr` + the quantise/gather epilogue + the frame to host memory.
-static int render_frame(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_params* p, SampleRange sr, uint8_t* out_rgba, rtiow_stats* stats)
+// One launch per device over the sample range `sr` + the quantise/gather epilogue + the frame to host memory.  aov (the whole
+// frame only, sr = {0, spp}): every device also records its camera rays' first hits and copies its rows of the requested float
+// buffers to their places in the caller's (copy_aovs).
+static int render_frame(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_params* p, SampleRange sr, uint8_t* out_rgba, rtiow_stats* stats,
+                        const AovOut* aov = nullptr)
 {
     int rc = RTIOW_OK;
     const double t0 = now_ms();
@@ -1012,7 +1075,7 @@ static int render_frame(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_param
     std::vector<Part> parts(world);
     const uint32_t* d_final = nullptr;
     if (world == 1) {
-        rc = render_single(c, d0, cam, p, sr, d0.stream, d0.ev0, d0.ev1, &launches, &parts[0], &d_final); if (rc) return rc;
+        rc = render_single(c, d0, cam, p, sr, d0.stream, d0.ev0, d0.ev1, &launches, &parts[0], &d_final, 0, aov != nullptr); if (rc) return rc;
     } else {
         // interleaved row tiles on every GPU.  Three gathers:
         //   fused (default with NVLink peer access, every B200 box): each rank's epilogue stores its pixels straight into device
@@ -1038,7 +1101,7 @@ static int render_frame(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_param
             Dest dst{ d0.frame.p, true };
             if (use_nccl) { CU(d.tiles.resize(tile_px)); CU(d.gathered.resize(tile_px * world)); dst = Dest{ d.tiles.p, false }; }
             else if (!fused) { if (r == 0) dst = Dest{ d0.gathered.p, false }; else { CU(d.tiles.resize(tile_px)); dst = Dest{ d.tiles.p, false }; } }
-            rc = render_step(c, d, cam, p, r, world, sr, dst, d.stream, d.ev0, d.ev1, &launches, &parts[r]); if (rc) return rc;
+            rc = render_step(c, d, cam, p, r, world, sr, dst, d.stream, d.ev0, d.ev1, &launches, &parts[r], 0, aov != nullptr); if (rc) return rc;
             if (r != 0 && !use_nccl) {
                 if (!fused) {
                     const size_t bytes = (size_t)rows_of_rank(p->height, tile_rows_of(p), world, r) * p->width * 4;
@@ -1068,8 +1131,12 @@ static int render_frame(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_param
         c->gather_note = note;
         d_final = d0.frame.p;
     }
+    uint64_t aov_bytes = 0;
+    if (aov)
+        for (uint32_t r = 0; r < world; ++r) { rc = copy_aovs(c->dev[r], *aov, p, world, r, &aov_bytes); if (rc) return rc; }
+    CU(cudaSetDevice(d0.device));
     rc = parts[0].start_copy(out_rgba, d_final, frame_bytes); if (rc) return rc;
-    return finish_call(parts.data(), world, t0, launches, world, kCallH2D, frame_bytes + 16, stats);
+    return finish_call(parts.data(), world, t0, launches, world, kCallH2D, frame_bytes + 16 + aov_bytes, stats);
 }
 
 extern "C" int rtiow_render(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_params* p, uint8_t* out_rgba, rtiow_stats* stats)
@@ -1077,6 +1144,22 @@ extern "C" int rtiow_render(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_p
     if (!c || !cam || !out_rgba) return fail(RTIOW_ERR_INVALID_ARG, "NULL argument");
     int rc = check_params(p); if (rc) return rc;
     return render_frame(c, cam, p, SampleRange{ 0u, p->spp }, out_rgba, stats);
+}
+
+// A frame exactly as rtiow_render renders it, plus the float buffers a denoiser takes: the frame's own sums as linear colour and
+// the first hit of every camera ray (rt_render.cuh, record_first_hit).  Only the render kernel (render_aov_kernel: the frame's
+// loop with kAov) and one more epilogue (finalize_aov_kernel) differ from rtiow_render; with every float buffer NULL the call
+// is rtiow_render.  An n-GPU ctx renders its interleaved row tiles as rtiow_render does and each device copies its rows of the
+// float buffers to their top-down places.
+extern "C" int rtiow_render_aov(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_params* p, uint8_t* out_rgba, float* out_color, float* out_albedo,
+                                float* out_normal, float* out_depth, rtiow_stats* stats)
+{
+    if (!c || !cam || !out_rgba) return fail(RTIOW_ERR_INVALID_ARG, "NULL argument");
+    int rc = check_params(p); if (rc) return rc;
+    if (c->world > 1) return fail(RTIOW_ERR_UNSUPPORTED, "rtiow_render_aov: a rank ctx with world > 1 renders collective frames (rtiow_render_rank), without AOVs");
+    const AovOut aov{ out_color, out_albedo, out_normal, out_depth };
+    const bool any = out_color || out_albedo || out_normal || out_depth;
+    return render_frame(c, cam, p, SampleRange{ 0u, p->spp }, out_rgba, stats, any ? &aov : nullptr);
 }
 
 // Many cameras of one scene (turntables, stereo pairs, camera sweeps) in one render launch per device: CTA start-up, the

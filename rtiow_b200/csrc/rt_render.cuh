@@ -38,6 +38,23 @@ template <typename T> struct RenderArgs {
 
 #define RT_FIX_SCALE 4294967296.0f   // 2^32
 
+// The first-hit accumulators of rtiow_render_aov (render_aov_kernel), beside RenderArgs::accum and over the same local pixels.
+// Every camera ray adds one fixed-point sample per channel with an integer RED.ADD, so the AOVs are bit-identical for any grid,
+// chunking or GPU count.  Each per-sample value is clamped to a range whose sum over 2^32 - 1 samples stays below 2^64, so no
+// sum can wrap at any spp and none needs add_saturating:
+//   albedo  [3][n_lp]  per sample in [0, 1] (the range a denoiser's albedo guide takes), scale 2^32;
+//   normal  [3][n_lp]  per sample n + 1 in [0, 2] (a unit normal, offset so that a sample is never negative), scale 2^31;
+//   depth   [n_lp]     per sample in [0, 65536] scene units, scale 2^16 (resolution 1.5e-5);
+//   hits    [n_lp]     camera rays that hit a sphere (32-bit: at most spp of them).
+// A miss adds its sky value to the albedo and nothing else, so finalize_aov_kernel removes the offset of the hits alone.
+struct AovArgs {
+    unsigned long long* sum;       // [7][n_lp]: albedo r, g, b, normal x, y, z, depth
+    unsigned int* hits;            // [n_lp]
+};
+#define RT_AOV_NORMAL_SCALE 2147483648.0   // 2^31
+#define RT_AOV_DEPTH_SCALE 65536.0         // 2^16
+#define RT_AOV_DEPTH_MAX 65536.0           // a farther hit is recorded at this distance
+
 // A sample's 32.32 value, clamped to [0, cap].  NaN/negative -> 0: a poisoned sample contributes nothing (the reference would
 // turn the whole pixel black through NaN -> `as u8` = 0, vec3.rs:415-417; the upload rejects non-finite materials, so only
 // an overflow to inf x 0 can make one).  cap = min(1e9, total spp) changes no byte: a sample of >= spp alone brings the
@@ -287,13 +304,52 @@ __device__ __forceinline__ bool next_ray(const RenderArgs<T>& a, const CameraT<T
     return active;
 }
 
-// Step 4 for one lane after the scan found (t_hit, idx, code); on a hit the lane moves to the hit point and keeps the
-// sphere in *hit_idx, *hit_code.  Returns whether a scatter is now pending.
+// a per-sample AOV value clamped to [0, hi] in fixed point (AovArgs); NaN -> 0
+__device__ __forceinline__ unsigned long long aov_fix(float v, float hi, float scale) { return __float2ull_rn(fminf(fmaxf(v, 0.0f), hi) * scale); }
+__device__ __forceinline__ unsigned long long aov_fix(double v, double hi, double scale) { return __double2ull_rn(fmin(fmax(v, 0.0), hi) * scale); }
+
+// The first hit of a camera ray into the AOV accumulators (AovArgs): the albedo of the material hit (Lambertian / Metal: its
+// albedo, Dielectric: 1) or the sky value on a miss (main.rs:54-56), and on a hit HitRecord::new's normal (hit_record) and
+// the distance t_hit (the ray's direction is unit: rt_render.cuh, start_ray).
 template <typename T>
-__device__ __forceinline__ bool take_hit(const RenderArgs<T>& a, PathState<T>& ps, bool active, uint32_t acc_lp, T t_hit, int idx, int code,
-                                         int* hit_idx, int* hit_code)
+__device__ __forceinline__ void record_first_hit(const RenderArgs<T>& a, const AovArgs& aov, const PathState<T>& ps, uint32_t acc_lp, T t_hit, int idx)
+{
+    const size_t n_lp = (size_t)a.local_rows * a.width;
+    unsigned long long* const sum = aov.sum + acc_lp;
+    V3<T> alb;
+    if (idx < 0) {
+        alb = sky<T, sizeof(T) == 4>(ps.dhat);
+    } else {
+        V3<T> cen; T rad;
+        if (sizeof(T) == 4) {
+            const float4 s = a.scene.sph[idx], m = a.scene.mat[idx];
+            cen = mk<T>(s.x, s.y, s.z); rad = s.w; alb = mk<T>(m.x, m.y, m.z);
+        } else {
+            const double4 s = a.scene.sphd[idx], m = a.scene.matd[idx];
+            cen = mk<T>(s.x, s.y, s.z); rad = s.w; alb = mk<T>(m.x, m.y, m.z);
+        }
+        if (a.scene.kind[idx] == MAT_DIELECTRIC) alb = mk<T>(1, 1, 1);
+        V3<T> n; bool ff; hit_record(ps.o + ps.dhat * t_hit, cen, rad, ps.dhat, &n, &ff);          // sphere.rs:36-39
+        atomicAdd(sum + 3 * n_lp, aov_fix(n.x + T(1), T(2), T(RT_AOV_NORMAL_SCALE)));
+        atomicAdd(sum + 4 * n_lp, aov_fix(n.y + T(1), T(2), T(RT_AOV_NORMAL_SCALE)));
+        atomicAdd(sum + 5 * n_lp, aov_fix(n.z + T(1), T(2), T(RT_AOV_NORMAL_SCALE)));
+        atomicAdd(sum + 6 * n_lp, aov_fix(t_hit, T(RT_AOV_DEPTH_MAX), T(RT_AOV_DEPTH_SCALE)));
+        atomicAdd(aov.hits + acc_lp, 1u);
+    }
+    atomicAdd(sum, aov_fix(alb.x, T(1), T(RT_FIX_SCALE)));
+    atomicAdd(sum + n_lp, aov_fix(alb.y, T(1), T(RT_FIX_SCALE)));
+    atomicAdd(sum + 2 * n_lp, aov_fix(alb.z, T(1), T(RT_FIX_SCALE)));
+}
+
+// Step 4 for one lane after the scan found (t_hit, idx, code); on a hit the lane moves to the hit point and keeps the
+// sphere in *hit_idx, *hit_code.  Returns whether a scatter is now pending.  kAov: a camera ray (depth still max_depth)
+// also records its first hit (record_first_hit).
+template <bool kAov, typename T>
+__device__ __forceinline__ bool take_hit(const RenderArgs<T>& a, const AovArgs& aov, PathState<T>& ps, bool active, uint32_t acc_lp, T t_hit, int idx,
+                                         int code, int* hit_idx, int* hit_code)
 {
     if (!active) return false;
+    if (kAov && ps.depth == a.max_depth) record_first_hit(a, aov, ps, acc_lp, t_hit, idx);
     if (idx < 0) { accumulate(a, acc_lp, ps.thr * sky<T, sizeof(T) == 4>(ps.dhat)); return false; }     // miss: sky (main.rs:54-56)
     ps.o = ps.o + ps.dhat * t_hit; *hit_idx = idx; *hit_code = code;                                    // ray.rs:15-17
     return true;
@@ -307,9 +363,10 @@ __device__ __forceinline__ bool take_hit(const RenderArgs<T>& a, PathState<T>& p
 //   3. the scan (world.hit) for all 32 lanes;
 //   4. miss -> throughput x sky is added to the pixel and the lane is free again; hit -> the lane keeps the hit for step 2.
 // Steps 2 and 4 are next_ray and take_hit, which the tensor-core kernel below calls too.  render_kernel renders a frame
-// (or a rank's rows of one); render_views_kernel runs the same loop over a batch of views, one camera per view in `cams`.
-template <typename T, bool kSmem, int kThreads, bool kViews>
-__device__ __forceinline__ void render_loop(const RenderArgs<T>& a, const CameraT<T>* cams)
+// (or a rank's rows of one); render_views_kernel runs the same loop over a batch of views, one camera per view in `cams`;
+// render_aov_kernel renders a frame and records every camera ray's first hit in `aov` (AovArgs).
+template <typename T, bool kSmem, int kThreads, bool kViews, bool kAov>
+__device__ __forceinline__ void render_loop(const RenderArgs<T>& a, const CameraT<T>* cams, const AovArgs& aov)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     uint16_t* cand;
@@ -333,7 +390,7 @@ __device__ __forceinline__ void render_loop(const RenderArgs<T>& a, const Camera
         n_rays_w += __popc(__ballot_sync(RT_FULL, active));          // world.hit call count (main.rs:44)
         T t_hit; int idx, code;
         world_hit<T, kSmem>(a.scene, table, cand, kThreads, ps, &t_hit, &idx, &code);
-        pending = take_hit(a, ps, active, acc_lp, t_hit, idx, code, &hit_idx, &hit_code);
+        pending = take_hit<kAov>(a, aov, ps, active, acc_lp, t_hit, idx, code, &hit_idx, &hit_code);
     }
     if (lane == 0) atomicAdd(a.ray_counter, (unsigned long long)n_rays_w);
 }
@@ -341,12 +398,17 @@ __device__ __forceinline__ void render_loop(const RenderArgs<T>& a, const Camera
 template <typename T, bool kSmem, int kThreads, int kMinCtas>
 __global__ void __launch_bounds__(kThreads, kMinCtas) render_kernel(const RenderArgs<T> a)
 {
-    render_loop<T, kSmem, kThreads, false>(a, nullptr);
+    render_loop<T, kSmem, kThreads, false, false>(a, nullptr, AovArgs{});
 }
 template <typename T, bool kSmem, int kThreads, int kMinCtas>
 __global__ void __launch_bounds__(kThreads, kMinCtas) render_views_kernel(const RenderArgs<T> a, const CameraT<T>* __restrict__ cams)
 {
-    render_loop<T, kSmem, kThreads, true>(a, cams);
+    render_loop<T, kSmem, kThreads, true, false>(a, cams, AovArgs{});
+}
+template <typename T, bool kSmem, int kThreads, int kMinCtas>
+__global__ void __launch_bounds__(kThreads, kMinCtas) render_aov_kernel(const RenderArgs<T> a, const AovArgs aov)
+{
+    render_loop<T, kSmem, kThreads, false, true>(a, nullptr, aov);
 }
 
 // The same render loop with the sphere filter on the tensor cores (rt_umma_scan.cuh): G groups of 128 ray threads + G
@@ -355,8 +417,8 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) render_views_kernel(const 
 // filter's survivors and the f64 large-sphere test; only the filter moves from 7 FFMA2 per sphere pair to three
 // tcgen05.mma per 128 rays x NC spheres, and the warp-level "any lane alive" vote becomes a 128-thread one, because a
 // group's 128 rays form one MMA.
-template <int G, int NC, bool kViews>
-__device__ __forceinline__ void render_loop_umma(const RenderArgs<float>& a, const CameraT<float>* cams)
+template <int G, int NC, bool kViews, bool kAov>
+__device__ __forceinline__ void render_loop_umma(const RenderArgs<float>& a, const CameraT<float>* cams, const AovArgs& aov)
 {
     extern __shared__ __align__(1024) unsigned char smem_umma[];
     uint32_t tmem_base;
@@ -389,7 +451,7 @@ __device__ __forceinline__ void render_loop_umma(const RenderArgs<float>& a, con
             RT_STAMP(4);
             const HitF h = closest_hit_umma<G, NC>(ux, a.scene, ps.o, ps.dhat, ps.tmin_n, ps.self_code, ps.self_n, active);
             RT_STAMP(9);
-            pending = take_hit(a, ps, active, acc_lp, h.t, h.idx, h.code, &hit_idx, &hit_code);
+            pending = take_hit<kAov>(a, aov, ps, active, acc_lp, h.t, h.idx, h.code, &hit_idx, &hit_code);
         }
         if (lane == 0) atomicAdd(a.ray_counter, (unsigned long long)n_rays_w);
     }
@@ -399,12 +461,17 @@ __device__ __forceinline__ void render_loop_umma(const RenderArgs<float>& a, con
 template <int G, int NC>
 __global__ void __launch_bounds__(UmmaShape<G, NC>::kRenderThreads, 1) render_kernel_umma(const RenderArgs<float> a)
 {
-    render_loop_umma<G, NC, false>(a, nullptr);
+    render_loop_umma<G, NC, false, false>(a, nullptr, AovArgs{});
 }
 template <int G, int NC>
 __global__ void __launch_bounds__(UmmaShape<G, NC>::kRenderThreads, 1) render_views_kernel_umma(const RenderArgs<float> a, const CameraT<float>* __restrict__ cams)
 {
-    render_loop_umma<G, NC, true>(a, cams);
+    render_loop_umma<G, NC, true, false>(a, cams, AovArgs{});
+}
+template <int G, int NC>
+__global__ void __launch_bounds__(UmmaShape<G, NC>::kRenderThreads, 1) render_aov_kernel_umma(const RenderArgs<float> a, const AovArgs aov)
+{
+    render_loop_umma<G, NC, false, true>(a, nullptr, aov);
 }
 
 // Color::to_rgba (vec3.rs:404-420) + the row flip (main.rs:141-145): fixed-point sums -> top-down
@@ -417,6 +484,26 @@ __global__ void finalize_kernel(const unsigned long long* __restrict__ accum, ui
     const double k = 1.0 / 4294967296.0;
     const V3<double> sum = mk<double>((double)accum[i] * k, (double)accum[n_lp + i] * k, (double)accum[2 * (size_t)n_lp + i] * k);
     out_rgba[i] = to_rgba<double>(sum, alpha, (uint64_t)spp);
+}
+
+// The float epilogue of rtiow_render_aov: the frame's sums and the AOV accumulators (AovArgs) -> per-pixel means in this
+// rank's local row order, each buffer [n_lp][3] (depth [n_lp]) one after the other in `out`: colour = sum / spp, albedo =
+// sum / spp, normal = (sum - hits x 2^31) / 2^31 / spp (exact in 64-bit integers: the hits' offsets come off before any
+// rounding, misses add 0), depth = sum / 2^16 / hits, or +inf when no camera ray of the pixel hit anything.
+__global__ void finalize_aov_kernel(const unsigned long long* __restrict__ accum, const unsigned long long* __restrict__ aov_sum,
+                                    const unsigned int* __restrict__ hits, uint32_t n_lp, uint32_t spp, float* __restrict__ out)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_lp) return;
+    const double inv_spp = 1.0 / (double)spp;
+    const uint32_t h = hits[i];
+    for (int c = 0; c < 3; ++c) {
+        out[3 * (size_t)i + c] = (float)((double)accum[c * (size_t)n_lp + i] * (inv_spp / 4294967296.0));
+        out[3 * ((size_t)n_lp + i) + c] = (float)((double)aov_sum[c * (size_t)n_lp + i] * (inv_spp / 4294967296.0));
+        const long long nrm = (long long)(aov_sum[(3 + c) * (size_t)n_lp + i] - ((unsigned long long)h << 31));
+        out[3 * (2 * (size_t)n_lp + i) + c] = (float)((double)nrm * (inv_spp / RT_AOV_NORMAL_SCALE));
+    }
+    out[9 * (size_t)n_lp + i] = h ? (float)((double)aov_sum[6 * (size_t)n_lp + i] / (RT_AOV_DEPTH_SCALE * h)) : __int_as_float(0x7f800000);
 }
 
 // The same epilogue FUSED with the gather (single-process multi-GPU): each rank's quantised pixel is stored straight

@@ -3,9 +3,11 @@
 // into flags (SURVEY §8f #3).  No preview window (main.rs:151-171 cannot run headless).
 //
 //   rtiow_host_example [--width W] [--height H] [--spp N] [--depth D] [--seed S] [--scene-seed S] [--gpus G]
-//                      [--grid HALF_EXTENT] [--materials 0..3] [--f64] [--passes N] [--views N] [--out image.png|image.ppm] [--selftest]
+//                      [--grid HALF_EXTENT] [--materials 0..3] [--f64] [--passes N] [--views N] [--aov] [--out image.png|image.ppm] [--selftest]
 // --views N renders N cameras orbiting the look-at point about the vertical axis in one call and writes out_000.png ...
 // (with --out, the frames are named after its stem: --out orbit.ppm writes orbit_000.ppm ...).
+// --aov also writes the inputs of a denoiser beside the image: <stem>_color.pfm (linear colour), <stem>_albedo.png and
+// <stem>_normal.png (0.5 n + 0.5).
 #include <algorithm>
 #include <chrono>
 #include <cstdlib>
@@ -91,6 +93,14 @@ static int selftest()
       }
       expect(same && std::equal(v.begin(), v.begin() + fb, a.begin()), "render_views: every view equals its own render() byte for byte");
       expect(sv.paths == 3ull * p.width * p.height * p.spp && sv.rays_traced == rays, "render_views stats: paths and rays of the batch"); }
+    // the frame with AOVs: out_rgba byte-identical to render()'s, the colour its own sums, albedo and normal in range
+    { Aovs av; rtiow_stats sa{};
+      std::vector<uint8_t> f = render_aov(cam, random_scene(1), p, &av, &sa);
+      const size_t n = size_t(p.width) * p.height;
+      expect(f == a && sa.rays_traced == st.rays_traced, "render_aov: the frame equals render()'s byte for byte");
+      bool sized = av.color.size() == 3 * n && av.albedo.size() == 3 * n && av.normal.size() == 3 * n && av.depth.size() == n, ranged = sized;
+      for (size_t i = 0; ranged && i < 3 * n; ++i) ranged = av.color[i] >= 0 && av.albedo[i] >= 0 && av.albedo[i] <= 1 && std::fabs(av.normal[i]) <= 1.0f + 1e-5f;
+      expect(ranged && std::isinf(av.depth[0]) && av.depth[n - 1] > 0 && av.depth[n - 1] < 100, "render_aov: buffers sized, in range, sky depth inf, ground depth finite"); }
     // the files below go to a private directory: a fixed name in the shared temporary directory may belong to another user
     std::string dir = (std::filesystem::temp_directory_path() / "rtiow_selftest_XXXXXX").string();
     if (!mkdtemp(dir.data())) { std::cerr << "FAIL: cannot create a temporary directory\nselftest FAILED\n"; return 1; }
@@ -111,7 +121,7 @@ int main(int argc, char** argv)
 {
     RenderParams p; p.width = 200; p.height = 133;                       // main.rs:24-28
     uint64_t scene_seed = 1; int grid = 11, materials = 0; std::string out = "image.png";     // main.rs:177
-    bool explicit_h = false, explicit_out = false; uint32_t passes = 0, views = 0; std::string scene_file, dump_scene;
+    bool explicit_h = false, explicit_out = false, aov = false; uint32_t passes = 0, views = 0; std::string scene_file, dump_scene;
     for (int i = 1; i < argc; ++i) {
         auto next = [&]() -> const char* { if (i + 1 >= argc) { std::cerr << "missing value for " << argv[i] << "\n"; std::exit(2); } return argv[++i]; };
         if (!std::strcmp(argv[i], "--width")) p.width = std::atoi(next());
@@ -126,6 +136,7 @@ int main(int argc, char** argv)
         else if (!std::strcmp(argv[i], "--f64")) p.f64 = true;
         else if (!std::strcmp(argv[i], "--passes")) passes = uint32_t(std::atoi(next()));
         else if (!std::strcmp(argv[i], "--views")) views = uint32_t(std::atoi(next()));
+        else if (!std::strcmp(argv[i], "--aov")) aov = true;
         else if (!std::strcmp(argv[i], "--out")) { out = next(); explicit_out = true; }
         else if (!std::strcmp(argv[i], "--scene")) scene_file = next();               // render the world of a scene file instead of random_scene
         else if (!std::strcmp(argv[i], "--dump-scene")) dump_scene = next();          // write the world to a scene file (for the oracle / a cargo build)
@@ -156,6 +167,19 @@ int main(int argc, char** argv)
                 if (!(ppm ? write_ppm(path, p.width, p.height, f) : write_png(path, p.width, p.height, f))) { std::cerr << "could not write " << path << "\n"; return 1; }
                 std::cout << path << " saved\n";
             }
+            return 0;
+        }
+        if (aov) {                                                        // the frame plus a denoiser's inputs
+            Aovs av;
+            std::vector<uint8_t> pixels = render_aov(cam, world, p, &av, &st);
+            std::cout << p.width << "x" << p.height << " @ " << p.spp << " spp with AOVs on " << st.n_gpus << " GPU(s): kernel " << st.kernel_ms << " ms\n";
+            const std::string stem = out.substr(0, out.rfind('.') == std::string::npos ? out.size() : out.rfind('.'));
+            const bool ok = (ppm ? write_ppm(out, p.width, p.height, pixels) : write_png(out, p.width, p.height, pixels)) &&
+                            write_pfm(stem + "_color.pfm", p.width, p.height, av.color) &&
+                            write_png(stem + "_albedo.png", p.width, p.height, unit_rgb_to_rgba(av.albedo)) &&
+                            write_png(stem + "_normal.png", p.width, p.height, unit_rgb_to_rgba(av.normal, 0.5f, 0.5f));
+            if (!ok) { std::cerr << "could not write " << out << " and its AOV files\n"; return 1; }
+            std::cout << out << ", " << stem << "_color.pfm, " << stem << "_albedo.png, " << stem << "_normal.png saved\n";
             return 0;
         }
         auto t0 = std::chrono::steady_clock::now();

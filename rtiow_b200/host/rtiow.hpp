@@ -11,6 +11,7 @@
 // reach the GPU through the defaulted describe() methods, and anything that does not describe
 // itself is RenderError::Unsupported — there is no CPU fallback.
 #pragma once
+#include <algorithm>
 #include <array>
 #include <cmath>
 #include <cstdint>
@@ -287,10 +288,14 @@ inline int progress_trampoline(void* user, uint32_t pass, uint32_t n_passes, uin
 }
 }  // namespace detail
 
+// The float buffers of render_aov(), top-down: color, albedo and normal hold 3 floats per pixel, depth one (include/rtiow_cuda.h,
+// rtiow_render_aov).
+struct Aovs { std::vector<float> color, albedo, normal, depth; };
+
 // The world as the GPU sees it + one render call; n_passes == 0: rtiow_render, else rtiow_render_progressive; with `views`:
-// rtiow_render_views of those cameras (cam is not used).
+// rtiow_render_views of those cameras (cam is not used); with `aovs`: rtiow_render_aov into them.
 inline std::vector<uint8_t> render_impl(const Camera& cam, const HittableList& world, const RenderParams& p, rtiow_stats* stats, uint32_t n_passes,
-                                        const ProgressFn* on_pass, const std::vector<Camera>* views = nullptr)
+                                        const ProgressFn* on_pass, const std::vector<Camera>* views = nullptr, Aovs* aovs = nullptr)
 {
     std::vector<double> cx, cy, cz, rad, ar, ag, ab, prm; std::vector<uint32_t> mi, kind;
     std::vector<const Scatter*> seen;
@@ -322,6 +327,10 @@ inline std::vector<uint8_t> render_impl(const Camera& cam, const HittableList& w
     if (views) {
         std::vector<rtiow_camera> raw; for (const Camera& v : *views) raw.push_back(v.raw());
         check(rtiow_render_views(ctx, raw.data(), uint32_t(raw.size()), &rp, out.data(), stats));
+    } else if (aovs) {
+        const size_t n = size_t(p.width) * p.height;
+        aovs->color.resize(3 * n); aovs->albedo.resize(3 * n); aovs->normal.resize(3 * n); aovs->depth.resize(n);
+        check(rtiow_render_aov(ctx, &cam.raw(), &rp, out.data(), aovs->color.data(), aovs->albedo.data(), aovs->normal.data(), aovs->depth.data(), stats));
     } else if (n_passes == 0) check(rtiow_render(ctx, &cam.raw(), &rp, out.data(), stats));
     else {
         detail::ProgressCtx pc{ on_pass, &out };
@@ -344,6 +353,14 @@ inline std::vector<uint8_t> render_views(const std::vector<Camera>& cams, const 
 {
     if (cams.empty()) throw RenderError(RTIOW_ERR_INVALID_ARG, "render_views needs at least one camera");
     return render_impl(cams.front(), world, p, stats, 0, nullptr, &cams);
+}
+
+// render_aov(): render()'s frame, byte for byte, plus the float buffers a denoiser takes in *aovs: linear colour, and the
+// albedo, normal and distance of each camera ray's first hit, averaged over the samples.
+inline std::vector<uint8_t> render_aov(const Camera& cam, const HittableList& world, const RenderParams& p, Aovs* aovs, rtiow_stats* stats = nullptr)
+{
+    if (!aovs) throw RenderError(RTIOW_ERR_INVALID_ARG, "render_aov needs an Aovs to fill");
+    return render_impl(cam, world, p, stats, 0, nullptr, nullptr, aovs);
 }
 
 // render_progressive(): the same frame in n_passes slices of the samples, with a preview after each — what the reference's
@@ -443,6 +460,22 @@ inline bool write_png(const std::string& path, uint32_t w, uint32_t h, const std
     FILE* f = std::fopen(path.c_str(), "wb"); if (!f) return false;
     std::fwrite(out.data(), 1, out.size(), f);
     return std::fclose(f) == 0;
+}
+// top-down float RGB (render_aov's colour) -> PFM ("PF", scale -1: little-endian floats, rows stored bottom-up)
+inline bool write_pfm(const std::string& path, uint32_t w, uint32_t h, const std::vector<float>& rgb)
+{
+    FILE* f = std::fopen(path.c_str(), "wb"); if (!f) return false;
+    std::fprintf(f, "PF\n%u %u\n-1.0\n", w, h);
+    for (uint32_t y = h; y-- > 0;) std::fwrite(&rgb[size_t(y) * w * 3], sizeof(float), size_t(w) * 3, f);
+    return std::fclose(f) == 0;
+}
+// float RGB in [0, 1] per channel (render_aov's albedo, or 0.5 n + 0.5 of its normal) -> RGBA8 for write_png
+inline std::vector<uint8_t> unit_rgb_to_rgba(const std::vector<float>& rgb, float scale = 1.0f, float offset = 0.0f)
+{
+    std::vector<uint8_t> out(rgb.size() / 3 * 4, 255);
+    for (size_t i = 0; i < rgb.size() / 3; ++i)
+        for (int c = 0; c < 3; ++c) out[4 * i + c] = uint8_t(std::lround(255.0f * std::min(1.0f, std::max(0.0f, scale * rgb[3 * i + c] + offset))));
+    return out;
 }
 
 }  // namespace rtiow

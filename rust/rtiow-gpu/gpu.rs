@@ -76,6 +76,29 @@ pub fn render_views(cams: &[Camera], world: &HittableList, p: &RenderParams) -> 
     }
 }
 
+/// The float buffers of `render_aov`, top-down: `color`, `albedo` and `normal` hold 3 floats per pixel, `depth` one.
+pub struct Aovs { pub color: Vec<f32>, pub albedo: Vec<f32>, pub normal: Vec<f32>, pub depth: Vec<f32> }
+
+/// `render`'s frame, byte for byte, plus the float buffers a denoiser takes: linear colour, and the albedo, normal and distance of
+/// each camera ray's first hit, averaged over the samples (include/rtiow_cuda.h, rtiow_render_aov).
+pub fn render_aov(cam: &Camera, world: &HittableList, p: &RenderParams) -> Result<(Vec<u8>, Aovs), RenderError> {
+    unsafe {
+        let mut raw: *mut sys::rtiow_ctx = ptr::null_mut();
+        let rc = sys::rtiow_ctx_create(p.n_gpus, &mut raw);
+        if rc != sys::RTIOW_OK { return Err(err(rc)); }
+        let ctx = Ctx(raw);
+        upload(&ctx, world)?;
+        let prm = raw_params(p);
+        let n = p.width as usize * p.height as usize;
+        let mut pixels = vec![0u8; 4 * n];
+        let mut a = Aovs { color: vec![0.0; 3 * n], albedo: vec![0.0; 3 * n], normal: vec![0.0; 3 * n], depth: vec![0.0; n] };
+        let rc = sys::rtiow_render_aov(ctx.0, &cam.raw(), &prm, pixels.as_mut_ptr(), a.color.as_mut_ptr(), a.albedo.as_mut_ptr(),
+                                       a.normal.as_mut_ptr(), a.depth.as_mut_ptr(), ptr::null_mut());
+        if rc != sys::RTIOW_OK { return Err(err(rc)); }
+        Ok((pixels, a))
+    }
+}
+
 /// The same frame in `n_passes` slices of the samples, with the frame so far handed to `on_pass(pass, n_passes, spp_done, rgba)`
 /// after each — the role of the indicatif bar (main.rs:120,124) and the piston preview window (main.rs:151-171).  The returned
 /// frame is bit-identical to `render`'s.  `on_pass` returning `true` stops the render: `Err(RenderError::Cancelled)`.
