@@ -188,6 +188,32 @@ int rtiow_render(rtiow_ctx* ctx, const rtiow_camera* cam, const rtiow_params* p,
 int rtiow_render_aov(rtiow_ctx* ctx, const rtiow_camera* cam, const rtiow_params* p, uint8_t* out_rgba, float* out_color,
                      float* out_albedo, float* out_normal, float* out_depth, rtiow_stats* stats);
 
+/* Adaptive sampling: each pixel gets as many samples as its own noise asks for, between min_spp and p->spp (the maximum).
+ *   Schedule   boundaries b_0 = min_spp, b_(k+1) = min(2 b_k, p->spp).  Round 0 renders samples [0, b_0) of every pixel;
+ *              round k >= 1 renders samples [b_(k-1), b_k) of the pixels still active.  (min_spp 16, spp 500: 16, 32, 64, 128,
+ *              256, 500.)
+ *   Noise      every sample that ends on the sky adds y = clamp((r + g + b) / 3, 0, 1) of its radiance, computed in the
+ *              render's precision, to two u64 per-pixel sums: S1 += round(y 2^32), S2 += round(y^2 2^32).  Black paths add
+ *              nothing, as they add nothing to the colour sums.
+ *   Error      at a boundary of n samples, in IEEE double, each operation rounded on its own: m = S1 2^-32 / n,
+ *              q = S2 2^-32 / n, err = 128 sqrt(max(0, q - m^2) / ((n - 1) max(m, 2^-16))), then rounded to float; +inf for
+ *              n = 1.  That is one standard error of the displayed value 256 sqrt(m) (to_rgba, vec3.rs:404-420) in 8-bit levels.
+ *   Rule       at boundary b_k a pixel stays active iff its (float) err > tolerance and b_k < p->spp.
+ *   Exactness  a pixel that stops at n samples has exactly the bytes rtiow_render gives it at spp = n: the samples are keyed by
+ *              (seed; pixel, sample, bounce) and summed as integers.  The per-sample clamp is min(1e9, p->spp) instead of
+ *              min(1e9, n), but a sample >= n brings the mean to >= 1 under either clamp, which quantises to 255.  (Per channel;
+ *              for n <= 65535 neither call saturates.)  With min_spp == p->spp the call is rtiow_render (same bytes and
+ *              rays_traced); with tolerance = +inf it is rtiow_render at spp = min_spp.
+ * Outputs (top-down, caller-owned HOST memory): out_rgba [H][W] RGBA8, each pixel quantised at its own count n_p; out_spp
+ * [H][W] n_p; out_error [H][W] err at the last boundary the pixel reached (the final boundary p->spp included).  out_spp and
+ * out_error may be NULL.  Stats: paths = sum of n_p; rays_traced, kernel_launches and d2h_bytes cover every round; kernel_ms is
+ * the rounds' and the epilogue's GPU time, without the host's gaps between rounds (one synchronisation per round), on the
+ * slowest device.  min_spp must be in [1, p->spp] and tolerance >= 0 (+inf allowed), else RTIOW_ERR_INVALID_ARG.  Every output
+ * is identical for any GPU count.  An n-GPU ctx renders its row tiles as rtiow_render does, each device running its own rounds.
+ * A rank ctx with world > 1 returns RTIOW_ERR_UNSUPPORTED. */
+int rtiow_render_adaptive(rtiow_ctx* ctx, const rtiow_camera* cam, const rtiow_params* p, uint32_t min_spp, double tolerance,
+                          uint8_t* out_rgba, uint32_t* out_spp, float* out_error, rtiow_stats* stats);
+
 /* Many views of one scene (turntables, animations, stereo pairs, camera sweeps) in one call: out_rgba receives n_views top-down
  * RGBA8 frames of 4*width*height bytes each, in view order, in caller-owned HOST memory.  Frame v equals
  * rtiow_render(ctx, &cams[v], p, ...) byte for byte, so the views share their sample streams (same seed, same pixel keys);

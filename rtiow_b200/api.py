@@ -117,6 +117,16 @@ def render_aov(cam: capi.Camera, world: HittableList, params: capi.Params, n_gpu
     return img, aovs
 
 
+def render_adaptive(cam: capi.Camera, world: HittableList, params: capi.Params, min_spp: int, tolerance: float, n_gpus: int = 1):
+    """Adaptive sampling: each pixel gets between min_spp and params.spp samples, as many as its own noise asks for, and equals
+    render() at its own count byte for byte -> (rgba[H,W,4], {"spp": uint32[H,W], "error": float32[H,W]}) (include/rtiow_cuda.h,
+    rtiow_render_adaptive: the error is one standard error of the displayed value in 8-bit levels, compared with tolerance)."""
+    with capi.Context(n_gpus) as ctx:
+        ctx.upload_scene(**world.to_arrays())
+        img, maps, _ = ctx.render_adaptive(cam, params, min_spp, tolerance)
+    return img, maps
+
+
 def render_views(cams, world: HittableList, params: capi.Params, n_gpus: int = 1):
     """Many cameras of one world in one call: [K,H,W,4] top-down RGBA8, frame v byte-identical to render(cams[v], ...)."""
     with capi.Context(n_gpus) as ctx:

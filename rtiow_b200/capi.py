@@ -30,7 +30,7 @@ PROGRESS_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint3
 SYMBOLS = [
     "rtiow_abi_version", "rtiow_last_error", "rtiow_device_count", "rtiow_ctx_create", "rtiow_ctx_create_on_device",
     "rtiow_ctx_destroy", "rtiow_ctx_set_scan_backend", "rtiow_ctx_set_filter_bypass", "rtiow_nccl_unique_id", "rtiow_ctx_create_rank", "rtiow_ctx_set_gather", "rtiow_ctx_set_stream",
-    "rtiow_ctx_gather_info", "rtiow_render_rank", "rtiow_render_rank_device", "rtiow_render_rank_enqueue", "rtiow_ctx_synchronize", "rtiow_scene_upload", "rtiow_camera_new", "rtiow_params_default", "rtiow_render", "rtiow_render_aov", "rtiow_render_views", "rtiow_render_progressive",
+    "rtiow_ctx_gather_info", "rtiow_render_rank", "rtiow_render_rank_device", "rtiow_render_rank_enqueue", "rtiow_ctx_synchronize", "rtiow_scene_upload", "rtiow_camera_new", "rtiow_params_default", "rtiow_render", "rtiow_render_aov", "rtiow_render_adaptive", "rtiow_render_views", "rtiow_render_progressive",
     "rtiow_tile_buffer_bytes", "rtiow_render_tiles_device", "rtiow_render_to_frame_device", "rtiow_deinterleave_device", "rtiow_sphere_hit_batch",
     "rtiow_hitlist_batch", "rtiow_scatter_batch", "rtiow_get_ray_batch", "rtiow_to_rgba_batch", "rtiow_reflect_batch",
     "rtiow_refract_batch", "rtiow_ray_color_batch", "rtiow_ray_color_trace_batch", "rtiow_sampler_batch", "rtiow_fp32_peak_probe", "rtiow_flush_l2",
@@ -121,6 +121,7 @@ def _declare(L):
         "rtiow_params_default": (None, [C.POINTER(Params)]),
         "rtiow_render": (C.c_int, [P, C.POINTER(Camera), C.POINTER(Params), P, C.POINTER(Stats)]),
         "rtiow_render_aov": (C.c_int, [P, C.POINTER(Camera), C.POINTER(Params), P, P, P, P, P, C.POINTER(Stats)]),
+        "rtiow_render_adaptive": (C.c_int, [P, C.POINTER(Camera), C.POINTER(Params), u32, d, P, P, P, C.POINTER(Stats)]),
         "rtiow_render_views": (C.c_int, [P, C.POINTER(Camera), C.c_uint32, C.POINTER(Params), P, C.POINTER(Stats)]),
         "rtiow_render_progressive": (C.c_int, [P, C.POINTER(Camera), C.POINTER(Params), C.c_uint32, PROGRESS_FN, P, P, C.POINTER(Stats)]),
         "rtiow_render_rank_enqueue": (C.c_int, [P, C.POINTER(Camera), C.POINTER(Params), C.POINTER(C.c_void_p)]),
@@ -389,6 +390,32 @@ class Context:
         ptrs = [_p(bufs[k]) if k in bufs else None for k in self.AOVS]
         _check(lib().rtiow_render_aov(self._h, C.byref(cam), C.byref(params), _p(out), *ptrs, C.byref(st)))
         return out.reshape(h, w, 4), bufs, st.as_dict()
+
+    def render_adaptive(self, cam: Camera, params: Params, min_spp: int, tolerance: float, out: np.ndarray | None = None, spp_map=True,
+                        error_map=True):
+        """rtiow_render_adaptive: per-pixel sample counts in [min_spp, params.spp] driven by each pixel's own noise, every pixel
+        byte-identical to render() at its own count -> (rgba[H,W,4] uint8, {"spp": uint32[H,W], "error": float32[H,W]}, stats).
+        spp_map / error_map are True (allocate), False / None (not returned: NULL, absent from the dict) or a C-contiguous array
+        of H*W uint32 / float32 that receives it.  Schedule, noise sums, error and rule are defined in include/rtiow_cuda.h."""
+        h, w = params.height, params.width
+        if out is None:
+            out = np.empty((h, w, 4), np.uint8)
+        if not isinstance(out, np.ndarray) or out.dtype != np.uint8 or out.size != h * w * 4 or not out.flags.c_contiguous:
+            raise ValueError(f"out must be a C-contiguous uint8 array with {h * w * 4} elements")
+        maps = {}
+        for name, arg, dt in (("spp", spp_map, np.uint32), ("error", error_map, np.float32)):
+            if arg is None or arg is False:
+                continue
+            if arg is True:
+                arg = np.empty((h, w), dt)
+            elif not isinstance(arg, np.ndarray) or arg.dtype != dt or arg.size != h * w or not arg.flags.c_contiguous:
+                raise ValueError(f"{name} must be a C-contiguous {np.dtype(dt).name} array with {h * w} elements")
+            maps[name] = arg.reshape(h, w)
+        st = Stats()
+        _check(lib().rtiow_render_adaptive(self._h, C.byref(cam), C.byref(params), min_spp, tolerance, _p(out),
+                                           _p(maps["spp"]) if "spp" in maps else None, _p(maps["error"]) if "error" in maps else None,
+                                           C.byref(st)))
+        return out.reshape(h, w, 4), maps, st.as_dict()
 
     def render_views(self, cams, params: Params, out=None):
         """rtiow_render_views: many cameras of the uploaded scene in one call -> (rgba[K,H,W,4] uint8, stats of the batch).

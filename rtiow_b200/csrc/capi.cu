@@ -97,6 +97,12 @@ struct DeviceState {
     DevBuf<unsigned char> cams; HostBuf<unsigned char> cams_stage;   // the cameras of a batch of views (rtiow_render_views) and their staging
     // rtiow_render_aov: the first-hit accumulators (AovArgs, rt_render.cuh) and the float buffers of finalize_aov_kernel
     DevBuf<unsigned long long> aov_sum; DevBuf<unsigned int> aov_hits; DevBuf<float> aov_out;
+    // rtiow_render_adaptive: the active pixels of this round and of the next ([2][n_lp]), the noise sums (AdaptArgs), each pixel's
+    // count and error, the select kernel's per-block counts, the next list's length (on the device and page-locked), and what the
+    // rounds of the call did here: their paths and their summed kernel time
+    DevBuf<uint32_t> adapt_list; DevBuf<unsigned long long> adapt_lum; DevBuf<uint32_t> adapt_spp; DevBuf<float> adapt_err;
+    DevBuf<uint32_t> adapt_blocks; DevBuf<uint32_t> adapt_n; HostBuf<uint32_t> adapt_n_host;
+    uint64_t adapt_paths = 0; float adapt_ms = 0;
     // measurement
     DevBuf<uint4> flush; DevBuf<float> probe;
     int last_backend = RTIOW_SCAN_FP32;                // which filter the last render launch used (rtiow_stats.scan_backend)
@@ -363,6 +369,8 @@ extern "C" void rtiow_ctx_destroy(rtiow_ctx* c)
         d.flush.release(); d.probe.release();
         d.pinned.release(); d.pinned_cnt.release(); d.cams.release(); d.cams_stage.release();
         d.aov_sum.release(); d.aov_hits.release(); d.aov_out.release();
+        d.adapt_list.release(); d.adapt_lum.release(); d.adapt_spp.release(); d.adapt_err.release(); d.adapt_blocks.release(); d.adapt_n.release();
+        d.adapt_n_host.release();
         if (d.ev0) cudaEventDestroy(d.ev0);
         if (d.ev1) cudaEventDestroy(d.ev1);
         if (d.ev_done) cudaEventDestroy(d.ev_done);
@@ -749,7 +757,8 @@ template <typename T> static void size_fetch(RenderArgs<T>& a, int grid, int thr
 }
 
 // a persistent render kernel: as many CTAs as fit on the SMs at once.  `extra` is the kernel's argument after RenderArgs, if any:
-// the device array of the cameras for a batch of views (render_views_kernel), the AOV accumulators (render_aov_kernel)
+// the device array of the cameras for a batch of views (render_views_kernel), the AOV accumulators (render_aov_kernel), the
+// round's pixel list and noise sums (render_adaptive_kernel)
 template <typename T, typename K, typename... V> static int launch_persistent(K kernel, RenderArgs<T>& a, int threads, size_t smem, int sms, cudaStream_t st, V... extra)
 {
     int rc = allow_smem(kernel, smem); if (rc) return rc;
@@ -763,18 +772,20 @@ template <typename T, typename K, typename... V> static int launch_persistent(K 
 }
 
 // What a render launch produces, which picks the kernel of a scan arm (the same loop, rt_render.cuh): a frame, a batch of views,
-// or a frame with its first-hit AOVs
-enum class Loop { Frame, Views, Aov };
+// a frame with its first-hit AOVs, or one round of an adaptive frame
+enum class Loop { Frame, Views, Aov, Adaptive };
 template <Loop L, typename T, bool kSmem, int kThreads, int kMinCtas> static auto render_entry()
 {
     if constexpr (L == Loop::Views) return render_views_kernel<T, kSmem, kThreads, kMinCtas>;
     else if constexpr (L == Loop::Aov) return render_aov_kernel<T, kSmem, kThreads, kMinCtas>;
+    else if constexpr (L == Loop::Adaptive) return render_adaptive_kernel<T, kSmem, kThreads, kMinCtas>;
     else return render_kernel<T, kSmem, kThreads, kMinCtas>;
 }
 template <Loop L> static auto render_entry_umma()
 {
     if constexpr (L == Loop::Views) return render_views_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
     else if constexpr (L == Loop::Aov) return render_aov_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
+    else if constexpr (L == Loop::Adaptive) return render_adaptive_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
     else return render_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
 }
 
@@ -811,6 +822,28 @@ static int launch_render_kernel(const ScanPlan& plan, const DeviceState& d, Rend
 // a whole frame that may live on another GPU (fused quantise + gather: finalize_to_frame_kernel)
 struct Dest { uint32_t* p; bool whole_frame; };
 
+// The arguments of a render launch over samples `sr` of `local_rows` rows (rank `rank` of `world`, or a batch of views) of
+// every pixel; d.accum must hold 3 x local_rows x width sums.
+template <typename T>
+static RenderArgs<T> render_args(const DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, uint32_t rank, uint32_t world, SampleRange sr,
+                                 uint32_t local_rows)
+{
+    RenderArgs<T> a;
+    a.scene = d.scene; a.cam = to_dev_camera<T>(*cam);
+    a.width = p->width; a.height = p->height; a.spp = sr.count; a.smp_begin = sr.begin; a.max_depth = p->max_depth; a.t_min = (T)p->t_min; a.key = philox_key(p->seed);
+    a.inv_wm1 = (T)(1.0 / (double)(p->width - 1)); a.inv_hm1 = (T)(1.0 / (double)(p->height - 1));
+    a.rank = rank; a.world = world; a.tile_rows = tile_rows_of(p);
+    a.local_rows = local_rows;
+    a.chunk_samples = std::min<uint32_t>(sr.count, 64u);
+    a.chunks_per_pixel = (sr.count + a.chunk_samples - 1) / a.chunk_samples;
+    a.chunks_per_fetch = std::max<uint32_t>(1u, 256u / a.chunk_samples);
+    a.n_chunks = (uint64_t)local_rows * p->width * a.chunks_per_pixel;
+    a.sample_cap = (T)std::min(1e9, (double)p->spp);        // the whole frame's spp: every pass of a progressive render adds the same
+    a.saturate = p->spp > 65535u;
+    a.accum = d.accum.p; a.work_counter = d.counters.p; a.ray_counter = d.counters.p + 1;
+    return a;
+}
+
 // n_views = 0: a frame (or a rank's rows of one) of camera *cam.  n_views > 0 (world 1): a batch of views, the cameras
 // cam[0 .. n_views), rendered as one frame n_views * height rows tall whose epilogue writes the views' frames one after the other.
 // aov (n_views = 0): the launch also records every camera ray's first hit (render_aov_kernel) and a second epilogue turns the sums
@@ -820,22 +853,11 @@ template <typename T>
 static int launch_render(const ScanPlan& plan, DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, uint32_t rank, uint32_t world, SampleRange sr,
                          Dest dst, cudaStream_t st, uint32_t* launches, uint64_t* paths, uint32_t n_views, bool aov)
 {
-    RenderArgs<T> a;
-    a.scene = d.scene; a.cam = to_dev_camera<T>(*cam);
-    a.width = p->width; a.height = p->height; a.spp = sr.count; a.smp_begin = sr.begin; a.max_depth = p->max_depth; a.t_min = (T)p->t_min; a.key = philox_key(p->seed);
-    a.inv_wm1 = (T)(1.0 / (double)(p->width - 1)); a.inv_hm1 = (T)(1.0 / (double)(p->height - 1));
-    a.rank = rank; a.world = world; a.tile_rows = tile_rows_of(p);
-    a.local_rows = n_views ? n_views * p->height : rows_of_rank(p->height, tile_rows_of(p), world, rank);
-    a.chunk_samples = std::min<uint32_t>(sr.count, 64u);
-    a.chunks_per_pixel = (sr.count + a.chunk_samples - 1) / a.chunk_samples;
-    a.chunks_per_fetch = std::max<uint32_t>(1u, 256u / a.chunk_samples);
-    const uint64_t n_lp = (uint64_t)a.local_rows * p->width;
-    a.n_chunks = n_lp * a.chunks_per_pixel;
-    a.sample_cap = (T)std::min(1e9, (double)p->spp);        // the whole frame's spp: every pass of a progressive render adds the same
-    a.saturate = p->spp > 65535u;
+    const uint32_t local_rows = n_views ? n_views * p->height : rows_of_rank(p->height, tile_rows_of(p), world, rank);
+    const uint64_t n_lp = (uint64_t)local_rows * p->width;
     *paths = n_lp * sr.count;
     CU(d.accum.resize(3 * n_lp));
-    a.accum = d.accum.p; a.work_counter = d.counters.p; a.ray_counter = d.counters.p + 1;
+    RenderArgs<T> a = render_args<T>(d, cam, p, rank, world, sr, local_rows);
     if (sr.begin == 0) CU(cudaMemsetAsync(d.accum.p, 0, 3 * n_lp * sizeof(unsigned long long), st));     // later passes add to the same sums
     CU(cudaMemsetAsync(d.counters.p, 0, 2 * sizeof(unsigned long long), st));
     if (n_lp == 0) return RTIOW_OK;
@@ -879,6 +901,7 @@ static int launch_render(const ScanPlan& plan, DeviceState& d, const rtiow_camer
 struct Part {
     DeviceState* d = nullptr; cudaStream_t st = nullptr; cudaEvent_t e0 = nullptr, e1 = nullptr;
     uint64_t paths = 0;
+    float ms_before = 0;         // kernel time of the call's earlier launches on this device, timed on their own (adaptive rounds)
     uint8_t* out = nullptr; const uint8_t* staged = nullptr; size_t copy_bytes = 0;
     int start_copy(uint8_t* dst, const uint32_t* d_frame, size_t n)
     {
@@ -896,11 +919,120 @@ struct Part {
     }
 };
 
+// ---- rtiow_render_adaptive ---------------------------------------------------------------------------------------------
+// One round on one device: samples `sr` of the n_act pixels of `list` (render_adaptive_kernel), then the select kernel, which
+// gives each of them its count sr.begin + sr.count and its error, and the compact kernel, which writes the pixels that stay
+// active to `next`, in order, and their number to d.adapt_n.  The ray counter is not reset: it adds up over the rounds.
+template <typename T>
+static int adaptive_round(const ScanPlan& plan, DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, uint32_t rank, uint32_t world, SampleRange sr,
+                          const uint32_t* list, uint32_t n_act, uint32_t* next, double tol, cudaStream_t st, uint32_t* launches)
+{
+    const uint32_t local_rows = rows_of_rank(p->height, tile_rows_of(p), world, rank);
+    const uint32_t n_lp = local_rows * p->width;
+    RenderArgs<T> a = render_args<T>(d, cam, p, rank, world, sr, local_rows);
+    a.n_chunks = (uint64_t)n_act * a.chunks_per_pixel;
+    CU(cudaMemsetAsync(d.counters.p, 0, sizeof(unsigned long long), st));           // the work counter only
+    int rc = launch_render_kernel<Loop::Adaptive>(plan, d, a, st, AdaptArgs{ list, d.adapt_lum.p }); if (rc) return rc;
+    CU(cudaGetLastError());
+    const uint32_t blocks = (n_act + RT_ADAPT_BLOCK - 1) / RT_ADAPT_BLOCK, n = sr.begin + sr.count;
+    adapt_select_kernel<<<blocks, RT_ADAPT_BLOCK, 0, st>>>(list, n_act, d.adapt_lum.p, n_lp, n, p->spp, tol, d.adapt_spp.p, d.adapt_err.p, d.adapt_blocks.p);
+    adapt_compact_kernel<<<blocks, RT_ADAPT_BLOCK, 0, st>>>(list, n_act, d.adapt_err.p, n, p->spp, tol, d.adapt_blocks.p, next, d.adapt_n.p);
+    CU(cudaGetLastError());
+    *launches += 3;
+    return RTIOW_OK;
+}
+
+// Every round of rtiow_render_adaptive on every device of the ctx, each over its own interleaved row tiles (the rule is per
+// pixel, so the devices need not agree on anything).  Round 0 renders samples [0, min_spp) of every pixel; round k renders
+// [b_(k-1), b_k) of the pixels still active, b_k = min(2 b_(k-1), spp).  After each round the host reads every device's
+// active count (4 bytes into page-locked memory, one synchronisation per round) and stops when none is left.  Leaves the
+// sums in d.accum, each pixel's count and error in d.adapt_spp / d.adapt_err, and the paths and summed kernel time (event pairs
+// per round, without the host's gaps between rounds) in d.adapt_paths / d.adapt_ms.
+static int adaptive_rounds(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_params* p, uint32_t min_spp, double tol, uint32_t* launches,
+                           uint64_t* d2h_bytes)
+{
+    const uint32_t world = (uint32_t)c->dev.size();
+    std::vector<ScanPlan> plans(world);
+    std::vector<uint32_t> n_act(world, 0), cur(world, 0);
+    for (uint32_t r = 0; r < world; ++r) {
+        DeviceState& d = c->dev[r];
+        if (!d.has_scene) return fail(RTIOW_ERR_INVALID_ARG, "no scene uploaded (call rtiow_scene_upload first)");
+        CU(cudaSetDevice(d.device));
+        int rc = plan_scan(c, d, p->precision, &plans[r]); if (rc) return rc;
+        const uint32_t n_lp = rows_of_rank(p->height, tile_rows_of(p), world, r) * p->width;
+        const uint32_t blocks = (n_lp + RT_ADAPT_BLOCK - 1) / RT_ADAPT_BLOCK;
+        CU(d.accum.resize(3 * (size_t)n_lp)); CU(d.adapt_lum.resize(2 * (size_t)n_lp)); CU(d.adapt_list.resize(2 * (size_t)n_lp));
+        CU(d.adapt_spp.resize(n_lp)); CU(d.adapt_err.resize(n_lp)); CU(d.adapt_blocks.resize(blocks)); CU(d.adapt_n.resize(1)); CU(d.adapt_n_host.resize(1));
+        CU(cudaMemsetAsync(d.counters.p, 0, 2 * sizeof(unsigned long long), d.stream));
+        CU(cudaMemsetAsync(d.accum.p, 0, 3 * (size_t)n_lp * sizeof(unsigned long long), d.stream));
+        CU(cudaMemsetAsync(d.adapt_lum.p, 0, 2 * (size_t)n_lp * sizeof(unsigned long long), d.stream));
+        d.adapt_paths = 0; d.adapt_ms = 0;
+        d.last_backend = plans[r].scan == Scan::Tensor ? RTIOW_SCAN_TENSOR : RTIOW_SCAN_FP32;
+        if (n_lp == 0) continue;                                    // more devices than row tiles
+        adapt_first_list_kernel<<<blocks, RT_ADAPT_BLOCK, 0, d.stream>>>(n_lp, d.adapt_list.p);
+        CU(cudaGetLastError());
+        ++*launches;
+        n_act[r] = n_lp;
+    }
+    for (SampleRange sr{ 0u, min_spp };;) {
+        for (uint32_t r = 0; r < world; ++r) {
+            if (!n_act[r]) continue;
+            DeviceState& d = c->dev[r];
+            CU(cudaSetDevice(d.device));
+            const size_t half = d.adapt_list.n / 2;                   // the buffer only grows: its halves hold >= n_lp pixels
+            const uint32_t* list = d.adapt_list.p + cur[r] * half;
+            uint32_t* next = d.adapt_list.p + (1 - cur[r]) * half;
+            CU(cudaEventRecord(d.ev0, d.stream));
+            int rc = plans[r].scan == Scan::F64 ? adaptive_round<double>(plans[r], d, cam, p, r, world, sr, list, n_act[r], next, tol, d.stream, launches)
+                                                : adaptive_round<float>(plans[r], d, cam, p, r, world, sr, list, n_act[r], next, tol, d.stream, launches);
+            if (rc) return rc;
+            CU(cudaEventRecord(d.ev1, d.stream));
+            CU(cudaMemcpyAsync(d.adapt_n_host.p, d.adapt_n.p, sizeof(uint32_t), cudaMemcpyDeviceToHost, d.stream));
+            d.adapt_paths += (uint64_t)n_act[r] * sr.count;
+            *d2h_bytes += sizeof(uint32_t);
+        }
+        bool any = false;
+        for (uint32_t r = 0; r < world; ++r) {
+            if (!n_act[r]) continue;
+            DeviceState& d = c->dev[r];
+            CU(cudaSetDevice(d.device));
+            CU(cudaStreamSynchronize(d.stream));
+            float ms = 0; CU(cudaEventElapsedTime(&ms, d.ev0, d.ev1));
+            d.adapt_ms += ms;
+            n_act[r] = *d.adapt_n_host.p; cur[r] ^= 1u;
+            any = any || n_act[r] > 0;
+        }
+        if (!any) return RTIOW_OK;                                   // the round that reaches spp keeps no pixel active
+        const uint32_t end = sr.begin + sr.count;
+        sr = SampleRange{ end, (uint32_t)std::min<uint64_t>(2ull * end, p->spp) - end };
+    }
+}
+
+// the epilogue of rtiow_render_adaptive on one device: its pixels quantised at their own counts (d.adapt_spp), into `dst` as
+// launch_render's epilogue stores a frame's.  *paths: the paths of the rounds.
+static int finalize_adaptive(DeviceState& d, const rtiow_params* p, uint32_t rank, uint32_t world, Dest dst, cudaStream_t st, uint32_t* launches,
+                             uint64_t* paths)
+{
+    const uint32_t n_lp = rows_of_rank(p->height, tile_rows_of(p), world, rank) * p->width;
+    *paths = d.adapt_paths;
+    if (n_lp == 0) return RTIOW_OK;
+    const unsigned blocks = (n_lp + 255) / 256;
+    if (dst.whole_frame)
+        finalize_adaptive_to_frame_kernel<<<blocks, 256, 0, st>>>(d.accum.p, n_lp, d.adapt_spp.p, p->alpha, p->width, tile_rows_of(p), world, rank, dst.p);
+    else
+        finalize_adaptive_kernel<<<blocks, 256, 0, st>>>(d.accum.p, n_lp, d.adapt_spp.p, p->alpha, dst.p);
+    CU(cudaGetLastError());
+    ++*launches;
+    return RTIOW_OK;
+}
+
 // One device's part of a frame: samples `sr` of the rows {y : (y / tile_rows) % world == rank}, quantised into `dst`, with the
 // events e0 / e1 around the work and its kernel launches added to *launches.  n_views > 0: the batch of views cam[0 .. n_views)
-// (launch_render).  aov: the frame's first-hit AOVs too, left in d.aov_out (launch_render).
+// (launch_render).  aov: the frame's first-hit AOVs too, left in d.aov_out (launch_render).  adaptive: the rounds of
+// rtiow_render_adaptive already ran (adaptive_rounds); only their epilogue is left (finalize_adaptive).
 static int render_step(const rtiow_ctx* c, DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, uint32_t rank, uint32_t world, SampleRange sr,
-                       Dest dst, cudaStream_t st, cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches, Part* part, uint32_t n_views = 0, bool aov = false)
+                       Dest dst, cudaStream_t st, cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches, Part* part, uint32_t n_views = 0, bool aov = false,
+                       bool adaptive = false)
 {
     if (!d.has_scene) return fail(RTIOW_ERR_INVALID_ARG, "no scene uploaded (call rtiow_scene_upload first)");
     CU(cudaSetDevice(d.device));
@@ -908,8 +1040,9 @@ static int render_step(const rtiow_ctx* c, DeviceState& d, const rtiow_camera* c
     int rc = plan_scan(c, d, p->precision, &plan); if (rc) return rc;
     *part = Part{ &d, st, e0, e1 };
     CU(cudaEventRecord(e0, st));
-    rc = plan.scan == Scan::F64 ? launch_render<double>(plan, d, cam, p, rank, world, sr, dst, st, launches, &part->paths, n_views, aov)
-                                : launch_render<float>(plan, d, cam, p, rank, world, sr, dst, st, launches, &part->paths, n_views, aov);
+    if (adaptive) { part->ms_before = d.adapt_ms; rc = finalize_adaptive(d, p, rank, world, dst, st, launches, &part->paths); }
+    else rc = plan.scan == Scan::F64 ? launch_render<double>(plan, d, cam, p, rank, world, sr, dst, st, launches, &part->paths, n_views, aov)
+                                     : launch_render<float>(plan, d, cam, p, rank, world, sr, dst, st, launches, &part->paths, n_views, aov);
     if (rc) return rc;
     CU(cudaEventRecord(e1, st));
     return RTIOW_OK;
@@ -917,10 +1050,11 @@ static int render_step(const rtiow_ctx* c, DeviceState& d, const rtiow_camera* c
 
 // a frame on one device: its rank-local order IS top-down (and a batch of n_views views is their frames one after the other)
 static int render_single(const rtiow_ctx* c, DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, SampleRange sr, cudaStream_t st,
-                         cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches, Part* part, const uint32_t** d_frame, uint32_t n_views = 0, bool aov = false)
+                         cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches, Part* part, const uint32_t** d_frame, uint32_t n_views = 0, bool aov = false,
+                         bool adaptive = false)
 {
     CU(d.tiles.resize((size_t)p->width * p->height * std::max<uint32_t>(n_views, 1)));
-    int rc = render_step(c, d, cam, p, 0, 1, sr, Dest{ d.tiles.p, false }, st, e0, e1, launches, part, n_views, aov); if (rc) return rc;
+    int rc = render_step(c, d, cam, p, 0, 1, sr, Dest{ d.tiles.p, false }, st, e0, e1, launches, part, n_views, aov, adaptive); if (rc) return rc;
     *d_frame = d.tiles.p;
     return RTIOW_OK;
 }
@@ -964,7 +1098,7 @@ static int finish_call(Part* parts, size_t n, double t0, uint32_t launches, uint
         CU(cudaStreamSynchronize(pt.st));
         if (pt.staged) memcpy(pt.out, pt.staged, pt.copy_bytes);
         float mp = 0; if (stats) CU(cudaEventElapsedTime(&mp, pt.e0, pt.e1));
-        ms = std::max(ms, mp); paths += pt.paths; rays += pt.d->pinned_cnt.p[1];          // the slowest device's kernels
+        ms = std::max(ms, pt.ms_before + mp); paths += pt.paths; rays += pt.d->pinned_cnt.p[1];          // the slowest device's kernels
     }
     CU(cudaSetDevice(parts[0].d->device));
     if (stats) *stats = make_stats(*parts[0].d, ms, now_ms() - t0, paths, rays, launches, n_gpus, h2d_bytes, d2h_bytes);
@@ -1019,15 +1153,17 @@ extern "C" int rtiow_deinterleave_device(rtiow_ctx* c, const void* d_gathered, c
 // The host buffers of rtiow_render_aov; any may be NULL
 struct AovOut { float* color; float* albedo; float* normal; float* depth; };
 
-// Device `rank`'s rows of one float buffer of d.aov_out (`elems` floats per pixel, rank-local row order) into their top-down rows
-// of the caller's host buffer.  The rank's tiles rank, rank + world, ... sit equally spaced in the frame and back to back in
-// src, so one 2D copy moves every whole tile; the frame's last tile, which may be short, goes on its own.
-static int copy_aov_rows(float* dst, const float* src, uint32_t elems, const rtiow_params* p, uint32_t world, uint32_t rank, cudaStream_t st,
-                         uint64_t* bytes)
+// Device `rank`'s rows of one per-pixel buffer (`elems` 4-byte values per pixel, rank-local row order: a float buffer of
+// d.aov_out, or rtiow_render_adaptive's counts or errors) into their top-down rows of the caller's host buffer.  The rank's tiles
+// rank, rank + world, ... sit equally spaced in the frame and back to back in src, so one 2D copy moves every whole tile; the
+// frame's last tile, which may be short, goes on its own.
+template <typename E>
+static int copy_aov_rows(E* dst, const E* src, uint32_t elems, const rtiow_params* p, uint32_t world, uint32_t rank, cudaStream_t st, uint64_t* bytes)
 {
+    static_assert(sizeof(E) == 4, "a per-pixel buffer of 4-byte values");
     const uint32_t tr = tile_rows_of(p), n_tiles = (p->height + tr - 1) / tr;
     if (rank >= n_tiles) return RTIOW_OK;
-    const size_t row = (size_t)p->width * elems * sizeof(float), tile = tr * row;
+    const size_t row = (size_t)p->width * elems * sizeof(E), tile = tr * row;
     const uint32_t mine = (n_tiles - 1 - rank) / world + 1, last_rows = p->height - (n_tiles - 1) * tr;
     const uint32_t whole = mine - (rank + (mine - 1) * world == n_tiles - 1 && last_rows < tr ? 1u : 0u);
     char* const d = reinterpret_cast<char*>(dst);
@@ -1057,12 +1193,17 @@ static int copy_aovs(const DeviceState& d, const AovOut& aov, const rtiow_params
     return RTIOW_OK;
 }
 
+// rtiow_render_adaptive's arguments beyond rtiow_render's; the host buffers may be NULL
+struct AdaptOut { uint32_t min_spp; double tolerance; uint32_t* spp; float* error; };
+
 // THE drop-in call (main.rs:122-145)
 // One launch per device over the sample range `sr` + the quantise/gather epilogue + the frame to host memory.  aov (the whole
 // frame only, sr = {0, spp}): every device also records its camera rays' first hits and copies its rows of the requested float
-// buffers to their places in the caller's (copy_aovs).
+// buffers to their places in the caller's (copy_aovs).  adapt (sr = {0, spp}): the rounds of rtiow_render_adaptive run first on
+// every device (adaptive_rounds), the epilogue quantises each pixel at its own count, and every device copies its rows of the
+// requested counts and errors to their places in the caller's buffers.
 static int render_frame(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_params* p, SampleRange sr, uint8_t* out_rgba, rtiow_stats* stats,
-                        const AovOut* aov = nullptr)
+                        const AovOut* aov = nullptr, const AdaptOut* adapt = nullptr)
 {
     int rc = RTIOW_OK;
     const double t0 = now_ms();
@@ -1071,11 +1212,13 @@ static int render_frame(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_param
     const size_t tile_px = (size_t)max_rows_per_rank(p->height, tile_rows_of(p), world) * p->width;
     DeviceState& d0 = c->dev[0];
     uint32_t launches = 0;
+    uint64_t extra_d2h = 0;
+    if (adapt) { rc = adaptive_rounds(c, cam, p, adapt->min_spp, adapt->tolerance, &launches, &extra_d2h); if (rc) return rc; }
     CU(cudaSetDevice(d0.device));
     std::vector<Part> parts(world);
     const uint32_t* d_final = nullptr;
     if (world == 1) {
-        rc = render_single(c, d0, cam, p, sr, d0.stream, d0.ev0, d0.ev1, &launches, &parts[0], &d_final, 0, aov != nullptr); if (rc) return rc;
+        rc = render_single(c, d0, cam, p, sr, d0.stream, d0.ev0, d0.ev1, &launches, &parts[0], &d_final, 0, aov != nullptr, adapt != nullptr); if (rc) return rc;
     } else {
         // interleaved row tiles on every GPU.  Three gathers:
         //   fused (default with NVLink peer access, every B200 box): each rank's epilogue stores its pixels straight into device
@@ -1101,7 +1244,7 @@ static int render_frame(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_param
             Dest dst{ d0.frame.p, true };
             if (use_nccl) { CU(d.tiles.resize(tile_px)); CU(d.gathered.resize(tile_px * world)); dst = Dest{ d.tiles.p, false }; }
             else if (!fused) { if (r == 0) dst = Dest{ d0.gathered.p, false }; else { CU(d.tiles.resize(tile_px)); dst = Dest{ d.tiles.p, false }; } }
-            rc = render_step(c, d, cam, p, r, world, sr, dst, d.stream, d.ev0, d.ev1, &launches, &parts[r], 0, aov != nullptr); if (rc) return rc;
+            rc = render_step(c, d, cam, p, r, world, sr, dst, d.stream, d.ev0, d.ev1, &launches, &parts[r], 0, aov != nullptr, adapt != nullptr); if (rc) return rc;
             if (r != 0 && !use_nccl) {
                 if (!fused) {
                     const size_t bytes = (size_t)rows_of_rank(p->height, tile_rows_of(p), world, r) * p->width * 4;
@@ -1131,12 +1274,18 @@ static int render_frame(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_param
         c->gather_note = note;
         d_final = d0.frame.p;
     }
-    uint64_t aov_bytes = 0;
     if (aov)
-        for (uint32_t r = 0; r < world; ++r) { rc = copy_aovs(c->dev[r], *aov, p, world, r, &aov_bytes); if (rc) return rc; }
+        for (uint32_t r = 0; r < world; ++r) { rc = copy_aovs(c->dev[r], *aov, p, world, r, &extra_d2h); if (rc) return rc; }
+    if (adapt)
+        for (uint32_t r = 0; r < world; ++r) {
+            const DeviceState& d = c->dev[r];
+            CU(cudaSetDevice(d.device));
+            if (adapt->spp) { rc = copy_aov_rows(adapt->spp, d.adapt_spp.p, 1, p, world, r, d.stream, &extra_d2h); if (rc) return rc; }
+            if (adapt->error) { rc = copy_aov_rows(adapt->error, d.adapt_err.p, 1, p, world, r, d.stream, &extra_d2h); if (rc) return rc; }
+        }
     CU(cudaSetDevice(d0.device));
     rc = parts[0].start_copy(out_rgba, d_final, frame_bytes); if (rc) return rc;
-    return finish_call(parts.data(), world, t0, launches, world, kCallH2D, frame_bytes + 16 + aov_bytes, stats);
+    return finish_call(parts.data(), world, t0, launches, world, kCallH2D, frame_bytes + 16 + extra_d2h, stats);
 }
 
 extern "C" int rtiow_render(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_params* p, uint8_t* out_rgba, rtiow_stats* stats)
@@ -1160,6 +1309,24 @@ extern "C" int rtiow_render_aov(rtiow_ctx* c, const rtiow_camera* cam, const rti
     const AovOut aov{ out_color, out_albedo, out_normal, out_depth };
     const bool any = out_color || out_albedo || out_normal || out_depth;
     return render_frame(c, cam, p, SampleRange{ 0u, p->spp }, out_rgba, stats, any ? &aov : nullptr);
+}
+
+// Per-pixel sample counts from each pixel's own noise (include/rtiow_cuda.h).  The rounds (adaptive_rounds) render sample ranges
+// of shrinking pixel lists into the frame's own 32.32 sums and are keyed by (seed; pixel, sample, bounce) like every other
+// call, so a pixel that stops at n samples holds exactly the sums rtiow_render(spp = n) gives it: the only difference is the
+// per-sample clamp sample_cap = min(1e9, spp) instead of min(1e9, n), and a sample >= n brings the mean to >= 1 under either
+// cap, which quantises to 255 (to_fix).  So each byte is rtiow_render's at the pixel's count.  An n-GPU ctx runs the rounds of
+// its interleaved row tiles on each device and gathers the frame as rtiow_render does.
+extern "C" int rtiow_render_adaptive(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_params* p, uint32_t min_spp, double tolerance, uint8_t* out_rgba,
+                                     uint32_t* out_spp, float* out_error, rtiow_stats* stats)
+{
+    if (!c || !cam || !out_rgba) return fail(RTIOW_ERR_INVALID_ARG, "NULL argument");
+    int rc = check_params(p); if (rc) return rc;
+    if (min_spp < 1 || min_spp > p->spp) return fail(RTIOW_ERR_INVALID_ARG, "min_spp must be in [1, spp]");
+    if (!(tolerance >= 0.0)) return fail(RTIOW_ERR_INVALID_ARG, "tolerance must be >= 0 (not NaN)");
+    if (c->world > 1) return fail(RTIOW_ERR_UNSUPPORTED, "rtiow_render_adaptive: a rank ctx with world > 1 renders collective frames (rtiow_render_rank), not adaptive ones");
+    const AdaptOut adapt{ min_spp, tolerance, out_spp, out_error };
+    return render_frame(c, cam, p, SampleRange{ 0u, p->spp }, out_rgba, stats, nullptr, &adapt);
 }
 
 // Many cameras of one scene (turntables, stereo pairs, camera sweeps) in one render launch per device: CTA start-up, the

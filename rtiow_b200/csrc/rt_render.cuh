@@ -55,6 +55,15 @@ struct AovArgs {
 #define RT_AOV_DEPTH_SCALE 65536.0         // 2^16
 #define RT_AOV_DEPTH_MAX 65536.0           // a farther hit is recorded at this distance
 
+// One round of rtiow_render_adaptive (render_adaptive_kernel): the launch renders its sample range of the pixels in `list`
+// only (local pixel indices, n_chunks / chunks_per_pixel of them), and every finished non-black path also adds its noise value
+// y = clamp((r + g + b) / 3, 0, 1) to two per-pixel fixed-point sums, S1 += round(y 2^32) and S2 += round(y^2 2^32).  Each
+// value is at most 2^32, so neither sum can wrap at any u32 spp.  The pixels' own radiance sums stay RenderArgs::accum.
+struct AdaptArgs {
+    const uint32_t* list;          // the round's active local pixels, in the frame's bottom-up drawing order
+    unsigned long long* lum_sum;   // [2][n_lp]: S1, S2
+};
+
 // A sample's 32.32 value, clamped to [0, cap].  NaN/negative -> 0: a poisoned sample contributes nothing (the reference would
 // turn the whole pixel black through NaN -> `as u8` = 0, vec3.rs:415-417; the upload rejects non-finite materials, so only
 // an overflow to inf x 0 can make one).  cap = min(1e9, total spp) changes no byte: a sample of >= spp alone brings the
@@ -200,9 +209,10 @@ struct WorkCursor {
 // kViews: the launch renders a batch of views (rtiow_render_views) on one device as ONE frame n_views * height rows tall, so
 // local row lr is row lr % height of view lr / height.  *pv receives the view; pj and the Philox pixel key are those of the
 // row within the view, exactly as the view's own frame computes them, which makes every view byte-identical to it.
-template <bool kViews, typename T>
-__device__ __forceinline__ bool assign_work(const RenderArgs<T>& a, WorkCursor& wc, unsigned lt_mask, bool busy, PathState<T>& ps, uint32_t& acc_lp,
-                                            uint32_t* px, uint32_t* pj, uint32_t* pv)
+// kAdapt: chunk c belongs to pixel ad.list[c / chunks_per_pixel] (AdaptArgs), a round's subset of the pixels in the same order.
+template <bool kViews, bool kAdapt, typename T>
+__device__ __forceinline__ bool assign_work(const RenderArgs<T>& a, const AdaptArgs& ad, WorkCursor& wc, unsigned lt_mask, bool busy, PathState<T>& ps,
+                                            uint32_t& acc_lp, uint32_t* px, uint32_t* pj, uint32_t* pv)
 {
     bool fresh = false;
     unsigned need = __ballot_sync(RT_FULL, !busy);
@@ -227,7 +237,7 @@ __device__ __forceinline__ bool assign_work(const RenderArgs<T>& a, WorkCursor& 
             const unsigned long long c = wc.cc++;
             const uint32_t pix = (uint32_t)(c / a.chunks_per_pixel);
             const uint32_t part = (uint32_t)(c - (unsigned long long)pix * a.chunks_per_pixel);
-            wc.c_lp = a.local_rows * a.width - 1u - pix;
+            wc.c_lp = kAdapt ? ad.list[pix] : a.local_rows * a.width - 1u - pix;
             wc.cs = part * a.chunk_samples; wc.ce = min(wc.cs + a.chunk_samples, a.spp);
             const uint32_t lr = wc.c_lp / a.width;
             wc.c_x = wc.c_lp - lr * a.width;
@@ -341,16 +351,36 @@ __device__ __forceinline__ void record_first_hit(const RenderArgs<T>& a, const A
     atomicAdd(sum + 2 * n_lp, aov_fix(alb.z, T(1), T(RT_FIX_SCALE)));
 }
 
+// A finished path's noise value into the sums of rtiow_render_adaptive (AdaptArgs): y = clamp((r + g + b) / 3, 0, 1) of its
+// radiance in the render's precision, S1 += round(y 2^32), S2 += round(y^2 2^32).  A black path adds nothing, as in accumulate.
+template <typename T>
+__device__ __forceinline__ void accumulate_noise(const RenderArgs<T>& a, const AdaptArgs& ad, uint32_t acc_lp, V3<T> rad)
+{
+    if (rad.x != T(0) || rad.y != T(0) || rad.z != T(0)) {
+        const size_t n_lp = (size_t)a.local_rows * a.width;
+        const T y = (rad.x + rad.y + rad.z) / T(3);
+        const T yc = y > T(0) ? (y < T(1) ? y : T(1)) : T(0);                  // NaN -> 0, as to_fix does
+        atomicAdd(ad.lum_sum + acc_lp, aov_fix(yc, T(1), T(RT_FIX_SCALE)));
+        atomicAdd(ad.lum_sum + n_lp + acc_lp, aov_fix(yc * yc, T(1), T(RT_FIX_SCALE)));
+    }
+}
+
 // Step 4 for one lane after the scan found (t_hit, idx, code); on a hit the lane moves to the hit point and keeps the
 // sphere in *hit_idx, *hit_code.  Returns whether a scatter is now pending.  kAov: a camera ray (depth still max_depth)
-// also records its first hit (record_first_hit).
-template <bool kAov, typename T>
-__device__ __forceinline__ bool take_hit(const RenderArgs<T>& a, const AovArgs& aov, PathState<T>& ps, bool active, uint32_t acc_lp, T t_hit, int idx,
-                                         int code, int* hit_idx, int* hit_code)
+// also records its first hit (record_first_hit).  kAdapt: a path that ends on the sky also adds its noise value
+// (accumulate_noise); paths that end black add nothing anywhere.
+template <bool kAov, bool kAdapt, typename T>
+__device__ __forceinline__ bool take_hit(const RenderArgs<T>& a, const AovArgs& aov, const AdaptArgs& ad, PathState<T>& ps, bool active, uint32_t acc_lp,
+                                         T t_hit, int idx, int code, int* hit_idx, int* hit_code)
 {
     if (!active) return false;
     if (kAov && ps.depth == a.max_depth) record_first_hit(a, aov, ps, acc_lp, t_hit, idx);
-    if (idx < 0) { accumulate(a, acc_lp, ps.thr * sky<T, sizeof(T) == 4>(ps.dhat)); return false; }     // miss: sky (main.rs:54-56)
+    if (idx < 0) {                                                                                        // miss: sky (main.rs:54-56)
+        const V3<T> rad = ps.thr * sky<T, sizeof(T) == 4>(ps.dhat);
+        accumulate(a, acc_lp, rad);
+        if (kAdapt) accumulate_noise(a, ad, acc_lp, rad);
+        return false;
+    }
     ps.o = ps.o + ps.dhat * t_hit; *hit_idx = idx; *hit_code = code;                                    // ray.rs:15-17
     return true;
 }
@@ -364,9 +394,10 @@ __device__ __forceinline__ bool take_hit(const RenderArgs<T>& a, const AovArgs& 
 //   4. miss -> throughput x sky is added to the pixel and the lane is free again; hit -> the lane keeps the hit for step 2.
 // Steps 2 and 4 are next_ray and take_hit, which the tensor-core kernel below calls too.  render_kernel renders a frame
 // (or a rank's rows of one); render_views_kernel runs the same loop over a batch of views, one camera per view in `cams`;
-// render_aov_kernel renders a frame and records every camera ray's first hit in `aov` (AovArgs).
-template <typename T, bool kSmem, int kThreads, bool kViews, bool kAov>
-__device__ __forceinline__ void render_loop(const RenderArgs<T>& a, const CameraT<T>* cams, const AovArgs& aov)
+// render_aov_kernel renders a frame and records every camera ray's first hit in `aov` (AovArgs); render_adaptive_kernel renders
+// one round of rtiow_render_adaptive: the pixels of `ad.list` only, with their noise sums (AdaptArgs).
+template <typename T, bool kSmem, int kThreads, bool kViews, bool kAov, bool kAdapt>
+__device__ __forceinline__ void render_loop(const RenderArgs<T>& a, const CameraT<T>* cams, const AovArgs& aov, const AdaptArgs& ad)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     uint16_t* cand;
@@ -383,14 +414,14 @@ __device__ __forceinline__ void render_loop(const RenderArgs<T>& a, const Camera
 
     for (;;) {
         uint32_t px = 0, pj = 0, pv = 0;
-        const bool fresh = assign_work<kViews>(a, wc, lt_mask, pending, ps, acc_lp, &px, &pj, &pv);
+        const bool fresh = assign_work<kViews, kAdapt>(a, ad, wc, lt_mask, pending, ps, acc_lp, &px, &pj, &pv);
         if (!__any_sync(RT_FULL, fresh || pending)) break;
 
         const bool active = next_ray<kViews>(a, cams, ps, fresh, pending, hit_idx, hit_code, px, pj, pv);
         n_rays_w += __popc(__ballot_sync(RT_FULL, active));          // world.hit call count (main.rs:44)
         T t_hit; int idx, code;
         world_hit<T, kSmem>(a.scene, table, cand, kThreads, ps, &t_hit, &idx, &code);
-        pending = take_hit<kAov>(a, aov, ps, active, acc_lp, t_hit, idx, code, &hit_idx, &hit_code);
+        pending = take_hit<kAov, kAdapt>(a, aov, ad, ps, active, acc_lp, t_hit, idx, code, &hit_idx, &hit_code);
     }
     if (lane == 0) atomicAdd(a.ray_counter, (unsigned long long)n_rays_w);
 }
@@ -398,17 +429,22 @@ __device__ __forceinline__ void render_loop(const RenderArgs<T>& a, const Camera
 template <typename T, bool kSmem, int kThreads, int kMinCtas>
 __global__ void __launch_bounds__(kThreads, kMinCtas) render_kernel(const RenderArgs<T> a)
 {
-    render_loop<T, kSmem, kThreads, false, false>(a, nullptr, AovArgs{});
+    render_loop<T, kSmem, kThreads, false, false, false>(a, nullptr, AovArgs{}, AdaptArgs{});
 }
 template <typename T, bool kSmem, int kThreads, int kMinCtas>
 __global__ void __launch_bounds__(kThreads, kMinCtas) render_views_kernel(const RenderArgs<T> a, const CameraT<T>* __restrict__ cams)
 {
-    render_loop<T, kSmem, kThreads, true, false>(a, cams, AovArgs{});
+    render_loop<T, kSmem, kThreads, true, false, false>(a, cams, AovArgs{}, AdaptArgs{});
 }
 template <typename T, bool kSmem, int kThreads, int kMinCtas>
 __global__ void __launch_bounds__(kThreads, kMinCtas) render_aov_kernel(const RenderArgs<T> a, const AovArgs aov)
 {
-    render_loop<T, kSmem, kThreads, false, true>(a, nullptr, aov);
+    render_loop<T, kSmem, kThreads, false, true, false>(a, nullptr, aov, AdaptArgs{});
+}
+template <typename T, bool kSmem, int kThreads, int kMinCtas>
+__global__ void __launch_bounds__(kThreads, kMinCtas) render_adaptive_kernel(const RenderArgs<T> a, const AdaptArgs ad)
+{
+    render_loop<T, kSmem, kThreads, false, false, true>(a, nullptr, AovArgs{}, ad);
 }
 
 // The same render loop with the sphere filter on the tensor cores (rt_umma_scan.cuh): G groups of 128 ray threads + G
@@ -417,8 +453,8 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) render_aov_kernel(const Re
 // filter's survivors and the f64 large-sphere test; only the filter moves from 7 FFMA2 per sphere pair to three
 // tcgen05.mma per 128 rays x NC spheres, and the warp-level "any lane alive" vote becomes a 128-thread one, because a
 // group's 128 rays form one MMA.
-template <int G, int NC, bool kViews, bool kAov>
-__device__ __forceinline__ void render_loop_umma(const RenderArgs<float>& a, const CameraT<float>* cams, const AovArgs& aov)
+template <int G, int NC, bool kViews, bool kAov, bool kAdapt>
+__device__ __forceinline__ void render_loop_umma(const RenderArgs<float>& a, const CameraT<float>* cams, const AovArgs& aov, const AdaptArgs& ad)
 {
     extern __shared__ __align__(1024) unsigned char smem_umma[];
     uint32_t tmem_base;
@@ -441,7 +477,7 @@ __device__ __forceinline__ void render_loop_umma(const RenderArgs<float>& a, con
         for (;;) {
             uint32_t px = 0, pj = 0, pv = 0;
             RT_STAMP(1);
-            const bool fresh = assign_work<kViews>(a, wc, lt_mask, pending, ps, acc_lp, &px, &pj, &pv);
+            const bool fresh = assign_work<kViews, kAdapt>(a, ad, wc, lt_mask, pending, ps, acc_lp, &px, &pj, &pv);
             RT_STAMP(2);
             if (!umma_group_any(ux, fresh || pending)) { umma_group_quit(ux); break; }
             RT_STAMP(3);
@@ -451,7 +487,7 @@ __device__ __forceinline__ void render_loop_umma(const RenderArgs<float>& a, con
             RT_STAMP(4);
             const HitF h = closest_hit_umma<G, NC>(ux, a.scene, ps.o, ps.dhat, ps.tmin_n, ps.self_code, ps.self_n, active);
             RT_STAMP(9);
-            pending = take_hit<kAov>(a, aov, ps, active, acc_lp, h.t, h.idx, h.code, &hit_idx, &hit_code);
+            pending = take_hit<kAov, kAdapt>(a, aov, ad, ps, active, acc_lp, h.t, h.idx, h.code, &hit_idx, &hit_code);
         }
         if (lane == 0) atomicAdd(a.ray_counter, (unsigned long long)n_rays_w);
     }
@@ -461,17 +497,22 @@ __device__ __forceinline__ void render_loop_umma(const RenderArgs<float>& a, con
 template <int G, int NC>
 __global__ void __launch_bounds__(UmmaShape<G, NC>::kRenderThreads, 1) render_kernel_umma(const RenderArgs<float> a)
 {
-    render_loop_umma<G, NC, false, false>(a, nullptr, AovArgs{});
+    render_loop_umma<G, NC, false, false, false>(a, nullptr, AovArgs{}, AdaptArgs{});
 }
 template <int G, int NC>
 __global__ void __launch_bounds__(UmmaShape<G, NC>::kRenderThreads, 1) render_views_kernel_umma(const RenderArgs<float> a, const CameraT<float>* __restrict__ cams)
 {
-    render_loop_umma<G, NC, true, false>(a, cams, AovArgs{});
+    render_loop_umma<G, NC, true, false, false>(a, cams, AovArgs{}, AdaptArgs{});
 }
 template <int G, int NC>
 __global__ void __launch_bounds__(UmmaShape<G, NC>::kRenderThreads, 1) render_aov_kernel_umma(const RenderArgs<float> a, const AovArgs aov)
 {
-    render_loop_umma<G, NC, false, true>(a, nullptr, aov);
+    render_loop_umma<G, NC, false, true, false>(a, nullptr, aov, AdaptArgs{});
+}
+template <int G, int NC>
+__global__ void __launch_bounds__(UmmaShape<G, NC>::kRenderThreads, 1) render_adaptive_kernel_umma(const RenderArgs<float> a, const AdaptArgs ad)
+{
+    render_loop_umma<G, NC, false, false, true>(a, nullptr, AovArgs{}, ad);
 }
 
 // Color::to_rgba (vec3.rs:404-420) + the row flip (main.rs:141-145): fixed-point sums -> top-down
@@ -520,6 +561,113 @@ __global__ void finalize_to_frame_kernel(const unsigned long long* __restrict__ 
     const uint32_t lr = i / width, x = i - lr * width;
     const uint32_t y = local_to_global_row(lr, tile_rows, world, rank);
     frame[(size_t)y * width + x] = to_rgba<double>(sum, alpha, (uint64_t)spp);
+}
+
+// ---- rtiow_render_adaptive: the rounds' bookkeeping and the epilogue at per-pixel counts --------------------------------
+// The error of a pixel at a boundary of n samples (include/rtiow_cuda.h): with m = S1 2^-32 / n and q = S2 2^-32 / n,
+// err = 128 sqrt(max(0, q - m^2) / ((n - 1) max(m, 2^-16))), one standard error of the displayed value 256 sqrt(m) in 8-bit
+// levels; +inf for n = 1.  Every operation is rounded on its own (no contraction), so a restatement in IEEE double from the
+// same sums gives the same bits.
+__device__ __forceinline__ double adapt_error(unsigned long long s1, unsigned long long s2, uint32_t n)
+{
+    if (n <= 1) return __longlong_as_double(0x7ff0000000000000ll);
+    const double k = 1.0 / 4294967296.0, nd = (double)n;
+    const double m = __ddiv_rn(__dmul_rn(__ull2double_rn(s1), k), nd);
+    const double q = __ddiv_rn(__dmul_rn(__ull2double_rn(s2), k), nd);
+    const double var = fmax(0.0, __dadd_rn(q, -__dmul_rn(m, m)));
+    const double den = __dmul_rn((double)(n - 1), fmax(m, 1.0 / 65536.0));
+    return __dmul_rn(128.0, __dsqrt_rn(__ddiv_rn(var, den)));
+}
+
+// the rule: a pixel at boundary n stays active iff its error, as out_error reports it (float), exceeds the tolerance and n is
+// not the maximum
+__device__ __forceinline__ bool adapt_keep(float err, double tol, uint32_t n, uint32_t n_max) { return n < n_max && (double)err > tol; }
+
+#define RT_ADAPT_BLOCK 1024   // the select and compact kernels share their blocks: one list entry per thread, 32 warps
+
+// the first round's list: every local pixel, bottom-up like the frame's chunks (assign_work)
+__global__ void adapt_first_list_kernel(uint32_t n_lp, uint32_t* __restrict__ list)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n_lp) list[i] = n_lp - 1u - i;
+}
+
+// After a round that brought every pixel of `list` to n samples: each gets its count and error, and each block counts the
+// pixels that stay active (adapt_keep) into block_keep[block].
+__global__ void __launch_bounds__(RT_ADAPT_BLOCK) adapt_select_kernel(const uint32_t* __restrict__ list, uint32_t n_act,
+                                                                      const unsigned long long* __restrict__ lum_sum, uint32_t n_lp, uint32_t n,
+                                                                      uint32_t n_max, double tol, uint32_t* __restrict__ spp_out,
+                                                                      float* __restrict__ err_out, uint32_t* __restrict__ block_keep)
+{
+    const uint32_t i = blockIdx.x * RT_ADAPT_BLOCK + threadIdx.x;
+    bool keep = false;
+    if (i < n_act) {
+        const uint32_t lp = list[i];
+        const float err = (float)adapt_error(lum_sum[lp], lum_sum[n_lp + lp], n);
+        spp_out[lp] = n; err_out[lp] = err;
+        keep = adapt_keep(err, tol, n, n_max);
+    }
+    const int kept = __syncthreads_count(keep);
+    if (threadIdx.x == 0) block_keep[blockIdx.x] = (uint32_t)kept;
+}
+
+// The next round's list: the active pixels of `list` in their order (a stable compaction, so every round still walks the frame
+// bottom-up and ends on the sky rows).  A block's offset is the sum of the counts of the blocks before it; the last block also
+// writes the length of the new list to *n_next.
+__global__ void __launch_bounds__(RT_ADAPT_BLOCK) adapt_compact_kernel(const uint32_t* __restrict__ list, uint32_t n_act,
+                                                                       const float* __restrict__ err_out, uint32_t n, uint32_t n_max, double tol,
+                                                                       const uint32_t* __restrict__ block_keep, uint32_t* __restrict__ next,
+                                                                       uint32_t* __restrict__ n_next)
+{
+    __shared__ uint32_t warp_n[32];
+    __shared__ uint32_t base;
+    const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+    uint32_t before = 0;
+    for (uint32_t b = threadIdx.x; b < blockIdx.x; b += RT_ADAPT_BLOCK) before += block_keep[b];
+    before = __reduce_add_sync(RT_FULL, before);
+    if (lane == 0) warp_n[warp] = before;
+    __syncthreads();
+    if (threadIdx.x == 0) { uint32_t s = 0; for (int w = 0; w < 32; ++w) s += warp_n[w]; base = s; }
+    __syncthreads();
+    const uint32_t i = blockIdx.x * RT_ADAPT_BLOCK + threadIdx.x;
+    const bool keep = i < n_act && adapt_keep(err_out[list[i]], tol, n, n_max);
+    const unsigned kept = __ballot_sync(RT_FULL, keep);
+    if (lane == 0) warp_n[warp] = __popc(kept);
+    __syncthreads();
+    if (warp == 0) {                                          // exclusive scan of the 32 warps' counts
+        const uint32_t v = warp_n[lane];
+        uint32_t incl = v;
+        for (int o = 1; o < 32; o <<= 1) { const uint32_t u = __shfl_up_sync(RT_FULL, incl, o); if (lane >= (unsigned)o) incl += u; }
+        warp_n[lane] = incl - v;
+    }
+    __syncthreads();
+    if (keep) next[base + warp_n[warp] + __popc(kept & ((1u << lane) - 1u))] = list[i];
+    if (blockIdx.x == gridDim.x - 1 && threadIdx.x == 0) *n_next = base + block_keep[blockIdx.x];
+}
+
+// finalize_kernel with each pixel quantised at its own sample count spp[i] (vec3.rs:404-420)
+__global__ void finalize_adaptive_kernel(const unsigned long long* __restrict__ accum, uint32_t n_lp, const uint32_t* __restrict__ spp, uint32_t alpha,
+                                         uint32_t* __restrict__ out_rgba)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_lp) return;
+    const double k = 1.0 / 4294967296.0;
+    const V3<double> sum = mk<double>((double)accum[i] * k, (double)accum[n_lp + i] * k, (double)accum[2 * (size_t)n_lp + i] * k);
+    out_rgba[i] = to_rgba<double>(sum, alpha, (uint64_t)spp[i]);
+}
+
+// finalize_to_frame_kernel with each pixel quantised at its own sample count spp[i]
+__global__ void finalize_adaptive_to_frame_kernel(const unsigned long long* __restrict__ accum, uint32_t n_lp, const uint32_t* __restrict__ spp,
+                                                  uint32_t alpha, uint32_t width, uint32_t tile_rows, uint32_t world, uint32_t rank,
+                                                  uint32_t* __restrict__ frame)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_lp) return;
+    const double k = 1.0 / 4294967296.0;
+    const V3<double> sum = mk<double>((double)accum[i] * k, (double)accum[n_lp + i] * k, (double)accum[2 * (size_t)n_lp + i] * k);
+    const uint32_t lr = i / width, x = i - lr * width;
+    const uint32_t y = local_to_global_row(lr, tile_rows, world, rank);
+    frame[(size_t)y * width + x] = to_rgba<double>(sum, alpha, (uint64_t)spp[i]);
 }
 
 // gathered tile buffers (rank-major, rank-local rows) -> top-down frame

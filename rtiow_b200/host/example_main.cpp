@@ -3,11 +3,15 @@
 // into flags (SURVEY §8f #3).  No preview window (main.rs:151-171 cannot run headless).
 //
 //   rtiow_host_example [--width W] [--height H] [--spp N] [--depth D] [--seed S] [--scene-seed S] [--gpus G]
-//                      [--grid HALF_EXTENT] [--materials 0..3] [--f64] [--passes N] [--views N] [--aov] [--out image.png|image.ppm] [--selftest]
+//                      [--grid HALF_EXTENT] [--materials 0..3] [--f64] [--passes N] [--views N] [--aov]
+//                      [--adaptive TOL [--min-spp N]] [--out image.png|image.ppm] [--selftest]
 // --views N renders N cameras orbiting the look-at point about the vertical axis in one call and writes out_000.png ...
 // (with --out, the frames are named after its stem: --out orbit.ppm writes orbit_000.ppm ...).
 // --aov also writes the inputs of a denoiser beside the image: <stem>_color.pfm (linear colour), <stem>_albedo.png and
 // <stem>_normal.png (0.5 n + 0.5).
+// --adaptive TOL renders with adaptive sampling (render_adaptive): between --min-spp N (default 16, at most --spp) and --spp
+// samples per pixel, until a pixel's error is at most TOL 8-bit levels; it also writes <stem>_spp.png, a heat map of the
+// per-pixel counts (blue: min-spp, red: spp, log scale).
 #include <algorithm>
 #include <chrono>
 #include <cstdlib>
@@ -101,6 +105,12 @@ static int selftest()
       bool sized = av.color.size() == 3 * n && av.albedo.size() == 3 * n && av.normal.size() == 3 * n && av.depth.size() == n, ranged = sized;
       for (size_t i = 0; ranged && i < 3 * n; ++i) ranged = av.color[i] >= 0 && av.albedo[i] >= 0 && av.albedo[i] <= 1 && std::fabs(av.normal[i]) <= 1.0f + 1e-5f;
       expect(ranged && std::isinf(av.depth[0]) && av.depth[n - 1] > 0 && av.depth[n - 1] < 100, "render_aov: buffers sized, in range, sky depth inf, ground depth finite"); }
+    // adaptive sampling with min_spp == spp renders every pixel at spp: render()'s frame, rays and paths
+    { AdaptiveMaps am; rtiow_stats sd{};
+      std::vector<uint8_t> f = render_adaptive(cam, random_scene(1), p, p.spp, 1.0, &am, &sd);
+      bool flat = am.spp.size() == size_t(p.width) * p.height;
+      for (size_t i = 0; flat && i < am.spp.size(); ++i) flat = am.spp[i] == p.spp;
+      expect(f == a && sd.rays_traced == st.rays_traced && sd.paths == st.paths && flat, "render_adaptive with min_spp == spp equals render() byte for byte"); }
     // the files below go to a private directory: a fixed name in the shared temporary directory may belong to another user
     std::string dir = (std::filesystem::temp_directory_path() / "rtiow_selftest_XXXXXX").string();
     if (!mkdtemp(dir.data())) { std::cerr << "FAIL: cannot create a temporary directory\nselftest FAILED\n"; return 1; }
@@ -122,6 +132,7 @@ int main(int argc, char** argv)
     RenderParams p; p.width = 200; p.height = 133;                       // main.rs:24-28
     uint64_t scene_seed = 1; int grid = 11, materials = 0; std::string out = "image.png";     // main.rs:177
     bool explicit_h = false, explicit_out = false, aov = false; uint32_t passes = 0, views = 0; std::string scene_file, dump_scene;
+    double adaptive = -1.0; uint32_t min_spp = 16;
     for (int i = 1; i < argc; ++i) {
         auto next = [&]() -> const char* { if (i + 1 >= argc) { std::cerr << "missing value for " << argv[i] << "\n"; std::exit(2); } return argv[++i]; };
         if (!std::strcmp(argv[i], "--width")) p.width = std::atoi(next());
@@ -137,6 +148,8 @@ int main(int argc, char** argv)
         else if (!std::strcmp(argv[i], "--passes")) passes = uint32_t(std::atoi(next()));
         else if (!std::strcmp(argv[i], "--views")) views = uint32_t(std::atoi(next()));
         else if (!std::strcmp(argv[i], "--aov")) aov = true;
+        else if (!std::strcmp(argv[i], "--adaptive")) adaptive = std::atof(next());
+        else if (!std::strcmp(argv[i], "--min-spp")) min_spp = uint32_t(std::atoi(next()));
         else if (!std::strcmp(argv[i], "--out")) { out = next(); explicit_out = true; }
         else if (!std::strcmp(argv[i], "--scene")) scene_file = next();               // render the world of a scene file instead of random_scene
         else if (!std::strcmp(argv[i], "--dump-scene")) dump_scene = next();          // write the world to a scene file (for the oracle / a cargo build)
@@ -180,6 +193,18 @@ int main(int argc, char** argv)
                             write_png(stem + "_normal.png", p.width, p.height, unit_rgb_to_rgba(av.normal, 0.5f, 0.5f));
             if (!ok) { std::cerr << "could not write " << out << " and its AOV files\n"; return 1; }
             std::cout << out << ", " << stem << "_color.pfm, " << stem << "_albedo.png, " << stem << "_normal.png saved\n";
+            return 0;
+        }
+        if (adaptive >= 0.0) {                                            // per-pixel sample counts + their heat map
+            AdaptiveMaps am;
+            std::vector<uint8_t> pixels = render_adaptive(cam, world, p, std::min(min_spp, p.spp), adaptive, &am, &st);
+            std::cout << p.width << "x" << p.height << " @ " << std::min(min_spp, p.spp) << ".." << p.spp << " spp (tolerance " << adaptive << ") on "
+                      << st.n_gpus << " GPU(s): kernel " << st.kernel_ms << " ms, " << double(st.paths) / (double(p.width) * p.height) << " spp on average\n";
+            const std::string stem = out.substr(0, out.rfind('.') == std::string::npos ? out.size() : out.rfind('.'));
+            const bool ok = (ppm ? write_ppm(out, p.width, p.height, pixels) : write_png(out, p.width, p.height, pixels)) &&
+                            write_png(stem + "_spp.png", p.width, p.height, spp_heat_map(am.spp, std::min(min_spp, p.spp), p.spp));
+            if (!ok) { std::cerr << "could not write " << out << " and its heat map\n"; return 1; }
+            std::cout << out << ", " << stem << "_spp.png saved\n";
             return 0;
         }
         auto t0 = std::chrono::steady_clock::now();

@@ -292,10 +292,17 @@ inline int progress_trampoline(void* user, uint32_t pass, uint32_t n_passes, uin
 // rtiow_render_aov).
 struct Aovs { std::vector<float> color, albedo, normal, depth; };
 
+// The per-pixel results of render_adaptive(), top-down: each pixel's sample count and its error at the last boundary it reached
+// (include/rtiow_cuda.h, rtiow_render_adaptive).
+struct AdaptiveMaps { std::vector<uint32_t> spp; std::vector<float> error; };
+namespace detail { struct Adaptive { uint32_t min_spp; double tolerance; AdaptiveMaps* maps; }; }
+
 // The world as the GPU sees it + one render call; n_passes == 0: rtiow_render, else rtiow_render_progressive; with `views`:
-// rtiow_render_views of those cameras (cam is not used); with `aovs`: rtiow_render_aov into them.
+// rtiow_render_views of those cameras (cam is not used); with `aovs`: rtiow_render_aov into them; with `adaptive`:
+// rtiow_render_adaptive into its maps.
 inline std::vector<uint8_t> render_impl(const Camera& cam, const HittableList& world, const RenderParams& p, rtiow_stats* stats, uint32_t n_passes,
-                                        const ProgressFn* on_pass, const std::vector<Camera>* views = nullptr, Aovs* aovs = nullptr)
+                                        const ProgressFn* on_pass, const std::vector<Camera>* views = nullptr, Aovs* aovs = nullptr,
+                                        const detail::Adaptive* adaptive = nullptr)
 {
     std::vector<double> cx, cy, cz, rad, ar, ag, ab, prm; std::vector<uint32_t> mi, kind;
     std::vector<const Scatter*> seen;
@@ -331,6 +338,11 @@ inline std::vector<uint8_t> render_impl(const Camera& cam, const HittableList& w
         const size_t n = size_t(p.width) * p.height;
         aovs->color.resize(3 * n); aovs->albedo.resize(3 * n); aovs->normal.resize(3 * n); aovs->depth.resize(n);
         check(rtiow_render_aov(ctx, &cam.raw(), &rp, out.data(), aovs->color.data(), aovs->albedo.data(), aovs->normal.data(), aovs->depth.data(), stats));
+    } else if (adaptive) {
+        const size_t n = size_t(p.width) * p.height;
+        adaptive->maps->spp.resize(n); adaptive->maps->error.resize(n);
+        check(rtiow_render_adaptive(ctx, &cam.raw(), &rp, adaptive->min_spp, adaptive->tolerance, out.data(), adaptive->maps->spp.data(),
+                                    adaptive->maps->error.data(), stats));
     } else if (n_passes == 0) check(rtiow_render(ctx, &cam.raw(), &rp, out.data(), stats));
     else {
         detail::ProgressCtx pc{ on_pass, &out };
@@ -361,6 +373,17 @@ inline std::vector<uint8_t> render_aov(const Camera& cam, const HittableList& wo
 {
     if (!aovs) throw RenderError(RTIOW_ERR_INVALID_ARG, "render_aov needs an Aovs to fill");
     return render_impl(cam, world, p, stats, 0, nullptr, nullptr, aovs);
+}
+
+// render_adaptive(): adaptive sampling.  Each pixel gets between min_spp and p.spp samples, as many as its own noise asks for
+// (its error, one standard error of the displayed value in 8-bit levels, at most `tolerance`), and is byte-identical to
+// render() at its own count; *maps receives every pixel's count and error.
+inline std::vector<uint8_t> render_adaptive(const Camera& cam, const HittableList& world, const RenderParams& p, uint32_t min_spp, double tolerance,
+                                            AdaptiveMaps* maps, rtiow_stats* stats = nullptr)
+{
+    if (!maps) throw RenderError(RTIOW_ERR_INVALID_ARG, "render_adaptive needs an AdaptiveMaps to fill");
+    const detail::Adaptive a{ min_spp, tolerance, maps };
+    return render_impl(cam, world, p, stats, 0, nullptr, nullptr, nullptr, &a);
 }
 
 // render_progressive(): the same frame in n_passes slices of the samples, with a preview after each — what the reference's
@@ -468,6 +491,18 @@ inline bool write_pfm(const std::string& path, uint32_t w, uint32_t h, const std
     std::fprintf(f, "PF\n%u %u\n-1.0\n", w, h);
     for (uint32_t y = h; y-- > 0;) std::fwrite(&rgb[size_t(y) * w * 3], sizeof(float), size_t(w) * 3, f);
     return std::fclose(f) == 0;
+}
+// per-pixel sample counts (render_adaptive's) -> RGBA8 heat map for write_png: blue at lo samples to red at hi, on a log scale
+inline std::vector<uint8_t> spp_heat_map(const std::vector<uint32_t>& spp, uint32_t lo, uint32_t hi)
+{
+    std::vector<uint8_t> out(spp.size() * 4, 255);
+    const double span = hi > lo ? std::log(double(hi) / double(lo)) : 1.0;
+    for (size_t i = 0; i < spp.size(); ++i) {
+        const double v = std::min(1.0, std::max(0.0, std::log(double(std::max(spp[i], lo)) / double(lo)) / span));
+        out[4 * i] = uint8_t(std::lround(255.0 * v)); out[4 * i + 1] = uint8_t(std::lround(255.0 * (1.0 - std::fabs(2.0 * v - 1.0))));
+        out[4 * i + 2] = uint8_t(std::lround(255.0 * (1.0 - v)));
+    }
+    return out;
 }
 // float RGB in [0, 1] per channel (render_aov's albedo, or 0.5 n + 0.5 of its normal) -> RGBA8 for write_png
 inline std::vector<uint8_t> unit_rgb_to_rgba(const std::vector<float>& rgb, float scale = 1.0f, float offset = 0.0f)

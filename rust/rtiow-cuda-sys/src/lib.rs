@@ -108,6 +108,8 @@ extern "C" {
                         stats: *mut rtiow_stats) -> c_int;
     pub fn rtiow_render_aov(ctx: *mut rtiow_ctx, cam: *const rtiow_camera, p: *const rtiow_params, out_rgba: *mut u8, out_color: *mut f32,
                             out_albedo: *mut f32, out_normal: *mut f32, out_depth: *mut f32, stats: *mut rtiow_stats) -> c_int;
+    pub fn rtiow_render_adaptive(ctx: *mut rtiow_ctx, cam: *const rtiow_camera, p: *const rtiow_params, min_spp: u32, tolerance: f64,
+                                 out_rgba: *mut u8, out_spp: *mut u32, out_error: *mut f32, stats: *mut rtiow_stats) -> c_int;
     pub fn rtiow_render_views(ctx: *mut rtiow_ctx, cams: *const rtiow_camera, n_views: u32, p: *const rtiow_params, out_rgba: *mut u8,
                               stats: *mut rtiow_stats) -> c_int;
     pub fn rtiow_render_progressive(ctx: *mut rtiow_ctx, cam: *const rtiow_camera, p: *const rtiow_params, n_passes: u32,

@@ -99,6 +99,29 @@ pub fn render_aov(cam: &Camera, world: &HittableList, p: &RenderParams) -> Resul
     }
 }
 
+/// Adaptive sampling: each pixel gets between `min_spp` and `p.spp` samples, as many as its own noise asks for, and is
+/// byte-identical to `render` at its own count.  Returns the frame, each pixel's count and its error at the last boundary it
+/// reached (one standard error of the displayed value in 8-bit levels; include/rtiow_cuda.h, rtiow_render_adaptive).
+pub fn render_adaptive(cam: &Camera, world: &HittableList, p: &RenderParams, min_spp: u32, tolerance: f64)
+                       -> Result<(Vec<u8>, Vec<u32>, Vec<f32>), RenderError> {
+    unsafe {
+        let mut raw: *mut sys::rtiow_ctx = ptr::null_mut();
+        let rc = sys::rtiow_ctx_create(p.n_gpus, &mut raw);
+        if rc != sys::RTIOW_OK { return Err(err(rc)); }
+        let ctx = Ctx(raw);
+        upload(&ctx, world)?;
+        let prm = raw_params(p);
+        let n = p.width as usize * p.height as usize;
+        let mut pixels = vec![0u8; 4 * n];
+        let mut spp = vec![0u32; n];
+        let mut error = vec![0.0f32; n];
+        let rc = sys::rtiow_render_adaptive(ctx.0, &cam.raw(), &prm, min_spp, tolerance, pixels.as_mut_ptr(), spp.as_mut_ptr(),
+                                            error.as_mut_ptr(), ptr::null_mut());
+        if rc != sys::RTIOW_OK { return Err(err(rc)); }
+        Ok((pixels, spp, error))
+    }
+}
+
 /// The same frame in `n_passes` slices of the samples, with the frame so far handed to `on_pass(pass, n_passes, spp_done, rgba)`
 /// after each — the role of the indicatif bar (main.rs:120,124) and the piston preview window (main.rs:151-171).  The returned
 /// frame is bit-identical to `render`'s.  `on_pass` returning `true` stops the render: `Err(RenderError::Cancelled)`.
