@@ -214,6 +214,48 @@ int rtiow_render_aov(rtiow_ctx* ctx, const rtiow_camera* cam, const rtiow_params
 int rtiow_render_adaptive(rtiow_ctx* ctx, const rtiow_camera* cam, const rtiow_params* p, uint32_t min_spp, double tolerance,
                           uint8_t* out_rgba, uint32_t* out_spp, float* out_error, rtiow_stats* stats);
 
+/* An edge-avoiding a-trous wavelet denoiser (Dammertz et al., HPG 2010) for the buffers of rtiow_render_aov, guided by the first
+ * hit's albedo, normal and depth.  Every output bit is pinned below (tests/np_denoise.py restates it in numpy float32).
+ *   Inputs     color, albedo, normal [H][W][3] and depth [H][W], top-down, caller-owned HOST memory, as rtiow_render_aov writes
+ *              them; all four are required.  Each value must lie in the range those buffers can take: colour in [0, 2^32],
+ *              albedo in [0, 1], normal components in [-1, 1], depth in [0, 65536] or +inf, and no NaN anywhere; else the call
+ *              returns RTIOW_ERR_INVALID_ARG and writes no output.  The ranges keep every intermediate below float's limits, so
+ *              no weight is ever NaN.
+ *   Arithmetic every operation is one correctly rounded fp32 +, -, x or /, min or max, in the order given; nothing contracts into
+ *              an FMA and denormals are kept.  Host doubles (the sigmas) are narrowed to float with round-to-nearest.
+ *   1. Demodulate  a_c = max(albedo_c, 2^-8), x_c = color_c / a_c.
+ *   2. Level i = 0 .. levels-1, step s = 2^i:
+ *        k_c = 1 / ((sigma_color 2^-i) (sigma_color 2^-i)), k_n = 1 / (sigma_normal sigma_normal), k_z = 1 / (sigma_depth
+ *        sigma_depth), in float (a sigma of +inf gives k = 0: that term is off).  For each pixel p, the taps q = p + s (dx, dy),
+ *        dy = -2..2 outer, dx = -2..2 inner; a tap outside the image is skipped (not clamped):
+ *          h  = h1[dy] h1[dx], h1 = (1/16, 1/4, 3/8, 1/4, 1/16) (exact)
+ *          Dc = sum over r, g, b in order of (x_p - x_q)^2 (x: this level's input),  wc = 1 / (1 + Dc k_c)
+ *          Dn = sum over x, y, z in order of (n_p - n_q)^2,                         wn = 1 / (1 + Dn k_n)
+ *          wz = 1 / (1 + Dz k_z), Dz = t t, t = (z_p - z_q) / (s max(max(z_p, z_q), 2^-16)) when both depths are finite;
+ *               1 when both are +inf; 0 when exactly one is (sky never blends into geometry)
+ *          w  = ((h wc) wn) wz;  num_c += w x_c(q) and den += w, in tap order
+ *        and the level's output is num_c / den (den >= 9/64: the centre tap).
+ *   3. Remodulate  y_c = out_c a_c: out_color.  out_rgba quantises y as a frame's epilogue quantises a pixel of one sample
+ *              (to_rgba at spp = 1, in double, vec3.rs:404-420), with alpha byte dp->alpha.
+ * out_color [H][W][3] float and out_rgba [H][W] RGBA8 (caller-owned HOST memory) may each be NULL, but not both.
+ * RTIOW_ERR_INVALID_ARG also for a NULL input or dp, width or height 0, levels > 10, or a sigma that is NaN or below 1e-12
+ * (+inf allowed).  The call is local: it runs on the ctx's first device and stream (device 0 of an n-GPU ctx, a rank ctx's own
+ * device for any world) and needs no uploaded scene.  Stats: kernel_ms (the denoise kernels), total_ms, h2d_bytes = 40 W H,
+ * d2h_bytes = 12 W H with out_color plus 4 W H with out_rgba, kernel_launches = levels + 2, n_gpus = 1; every other field 0. */
+typedef struct {
+    uint32_t levels;          /* a-trous levels, step 2^i at level i; 0..10 */
+    double   sigma_color;     /* edge-stopping widths: each >= 1e-12 or +inf (+inf turns that term off) */
+    double   sigma_normal;
+    double   sigma_depth;
+    uint8_t  alpha;           /* alpha byte of out_rgba (255 as at main.rs:137) */
+    uint8_t  reserved[7];
+} rtiow_denoise_params;
+/* the defaults tools/denoise_probe.py chose on the final scene (profiles/denoise_probe.json): levels 4, sigma_color 0.1,
+ * sigma_normal +inf (the normal term off), sigma_depth 0.1, alpha 255 */
+void rtiow_denoise_params_default(rtiow_denoise_params* dp);
+int  rtiow_denoise(rtiow_ctx* ctx, uint32_t width, uint32_t height, const float* color, const float* albedo, const float* normal,
+                   const float* depth, const rtiow_denoise_params* dp, float* out_color, uint8_t* out_rgba, rtiow_stats* stats);
+
 /* Many views of one scene (turntables, animations, stereo pairs, camera sweeps) in one call: out_rgba receives n_views top-down
  * RGBA8 frames of 4*width*height bytes each, in view order, in caller-owned HOST memory.  Frame v equals
  * rtiow_render(ctx, &cams[v], p, ...) byte for byte, so the views share their sample streams (same seed, same pixel keys);

@@ -127,6 +127,14 @@ def render_adaptive(cam: capi.Camera, world: HittableList, params: capi.Params, 
     return img, maps
 
 
+def denoise(color, albedo, normal, depth, params: capi.DenoiseParams | None = None, n_gpus: int = 1):
+    """An edge-avoiding a-trous denoiser over render_aov()'s buffers (include/rtiow_cuda.h, rtiow_denoise; default parameters when
+    params is None) -> (linear colour float32[H,W,3], rgba uint8[H,W,4]).  Needs no scene: it runs on the first GPU."""
+    with capi.Context(n_gpus) as ctx:
+        outs, _ = ctx.denoise(color, albedo, normal, depth, params)
+    return outs["color"], outs["rgba"]
+
+
 def render_views(cams, world: HittableList, params: capi.Params, n_gpus: int = 1):
     """Many cameras of one world in one call: [K,H,W,4] top-down RGBA8, frame v byte-identical to render(cams[v], ...)."""
     with capi.Context(n_gpus) as ctx:

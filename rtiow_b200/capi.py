@@ -31,6 +31,7 @@ SYMBOLS = [
     "rtiow_abi_version", "rtiow_last_error", "rtiow_device_count", "rtiow_ctx_create", "rtiow_ctx_create_on_device",
     "rtiow_ctx_destroy", "rtiow_ctx_set_scan_backend", "rtiow_ctx_set_filter_bypass", "rtiow_nccl_unique_id", "rtiow_ctx_create_rank", "rtiow_ctx_set_gather", "rtiow_ctx_set_stream",
     "rtiow_ctx_gather_info", "rtiow_render_rank", "rtiow_render_rank_device", "rtiow_render_rank_enqueue", "rtiow_ctx_synchronize", "rtiow_scene_upload", "rtiow_camera_new", "rtiow_params_default", "rtiow_render", "rtiow_render_aov", "rtiow_render_adaptive", "rtiow_render_views", "rtiow_render_progressive",
+    "rtiow_denoise_params_default", "rtiow_denoise",
     "rtiow_tile_buffer_bytes", "rtiow_render_tiles_device", "rtiow_render_to_frame_device", "rtiow_deinterleave_device", "rtiow_sphere_hit_batch",
     "rtiow_hitlist_batch", "rtiow_scatter_batch", "rtiow_get_ray_batch", "rtiow_to_rgba_batch", "rtiow_reflect_batch",
     "rtiow_refract_batch", "rtiow_ray_color_batch", "rtiow_ray_color_trace_batch", "rtiow_sampler_batch", "rtiow_fp32_peak_probe", "rtiow_flush_l2",
@@ -72,6 +73,11 @@ class Stats(C.Structure):
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_}
+
+
+class DenoiseParams(C.Structure):
+    _fields_ = [("levels", C.c_uint32), ("sigma_color", C.c_double), ("sigma_normal", C.c_double), ("sigma_depth", C.c_double),
+                ("alpha", C.c_uint8), ("reserved", C.c_uint8 * 7)]
 
 
 _lib = None
@@ -124,6 +130,8 @@ def _declare(L):
         "rtiow_render_adaptive": (C.c_int, [P, C.POINTER(Camera), C.POINTER(Params), u32, d, P, P, P, C.POINTER(Stats)]),
         "rtiow_render_views": (C.c_int, [P, C.POINTER(Camera), C.c_uint32, C.POINTER(Params), P, C.POINTER(Stats)]),
         "rtiow_render_progressive": (C.c_int, [P, C.POINTER(Camera), C.POINTER(Params), C.c_uint32, PROGRESS_FN, P, P, C.POINTER(Stats)]),
+        "rtiow_denoise_params_default": (None, [C.POINTER(DenoiseParams)]),
+        "rtiow_denoise": (C.c_int, [P, u32, u32, P, P, P, P, C.POINTER(DenoiseParams), P, P, C.POINTER(Stats)]),
         "rtiow_render_rank_enqueue": (C.c_int, [P, C.POINTER(Camera), C.POINTER(Params), C.POINTER(C.c_void_p)]),
         "rtiow_ctx_synchronize": (C.c_int, [P, C.POINTER(Stats)]),
         "rtiow_tile_buffer_bytes": (C.c_int, [C.POINTER(Params), C.c_int, C.POINTER(C.c_size_t)]),
@@ -196,6 +204,15 @@ def default_params(**kw) -> Params:
     for k, v in kw.items():
         setattr(p, k, v)
     return p
+
+
+def default_denoise_params(**kw) -> DenoiseParams:
+    """rtiow_denoise_params_default (the defaults tools/denoise_probe.py chose), with any field overridden by keyword"""
+    dp = DenoiseParams()
+    lib().rtiow_denoise_params_default(C.byref(dp))
+    for k, v in kw.items():
+        setattr(dp, k, v)
+    return dp
 
 
 def random_scene(seed: int = 1, half_extent: int = 11, material_mode: int = 0):
@@ -416,6 +433,38 @@ class Context:
                                            _p(maps["spp"]) if "spp" in maps else None, _p(maps["error"]) if "error" in maps else None,
                                            C.byref(st)))
         return out.reshape(h, w, 4), maps, st.as_dict()
+
+    def denoise(self, color, albedo, normal, depth, params: DenoiseParams | None = None, out_color=True, out_rgba=True):
+        """rtiow_denoise: the edge-avoiding a-trous filter over render_aov's buffers (colour, albedo, normal float32 [H,W,3], depth
+        float32 [H,W], each C-contiguous) -> ({"color": float32[H,W,3], "rgba": uint8[H,W,4]}, stats).  out_color / out_rgba are
+        True (allocate), False / None (not computed: NULL, absent from the dict) or a C-contiguous array of the right dtype and
+        size that receives it.  The filter, bit for bit, and the input ranges are defined in include/rtiow_cuda.h."""
+        if not isinstance(depth, np.ndarray) or depth.ndim != 2:
+            raise ValueError("depth must be a float32 array of shape (H, W)")
+        h, w = depth.shape
+        ins = {}
+        for name, arr, per_px in (("color", color, 3), ("albedo", albedo, 3), ("normal", normal, 3), ("depth", depth, 1)):
+            if (not isinstance(arr, np.ndarray) or arr.dtype != np.float32 or arr.size != h * w * per_px or not arr.flags.c_contiguous):
+                raise ValueError(f"{name} must be a C-contiguous float32 array with {h * w * per_px} elements")
+            ins[name] = arr
+        outs = {}
+        for name, arg, dt, shape in (("color", out_color, np.float32, (h, w, 3)), ("rgba", out_rgba, np.uint8, (h, w, 4))):
+            if arg is None or arg is False:
+                continue
+            if arg is True:
+                arg = np.empty(shape, dt)
+            elif (not isinstance(arg, np.ndarray) or arg.dtype != dt or arg.size != int(np.prod(shape)) or not arg.flags.c_contiguous):
+                raise ValueError(f"out_{name} must be a C-contiguous {np.dtype(dt).name} array with {int(np.prod(shape))} elements")
+            outs[name] = arg.reshape(shape)
+        if not outs:
+            raise ValueError("out_color and out_rgba cannot both be None")
+        if params is None:
+            params = default_denoise_params()
+        st = Stats()
+        _check(lib().rtiow_denoise(self._h, w, h, _p(ins["color"]), _p(ins["albedo"]), _p(ins["normal"]), _p(ins["depth"]), C.byref(params),
+                                   _p(outs["color"]) if "color" in outs else None, _p(outs["rgba"]) if "rgba" in outs else None,
+                                   C.byref(st)))
+        return outs, st.as_dict()
 
     def render_views(self, cams, params: Params, out=None):
         """rtiow_render_views: many cameras of the uploaded scene in one call -> (rgba[K,H,W,4] uint8, stats of the batch).

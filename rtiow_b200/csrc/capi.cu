@@ -4,6 +4,7 @@
 // CUDA device every compute entry point returns RTIOW_ERR_NO_DEVICE.
 #include "../../include/rtiow_cuda.h"
 #include "rt_unit.cuh"
+#include "rt_denoise.cuh"
 
 #include <nccl.h>
 #include <dlfcn.h>
@@ -103,6 +104,10 @@ struct DeviceState {
     DevBuf<uint32_t> adapt_list; DevBuf<unsigned long long> adapt_lum; DevBuf<uint32_t> adapt_spp; DevBuf<float> adapt_err;
     DevBuf<uint32_t> adapt_blocks; DevBuf<uint32_t> adapt_n; HostBuf<uint32_t> adapt_n_host;
     uint64_t adapt_paths = 0; float adapt_ms = 0;
+    // rtiow_denoise: the caller's four input buffers back to back, the float4 ping-pong pair and the guides ([3][n]), the outputs,
+    // and the range flag of the prepare kernel (on the device and page-locked)
+    DevBuf<float> dn_in; DevBuf<float4> dn_work; DevBuf<float> dn_color; DevBuf<uint32_t> dn_rgba;
+    DevBuf<uint32_t> dn_bad; HostBuf<uint32_t> dn_bad_host;
     // measurement
     DevBuf<uint4> flush; DevBuf<float> probe;
     int last_backend = RTIOW_SCAN_FP32;                // which filter the last render launch used (rtiow_stats.scan_backend)
@@ -371,6 +376,7 @@ extern "C" void rtiow_ctx_destroy(rtiow_ctx* c)
         d.aov_sum.release(); d.aov_hits.release(); d.aov_out.release();
         d.adapt_list.release(); d.adapt_lum.release(); d.adapt_spp.release(); d.adapt_err.release(); d.adapt_blocks.release(); d.adapt_n.release();
         d.adapt_n_host.release();
+        d.dn_in.release(); d.dn_work.release(); d.dn_color.release(); d.dn_rgba.release(); d.dn_bad.release(); d.dn_bad_host.release();
         if (d.ev0) cudaEventDestroy(d.ev0);
         if (d.ev1) cudaEventDestroy(d.ev1);
         if (d.ev_done) cudaEventDestroy(d.ev_done);
@@ -1590,6 +1596,68 @@ extern "C" int rtiow_ctx_synchronize(rtiow_ctx* c, rtiow_stats* stats)
             *stats = make_stats(d, sum / (double)d.ring_used, 0.0, d.enq_paths, d.pinned_cnt.p[1], d.enq_launches, d.enq_world, kCallH2D * d.ring_used, 16 * d.ring_used);
     }
     d.ring_used = 0; d.enq_launches = 0;
+    return RTIOW_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// rtiow_denoise: the edge-avoiding a-trous filter of rt_denoise.cuh over rtiow_render_aov's buffers
+// ------------------------------------------------------------------------------------------------
+extern "C" void rtiow_denoise_params_default(rtiow_denoise_params* dp)
+{
+    if (!dp) return;
+    memset(dp, 0, sizeof *dp);
+    // chosen by tools/denoise_probe.py on the final scene (profiles/denoise_probe.json).  The normal term is off: a pixel's normal
+    // is a mean over its samples, noisy at silhouettes and out of focus, and the best combinations the probe found leave it off.
+    dp->levels = 4; dp->sigma_color = 0.1; dp->sigma_normal = HUGE_VAL; dp->sigma_depth = 0.1;
+    dp->alpha = 255;
+}
+
+// Uploads the four buffers (40 B/px), runs prepare, the levels and finish on the ctx's first device and stream, reads the range
+// flag back and only then copies the requested outputs to the caller.  An input out of range still runs the kernels on the
+// device; it writes nothing to the caller and returns RTIOW_ERR_INVALID_ARG.
+extern "C" int rtiow_denoise(rtiow_ctx* c, uint32_t width, uint32_t height, const float* color, const float* albedo, const float* normal,
+                             const float* depth, const rtiow_denoise_params* dp, float* out_color, uint8_t* out_rgba, rtiow_stats* stats)
+{
+    if (!c || !color || !albedo || !normal || !depth || !dp) return fail(RTIOW_ERR_INVALID_ARG, "NULL argument");
+    if (!out_color && !out_rgba) return fail(RTIOW_ERR_INVALID_ARG, "rtiow_denoise: out_color and out_rgba are both NULL");
+    if (width == 0 || height == 0) return fail(RTIOW_ERR_INVALID_ARG, "rtiow_denoise: empty image (%u x %u)", width, height);
+    if (dp->levels > 10) return fail(RTIOW_ERR_INVALID_ARG, "rtiow_denoise: levels %u > 10", dp->levels);
+    const double sig[3] = { dp->sigma_color, dp->sigma_normal, dp->sigma_depth };
+    for (double s : sig)
+        if (!(s >= 1e-12)) return fail(RTIOW_ERR_INVALID_ARG, "rtiow_denoise: a sigma is NaN or below 1e-12 (%g)", s);
+    const double t0 = now_ms();
+    const size_t n = (size_t)width * height;
+    DeviceState& d = c->dev[0];
+    CU(cudaSetDevice(d.device));
+    const cudaStream_t st = d.stream;
+    CU(d.dn_in.resize(10 * n)); CU(d.dn_work.resize(3 * n)); CU(d.dn_bad.resize(1)); CU(d.dn_bad_host.resize(1));
+    if (out_color) CU(d.dn_color.resize(3 * n));
+    if (out_rgba) CU(d.dn_rgba.resize(n));
+    CU(cudaMemcpyAsync(d.dn_in.p, color, 3 * n * sizeof(float), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d.dn_in.p + 3 * n, albedo, 3 * n * sizeof(float), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d.dn_in.p + 6 * n, normal, 3 * n * sizeof(float), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d.dn_in.p + 9 * n, depth, n * sizeof(float), cudaMemcpyHostToDevice, st));
+    CU(cudaMemsetAsync(d.dn_bad.p, 0, sizeof(uint32_t), st));
+    CU(cudaEventRecord(d.ev0, st));
+    // the sigmas narrowed to float with round-to-nearest
+    CU(denoise_launch(d.dn_in.p, d.dn_work.p, d.dn_bad.p, width, height, dp->levels, (float)dp->sigma_color, (float)dp->sigma_normal,
+                      (float)dp->sigma_depth, dp->alpha, out_color ? d.dn_color.p : nullptr, out_rgba ? d.dn_rgba.p : nullptr, st));
+    CU(cudaEventRecord(d.ev1, st));
+    CU(cudaMemcpyAsync(d.dn_bad_host.p, d.dn_bad.p, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    if (*d.dn_bad_host.p)
+        return fail(RTIOW_ERR_INVALID_ARG, "rtiow_denoise: an input value lies outside the range of rtiow_render_aov's buffers (or is NaN)");
+    uint64_t d2h = 0;
+    if (out_color) { CU(cudaMemcpyAsync(out_color, d.dn_color.p, 3 * n * sizeof(float), cudaMemcpyDeviceToHost, st)); d2h += 12 * (uint64_t)n; }
+    if (out_rgba) { CU(cudaMemcpyAsync(out_rgba, d.dn_rgba.p, 4 * n, cudaMemcpyDeviceToHost, st)); d2h += 4 * (uint64_t)n; }
+    CU(cudaStreamSynchronize(st));
+    if (stats) {
+        float ms = 0; CU(cudaEventElapsedTime(&ms, d.ev0, d.ev1));
+        memset(stats, 0, sizeof *stats);
+        stats->kernel_ms = ms; stats->total_ms = now_ms() - t0;
+        stats->h2d_bytes = 40 * (uint64_t)n; stats->d2h_bytes = d2h;
+        stats->kernel_launches = dp->levels + 2; stats->n_gpus = 1;
+    }
     return RTIOW_OK;
 }
 

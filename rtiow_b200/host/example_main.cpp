@@ -4,11 +4,12 @@
 //
 //   rtiow_host_example [--width W] [--height H] [--spp N] [--depth D] [--seed S] [--scene-seed S] [--gpus G]
 //                      [--grid HALF_EXTENT] [--materials 0..3] [--f64] [--passes N] [--views N] [--aov]
-//                      [--adaptive TOL [--min-spp N]] [--out image.png|image.ppm] [--selftest]
+//                      [--denoise] [--adaptive TOL [--min-spp N]] [--out image.png|image.ppm] [--selftest]
 // --views N renders N cameras orbiting the look-at point about the vertical axis in one call and writes out_000.png ...
 // (with --out, the frames are named after its stem: --out orbit.ppm writes orbit_000.ppm ...).
 // --aov also writes the inputs of a denoiser beside the image: <stem>_color.pfm (linear colour), <stem>_albedo.png and
-// <stem>_normal.png (0.5 n + 0.5).
+// <stem>_normal.png (0.5 n + 0.5).  --denoise (implies --aov) also runs the library's a-trous denoiser (default parameters) over
+// them and writes <stem>_denoised.png.
 // --adaptive TOL renders with adaptive sampling (render_adaptive): between --min-spp N (default 16, at most --spp) and --spp
 // samples per pixel, until a pixel's error is at most TOL 8-bit levels; it also writes <stem>_spp.png, a heat map of the
 // per-pixel counts (blue: min-spp, red: spp, log scale).
@@ -104,7 +105,12 @@ static int selftest()
       expect(f == a && sa.rays_traced == st.rays_traced, "render_aov: the frame equals render()'s byte for byte");
       bool sized = av.color.size() == 3 * n && av.albedo.size() == 3 * n && av.normal.size() == 3 * n && av.depth.size() == n, ranged = sized;
       for (size_t i = 0; ranged && i < 3 * n; ++i) ranged = av.color[i] >= 0 && av.albedo[i] >= 0 && av.albedo[i] <= 1 && std::fabs(av.normal[i]) <= 1.0f + 1e-5f;
-      expect(ranged && std::isinf(av.depth[0]) && av.depth[n - 1] > 0 && av.depth[n - 1] < 100, "render_aov: buffers sized, in range, sky depth inf, ground depth finite"); }
+      expect(ranged && std::isinf(av.depth[0]) && av.depth[n - 1] > 0 && av.depth[n - 1] < 100, "render_aov: buffers sized, in range, sky depth inf, ground depth finite");
+      // the denoiser over those buffers: deterministic, sized, and its frame's bytes agree with its own colour's range
+      std::vector<float> dc; rtiow_stats sn{};
+      const std::vector<uint8_t> d1 = denoise(p.width, p.height, av, default_denoise_params(), &dc, &sn), d2 = denoise(p.width, p.height, av, default_denoise_params());
+      expect(d1 == d2 && d1.size() == 4 * n && dc.size() == 3 * n && d1[3] == 255, "denoise: the same bytes on a second call, sized 4*W*H, alpha 255");
+      expect(sn.h2d_bytes == 40ull * n && sn.d2h_bytes == 16ull * n && sn.n_gpus == 1 && sn.paths == 0, "denoise stats: 40 B/px up, 16 B/px down"); }
     // adaptive sampling with min_spp == spp renders every pixel at spp: render()'s frame, rays and paths
     { AdaptiveMaps am; rtiow_stats sd{};
       std::vector<uint8_t> f = render_adaptive(cam, random_scene(1), p, p.spp, 1.0, &am, &sd);
@@ -131,7 +137,7 @@ int main(int argc, char** argv)
 {
     RenderParams p; p.width = 200; p.height = 133;                       // main.rs:24-28
     uint64_t scene_seed = 1; int grid = 11, materials = 0; std::string out = "image.png";     // main.rs:177
-    bool explicit_h = false, explicit_out = false, aov = false; uint32_t passes = 0, views = 0; std::string scene_file, dump_scene;
+    bool explicit_h = false, explicit_out = false, aov = false, denoised = false; uint32_t passes = 0, views = 0; std::string scene_file, dump_scene;
     double adaptive = -1.0; uint32_t min_spp = 16;
     for (int i = 1; i < argc; ++i) {
         auto next = [&]() -> const char* { if (i + 1 >= argc) { std::cerr << "missing value for " << argv[i] << "\n"; std::exit(2); } return argv[++i]; };
@@ -148,6 +154,7 @@ int main(int argc, char** argv)
         else if (!std::strcmp(argv[i], "--passes")) passes = uint32_t(std::atoi(next()));
         else if (!std::strcmp(argv[i], "--views")) views = uint32_t(std::atoi(next()));
         else if (!std::strcmp(argv[i], "--aov")) aov = true;
+        else if (!std::strcmp(argv[i], "--denoise")) denoised = aov = true;        // implies --aov
         else if (!std::strcmp(argv[i], "--adaptive")) adaptive = std::atof(next());
         else if (!std::strcmp(argv[i], "--min-spp")) min_spp = uint32_t(std::atoi(next()));
         else if (!std::strcmp(argv[i], "--out")) { out = next(); explicit_out = true; }
@@ -193,6 +200,12 @@ int main(int argc, char** argv)
                             write_png(stem + "_normal.png", p.width, p.height, unit_rgb_to_rgba(av.normal, 0.5f, 0.5f));
             if (!ok) { std::cerr << "could not write " << out << " and its AOV files\n"; return 1; }
             std::cout << out << ", " << stem << "_color.pfm, " << stem << "_albedo.png, " << stem << "_normal.png saved\n";
+            if (denoised) {
+                rtiow_stats sd{};
+                const std::vector<uint8_t> dn = denoise(p.width, p.height, av, default_denoise_params(), nullptr, &sd);
+                if (!write_png(stem + "_denoised.png", p.width, p.height, dn)) { std::cerr << "could not write " << stem << "_denoised.png\n"; return 1; }
+                std::cout << "denoised: kernel " << sd.kernel_ms << " ms, call " << sd.total_ms << " ms; " << stem << "_denoised.png saved\n";
+            }
             return 0;
         }
         if (adaptive >= 0.0) {                                            // per-pixel sample counts + their heat map

@@ -386,6 +386,30 @@ inline std::vector<uint8_t> render_adaptive(const Camera& cam, const HittableLis
     return render_impl(cam, world, p, stats, 0, nullptr, nullptr, nullptr, &a);
 }
 
+// The parameters of denoise(): the defaults the library chose on the final scene (rtiow_denoise_params_default).
+inline rtiow_denoise_params default_denoise_params() { rtiow_denoise_params dp; rtiow_denoise_params_default(&dp); return dp; }
+
+// denoise(): an edge-avoiding a-trous filter over render_aov()'s buffers of a width x height frame (include/rtiow_cuda.h,
+// rtiow_denoise), on GPU 0.  Returns the denoised frame as top-down RGBA8; *color (may be null) receives its linear colour.
+inline std::vector<uint8_t> denoise(uint32_t width, uint32_t height, const Aovs& aovs, const rtiow_denoise_params& dp,
+                                    std::vector<float>* color = nullptr, rtiow_stats* stats = nullptr)
+{
+    const size_t n = size_t(width) * height;
+    if (aovs.color.size() != 3 * n || aovs.albedo.size() != 3 * n || aovs.normal.size() != 3 * n || aovs.depth.size() != n)
+        throw RenderError(RTIOW_ERR_INVALID_ARG, "denoise: the AOV buffers do not match width x height");
+    rtiow_ctx* ctx = nullptr;
+    int rc = rtiow_ctx_create(1, &ctx);
+    if (rc != RTIOW_OK) throw RenderError(rc, rtiow_last_error());
+    std::vector<uint8_t> out(4 * n);
+    if (color) color->resize(3 * n);
+    rc = rtiow_denoise(ctx, width, height, aovs.color.data(), aovs.albedo.data(), aovs.normal.data(), aovs.depth.data(), &dp,
+                       color ? color->data() : nullptr, out.data(), stats);
+    const std::string msg = rc != RTIOW_OK ? rtiow_last_error() : "";
+    rtiow_ctx_destroy(ctx);
+    if (rc != RTIOW_OK) throw RenderError(rc, msg);
+    return out;
+}
+
 // render_progressive(): the same frame in n_passes slices of the samples, with a preview after each — what the reference's
 // progress bar (main.rs:120,124) and preview window (main.rs:151-171) are for.  The returned frame is bit-identical to
 // render()'s.  A callback that returns true stops the render: RenderError::Cancelled.

@@ -83,6 +83,14 @@ pub struct rtiow_stats {
     pub kernel_launches: u32, pub n_gpus: u32, pub scan_backend: u32, pub reserved: u32,
 }
 
+#[repr(C)]
+#[derive(Clone, Copy, Debug, Default)]
+pub struct rtiow_denoise_params {
+    pub levels: u32,
+    pub sigma_color: f64, pub sigma_normal: f64, pub sigma_depth: f64,
+    pub alpha: u8, pub reserved: [u8; 7],
+}
+
 /// int (*)(void* user, uint32_t pass, uint32_t n_passes, uint32_t spp_done, const uint8_t* rgba); non-zero return cancels
 pub type rtiow_progress_fn = unsafe extern "C" fn(user: *mut c_void, pass: u32, n_passes: u32, spp_done: u32, rgba: *const u8) -> c_int;
 
@@ -110,6 +118,10 @@ extern "C" {
                             out_albedo: *mut f32, out_normal: *mut f32, out_depth: *mut f32, stats: *mut rtiow_stats) -> c_int;
     pub fn rtiow_render_adaptive(ctx: *mut rtiow_ctx, cam: *const rtiow_camera, p: *const rtiow_params, min_spp: u32, tolerance: f64,
                                  out_rgba: *mut u8, out_spp: *mut u32, out_error: *mut f32, stats: *mut rtiow_stats) -> c_int;
+    pub fn rtiow_denoise_params_default(dp: *mut rtiow_denoise_params);
+    pub fn rtiow_denoise(ctx: *mut rtiow_ctx, width: u32, height: u32, color: *const f32, albedo: *const f32, normal: *const f32,
+                         depth: *const f32, dp: *const rtiow_denoise_params, out_color: *mut f32, out_rgba: *mut u8,
+                         stats: *mut rtiow_stats) -> c_int;
     pub fn rtiow_render_views(ctx: *mut rtiow_ctx, cams: *const rtiow_camera, n_views: u32, p: *const rtiow_params, out_rgba: *mut u8,
                               stats: *mut rtiow_stats) -> c_int;
     pub fn rtiow_render_progressive(ctx: *mut rtiow_ctx, cam: *const rtiow_camera, p: *const rtiow_params, n_passes: u32,

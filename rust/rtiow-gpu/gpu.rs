@@ -122,6 +122,34 @@ pub fn render_adaptive(cam: &Camera, world: &HittableList, p: &RenderParams, min
     }
 }
 
+/// The parameters of `denoise`: the defaults the library chose on the final scene (`rtiow_denoise_params_default`).
+pub fn default_denoise_params() -> sys::rtiow_denoise_params {
+    let mut dp = sys::rtiow_denoise_params::default();
+    unsafe { sys::rtiow_denoise_params_default(&mut dp) };
+    dp
+}
+
+/// An edge-avoiding a-trous denoiser over `render_aov`'s buffers (include/rtiow_cuda.h, rtiow_denoise): returns the denoised
+/// linear colour (3 floats per pixel) and its top-down RGBA8 frame.  Runs on GPU 0 and needs no scene.
+pub fn denoise(width: u32, height: u32, aovs: &Aovs, dp: &sys::rtiow_denoise_params) -> Result<(Vec<f32>, Vec<u8>), RenderError> {
+    let n = width as usize * height as usize;
+    if aovs.color.len() != 3 * n || aovs.albedo.len() != 3 * n || aovs.normal.len() != 3 * n || aovs.depth.len() != n {
+        return Err(RenderError::InvalidArg("denoise: AOV buffers do not match width x height".into()));
+    }
+    unsafe {
+        let mut raw: *mut sys::rtiow_ctx = ptr::null_mut();
+        let rc = sys::rtiow_ctx_create(1, &mut raw);
+        if rc != sys::RTIOW_OK { return Err(err(rc)); }
+        let ctx = Ctx(raw);
+        let mut color = vec![0.0f32; 3 * n];
+        let mut pixels = vec![0u8; 4 * n];
+        let rc = sys::rtiow_denoise(ctx.0, width, height, aovs.color.as_ptr(), aovs.albedo.as_ptr(), aovs.normal.as_ptr(), aovs.depth.as_ptr(),
+                                    dp, color.as_mut_ptr(), pixels.as_mut_ptr(), ptr::null_mut());
+        if rc != sys::RTIOW_OK { return Err(err(rc)); }
+        Ok((color, pixels))
+    }
+}
+
 /// The same frame in `n_passes` slices of the samples, with the frame so far handed to `on_pass(pass, n_passes, spp_done, rgba)`
 /// after each — the role of the indicatif bar (main.rs:120,124) and the piston preview window (main.rs:151-171).  The returned
 /// frame is bit-identical to `render`'s.  `on_pass` returning `true` stops the render: `Err(RenderError::Cancelled)`.
