@@ -762,10 +762,10 @@ template <typename T> static void size_fetch(RenderArgs<T>& a, int grid, int thr
     a.guided_div = (uint32_t)std::max<uint64_t>(1, 2 * n_warps);
 }
 
-// a persistent render kernel: as many CTAs as fit on the SMs at once.  `extra` is the kernel's argument after RenderArgs, if any:
-// the device array of the cameras for a batch of views (render_views_kernel), the AOV accumulators (render_aov_kernel), the
-// round's pixel list and noise sums (render_adaptive_kernel)
-template <typename T, typename K, typename... V> static int launch_persistent(K kernel, RenderArgs<T>& a, int threads, size_t smem, int sms, cudaStream_t st, V... extra)
+// a persistent render kernel: as many CTAs as fit on the SMs at once.  Each kind of launch (Loop) reads the arguments after
+// RenderArgs that it needs and ignores the others.
+template <typename T, typename K>
+static int launch_persistent(K kernel, RenderArgs<T>& a, int threads, size_t smem, int sms, cudaStream_t st, const CameraT<T>* cams, AovArgs aov, AdaptArgs ad)
 {
     int rc = allow_smem(kernel, smem); if (rc) return rc;
     int per_sm = 0;
@@ -773,50 +773,33 @@ template <typename T, typename K, typename... V> static int launch_persistent(K 
     if (per_sm < 1) return fail(RTIOW_ERR_CUDA, "kernel does not fit on an SM (smem %zu)", smem);
     const int grid = per_sm * sms;
     size_fetch(a, grid, threads);
-    kernel<<<grid, threads, smem, st>>>(a, extra...);
+    kernel<<<grid, threads, smem, st>>>(a, cams, aov, ad);
     return RTIOW_OK;
 }
 
-// What a render launch produces, which picks the kernel of a scan arm (the same loop, rt_render.cuh): a frame, a batch of views,
-// a frame with its first-hit AOVs, or one round of an adaptive frame
-enum class Loop { Frame, Views, Aov, Adaptive };
-template <Loop L, typename T, bool kSmem, int kThreads, int kMinCtas> static auto render_entry()
-{
-    if constexpr (L == Loop::Views) return render_views_kernel<T, kSmem, kThreads, kMinCtas>;
-    else if constexpr (L == Loop::Aov) return render_aov_kernel<T, kSmem, kThreads, kMinCtas>;
-    else if constexpr (L == Loop::Adaptive) return render_adaptive_kernel<T, kSmem, kThreads, kMinCtas>;
-    else return render_kernel<T, kSmem, kThreads, kMinCtas>;
-}
-template <Loop L> static auto render_entry_umma()
-{
-    if constexpr (L == Loop::Views) return render_views_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
-    else if constexpr (L == Loop::Aov) return render_aov_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
-    else if constexpr (L == Loop::Adaptive) return render_adaptive_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
-    else return render_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK>;
-}
-
-template <Loop L, typename T, typename... V>
-static int launch_render_kernel(const ScanPlan& plan, const DeviceState& d, RenderArgs<T>& a, cudaStream_t st, V... extra)
+template <Loop L, typename T>
+static int launch_render_kernel(const ScanPlan& plan, const DeviceState& d, RenderArgs<T>& a, cudaStream_t st, const CameraT<T>* cams, AovArgs aov,
+                                AdaptArgs ad)
 {
     if constexpr (std::is_same<T, double>::value) {
-        return launch_persistent(render_entry<L, double, false, 256, 2>(), a, 256, plan.smem(256), d.sms, st, extra...);
+        return launch_persistent(render_kernel<double, false, 256, 2, L>, a, 256, plan.smem(256), d.sms, st, cams, aov, ad);
     } else {
         switch (plan.scan) {
         case Scan::Tensor: {     // one CTA per SM (it owns all of TMEM), G groups of 128 rays + G issuer warps
-            auto k = render_entry_umma<L>();
+            auto k = render_kernel_umma<RT_UMMA_GROUPS, RT_UMMA_CHUNK, L>;
             const size_t smem = plan.smem(UShape::kRenderThreads);
             int rc = allow_smem(k, smem); if (rc) return rc;
             size_fetch(a, d.sms, UShape::kRayThreads);          // the work is shared among the ray threads, not the whole block
-            k<<<d.sms, UShape::kRenderThreads, smem, st>>>(a, extra...);
+            k<<<d.sms, UShape::kRenderThreads, smem, st>>>(a, cams, aov, ad);
             return RTIOW_OK;
         }
         case Scan::Smem:         // 3 CTAs x 256 threads x 80 registers fills the 64K-register file
-            return launch_persistent(render_entry<L, float, true, 256, 3>(), a, 256, plan.smem(256), d.sms, st, extra...);
+            return launch_persistent(render_kernel<float, true, 256, 3, L>, a, 256, plan.smem(256), d.sms, st, cams, aov, ad);
         case Scan::Wide:         // one CTA per SM, 24 warps at 80 registers (+2.5 % over 512 threads at 104) when their lists fit
-            if (plan.smem(768) <= 227 * 1024) return launch_persistent(render_entry<L, float, true, 768, 1>(), a, 768, plan.smem(768), d.sms, st, extra...);
-            return launch_persistent(render_entry<L, float, true, 512, 1>(), a, 512, plan.smem(512), d.sms, st, extra...);
+            if (plan.smem(768) <= 227 * 1024) return launch_persistent(render_kernel<float, true, 768, 1, L>, a, 768, plan.smem(768), d.sms, st, cams, aov, ad);
+            return launch_persistent(render_kernel<float, true, 512, 1, L>, a, 512, plan.smem(512), d.sms, st, cams, aov, ad);
         case Scan::Global:
-            return launch_persistent(render_entry<L, float, false, 256, 4>(), a, 256, plan.smem(256), d.sms, st, extra...);
+            return launch_persistent(render_kernel<float, false, 256, 4, L>, a, 256, plan.smem(256), d.sms, st, cams, aov, ad);
         case Scan::F64:
             break;
         }
@@ -825,8 +808,19 @@ static int launch_render_kernel(const ScanPlan& plan, const DeviceState& d, Rend
 }
 
 // where a device's epilogue stores its pixels: its rows in rank-local order into a tile buffer, or into their top-down places in
-// a whole frame that may live on another GPU (fused quantise + gather: finalize_to_frame_kernel)
+// a whole frame that may live on another GPU (fused quantise + gather)
 struct Dest { uint32_t* p; bool whole_frame; };
+
+// The quantising epilogue (finalize_kernel) of device `rank`'s n_lp pixels into `dst`: each at `spp` samples, or at its own count
+// spp_px[i] when spp_px is given.  A tile buffer keeps rank-local order, which is the partition (1, 0).
+static int finalize_into(Dest dst, const DeviceState& d, const rtiow_params* p, uint32_t rank, uint32_t world, uint32_t n_lp, uint32_t spp,
+                         const uint32_t* spp_px, cudaStream_t st)
+{
+    const uint32_t w = dst.whole_frame ? world : 1u, r = dst.whole_frame ? rank : 0u;
+    finalize_kernel<<<(unsigned)(((uint64_t)n_lp + 255) / 256), 256, 0, st>>>(d.accum.p, n_lp, spp, spp_px, p->alpha, p->width, tile_rows_of(p), w, r, dst.p);
+    CU(cudaGetLastError());
+    return RTIOW_OK;
+}
 
 // The arguments of a render launch over samples `sr` of `local_rows` rows (rank `rank` of `world`, or a batch of views) of
 // every pixel; d.accum must hold 3 x local_rows x width sums.
@@ -850,16 +844,16 @@ static RenderArgs<T> render_args(const DeviceState& d, const rtiow_camera* cam, 
     return a;
 }
 
-// n_views = 0: a frame (or a rank's rows of one) of camera *cam.  n_views > 0 (world 1): a batch of views, the cameras
-// cam[0 .. n_views), rendered as one frame n_views * height rows tall whose epilogue writes the views' frames one after the other.
-// aov (n_views = 0): the launch also records every camera ray's first hit (render_aov_kernel) and a second epilogue turns the sums
-// into the float buffers of d.aov_out (finalize_aov_kernel), in this device's local row order.
-// *paths: the paths launched, local rows x width x samples.
+// The render launch of `loop` (the one place where a Loop chosen at run time picks its kernel) and its epilogue.  Frame: a frame
+// (or a rank's rows of one) of camera *cam.  Views (world 1): a batch of n_views views, the cameras cam[0 .. n_views), rendered
+// as one frame n_views * height rows tall whose epilogue writes the views' frames one after the other.  Aov: the launch also
+// records every camera ray's first hit and a second epilogue turns the sums into the float buffers of d.aov_out
+// (finalize_aov_kernel), in this device's local row order.  *paths: the paths launched, local rows x width x samples.
 template <typename T>
 static int launch_render(const ScanPlan& plan, DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, uint32_t rank, uint32_t world, SampleRange sr,
-                         Dest dst, cudaStream_t st, uint32_t* launches, uint64_t* paths, uint32_t n_views, bool aov)
+                         Dest dst, cudaStream_t st, uint32_t* launches, uint64_t* paths, Loop loop, uint32_t n_views)
 {
-    const uint32_t local_rows = n_views ? n_views * p->height : rows_of_rank(p->height, tile_rows_of(p), world, rank);
+    const uint32_t local_rows = loop == Loop::Views ? n_views * p->height : rows_of_rank(p->height, tile_rows_of(p), world, rank);
     const uint64_t n_lp = (uint64_t)local_rows * p->width;
     *paths = n_lp * sr.count;
     CU(d.accum.resize(3 * n_lp));
@@ -869,30 +863,26 @@ static int launch_render(const ScanPlan& plan, DeviceState& d, const rtiow_camer
     if (n_lp == 0) return RTIOW_OK;
     d.last_backend = plan.scan == Scan::Tensor ? RTIOW_SCAN_TENSOR : RTIOW_SCAN_FP32;
     int rc;
-    if (n_views) {              // the cameras go up in one copy; only a path's first ray reads its view's camera
+    if (loop == Loop::Views) {  // the cameras go up in one copy; only a path's first ray reads its view's camera
         const size_t bytes = (size_t)n_views * sizeof(CameraT<T>);
         CU(d.cams_stage.resize(bytes)); CU(d.cams.resize(bytes));
         CameraT<T>* staged = reinterpret_cast<CameraT<T>*>(d.cams_stage.p);
         for (uint32_t v = 0; v < n_views; ++v) staged[v] = to_dev_camera<T>(cam[v]);
         CU(cudaMemcpyAsync(d.cams.p, staged, bytes, cudaMemcpyHostToDevice, st));
-        rc = launch_render_kernel<Loop::Views>(plan, d, a, st, reinterpret_cast<const CameraT<T>*>(d.cams.p));
-    } else if (aov) {
+        rc = launch_render_kernel<Loop::Views, T>(plan, d, a, st, reinterpret_cast<const CameraT<T>*>(d.cams.p), AovArgs{}, AdaptArgs{});
+    } else if (loop == Loop::Aov) {
         CU(d.aov_sum.resize(7 * n_lp)); CU(d.aov_hits.resize(n_lp)); CU(d.aov_out.resize(10 * n_lp));
         CU(cudaMemsetAsync(d.aov_sum.p, 0, 7 * n_lp * sizeof(unsigned long long), st));
         CU(cudaMemsetAsync(d.aov_hits.p, 0, n_lp * sizeof(unsigned int), st));
-        rc = launch_render_kernel<Loop::Aov>(plan, d, a, st, AovArgs{ d.aov_sum.p, d.aov_hits.p });
+        rc = launch_render_kernel<Loop::Aov, T>(plan, d, a, st, nullptr, AovArgs{ d.aov_sum.p, d.aov_hits.p }, AdaptArgs{});
     } else {
-        rc = launch_render_kernel<Loop::Frame>(plan, d, a, st);
+        rc = launch_render_kernel<Loop::Frame, T>(plan, d, a, st, nullptr, AovArgs{}, AdaptArgs{});
     }
     if (rc) return rc;
     CU(cudaGetLastError());
-    if (dst.whole_frame)
-        finalize_to_frame_kernel<<<(unsigned)((n_lp + 255) / 256), 256, 0, st>>>(d.accum.p, (uint32_t)n_lp, sr.begin + sr.count, p->alpha, p->width, tile_rows_of(p), world, rank, dst.p);
-    else
-        finalize_kernel<<<(unsigned)((n_lp + 255) / 256), 256, 0, st>>>(d.accum.p, (uint32_t)n_lp, sr.begin + sr.count, p->alpha, dst.p);
-    CU(cudaGetLastError());
+    rc = finalize_into(dst, d, p, rank, world, (uint32_t)n_lp, sr.begin + sr.count, nullptr, st); if (rc) return rc;
     *launches += 2;
-    if (aov) {
+    if (loop == Loop::Aov) {
         finalize_aov_kernel<<<(unsigned)((n_lp + 255) / 256), 256, 0, st>>>(d.accum.p, d.aov_sum.p, d.aov_hits.p, (uint32_t)n_lp, sr.begin + sr.count, d.aov_out.p);
         CU(cudaGetLastError());
         ++*launches;
@@ -926,7 +916,7 @@ struct Part {
 };
 
 // ---- rtiow_render_adaptive ---------------------------------------------------------------------------------------------
-// One round on one device: samples `sr` of the n_act pixels of `list` (render_adaptive_kernel), then the select kernel, which
+// One round on one device: samples `sr` of the n_act pixels of `list` (Loop::Adaptive), then the select kernel, which
 // gives each of them its count sr.begin + sr.count and its error, and the compact kernel, which writes the pixels that stay
 // active to `next`, in order, and their number to d.adapt_n.  The ray counter is not reset: it adds up over the rounds.
 template <typename T>
@@ -938,7 +928,7 @@ static int adaptive_round(const ScanPlan& plan, DeviceState& d, const rtiow_came
     RenderArgs<T> a = render_args<T>(d, cam, p, rank, world, sr, local_rows);
     a.n_chunks = (uint64_t)n_act * a.chunks_per_pixel;
     CU(cudaMemsetAsync(d.counters.p, 0, sizeof(unsigned long long), st));           // the work counter only
-    int rc = launch_render_kernel<Loop::Adaptive>(plan, d, a, st, AdaptArgs{ list, d.adapt_lum.p }); if (rc) return rc;
+    int rc = launch_render_kernel<Loop::Adaptive, T>(plan, d, a, st, nullptr, AovArgs{}, AdaptArgs{ list, d.adapt_lum.p }); if (rc) return rc;
     CU(cudaGetLastError());
     const uint32_t blocks = (n_act + RT_ADAPT_BLOCK - 1) / RT_ADAPT_BLOCK, n = sr.begin + sr.count;
     adapt_select_kernel<<<blocks, RT_ADAPT_BLOCK, 0, st>>>(list, n_act, d.adapt_lum.p, n_lp, n, p->spp, tol, d.adapt_spp.p, d.adapt_err.p, d.adapt_blocks.p);
@@ -1014,31 +1004,13 @@ static int adaptive_rounds(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_pa
     }
 }
 
-// the epilogue of rtiow_render_adaptive on one device: its pixels quantised at their own counts (d.adapt_spp), into `dst` as
-// launch_render's epilogue stores a frame's.  *paths: the paths of the rounds.
-static int finalize_adaptive(DeviceState& d, const rtiow_params* p, uint32_t rank, uint32_t world, Dest dst, cudaStream_t st, uint32_t* launches,
-                             uint64_t* paths)
-{
-    const uint32_t n_lp = rows_of_rank(p->height, tile_rows_of(p), world, rank) * p->width;
-    *paths = d.adapt_paths;
-    if (n_lp == 0) return RTIOW_OK;
-    const unsigned blocks = (n_lp + 255) / 256;
-    if (dst.whole_frame)
-        finalize_adaptive_to_frame_kernel<<<blocks, 256, 0, st>>>(d.accum.p, n_lp, d.adapt_spp.p, p->alpha, p->width, tile_rows_of(p), world, rank, dst.p);
-    else
-        finalize_adaptive_kernel<<<blocks, 256, 0, st>>>(d.accum.p, n_lp, d.adapt_spp.p, p->alpha, dst.p);
-    CU(cudaGetLastError());
-    ++*launches;
-    return RTIOW_OK;
-}
-
 // One device's part of a frame: samples `sr` of the rows {y : (y / tile_rows) % world == rank}, quantised into `dst`, with the
-// events e0 / e1 around the work and its kernel launches added to *launches.  n_views > 0: the batch of views cam[0 .. n_views)
-// (launch_render).  aov: the frame's first-hit AOVs too, left in d.aov_out (launch_render).  adaptive: the rounds of
-// rtiow_render_adaptive already ran (adaptive_rounds); only their epilogue is left (finalize_adaptive).
+// events e0 / e1 around the work and its kernel launches added to *launches.  Frame, Views (the n_views cameras cam[0 .. n_views))
+// and Aov: launch_render.  Adaptive: the rounds of rtiow_render_adaptive already ran (adaptive_rounds); only their epilogue is
+// left, which quantises each pixel at its own count (d.adapt_spp).
 static int render_step(const rtiow_ctx* c, DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, uint32_t rank, uint32_t world, SampleRange sr,
-                       Dest dst, cudaStream_t st, cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches, Part* part, uint32_t n_views = 0, bool aov = false,
-                       bool adaptive = false)
+                       Dest dst, cudaStream_t st, cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches, Part* part, Loop loop = Loop::Frame,
+                       uint32_t n_views = 0)
 {
     if (!d.has_scene) return fail(RTIOW_ERR_INVALID_ARG, "no scene uploaded (call rtiow_scene_upload first)");
     CU(cudaSetDevice(d.device));
@@ -1046,9 +1018,14 @@ static int render_step(const rtiow_ctx* c, DeviceState& d, const rtiow_camera* c
     int rc = plan_scan(c, d, p->precision, &plan); if (rc) return rc;
     *part = Part{ &d, st, e0, e1 };
     CU(cudaEventRecord(e0, st));
-    if (adaptive) { part->ms_before = d.adapt_ms; rc = finalize_adaptive(d, p, rank, world, dst, st, launches, &part->paths); }
-    else rc = plan.scan == Scan::F64 ? launch_render<double>(plan, d, cam, p, rank, world, sr, dst, st, launches, &part->paths, n_views, aov)
-                                     : launch_render<float>(plan, d, cam, p, rank, world, sr, dst, st, launches, &part->paths, n_views, aov);
+    if (loop == Loop::Adaptive) {
+        const uint32_t n_lp = rows_of_rank(p->height, tile_rows_of(p), world, rank) * p->width;
+        part->ms_before = d.adapt_ms; part->paths = d.adapt_paths;
+        if (n_lp) { rc = finalize_into(dst, d, p, rank, world, n_lp, 0u, d.adapt_spp.p, st); ++*launches; }
+    } else {
+        rc = plan.scan == Scan::F64 ? launch_render<double>(plan, d, cam, p, rank, world, sr, dst, st, launches, &part->paths, loop, n_views)
+                                    : launch_render<float>(plan, d, cam, p, rank, world, sr, dst, st, launches, &part->paths, loop, n_views);
+    }
     if (rc) return rc;
     CU(cudaEventRecord(e1, st));
     return RTIOW_OK;
@@ -1056,11 +1033,11 @@ static int render_step(const rtiow_ctx* c, DeviceState& d, const rtiow_camera* c
 
 // a frame on one device: its rank-local order IS top-down (and a batch of n_views views is their frames one after the other)
 static int render_single(const rtiow_ctx* c, DeviceState& d, const rtiow_camera* cam, const rtiow_params* p, SampleRange sr, cudaStream_t st,
-                         cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches, Part* part, const uint32_t** d_frame, uint32_t n_views = 0, bool aov = false,
-                         bool adaptive = false)
+                         cudaEvent_t e0, cudaEvent_t e1, uint32_t* launches, Part* part, const uint32_t** d_frame, Loop loop = Loop::Frame,
+                         uint32_t n_views = 0)
 {
     CU(d.tiles.resize((size_t)p->width * p->height * std::max<uint32_t>(n_views, 1)));
-    int rc = render_step(c, d, cam, p, 0, 1, sr, Dest{ d.tiles.p, false }, st, e0, e1, launches, part, n_views, aov, adaptive); if (rc) return rc;
+    int rc = render_step(c, d, cam, p, 0, 1, sr, Dest{ d.tiles.p, false }, st, e0, e1, launches, part, loop, n_views); if (rc) return rc;
     *d_frame = d.tiles.p;
     return RTIOW_OK;
 }
@@ -1112,7 +1089,7 @@ static int finish_call(Part* parts, size_t n, double t0, uint32_t launches, uint
 }
 
 // shared body of the two per-rank entry points: this rank's rows into a tile buffer (rank-local order), or — with `to_frame` —
-// straight into their top-down place in a whole frame that may live on another GPU (finalize_to_frame_kernel)
+// straight into their top-down place in a whole frame that may live on another GPU (finalize_kernel under the partition)
 static int render_rank(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_params* p, int rank, int world, void* dst, bool to_frame, void* stream,
                        rtiow_stats* stats)
 {
@@ -1219,16 +1196,17 @@ static int render_frame(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_param
     DeviceState& d0 = c->dev[0];
     uint32_t launches = 0;
     uint64_t extra_d2h = 0;
+    const Loop loop = adapt ? Loop::Adaptive : aov ? Loop::Aov : Loop::Frame;
     if (adapt) { rc = adaptive_rounds(c, cam, p, adapt->min_spp, adapt->tolerance, &launches, &extra_d2h); if (rc) return rc; }
     CU(cudaSetDevice(d0.device));
     std::vector<Part> parts(world);
     const uint32_t* d_final = nullptr;
     if (world == 1) {
-        rc = render_single(c, d0, cam, p, sr, d0.stream, d0.ev0, d0.ev1, &launches, &parts[0], &d_final, 0, aov != nullptr, adapt != nullptr); if (rc) return rc;
+        rc = render_single(c, d0, cam, p, sr, d0.stream, d0.ev0, d0.ev1, &launches, &parts[0], &d_final, loop); if (rc) return rc;
     } else {
         // interleaved row tiles on every GPU.  Three gathers:
         //   fused (default with NVLink peer access, every B200 box): each rank's epilogue stores its pixels straight into device
-        //     0's top-down frame (finalize_to_frame_kernel): compute and gather are one kernel, nothing is staged;
+        //     0's top-down frame (finalize_kernel): compute and gather are one kernel, nothing is staged;
         //   NCCL (rtiow_ctx_set_gather(RTIOW_GATHER_NCCL); SURVEY §8e): ncclCommInitAll once, then per frame one grouped
         //     ncclAllGather of the equal-size (padded) tile buffers + the de-interleave kernel on device 0;
         //   without peer access and without NCCL: tile buffers + cudaMemcpyPeerAsync + de-interleave.
@@ -1250,7 +1228,7 @@ static int render_frame(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_param
             Dest dst{ d0.frame.p, true };
             if (use_nccl) { CU(d.tiles.resize(tile_px)); CU(d.gathered.resize(tile_px * world)); dst = Dest{ d.tiles.p, false }; }
             else if (!fused) { if (r == 0) dst = Dest{ d0.gathered.p, false }; else { CU(d.tiles.resize(tile_px)); dst = Dest{ d.tiles.p, false }; } }
-            rc = render_step(c, d, cam, p, r, world, sr, dst, d.stream, d.ev0, d.ev1, &launches, &parts[r], 0, aov != nullptr, adapt != nullptr); if (rc) return rc;
+            rc = render_step(c, d, cam, p, r, world, sr, dst, d.stream, d.ev0, d.ev1, &launches, &parts[r], loop); if (rc) return rc;
             if (r != 0 && !use_nccl) {
                 if (!fused) {
                     const size_t bytes = (size_t)rows_of_rank(p->height, tile_rows_of(p), world, r) * p->width * 4;
@@ -1302,8 +1280,8 @@ extern "C" int rtiow_render(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_p
 }
 
 // A frame exactly as rtiow_render renders it, plus the float buffers a denoiser takes: the frame's own sums as linear colour and
-// the first hit of every camera ray (rt_render.cuh, record_first_hit).  Only the render kernel (render_aov_kernel: the frame's
-// loop with kAov) and one more epilogue (finalize_aov_kernel) differ from rtiow_render; with every float buffer NULL the call
+// the first hit of every camera ray (rt_render.cuh, record_first_hit).  Only the render kernel (the frame's loop as Loop::Aov)
+// and one more epilogue (finalize_aov_kernel) differ from rtiow_render; with every float buffer NULL the call
 // is rtiow_render.  An n-GPU ctx renders its interleaved row tiles as rtiow_render does and each device copies its rows of the
 // float buffers to their top-down places.
 extern "C" int rtiow_render_aov(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_params* p, uint8_t* out_rgba, float* out_color, float* out_albedo,
@@ -1359,7 +1337,7 @@ extern "C" int rtiow_render_views(rtiow_ctx* c, const rtiow_camera* cams, uint32
         CU(cudaSetDevice(d.device));
         const uint32_t* d_frames = nullptr;
         Part part;
-        rc = render_single(c, d, cams + v0, p, SampleRange{ 0u, p->spp }, d.stream, d.ev0, d.ev1, &launches, &part, &d_frames, v1 - v0); if (rc) return rc;
+        rc = render_single(c, d, cams + v0, p, SampleRange{ 0u, p->spp }, d.stream, d.ev0, d.ev1, &launches, &part, &d_frames, Loop::Views, v1 - v0); if (rc) return rc;
         rc = part.start_copy(out_rgba + v0 * frame_bytes, d_frames, (v1 - v0) * frame_bytes); if (rc) return rc;
         parts.push_back(part);
     }

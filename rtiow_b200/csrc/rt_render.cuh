@@ -38,7 +38,14 @@ template <typename T> struct RenderArgs {
 
 #define RT_FIX_SCALE 4294967296.0f   // 2^32
 
-// The first-hit accumulators of rtiow_render_aov (render_aov_kernel), beside RenderArgs::accum and over the same local pixels.
+// What a render launch produces; every kind runs the same loop (render_kernel, render_kernel_umma):
+//   Frame     a frame, or a rank's rows of one;
+//   Views     a batch of views on one device, one camera per view in `cams` (rtiow_render_views);
+//   Aov       a frame, and every camera ray's first hit in `aov` (AovArgs, rtiow_render_aov);
+//   Adaptive  one round of rtiow_render_adaptive: the pixels of `ad.list` only, with their noise sums (AdaptArgs).
+enum class Loop { Frame, Views, Aov, Adaptive };
+
+// The first-hit accumulators of rtiow_render_aov (Loop::Aov), beside RenderArgs::accum and over the same local pixels.
 // Every camera ray adds one fixed-point sample per channel with an integer RED.ADD, so the AOVs are bit-identical for any grid,
 // chunking or GPU count.  Each per-sample value is clamped to a range whose sum over 2^32 - 1 samples stays below 2^64, so no
 // sum can wrap at any spp and none needs add_saturating:
@@ -47,7 +54,9 @@ template <typename T> struct RenderArgs {
 //   depth   [n_lp]     per sample in [0, 65536] scene units, scale 2^16 (resolution 1.5e-5);
 //   hits    [n_lp]     camera rays that hit a sphere (32-bit: at most spp of them).
 // A miss adds its sky value to the albedo and nothing else, so finalize_aov_kernel removes the offset of the hits alone.
-struct AovArgs {
+// 16-byte aligned: as a kernel parameter after the 8-byte `cams` it still starts on a 16-byte boundary, so the render loop
+// loads both pointers with one 128-bit constant load.
+struct __align__(16) AovArgs {
     unsigned long long* sum;       // [7][n_lp]: albedo r, g, b, normal x, y, z, depth
     unsigned int* hits;            // [n_lp]
 };
@@ -55,7 +64,7 @@ struct AovArgs {
 #define RT_AOV_DEPTH_SCALE 65536.0         // 2^16
 #define RT_AOV_DEPTH_MAX 65536.0           // a farther hit is recorded at this distance
 
-// One round of rtiow_render_adaptive (render_adaptive_kernel): the launch renders its sample range of the pixels in `list`
+// One round of rtiow_render_adaptive (Loop::Adaptive): the launch renders its sample range of the pixels in `list`
 // only (local pixel indices, n_chunks / chunks_per_pixel of them), and every finished non-black path also adds its noise value
 // y = clamp((r + g + b) / 3, 0, 1) to two per-pixel fixed-point sums, S1 += round(y 2^32) and S2 += round(y^2 2^32).  Each
 // value is at most 2^32, so neither sum can wrap at any u32 spp.  The pixels' own radiance sums stay RenderArgs::accum.
@@ -206,11 +215,11 @@ struct WorkCursor {
 
 // Every lane whose slot is free (`busy` false) takes the next (pixel, sample) of the warp's chunk (main.rs:130).  Returns
 // true for the lanes that received one; their pixel column / bottom-up row come back in *px, *pj.
-// kViews: the launch renders a batch of views (rtiow_render_views) on one device as ONE frame n_views * height rows tall, so
-// local row lr is row lr % height of view lr / height.  *pv receives the view; pj and the Philox pixel key are those of the
-// row within the view, exactly as the view's own frame computes them, which makes every view byte-identical to it.
-// kAdapt: chunk c belongs to pixel ad.list[c / chunks_per_pixel] (AdaptArgs), a round's subset of the pixels in the same order.
-template <bool kViews, bool kAdapt, typename T>
+// Loop::Views: the launch renders a batch of views on one device as ONE frame n_views * height rows tall, so local row lr is
+// row lr % height of view lr / height.  *pv receives the view; pj and the Philox pixel key are those of the row within the
+// view, exactly as the view's own frame computes them, which makes every view byte-identical to it.
+// Loop::Adaptive: chunk c belongs to pixel ad.list[c / chunks_per_pixel] (AdaptArgs), a round's subset of the pixels in the same order.
+template <Loop L, typename T>
 __device__ __forceinline__ bool assign_work(const RenderArgs<T>& a, const AdaptArgs& ad, WorkCursor& wc, unsigned lt_mask, bool busy, PathState<T>& ps,
                                             uint32_t& acc_lp, uint32_t* px, uint32_t* pj, uint32_t* pv)
 {
@@ -237,12 +246,12 @@ __device__ __forceinline__ bool assign_work(const RenderArgs<T>& a, const AdaptA
             const unsigned long long c = wc.cc++;
             const uint32_t pix = (uint32_t)(c / a.chunks_per_pixel);
             const uint32_t part = (uint32_t)(c - (unsigned long long)pix * a.chunks_per_pixel);
-            wc.c_lp = kAdapt ? ad.list[pix] : a.local_rows * a.width - 1u - pix;
+            wc.c_lp = L == Loop::Adaptive ? ad.list[pix] : a.local_rows * a.width - 1u - pix;
             wc.cs = part * a.chunk_samples; wc.ce = min(wc.cs + a.chunk_samples, a.spp);
             const uint32_t lr = wc.c_lp / a.width;
             wc.c_x = wc.c_lp - lr * a.width;
             wc.c_y = local_to_global_row(lr, a.tile_rows, a.world, a.rank);
-            if (kViews) { wc.c_v = lr / a.height; wc.c_y = lr - wc.c_v * a.height; }
+            if constexpr (L == Loop::Views) { wc.c_v = lr / a.height; wc.c_y = lr - wc.c_v * a.height; }
         }
         const uint32_t avail = wc.ce - wc.cs;
         const uint32_t r = __popc(need & lt_mask);
@@ -291,8 +300,8 @@ __device__ __forceinline__ void accumulate(const RenderArgs<T>& a, uint32_t acc_
 
 // Step 2 of the render iteration (below) for one lane: the camera ray of a fresh sample, or the scatter at the pending hit
 // on sphere hit_idx at ps.o.  Returns whether the lane has a ray for this iteration's scan.  The camera is a.cam, or with
-// kViews the camera of the sample's view pv.
-template <bool kViews, typename T>
+// Loop::Views the camera of the sample's view pv.
+template <Loop L, typename T>
 __device__ __forceinline__ bool next_ray(const RenderArgs<T>& a, const CameraT<T>* cams, PathState<T>& ps, bool fresh, bool pending, int hit_idx, int hit_code,
                                          uint32_t px, uint32_t pj, uint32_t pv)
 {
@@ -302,7 +311,7 @@ __device__ __forceinline__ bool next_ray(const RenderArgs<T>& a, const CameraT<T
     if (fresh) {
         const T su = (T(px) + u.u0) * a.inv_wm1;                 // main.rs:131
         const T sv = (T(pj) + u.u1) * a.inv_hm1;                 // main.rs:132
-        const CameraT<T>& cam = kViews ? cams[pv] : a.cam;
+        const CameraT<T>& cam = L == Loop::Views ? cams[pv] : a.cam;
         V3<T> ro, rd; get_ray(cam, su, sv, sa, sb, &ro, &rd);    // main.rs:134
         start_ray(ps, ro, rd, a.t_min);
         ps.thr = mk<T>(1, 1, 1); ps.self_code = RT_SELF_NONE;
@@ -366,19 +375,19 @@ __device__ __forceinline__ void accumulate_noise(const RenderArgs<T>& a, const A
 }
 
 // Step 4 for one lane after the scan found (t_hit, idx, code); on a hit the lane moves to the hit point and keeps the
-// sphere in *hit_idx, *hit_code.  Returns whether a scatter is now pending.  kAov: a camera ray (depth still max_depth)
-// also records its first hit (record_first_hit).  kAdapt: a path that ends on the sky also adds its noise value
+// sphere in *hit_idx, *hit_code.  Returns whether a scatter is now pending.  Loop::Aov: a camera ray (depth still max_depth)
+// also records its first hit (record_first_hit).  Loop::Adaptive: a path that ends on the sky also adds its noise value
 // (accumulate_noise); paths that end black add nothing anywhere.
-template <bool kAov, bool kAdapt, typename T>
+template <Loop L, typename T>
 __device__ __forceinline__ bool take_hit(const RenderArgs<T>& a, const AovArgs& aov, const AdaptArgs& ad, PathState<T>& ps, bool active, uint32_t acc_lp,
                                          T t_hit, int idx, int code, int* hit_idx, int* hit_code)
 {
     if (!active) return false;
-    if (kAov && ps.depth == a.max_depth) record_first_hit(a, aov, ps, acc_lp, t_hit, idx);
+    if (L == Loop::Aov && ps.depth == a.max_depth) record_first_hit(a, aov, ps, acc_lp, t_hit, idx);
     if (idx < 0) {                                                                                        // miss: sky (main.rs:54-56)
         const V3<T> rad = ps.thr * sky<T, sizeof(T) == 4>(ps.dhat);
         accumulate(a, acc_lp, rad);
-        if (kAdapt) accumulate_noise(a, ad, acc_lp, rad);
+        if constexpr (L == Loop::Adaptive) accumulate_noise(a, ad, acc_lp, rad);
         return false;
     }
     ps.o = ps.o + ps.dhat * t_hit; *hit_idx = idx; *hit_code = code;                                    // ray.rs:15-17
@@ -392,11 +401,8 @@ __device__ __forceinline__ bool take_hit(const RenderArgs<T>& a, const AovArgs& 
 //      common part runs once, converged, instead of once per divergent branch;
 //   3. the scan (world.hit) for all 32 lanes;
 //   4. miss -> throughput x sky is added to the pixel and the lane is free again; hit -> the lane keeps the hit for step 2.
-// Steps 2 and 4 are next_ray and take_hit, which the tensor-core kernel below calls too.  render_kernel renders a frame
-// (or a rank's rows of one); render_views_kernel runs the same loop over a batch of views, one camera per view in `cams`;
-// render_aov_kernel renders a frame and records every camera ray's first hit in `aov` (AovArgs); render_adaptive_kernel renders
-// one round of rtiow_render_adaptive: the pixels of `ad.list` only, with their noise sums (AdaptArgs).
-template <typename T, bool kSmem, int kThreads, bool kViews, bool kAov, bool kAdapt>
+// Steps 2 and 4 are next_ray and take_hit, which the tensor-core kernel below calls too.  L is what the launch produces (Loop).
+template <typename T, bool kSmem, int kThreads, Loop L>
 __device__ __forceinline__ void render_loop(const RenderArgs<T>& a, const CameraT<T>* cams, const AovArgs& aov, const AdaptArgs& ad)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -414,37 +420,23 @@ __device__ __forceinline__ void render_loop(const RenderArgs<T>& a, const Camera
 
     for (;;) {
         uint32_t px = 0, pj = 0, pv = 0;
-        const bool fresh = assign_work<kViews, kAdapt>(a, ad, wc, lt_mask, pending, ps, acc_lp, &px, &pj, &pv);
+        const bool fresh = assign_work<L>(a, ad, wc, lt_mask, pending, ps, acc_lp, &px, &pj, &pv);
         if (!__any_sync(RT_FULL, fresh || pending)) break;
 
-        const bool active = next_ray<kViews>(a, cams, ps, fresh, pending, hit_idx, hit_code, px, pj, pv);
+        const bool active = next_ray<L>(a, cams, ps, fresh, pending, hit_idx, hit_code, px, pj, pv);
         n_rays_w += __popc(__ballot_sync(RT_FULL, active));          // world.hit call count (main.rs:44)
         T t_hit; int idx, code;
         world_hit<T, kSmem>(a.scene, table, cand, kThreads, ps, &t_hit, &idx, &code);
-        pending = take_hit<kAov, kAdapt>(a, aov, ad, ps, active, acc_lp, t_hit, idx, code, &hit_idx, &hit_code);
+        pending = take_hit<L>(a, aov, ad, ps, active, acc_lp, t_hit, idx, code, &hit_idx, &hit_code);
     }
     if (lane == 0) atomicAdd(a.ray_counter, (unsigned long long)n_rays_w);
 }
 
-template <typename T, bool kSmem, int kThreads, int kMinCtas>
-__global__ void __launch_bounds__(kThreads, kMinCtas) render_kernel(const RenderArgs<T> a)
+template <typename T, bool kSmem, int kThreads, int kMinCtas, Loop L>
+__global__ void __launch_bounds__(kThreads, kMinCtas)
+render_kernel(const RenderArgs<T> a, const CameraT<T>* __restrict__ cams, const AovArgs aov, const AdaptArgs ad)
 {
-    render_loop<T, kSmem, kThreads, false, false, false>(a, nullptr, AovArgs{}, AdaptArgs{});
-}
-template <typename T, bool kSmem, int kThreads, int kMinCtas>
-__global__ void __launch_bounds__(kThreads, kMinCtas) render_views_kernel(const RenderArgs<T> a, const CameraT<T>* __restrict__ cams)
-{
-    render_loop<T, kSmem, kThreads, true, false, false>(a, cams, AovArgs{}, AdaptArgs{});
-}
-template <typename T, bool kSmem, int kThreads, int kMinCtas>
-__global__ void __launch_bounds__(kThreads, kMinCtas) render_aov_kernel(const RenderArgs<T> a, const AovArgs aov)
-{
-    render_loop<T, kSmem, kThreads, false, true, false>(a, nullptr, aov, AdaptArgs{});
-}
-template <typename T, bool kSmem, int kThreads, int kMinCtas>
-__global__ void __launch_bounds__(kThreads, kMinCtas) render_adaptive_kernel(const RenderArgs<T> a, const AdaptArgs ad)
-{
-    render_loop<T, kSmem, kThreads, false, false, true>(a, nullptr, AovArgs{}, ad);
+    render_loop<T, kSmem, kThreads, L>(a, cams, aov, ad);
 }
 
 // The same render loop with the sphere filter on the tensor cores (rt_umma_scan.cuh): G groups of 128 ray threads + G
@@ -453,7 +445,7 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) render_adaptive_kernel(con
 // filter's survivors and the f64 large-sphere test; only the filter moves from 7 FFMA2 per sphere pair to three
 // tcgen05.mma per 128 rays x NC spheres, and the warp-level "any lane alive" vote becomes a 128-thread one, because a
 // group's 128 rays form one MMA.
-template <int G, int NC, bool kViews, bool kAov, bool kAdapt>
+template <int G, int NC, Loop L>
 __device__ __forceinline__ void render_loop_umma(const RenderArgs<float>& a, const CameraT<float>* cams, const AovArgs& aov, const AdaptArgs& ad)
 {
     extern __shared__ __align__(1024) unsigned char smem_umma[];
@@ -477,54 +469,46 @@ __device__ __forceinline__ void render_loop_umma(const RenderArgs<float>& a, con
         for (;;) {
             uint32_t px = 0, pj = 0, pv = 0;
             RT_STAMP(1);
-            const bool fresh = assign_work<kViews, kAdapt>(a, ad, wc, lt_mask, pending, ps, acc_lp, &px, &pj, &pv);
+            const bool fresh = assign_work<L>(a, ad, wc, lt_mask, pending, ps, acc_lp, &px, &pj, &pv);
             RT_STAMP(2);
             if (!umma_group_any(ux, fresh || pending)) { umma_group_quit(ux); break; }
             RT_STAMP(3);
 
-            const bool active = next_ray<kViews>(a, cams, ps, fresh, pending, hit_idx, hit_code, px, pj, pv);
+            const bool active = next_ray<L>(a, cams, ps, fresh, pending, hit_idx, hit_code, px, pj, pv);
             n_rays_w += __popc(__ballot_sync(RT_FULL, active));              // world.hit call count (main.rs:44)
             RT_STAMP(4);
             const HitF h = closest_hit_umma<G, NC>(ux, a.scene, ps.o, ps.dhat, ps.tmin_n, ps.self_code, ps.self_n, active);
             RT_STAMP(9);
-            pending = take_hit<kAov, kAdapt>(a, aov, ad, ps, active, acc_lp, h.t, h.idx, h.code, &hit_idx, &hit_code);
+            pending = take_hit<L>(a, aov, ad, ps, active, acc_lp, h.t, h.idx, h.code, &hit_idx, &hit_code);
         }
         if (lane == 0) atomicAdd(a.ray_counter, (unsigned long long)n_rays_w);
     }
     umma_teardown(tmem_base);
 }
 
-template <int G, int NC>
-__global__ void __launch_bounds__(UmmaShape<G, NC>::kRenderThreads, 1) render_kernel_umma(const RenderArgs<float> a)
+template <int G, int NC, Loop L>
+__global__ void __launch_bounds__(UmmaShape<G, NC>::kRenderThreads, 1)
+render_kernel_umma(const RenderArgs<float> a, const CameraT<float>* __restrict__ cams, const AovArgs aov, const AdaptArgs ad)
 {
-    render_loop_umma<G, NC, false, false, false>(a, nullptr, AovArgs{}, AdaptArgs{});
-}
-template <int G, int NC>
-__global__ void __launch_bounds__(UmmaShape<G, NC>::kRenderThreads, 1) render_views_kernel_umma(const RenderArgs<float> a, const CameraT<float>* __restrict__ cams)
-{
-    render_loop_umma<G, NC, true, false, false>(a, cams, AovArgs{}, AdaptArgs{});
-}
-template <int G, int NC>
-__global__ void __launch_bounds__(UmmaShape<G, NC>::kRenderThreads, 1) render_aov_kernel_umma(const RenderArgs<float> a, const AovArgs aov)
-{
-    render_loop_umma<G, NC, false, true, false>(a, nullptr, aov, AdaptArgs{});
-}
-template <int G, int NC>
-__global__ void __launch_bounds__(UmmaShape<G, NC>::kRenderThreads, 1) render_adaptive_kernel_umma(const RenderArgs<float> a, const AdaptArgs ad)
-{
-    render_loop_umma<G, NC, false, false, true>(a, nullptr, AovArgs{}, ad);
+    render_loop_umma<G, NC, L>(a, cams, aov, ad);
 }
 
-// Color::to_rgba (vec3.rs:404-420) + the row flip (main.rs:141-145): fixed-point sums -> top-down
-// RGBA8 rows of this rank's tile buffer (rank-local row order).
-__global__ void finalize_kernel(const unsigned long long* __restrict__ accum, uint32_t n_lp, uint32_t spp, uint32_t alpha,
-                                uint32_t* __restrict__ out_rgba)
+// Color::to_rgba (vec3.rs:404-420) + the row flip (main.rs:141-145): fixed-point sums -> RGBA8, each pixel quantised at spp, or
+// at its own sample count spp_px[i] when spp_px is given (rtiow_render_adaptive).  Local pixel i is stored at its top-down place
+// in `out` under the partition (world, rank).  A tile buffer in rank-local row order is the partition (1, 0).  A whole frame
+// fuses the gather into the epilogue (single-process multi-GPU): `out` is then rank 0's frame, a peer pointer
+// (cudaDeviceEnablePeerAccess), so for ranks > 0 these are st.global over NVLink — no tile buffer, no copy, no de-interleave
+// pass.  Rows are written as whole 4-byte-per-pixel runs, i.e. coalesced 128-byte stores.
+__global__ void finalize_kernel(const unsigned long long* __restrict__ accum, uint32_t n_lp, uint32_t spp, const uint32_t* __restrict__ spp_px,
+                                uint32_t alpha, uint32_t width, uint32_t tile_rows, uint32_t world, uint32_t rank, uint32_t* __restrict__ out)
 {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_lp) return;
     const double k = 1.0 / 4294967296.0;
     const V3<double> sum = mk<double>((double)accum[i] * k, (double)accum[n_lp + i] * k, (double)accum[2 * (size_t)n_lp + i] * k);
-    out_rgba[i] = to_rgba<double>(sum, alpha, (uint64_t)spp);
+    const uint32_t lr = i / width, x = i - lr * width;
+    const uint32_t y = local_to_global_row(lr, tile_rows, world, rank);
+    out[(size_t)y * width + x] = to_rgba<double>(sum, alpha, (uint64_t)(spp_px ? spp_px[i] : spp));
 }
 
 // The float epilogue of rtiow_render_aov: the frame's sums and the AOV accumulators (AovArgs) -> per-pixel means in this
@@ -547,23 +531,7 @@ __global__ void finalize_aov_kernel(const unsigned long long* __restrict__ accum
     out[9 * (size_t)n_lp + i] = h ? (float)((double)aov_sum[6 * (size_t)n_lp + i] / (RT_AOV_DEPTH_SCALE * h)) : __int_as_float(0x7f800000);
 }
 
-// The same epilogue FUSED with the gather (single-process multi-GPU): each rank's quantised pixel is stored straight
-// into its top-down place in rank 0's frame.  `frame` is a peer pointer (cudaDeviceEnablePeerAccess), so for ranks > 0
-// these are st.global over NVLink — no tile buffer, no copy, no de-interleave pass.  Rows are written as whole
-// 4-byte-per-pixel runs, i.e. coalesced 128-byte stores.
-__global__ void finalize_to_frame_kernel(const unsigned long long* __restrict__ accum, uint32_t n_lp, uint32_t spp, uint32_t alpha,
-                                         uint32_t width, uint32_t tile_rows, uint32_t world, uint32_t rank, uint32_t* __restrict__ frame)
-{
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n_lp) return;
-    const double k = 1.0 / 4294967296.0;
-    const V3<double> sum = mk<double>((double)accum[i] * k, (double)accum[n_lp + i] * k, (double)accum[2 * (size_t)n_lp + i] * k);
-    const uint32_t lr = i / width, x = i - lr * width;
-    const uint32_t y = local_to_global_row(lr, tile_rows, world, rank);
-    frame[(size_t)y * width + x] = to_rgba<double>(sum, alpha, (uint64_t)spp);
-}
-
-// ---- rtiow_render_adaptive: the rounds' bookkeeping and the epilogue at per-pixel counts --------------------------------
+// ---- rtiow_render_adaptive: the rounds' bookkeeping (the epilogue is finalize_kernel at per-pixel counts) ---------------
 // The error of a pixel at a boundary of n samples (include/rtiow_cuda.h): with m = S1 2^-32 / n and q = S2 2^-32 / n,
 // err = 128 sqrt(max(0, q - m^2) / ((n - 1) max(m, 2^-16))), one standard error of the displayed value 256 sqrt(m) in 8-bit
 // levels; +inf for n = 1.  Every operation is rounded on its own (no contraction), so a restatement in IEEE double from the
@@ -643,31 +611,6 @@ __global__ void __launch_bounds__(RT_ADAPT_BLOCK) adapt_compact_kernel(const uin
     __syncthreads();
     if (keep) next[base + warp_n[warp] + __popc(kept & ((1u << lane) - 1u))] = list[i];
     if (blockIdx.x == gridDim.x - 1 && threadIdx.x == 0) *n_next = base + block_keep[blockIdx.x];
-}
-
-// finalize_kernel with each pixel quantised at its own sample count spp[i] (vec3.rs:404-420)
-__global__ void finalize_adaptive_kernel(const unsigned long long* __restrict__ accum, uint32_t n_lp, const uint32_t* __restrict__ spp, uint32_t alpha,
-                                         uint32_t* __restrict__ out_rgba)
-{
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n_lp) return;
-    const double k = 1.0 / 4294967296.0;
-    const V3<double> sum = mk<double>((double)accum[i] * k, (double)accum[n_lp + i] * k, (double)accum[2 * (size_t)n_lp + i] * k);
-    out_rgba[i] = to_rgba<double>(sum, alpha, (uint64_t)spp[i]);
-}
-
-// finalize_to_frame_kernel with each pixel quantised at its own sample count spp[i]
-__global__ void finalize_adaptive_to_frame_kernel(const unsigned long long* __restrict__ accum, uint32_t n_lp, const uint32_t* __restrict__ spp,
-                                                  uint32_t alpha, uint32_t width, uint32_t tile_rows, uint32_t world, uint32_t rank,
-                                                  uint32_t* __restrict__ frame)
-{
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n_lp) return;
-    const double k = 1.0 / 4294967296.0;
-    const V3<double> sum = mk<double>((double)accum[i] * k, (double)accum[n_lp + i] * k, (double)accum[2 * (size_t)n_lp + i] * k);
-    const uint32_t lr = i / width, x = i - lr * width;
-    const uint32_t y = local_to_global_row(lr, tile_rows, world, rank);
-    frame[(size_t)y * width + x] = to_rgba<double>(sum, alpha, (uint64_t)spp[i]);
 }
 
 // gathered tile buffers (rank-major, rank-local rows) -> top-down frame

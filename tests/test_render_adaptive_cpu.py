@@ -1,35 +1,12 @@
-"""CPU suite for rtiow_render_adaptive: the library carries one adaptive render kernel per scan-plan arm, the ctypes binding
-checks the buffers it is handed before it calls the library, and every layer exposes the call."""
+"""CPU suite for rtiow_render_adaptive: the ctypes binding checks the buffers it is handed before it calls the library, and every
+layer exposes the call.  test_kernel_inventory.py checks the library's adaptive render and round kernels."""
 import re
-import subprocess
 from pathlib import Path
 
 import numpy as np
 import pytest
 
 ROOT = Path(__file__).resolve().parent.parent
-ADAPTIVE_KERNELS = {
-    "render_adaptive_kernel<double, false, 256, 2>",     # F64
-    "render_adaptive_kernel<float, true, 256, 3>",       # Smem
-    "render_adaptive_kernel<float, true, 768, 1>",       # Wide, 768 threads
-    "render_adaptive_kernel<float, true, 512, 1>",       # Wide, 512 threads
-    "render_adaptive_kernel<float, false, 256, 4>",      # Global
-    "render_adaptive_kernel_umma<6, 64>",                # Tensor
-}
-
-
-def test_adaptive_kernels_are_the_plan_arms(capi):
-    """one render_adaptive_kernel per arm of the scan plan, the same instantiations as render_kernel's, and the round and
-    epilogue kernels"""
-    syms = subprocess.run(["cuobjdump", "-symbols", str(capi.lib_path())], capture_output=True, text=True, check=True).stdout
-    names = subprocess.run(["c++filt"], input=syms, capture_output=True, text=True, check=True).stdout
-    found = set(re.findall(r"rt::(render_adaptive_kernel(?:_umma)?<[^>]*>)", names))
-    assert found == ADAPTIVE_KERNELS, f"unexpected: {sorted(found - ADAPTIVE_KERNELS)}, missing: {sorted(ADAPTIVE_KERNELS - found)}"
-    frame = set(re.findall(r"rt::render_kernel((?:_umma)?<[^>]*>)", names))
-    assert {n.replace("render_adaptive_kernel", "") for n in ADAPTIVE_KERNELS} == frame
-    for k in ("adapt_first_list_kernel", "adapt_select_kernel", "adapt_compact_kernel", "finalize_adaptive_kernel",
-              "finalize_adaptive_to_frame_kernel"):
-        assert f"rt::{k}(" in names, k
 
 
 def _unbound_ctx(capi):

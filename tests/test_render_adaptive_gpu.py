@@ -1,7 +1,7 @@
 """GPU suite: rtiow_render_adaptive, per-pixel sample counts driven by each pixel's own noise.
 
 The rounds render sample ranges of shrinking pixel lists into the frame's own integer sums, keyed by (seed; pixel, sample,
-bounce) like every other call (rt_render.cuh, render_adaptive_kernel).  So:
+bounce) like every other call (rt_render.cuh, Loop::Adaptive).  So:
   * every pixel that stopped at n samples equals rtiow_render(spp = n) byte for byte, on every scan arm;
   * min_spp == spp is rtiow_render, and tolerance = +inf is rtiow_render at spp = min_spp (bytes, paths and rays);
   * the call with spp = b_k is the first k + 1 rounds of a call with a larger spp (the rule, exactly);

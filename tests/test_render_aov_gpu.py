@@ -1,6 +1,6 @@
 """GPU suite: rtiow_render_aov, a frame byte-identical to rtiow_render plus float AOVs for a denoiser.
 
-render_aov_kernel is the frame's render loop with kAov (rt_render.cuh): a camera ray also adds its first hit to integer
+The render kernel is the frame's loop as Loop::Aov (rt_render.cuh): a camera ray also adds its first hit to integer
 accumulators, and finalize_aov_kernel turns them into float buffers.  So:
   * the RGBA8 frame and rays_traced equal rtiow_render's on every scan arm, with the float buffers set and with them NULL;
   * the linear colour quantises to the frame (to_rgba, vec3.rs:404-420) except next to a quantisation step;

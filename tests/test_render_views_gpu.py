@@ -1,16 +1,14 @@
 """rtiow_render_views: many cameras of one scene in one call, each frame byte-identical to its own rtiow_render.
 
-A batch renders on one device as one frame n_views * height rows tall (rt_render.cuh, render_views_kernel): the work split,
+A batch renders on one device as one frame n_views * height rows tall (rt_render.cuh, Loop::Views): the work split,
 the accumulators and the epilogue are the frame's, and only a fresh path's row -> (view, row in the view) split and its camera
 differ.  A frame is a pure function of (scene, camera, params) and the accumulation is integer, so every view must equal
 rtiow_render of its camera exactly, on every arm plan_scan can choose, and where the work split puts view boundaries inside
 one fetch or one warp's assignment.
 
-The CPU tests at the end check the library's kernel inventory and the ctypes binding; everything else needs a GPU.
+The CPU tests at the end check the ctypes binding (test_kernel_inventory.py checks the kernels); everything else needs a GPU.
 """
 import ctypes as C
-import re
-import subprocess
 
 import numpy as np
 import pytest
@@ -216,26 +214,6 @@ def test_multi_gpu_matches_one_device(capi, final_scene):
 
 
 # ------------------------------------------------------------------------------------------------ CPU
-VIEW_KERNELS = {
-    "render_views_kernel<double, false, 256, 2>",     # F64
-    "render_views_kernel<float, true, 256, 3>",       # Smem
-    "render_views_kernel<float, true, 768, 1>",       # Wide, 768 threads
-    "render_views_kernel<float, true, 512, 1>",       # Wide, 512 threads
-    "render_views_kernel<float, false, 256, 4>",      # Global
-    "render_views_kernel_umma<6, 64>",                # Tensor
-}
-
-
-def test_views_kernels_are_the_plan_arms(capi):
-    """one render_views_kernel per arm of the scan plan, the same instantiations as render_kernel's"""
-    syms = subprocess.run(["cuobjdump", "-symbols", str(capi.lib_path())], capture_output=True, text=True, check=True).stdout
-    names = subprocess.run(["c++filt"], input=syms, capture_output=True, text=True, check=True).stdout
-    found = set(re.findall(r"rt::(render_views_kernel(?:_umma)?<[^>]*>)", names))
-    assert found == VIEW_KERNELS, f"unexpected: {sorted(found - VIEW_KERNELS)}, missing: {sorted(VIEW_KERNELS - found)}"
-    frame = set(re.findall(r"rt::render_kernel((?:_umma)?<[^>]*>)", names))
-    assert {n.replace("render_views_kernel", "") for n in VIEW_KERNELS} == frame
-
-
 @pytest.mark.parametrize("size", [0, 3 * 9 * 16 * 4 - 1, 3 * 9 * 16 * 4 + 4, 2 * 9 * 16 * 4])
 def test_binding_rejects_wrongly_sized_output(capi, size):
     """Context.render_views checks `out` before it calls the library (a ctx handle is not even needed)"""

@@ -1,6 +1,6 @@
 """Short single-GPU render used under ncu (profiles/): the bench workload's frame at reduced spp.
     python tools/profile_render.py [spp] [width] [height] [half_extent]
-Launch order per frame: render_kernel, finalize_kernel.  Two frames: the first warms up."""
+Launch order per frame: render_kernel<…, Loop::Frame> (or render_kernel_umma<6, 64, Loop::Frame>), finalize_kernel.  Two frames: the first warms up."""
 import sys
 from pathlib import Path
 sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
