@@ -256,6 +256,26 @@ void rtiow_denoise_params_default(rtiow_denoise_params* dp);
 int  rtiow_denoise(rtiow_ctx* ctx, uint32_t width, uint32_t height, const float* color, const float* albedo, const float* normal,
                    const float* depth, const rtiow_denoise_params* dp, float* out_color, uint8_t* out_rgba, rtiow_stats* stats);
 
+/* A denoised frame in one call: the render of rtiow_render_aov and the filter of rtiow_denoise back to back on the device, so the
+ * noisy frame and its four float buffers (40 B/px) never cross to the host and back.
+ *   Outputs    out_color [H][W][3] float and out_rgba [H][W] RGBA8, top-down, caller-owned HOST memory; either may be NULL, but
+ *              not both.  Both are bit-identical to
+ *                rtiow_render_aov(ctx, cam, p, frame, color, albedo, normal, depth, NULL);
+ *                rtiow_denoise(ctx, p->width, p->height, color, albedo, normal, depth, dp, out_color, out_rgba, NULL);
+ *              The AOVs' clamps keep every value inside rtiow_denoise's input ranges, so that sequence never rejects them.
+ *   Devices    the render runs as rtiow_render_aov runs it, on every device of an n-GPU ctx over interleaved row tiles; each
+ *              device copies its rows of the float buffers to device 0, and the filter runs on the ctx's first device and stream
+ *              as rtiow_denoise does.  A rank ctx with world > 1 returns RTIOW_ERR_UNSUPPORTED.
+ *   Errors     RTIOW_ERR_INVALID_ARG, checked before anything is launched and with nothing written, for what rtiow_render
+ *              rejects, for what rtiow_denoise rejects about dp (NULL, levels > 10, a sigma that is NaN or below 1e-12), for both
+ *              outputs NULL, and without an uploaded scene.
+ *   Stats      paths, rays_traced, sphere_tests, scan_backend and n_gpus as rtiow_render_aov reports them; kernel_ms = the
+ *              slowest device's render time plus the denoise kernels' time on device 0; total_ms the wall time; h2d_bytes =
+ *              sizeof(rtiow_camera) + sizeof(rtiow_params); d2h_bytes = 16 (the counters) + 12 W H with out_color + 4 W H with
+ *              out_rgba; kernel_launches = 3 per device that renders rows (render, frame epilogue, AOV epilogue) + levels + 2. */
+int  rtiow_render_denoised(rtiow_ctx* ctx, const rtiow_camera* cam, const rtiow_params* p, const rtiow_denoise_params* dp,
+                           float* out_color, uint8_t* out_rgba, rtiow_stats* stats);
+
 /* Many views of one scene (turntables, animations, stereo pairs, camera sweeps) in one call: out_rgba receives n_views top-down
  * RGBA8 frames of 4*width*height bytes each, in view order, in caller-owned HOST memory.  Frame v equals
  * rtiow_render(ctx, &cams[v], p, ...) byte for byte, so the views share their sample streams (same seed, same pixel keys);

@@ -135,6 +135,16 @@ def denoise(color, albedo, normal, depth, params: capi.DenoiseParams | None = No
     return outs["color"], outs["rgba"]
 
 
+def render_denoised(cam: capi.Camera, world: HittableList, params: capi.Params, dparams: capi.DenoiseParams | None = None, n_gpus: int = 1):
+    """A denoised frame in one call -> (linear colour float32[H,W,3], rgba uint8[H,W,4]), bit-identical to denoise() over
+    render_aov()'s buffers, which stay on the GPU (include/rtiow_cuda.h, rtiow_render_denoised; default denoise parameters when
+    dparams is None)."""
+    with capi.Context(n_gpus) as ctx:
+        ctx.upload_scene(**world.to_arrays())
+        outs, _ = ctx.render_denoised(cam, params, dparams)
+    return outs["color"], outs["rgba"]
+
+
 def render_views(cams, world: HittableList, params: capi.Params, n_gpus: int = 1):
     """Many cameras of one world in one call: [K,H,W,4] top-down RGBA8, frame v byte-identical to render(cams[v], ...)."""
     with capi.Context(n_gpus) as ctx:

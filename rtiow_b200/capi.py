@@ -31,7 +31,7 @@ SYMBOLS = [
     "rtiow_abi_version", "rtiow_last_error", "rtiow_device_count", "rtiow_ctx_create", "rtiow_ctx_create_on_device",
     "rtiow_ctx_destroy", "rtiow_ctx_set_scan_backend", "rtiow_ctx_set_filter_bypass", "rtiow_nccl_unique_id", "rtiow_ctx_create_rank", "rtiow_ctx_set_gather", "rtiow_ctx_set_stream",
     "rtiow_ctx_gather_info", "rtiow_render_rank", "rtiow_render_rank_device", "rtiow_render_rank_enqueue", "rtiow_ctx_synchronize", "rtiow_scene_upload", "rtiow_camera_new", "rtiow_params_default", "rtiow_render", "rtiow_render_aov", "rtiow_render_adaptive", "rtiow_render_views", "rtiow_render_progressive",
-    "rtiow_denoise_params_default", "rtiow_denoise",
+    "rtiow_denoise_params_default", "rtiow_denoise", "rtiow_render_denoised",
     "rtiow_tile_buffer_bytes", "rtiow_render_tiles_device", "rtiow_render_to_frame_device", "rtiow_deinterleave_device", "rtiow_sphere_hit_batch",
     "rtiow_hitlist_batch", "rtiow_scatter_batch", "rtiow_get_ray_batch", "rtiow_to_rgba_batch", "rtiow_reflect_batch",
     "rtiow_refract_batch", "rtiow_ray_color_batch", "rtiow_ray_color_trace_batch", "rtiow_sampler_batch", "rtiow_fp32_peak_probe", "rtiow_flush_l2",
@@ -132,6 +132,7 @@ def _declare(L):
         "rtiow_render_progressive": (C.c_int, [P, C.POINTER(Camera), C.POINTER(Params), C.c_uint32, PROGRESS_FN, P, P, C.POINTER(Stats)]),
         "rtiow_denoise_params_default": (None, [C.POINTER(DenoiseParams)]),
         "rtiow_denoise": (C.c_int, [P, u32, u32, P, P, P, P, C.POINTER(DenoiseParams), P, P, C.POINTER(Stats)]),
+        "rtiow_render_denoised": (C.c_int, [P, C.POINTER(Camera), C.POINTER(Params), C.POINTER(DenoiseParams), P, P, C.POINTER(Stats)]),
         "rtiow_render_rank_enqueue": (C.c_int, [P, C.POINTER(Camera), C.POINTER(Params), C.POINTER(C.c_void_p)]),
         "rtiow_ctx_synchronize": (C.c_int, [P, C.POINTER(Stats)]),
         "rtiow_tile_buffer_bytes": (C.c_int, [C.POINTER(Params), C.c_int, C.POINTER(C.c_size_t)]),
@@ -434,6 +435,23 @@ class Context:
                                            C.byref(st)))
         return out.reshape(h, w, 4), maps, st.as_dict()
 
+    @staticmethod
+    def _denoise_outputs(h, w, out_color, out_rgba):
+        """the output buffers of denoise / render_denoised: {"color": float32[H,W,3], "rgba": uint8[H,W,4]}, each allocated (True),
+        left out (False / None) or the caller's C-contiguous array of the right dtype and size"""
+        outs = {}
+        for name, arg, dt, shape in (("color", out_color, np.float32, (h, w, 3)), ("rgba", out_rgba, np.uint8, (h, w, 4))):
+            if arg is None or arg is False:
+                continue
+            if arg is True:
+                arg = np.empty(shape, dt)
+            elif (not isinstance(arg, np.ndarray) or arg.dtype != dt or arg.size != int(np.prod(shape)) or not arg.flags.c_contiguous):
+                raise ValueError(f"out_{name} must be a C-contiguous {np.dtype(dt).name} array with {int(np.prod(shape))} elements")
+            outs[name] = arg.reshape(shape)
+        if not outs:
+            raise ValueError("out_color and out_rgba cannot both be None")
+        return outs
+
     def denoise(self, color, albedo, normal, depth, params: DenoiseParams | None = None, out_color=True, out_rgba=True):
         """rtiow_denoise: the edge-avoiding a-trous filter over render_aov's buffers (colour, albedo, normal float32 [H,W,3], depth
         float32 [H,W], each C-contiguous) -> ({"color": float32[H,W,3], "rgba": uint8[H,W,4]}, stats).  out_color / out_rgba are
@@ -447,23 +465,27 @@ class Context:
             if (not isinstance(arr, np.ndarray) or arr.dtype != np.float32 or arr.size != h * w * per_px or not arr.flags.c_contiguous):
                 raise ValueError(f"{name} must be a C-contiguous float32 array with {h * w * per_px} elements")
             ins[name] = arr
-        outs = {}
-        for name, arg, dt, shape in (("color", out_color, np.float32, (h, w, 3)), ("rgba", out_rgba, np.uint8, (h, w, 4))):
-            if arg is None or arg is False:
-                continue
-            if arg is True:
-                arg = np.empty(shape, dt)
-            elif (not isinstance(arg, np.ndarray) or arg.dtype != dt or arg.size != int(np.prod(shape)) or not arg.flags.c_contiguous):
-                raise ValueError(f"out_{name} must be a C-contiguous {np.dtype(dt).name} array with {int(np.prod(shape))} elements")
-            outs[name] = arg.reshape(shape)
-        if not outs:
-            raise ValueError("out_color and out_rgba cannot both be None")
+        outs = self._denoise_outputs(h, w, out_color, out_rgba)
         if params is None:
             params = default_denoise_params()
         st = Stats()
         _check(lib().rtiow_denoise(self._h, w, h, _p(ins["color"]), _p(ins["albedo"]), _p(ins["normal"]), _p(ins["depth"]), C.byref(params),
                                    _p(outs["color"]) if "color" in outs else None, _p(outs["rgba"]) if "rgba" in outs else None,
                                    C.byref(st)))
+        return outs, st.as_dict()
+
+    def render_denoised(self, cam: Camera, params: Params, dparams: DenoiseParams | None = None, out_color=True, out_rgba=True):
+        """rtiow_render_denoised: render_aov's render and denoise's filter in one call, the AOVs kept on the device
+        -> ({"color": float32[H,W,3], "rgba": uint8[H,W,4]}, stats).  Both outputs are bit-identical to denoise() over
+        render_aov(cam, params)'s buffers (default denoise parameters when dparams is None).  out_color / out_rgba are as for
+        denoise()."""
+        outs = self._denoise_outputs(params.height, params.width, out_color, out_rgba)
+        if dparams is None:
+            dparams = default_denoise_params()
+        st = Stats()
+        _check(lib().rtiow_render_denoised(self._h, C.byref(cam), C.byref(params), C.byref(dparams),
+                                           _p(outs["color"]) if "color" in outs else None, _p(outs["rgba"]) if "rgba" in outs else None,
+                                           C.byref(st)))
         return outs, st.as_dict()
 
     def render_views(self, cams, params: Params, out=None):

@@ -108,6 +108,8 @@ struct DeviceState {
     // and the range flag of the prepare kernel (on the device and page-locked)
     DevBuf<float> dn_in; DevBuf<float4> dn_work; DevBuf<float> dn_color; DevBuf<uint32_t> dn_rgba;
     DevBuf<uint32_t> dn_bad; HostBuf<uint32_t> dn_bad_host;
+    // rtiow_render_denoised: the events around its filter, which runs after the render's own pair (ev0, ev1)
+    cudaEvent_t ev_dn0 = nullptr, ev_dn1 = nullptr;
     // measurement
     DevBuf<uint4> flush; DevBuf<float> probe;
     int last_backend = RTIOW_SCAN_FP32;                // which filter the last render launch used (rtiow_stats.scan_backend)
@@ -154,6 +156,7 @@ static int init_device(DeviceState& d, int device)
     d.sms = p.multiProcessorCount;
     CU(cudaStreamCreateWithFlags(&d.stream, cudaStreamNonBlocking));
     CU(cudaEventCreate(&d.ev0)); CU(cudaEventCreate(&d.ev1)); CU(cudaEventCreateWithFlags(&d.ev_done, cudaEventDisableTiming));
+    CU(cudaEventCreate(&d.ev_dn0)); CU(cudaEventCreate(&d.ev_dn1));
     CU(d.counters.resize(2));
     CU(d.pinned_cnt.resize(2));
     return RTIOW_OK;
@@ -380,6 +383,8 @@ extern "C" void rtiow_ctx_destroy(rtiow_ctx* c)
         if (d.ev0) cudaEventDestroy(d.ev0);
         if (d.ev1) cudaEventDestroy(d.ev1);
         if (d.ev_done) cudaEventDestroy(d.ev_done);
+        if (d.ev_dn0) cudaEventDestroy(d.ev_dn0);
+        if (d.ev_dn1) cudaEventDestroy(d.ev_dn1);
         for (auto& ev : d.ring) { cudaEventDestroy(ev.first); cudaEventDestroy(ev.second); }
         if (d.stream && d.owns_stream) cudaStreamDestroy(d.stream);
     }
@@ -1136,12 +1141,18 @@ extern "C" int rtiow_deinterleave_device(rtiow_ctx* c, const void* d_gathered, c
 // The host buffers of rtiow_render_aov; any may be NULL
 struct AovOut { float* color; float* albedo; float* normal; float* depth; };
 
+// Where copy_aov_rows puts the rows: the caller's host memory (the default), or device `dst_device`'s memory from device
+// `src_device`.  A copy between two devices is a cudaMemcpyPeerAsync; only with peer access (`peer`) is a 2D copy between them
+// valid, so without it every tile goes on its own.
+struct RowsTo { int src_device = -1, dst_device = -1; bool peer = true; };
+
 // Device `rank`'s rows of one per-pixel buffer (`elems` 4-byte values per pixel, rank-local row order: a float buffer of
-// d.aov_out, or rtiow_render_adaptive's counts or errors) into their top-down rows of the caller's host buffer.  The rank's tiles
-// rank, rank + world, ... sit equally spaced in the frame and back to back in src, so one 2D copy moves every whole tile; the
-// frame's last tile, which may be short, goes on its own.
+// d.aov_out, or rtiow_render_adaptive's counts or errors) into their top-down rows of `dst` (the caller's host buffer, or a
+// device buffer: `to`).  The rank's tiles rank, rank + world, ... sit equally spaced in the frame and back to back in src, so
+// one 2D copy moves every whole tile; the frame's last tile, which may be short, goes on its own.
 template <typename E>
-static int copy_aov_rows(E* dst, const E* src, uint32_t elems, const rtiow_params* p, uint32_t world, uint32_t rank, cudaStream_t st, uint64_t* bytes)
+static int copy_aov_rows(E* dst, const E* src, uint32_t elems, const rtiow_params* p, uint32_t world, uint32_t rank, cudaStream_t st, uint64_t* bytes,
+                         RowsTo to = RowsTo{})
 {
     static_assert(sizeof(E) == 4, "a per-pixel buffer of 4-byte values");
     const uint32_t tr = tile_rows_of(p), n_tiles = (p->height + tr - 1) / tr;
@@ -1151,14 +1162,19 @@ static int copy_aov_rows(E* dst, const E* src, uint32_t elems, const rtiow_param
     const uint32_t whole = mine - (rank + (mine - 1) * world == n_tiles - 1 && last_rows < tr ? 1u : 0u);
     char* const d = reinterpret_cast<char*>(dst);
     const char* const s = reinterpret_cast<const char*>(src);
+    const bool to_host = to.dst_device < 0, cross = !to_host && to.dst_device != to.src_device;
+    const cudaMemcpyKind kind = to_host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
+    auto copy = [&](char* dp, const char* sp, size_t n) {
+        return cross ? cudaMemcpyPeerAsync(dp, to.dst_device, sp, to.src_device, n, st) : cudaMemcpyAsync(dp, sp, n, kind, st);
+    };
     if (world == 1 || whole == 1) {
-        if (whole) CU(cudaMemcpyAsync(d + rank * tile, s, whole * tile, cudaMemcpyDeviceToHost, st));
-    } else if (world * tile <= (size_t)INT32_MAX) {          // the largest pitch a 2D copy takes
-        if (whole) CU(cudaMemcpy2DAsync(d + rank * tile, world * tile, s, tile, tile, whole, cudaMemcpyDeviceToHost, st));
+        if (whole) CU(copy(d + rank * tile, s, whole * tile));
+    } else if (world * tile <= (size_t)INT32_MAX && (!cross || to.peer)) {          // the largest pitch a 2D copy takes
+        if (whole) CU(cudaMemcpy2DAsync(d + rank * tile, world * tile, s, tile, tile, whole, kind, st));
     } else {
-        for (uint32_t k = 0; k < whole; ++k) CU(cudaMemcpyAsync(d + ((size_t)k * world + rank) * tile, s + k * tile, tile, cudaMemcpyDeviceToHost, st));
+        for (uint32_t k = 0; k < whole; ++k) CU(copy(d + ((size_t)k * world + rank) * tile, s + k * tile, tile));
     }
-    if (whole < mine) CU(cudaMemcpyAsync(d + (size_t)(n_tiles - 1) * tile, s + whole * tile, last_rows * row, cudaMemcpyDeviceToHost, st));
+    if (whole < mine) CU(copy(d + (size_t)(n_tiles - 1) * tile, s + whole * tile, last_rows * row));
     *bytes += (uint64_t)rows_of_rank(p->height, tr, world, rank) * row;
     return RTIOW_OK;
 }
@@ -1590,6 +1606,16 @@ extern "C" void rtiow_denoise_params_default(rtiow_denoise_params* dp)
     dp->alpha = 255;
 }
 
+// what both denoising calls check of a non-NULL dp: levels <= 10, and every sigma >= 1e-12 or +inf (not NaN)
+static int check_denoise_params(const char* call, const rtiow_denoise_params* dp)
+{
+    if (dp->levels > 10) return fail(RTIOW_ERR_INVALID_ARG, "%s: levels %u > 10", call, dp->levels);
+    const double sig[3] = { dp->sigma_color, dp->sigma_normal, dp->sigma_depth };
+    for (double s : sig)
+        if (!(s >= 1e-12)) return fail(RTIOW_ERR_INVALID_ARG, "%s: a sigma is NaN or below 1e-12 (%g)", call, s);
+    return RTIOW_OK;
+}
+
 // Uploads the four buffers (40 B/px), runs prepare, the levels and finish on the ctx's first device and stream, reads the range
 // flag back and only then copies the requested outputs to the caller.  An input out of range still runs the kernels on the
 // device; it writes nothing to the caller and returns RTIOW_ERR_INVALID_ARG.
@@ -1599,10 +1625,7 @@ extern "C" int rtiow_denoise(rtiow_ctx* c, uint32_t width, uint32_t height, cons
     if (!c || !color || !albedo || !normal || !depth || !dp) return fail(RTIOW_ERR_INVALID_ARG, "NULL argument");
     if (!out_color && !out_rgba) return fail(RTIOW_ERR_INVALID_ARG, "rtiow_denoise: out_color and out_rgba are both NULL");
     if (width == 0 || height == 0) return fail(RTIOW_ERR_INVALID_ARG, "rtiow_denoise: empty image (%u x %u)", width, height);
-    if (dp->levels > 10) return fail(RTIOW_ERR_INVALID_ARG, "rtiow_denoise: levels %u > 10", dp->levels);
-    const double sig[3] = { dp->sigma_color, dp->sigma_normal, dp->sigma_depth };
-    for (double s : sig)
-        if (!(s >= 1e-12)) return fail(RTIOW_ERR_INVALID_ARG, "rtiow_denoise: a sigma is NaN or below 1e-12 (%g)", s);
+    int rc = check_denoise_params("rtiow_denoise", dp); if (rc) return rc;
     const double t0 = now_ms();
     const size_t n = (size_t)width * height;
     DeviceState& d = c->dev[0];
@@ -1635,6 +1658,72 @@ extern "C" int rtiow_denoise(rtiow_ctx* c, uint32_t width, uint32_t height, cons
         stats->kernel_ms = ms; stats->total_ms = now_ms() - t0;
         stats->h2d_bytes = 40 * (uint64_t)n; stats->d2h_bytes = d2h;
         stats->kernel_launches = dp->levels + 2; stats->n_gpus = 1;
+    }
+    return RTIOW_OK;
+}
+
+// rtiow_render_aov's render and rtiow_denoise's filter back to back on the device.  Every device renders its row tiles with
+// Loop::Aov into its own tile buffer (the RGBA8 frame of that epilogue is not read: no gather).  On one device d.aov_out already
+// holds the filter's input, the four buffers back to back in top-down order; on several, each device copies its rows of them
+// to their top-down places in device 0's dn_in, and device 0's stream waits for every device's copies.  The filter then runs
+// on device 0 and only the requested outputs come down.  The range flag is not read back: the AOVs' clamps keep every value
+// inside the filter's ranges.
+extern "C" int rtiow_render_denoised(rtiow_ctx* c, const rtiow_camera* cam, const rtiow_params* p, const rtiow_denoise_params* dp,
+                                     float* out_color, uint8_t* out_rgba, rtiow_stats* stats)
+{
+    if (!c || !cam || !dp) return fail(RTIOW_ERR_INVALID_ARG, "NULL argument");
+    int rc = check_params(p); if (rc) return rc;
+    if (!out_color && !out_rgba) return fail(RTIOW_ERR_INVALID_ARG, "rtiow_render_denoised: out_color and out_rgba are both NULL");
+    rc = check_denoise_params("rtiow_render_denoised", dp); if (rc) return rc;
+    if (c->world > 1) return fail(RTIOW_ERR_UNSUPPORTED, "rtiow_render_denoised: a rank ctx with world > 1 renders collective frames (rtiow_render_rank), without AOVs");
+    for (const DeviceState& d : c->dev)
+        if (!d.has_scene) return fail(RTIOW_ERR_INVALID_ARG, "no scene uploaded (call rtiow_scene_upload first)");
+    const double t0 = now_ms();
+    const uint32_t world = (uint32_t)c->dev.size();
+    const size_t n = (size_t)p->width * p->height;
+    const size_t tile_px = (size_t)max_rows_per_rank(p->height, tile_rows_of(p), world) * p->width;
+    DeviceState& d0 = c->dev[0];
+    CU(cudaSetDevice(d0.device));
+    if (world > 1) CU(d0.dn_in.resize(10 * n));
+    CU(d0.dn_work.resize(3 * n)); CU(d0.dn_bad.resize(1));
+    if (out_color) CU(d0.dn_color.resize(3 * n));
+    if (out_rgba) CU(d0.dn_rgba.resize(n));
+    std::vector<Part> parts(world);
+    uint32_t launches = 0;
+    uint64_t no_d2h = 0;
+    for (uint32_t r = 0; r < world; ++r) {
+        DeviceState& d = c->dev[r];
+        CU(cudaSetDevice(d.device));
+        CU(d.tiles.resize(tile_px));
+        rc = render_step(c, d, cam, p, r, world, SampleRange{ 0u, p->spp }, Dest{ d.tiles.p, false }, d.stream, d.ev0, d.ev1, &launches, &parts[r], Loop::Aov);
+        if (rc) return rc;
+        if (world == 1) break;
+        // colour, albedo, normal and depth of this device's n_lp pixels into their rows of dn_in's four buffers
+        const size_t n_lp = (size_t)rows_of_rank(p->height, tile_rows_of(p), world, r) * p->width;
+        const RowsTo to{ d.device, d0.device, c->peer_ok };
+        for (int b = 0; b < 4; ++b) {
+            rc = copy_aov_rows(d0.dn_in.p + 3 * b * n, d.aov_out.p + 3 * b * n_lp, b < 3 ? 3u : 1u, p, world, r, d.stream, &no_d2h, to); if (rc) return rc;
+        }
+        if (r != 0) CU(cudaEventRecord(d.ev_done, d.stream));
+    }
+    CU(cudaSetDevice(d0.device));
+    for (uint32_t r = 1; r < world; ++r) CU(cudaStreamWaitEvent(d0.stream, c->dev[r].ev_done, 0));
+    CU(cudaEventRecord(d0.ev_dn0, d0.stream));
+    // the sigmas narrowed to float with round-to-nearest, as rtiow_denoise narrows them
+    CU(denoise_launch(world == 1 ? d0.aov_out.p : d0.dn_in.p, d0.dn_work.p, d0.dn_bad.p, p->width, p->height, dp->levels, (float)dp->sigma_color,
+                      (float)dp->sigma_normal, (float)dp->sigma_depth, dp->alpha, out_color ? d0.dn_color.p : nullptr, out_rgba ? d0.dn_rgba.p : nullptr,
+                      d0.stream));
+    CU(cudaEventRecord(d0.ev_dn1, d0.stream));
+    launches += dp->levels + 2;
+    uint64_t d2h = 16;
+    if (out_color) { CU(cudaMemcpyAsync(out_color, d0.dn_color.p, 3 * n * sizeof(float), cudaMemcpyDeviceToHost, d0.stream)); d2h += 12 * (uint64_t)n; }
+    if (out_rgba) { rc = parts[0].start_copy(out_rgba, d0.dn_rgba.p, 4 * n); if (rc) return rc; d2h += 4 * (uint64_t)n; }
+    rtiow_stats st;
+    rc = finish_call(parts.data(), world, t0, launches, world, kCallH2D, d2h, stats ? &st : nullptr); if (rc) return rc;
+    if (stats) {
+        float ms = 0; CU(cudaEventElapsedTime(&ms, d0.ev_dn0, d0.ev_dn1));
+        st.kernel_ms += ms; st.total_ms = now_ms() - t0;
+        *stats = st;
     }
     return RTIOW_OK;
 }

@@ -4,12 +4,13 @@
 //
 //   rtiow_host_example [--width W] [--height H] [--spp N] [--depth D] [--seed S] [--scene-seed S] [--gpus G]
 //                      [--grid HALF_EXTENT] [--materials 0..3] [--f64] [--passes N] [--views N] [--aov]
-//                      [--denoise] [--adaptive TOL [--min-spp N]] [--out image.png|image.ppm] [--selftest]
+//                      [--denoise] [--render-denoised] [--adaptive TOL [--min-spp N]] [--out image.png|image.ppm] [--selftest]
 // --views N renders N cameras orbiting the look-at point about the vertical axis in one call and writes out_000.png ...
 // (with --out, the frames are named after its stem: --out orbit.ppm writes orbit_000.ppm ...).
 // --aov also writes the inputs of a denoiser beside the image: <stem>_color.pfm (linear colour), <stem>_albedo.png and
 // <stem>_normal.png (0.5 n + 0.5).  --denoise (implies --aov) also runs the library's a-trous denoiser (default parameters) over
-// them and writes <stem>_denoised.png.
+// them and writes <stem>_denoised.png.  --render-denoised writes only <stem>_denoised.png, through one call that keeps the AOVs on
+// the GPU (render_denoised; the same bytes as --denoise's).
 // --adaptive TOL renders with adaptive sampling (render_adaptive): between --min-spp N (default 16, at most --spp) and --spp
 // samples per pixel, until a pixel's error is at most TOL 8-bit levels; it also writes <stem>_spp.png, a heat map of the
 // per-pixel counts (blue: min-spp, red: spp, log scale).
@@ -110,7 +111,13 @@ static int selftest()
       std::vector<float> dc; rtiow_stats sn{};
       const std::vector<uint8_t> d1 = denoise(p.width, p.height, av, default_denoise_params(), &dc, &sn), d2 = denoise(p.width, p.height, av, default_denoise_params());
       expect(d1 == d2 && d1.size() == 4 * n && dc.size() == 3 * n && d1[3] == 255, "denoise: the same bytes on a second call, sized 4*W*H, alpha 255");
-      expect(sn.h2d_bytes == 40ull * n && sn.d2h_bytes == 16ull * n && sn.n_gpus == 1 && sn.paths == 0, "denoise stats: 40 B/px up, 16 B/px down"); }
+      expect(sn.h2d_bytes == 40ull * n && sn.d2h_bytes == 16ull * n && sn.n_gpus == 1 && sn.paths == 0, "denoise stats: 40 B/px up, 16 B/px down");
+      // the same render and filter in one call, the AOVs kept on the GPU: the same bytes and colour bits
+      std::vector<float> rc; rtiow_stats sr{};
+      const std::vector<uint8_t> r1 = render_denoised(cam, random_scene(1), p, default_denoise_params(), &rc, &sr);
+      expect(r1 == d1 && rc.size() == dc.size() && std::memcmp(rc.data(), dc.data(), dc.size() * sizeof(float)) == 0,
+             "render_denoised equals denoise(render_aov(...)) byte for byte");
+      expect(sr.rays_traced == st.rays_traced && sr.d2h_bytes == 16 + 16ull * n, "render_denoised stats: render_aov's rays, 16 B/px + the counters down"); }
     // adaptive sampling with min_spp == spp renders every pixel at spp: render()'s frame, rays and paths
     { AdaptiveMaps am; rtiow_stats sd{};
       std::vector<uint8_t> f = render_adaptive(cam, random_scene(1), p, p.spp, 1.0, &am, &sd);
@@ -137,7 +144,7 @@ int main(int argc, char** argv)
 {
     RenderParams p; p.width = 200; p.height = 133;                       // main.rs:24-28
     uint64_t scene_seed = 1; int grid = 11, materials = 0; std::string out = "image.png";     // main.rs:177
-    bool explicit_h = false, explicit_out = false, aov = false, denoised = false; uint32_t passes = 0, views = 0; std::string scene_file, dump_scene;
+    bool explicit_h = false, explicit_out = false, aov = false, denoised = false, fused = false; uint32_t passes = 0, views = 0; std::string scene_file, dump_scene;
     double adaptive = -1.0; uint32_t min_spp = 16;
     for (int i = 1; i < argc; ++i) {
         auto next = [&]() -> const char* { if (i + 1 >= argc) { std::cerr << "missing value for " << argv[i] << "\n"; std::exit(2); } return argv[++i]; };
@@ -155,6 +162,7 @@ int main(int argc, char** argv)
         else if (!std::strcmp(argv[i], "--views")) views = uint32_t(std::atoi(next()));
         else if (!std::strcmp(argv[i], "--aov")) aov = true;
         else if (!std::strcmp(argv[i], "--denoise")) denoised = aov = true;        // implies --aov
+        else if (!std::strcmp(argv[i], "--render-denoised")) fused = true;
         else if (!std::strcmp(argv[i], "--adaptive")) adaptive = std::atof(next());
         else if (!std::strcmp(argv[i], "--min-spp")) min_spp = uint32_t(std::atoi(next()));
         else if (!std::strcmp(argv[i], "--out")) { out = next(); explicit_out = true; }
@@ -187,6 +195,15 @@ int main(int argc, char** argv)
                 if (!(ppm ? write_ppm(path, p.width, p.height, f) : write_png(path, p.width, p.height, f))) { std::cerr << "could not write " << path << "\n"; return 1; }
                 std::cout << path << " saved\n";
             }
+            return 0;
+        }
+        if (fused) {                                                      // the denoised frame only, its AOVs kept on the GPU
+            const std::vector<uint8_t> dn = render_denoised(cam, world, p, default_denoise_params(), nullptr, &st);
+            const std::string stem = out.substr(0, out.rfind('.') == std::string::npos ? out.size() : out.rfind('.'));
+            std::cout << p.width << "x" << p.height << " @ " << p.spp << " spp denoised on " << st.n_gpus << " GPU(s): kernel " << st.kernel_ms
+                      << " ms, call " << st.total_ms << " ms\n";
+            if (!write_png(stem + "_denoised.png", p.width, p.height, dn)) { std::cerr << "could not write " << stem << "_denoised.png\n"; return 1; }
+            std::cout << stem << "_denoised.png saved\n";
             return 0;
         }
         if (aov) {                                                        // the frame plus a denoiser's inputs

@@ -296,13 +296,14 @@ struct Aovs { std::vector<float> color, albedo, normal, depth; };
 // (include/rtiow_cuda.h, rtiow_render_adaptive).
 struct AdaptiveMaps { std::vector<uint32_t> spp; std::vector<float> error; };
 namespace detail { struct Adaptive { uint32_t min_spp; double tolerance; AdaptiveMaps* maps; }; }
+namespace detail { struct Denoised { const rtiow_denoise_params* dp; std::vector<float>* color; }; }
 
 // The world as the GPU sees it + one render call; n_passes == 0: rtiow_render, else rtiow_render_progressive; with `views`:
 // rtiow_render_views of those cameras (cam is not used); with `aovs`: rtiow_render_aov into them; with `adaptive`:
-// rtiow_render_adaptive into its maps.
+// rtiow_render_adaptive into its maps; with `denoised`: rtiow_render_denoised (the returned frame is the denoised one).
 inline std::vector<uint8_t> render_impl(const Camera& cam, const HittableList& world, const RenderParams& p, rtiow_stats* stats, uint32_t n_passes,
                                         const ProgressFn* on_pass, const std::vector<Camera>* views = nullptr, Aovs* aovs = nullptr,
-                                        const detail::Adaptive* adaptive = nullptr)
+                                        const detail::Adaptive* adaptive = nullptr, const detail::Denoised* denoised = nullptr)
 {
     std::vector<double> cx, cy, cz, rad, ar, ag, ab, prm; std::vector<uint32_t> mi, kind;
     std::vector<const Scatter*> seen;
@@ -343,6 +344,9 @@ inline std::vector<uint8_t> render_impl(const Camera& cam, const HittableList& w
         adaptive->maps->spp.resize(n); adaptive->maps->error.resize(n);
         check(rtiow_render_adaptive(ctx, &cam.raw(), &rp, adaptive->min_spp, adaptive->tolerance, out.data(), adaptive->maps->spp.data(),
                                     adaptive->maps->error.data(), stats));
+    } else if (denoised) {
+        if (denoised->color) denoised->color->resize(size_t(3) * p.width * p.height);
+        check(rtiow_render_denoised(ctx, &cam.raw(), &rp, denoised->dp, denoised->color ? denoised->color->data() : nullptr, out.data(), stats));
     } else if (n_passes == 0) check(rtiow_render(ctx, &cam.raw(), &rp, out.data(), stats));
     else {
         detail::ProgressCtx pc{ on_pass, &out };
@@ -408,6 +412,15 @@ inline std::vector<uint8_t> denoise(uint32_t width, uint32_t height, const Aovs&
     rtiow_ctx_destroy(ctx);
     if (rc != RTIOW_OK) throw RenderError(rc, msg);
     return out;
+}
+
+// render_denoised(): render_aov() and denoise() in one call, the AOVs kept on the GPU.  Returns the denoised frame as top-down
+// RGBA8; *color (may be null) receives its linear colour.  Both are bit-identical to denoise() over render_aov()'s buffers.
+inline std::vector<uint8_t> render_denoised(const Camera& cam, const HittableList& world, const RenderParams& p, const rtiow_denoise_params& dp,
+                                            std::vector<float>* color = nullptr, rtiow_stats* stats = nullptr)
+{
+    const detail::Denoised d{ &dp, color };
+    return render_impl(cam, world, p, stats, 0, nullptr, nullptr, nullptr, nullptr, &d);
 }
 
 // render_progressive(): the same frame in n_passes slices of the samples, with a preview after each — what the reference's

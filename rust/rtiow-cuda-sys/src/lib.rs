@@ -122,6 +122,8 @@ extern "C" {
     pub fn rtiow_denoise(ctx: *mut rtiow_ctx, width: u32, height: u32, color: *const f32, albedo: *const f32, normal: *const f32,
                          depth: *const f32, dp: *const rtiow_denoise_params, out_color: *mut f32, out_rgba: *mut u8,
                          stats: *mut rtiow_stats) -> c_int;
+    pub fn rtiow_render_denoised(ctx: *mut rtiow_ctx, cam: *const rtiow_camera, p: *const rtiow_params, dp: *const rtiow_denoise_params,
+                                 out_color: *mut f32, out_rgba: *mut u8, stats: *mut rtiow_stats) -> c_int;
     pub fn rtiow_render_views(ctx: *mut rtiow_ctx, cams: *const rtiow_camera, n_views: u32, p: *const rtiow_params, out_rgba: *mut u8,
                               stats: *mut rtiow_stats) -> c_int;
     pub fn rtiow_render_progressive(ctx: *mut rtiow_ctx, cam: *const rtiow_camera, p: *const rtiow_params, n_passes: u32,

@@ -150,6 +150,27 @@ pub fn denoise(width: u32, height: u32, aovs: &Aovs, dp: &sys::rtiow_denoise_par
     }
 }
 
+/// `render_aov` and `denoise` in one call, the AOVs kept on the GPU (include/rtiow_cuda.h, rtiow_render_denoised): returns the
+/// denoised linear colour (3 floats per pixel) and its top-down RGBA8 frame, both bit-identical to `denoise` over `render_aov`'s
+/// buffers.
+pub fn render_denoised(cam: &Camera, world: &HittableList, p: &RenderParams, dp: &sys::rtiow_denoise_params)
+                       -> Result<(Vec<f32>, Vec<u8>), RenderError> {
+    unsafe {
+        let mut raw: *mut sys::rtiow_ctx = ptr::null_mut();
+        let rc = sys::rtiow_ctx_create(p.n_gpus, &mut raw);
+        if rc != sys::RTIOW_OK { return Err(err(rc)); }
+        let ctx = Ctx(raw);
+        upload(&ctx, world)?;
+        let prm = raw_params(p);
+        let n = p.width as usize * p.height as usize;
+        let mut color = vec![0.0f32; 3 * n];
+        let mut pixels = vec![0u8; 4 * n];
+        let rc = sys::rtiow_render_denoised(ctx.0, &cam.raw(), &prm, dp, color.as_mut_ptr(), pixels.as_mut_ptr(), ptr::null_mut());
+        if rc != sys::RTIOW_OK { return Err(err(rc)); }
+        Ok((color, pixels))
+    }
+}
+
 /// The same frame in `n_passes` slices of the samples, with the frame so far handed to `on_pass(pass, n_passes, spp_done, rgba)`
 /// after each — the role of the indicatif bar (main.rs:120,124) and the piston preview window (main.rs:151-171).  The returned
 /// frame is bit-identical to `render`'s.  `on_pass` returning `true` stops the render: `Err(RenderError::Cancelled)`.
